@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- AMG-PCG solve of the 3D 7-point Poisson problem on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--n 256]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--n 256] [--dump-outputs DIR]
 
 A "step" is one complete `solve_pCG` (zero initial guess, AMG V-cycle preconditioner with 3+3
 Chebyshev sweeps, stop at ||r||/||r0|| < 1e-8: the reference's experiments/Poisson.cpp loop with
@@ -16,6 +16,12 @@ host-buffer entry point (pinned host rhs -> H2D -> solve -> D2H u inside the tim
 `roofline` = the dominant kernel's algorithmic bytes / its CUDA-event duration against the
 measured HBM peak; `cpu_baseline` = the reference's own CPU solve (oracle/_ref, the compiled
 reference) on a bounded sample.  `--impl reference` times only that CPU arm.
+
+`--dump-outputs DIR` writes what the last timed solve returned, as float64 .npy files: `u` (the
+solution, or a fixed seeded sample of at most DUMP_SAMPLE of its entries), `u_index` (their global
+row indices), `residual_history` and `iterations`.  The inputs depend only on the arguments, so two
+builds run with the same arguments can be compared output for output (to rounding: the setup picks
+each operator's kernel mapping by timing it).
 """
 from __future__ import annotations
 
@@ -37,6 +43,8 @@ UNIT = "Munknowns/s"
 OPTS = dict(max_iter=50, tol=1e-8, smoother="chebyshev", pre=3, post=3)   # data/options006_poisson.xml
 # reference arm: laplacian3D(mx) -> (mx-2)^3 = 48^3 unknowns (env override only for the contract test)
 CPU_SAMPLE_MX = int(os.environ.get("SAENA_BENCH_CPU_MX", 50))
+# --dump-outputs: entries of u written at most (16 MB of values + 16 MB of indices, whatever the problem size)
+DUMP_SAMPLE = 1 << 21
 
 
 def log(*a):
@@ -315,11 +323,41 @@ def nvlink_counters(device: int):
         return None
 
 
+def dump_outputs(out_dir: str, u_dev, iters: int, hist, row_offset: int, n_global: int, rank: int, world: int):
+    """--dump-outputs: u of the last solve at a fixed seeded sample of global rows (all rows when there are at most
+    DUMP_SAMPLE), gathered from the ranks' row blocks; rank 0 writes the files."""
+    import torch
+    if n_global > DUMP_SAMPLE:
+        idx = np.sort(np.random.default_rng(0).choice(n_global, DUMP_SAMPLE, replace=False))
+    else:
+        idx = np.arange(n_global)
+    lo, hi = (int(x) for x in np.searchsorted(idx, [row_offset, row_offset + u_dev.numel()]))
+    mine = u_dev[torch.from_numpy(idx[lo:hi] - row_offset).to(u_dev.device)].cpu().numpy()
+    parts = [(lo, mine)]
+    if world > 1:
+        import torch.distributed as dist
+        parts = [None] * world
+        dist.all_gather_object(parts, (lo, mine))
+    if rank != 0:
+        return
+    u = np.full(len(idx), np.nan)
+    for start, vals in parts:
+        u[start:start + len(vals)] = vals
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("u", u), ("u_index", idx), ("residual_history", hist), ("iterations", [iters])):
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 # ------------------------------------------------------------------------------------------------
 def main():
+    def at_least_one(s):
+        if int(s) < 1:
+            raise argparse.ArgumentTypeError(f"must be at least 1, got {s}")
+        return int(s)
+
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=at_least_one, default=10, help="timed solves")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--n", "--size", dest="n", type=int, default=int(os.environ.get("SAENA_BENCH_N", 256)),
@@ -341,7 +379,12 @@ def main():
     ap.add_argument("--rebalance-above", type=float, default=float(os.environ.get("SAENA_BENCH_REBALANCE", 1.10)),
                     help="N>1: a coarse level whose aligned row blocks leave one rank above this multiple of the mean "
                          "nnz is split by its own nnz balance (0: never)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed solves, write what the last one returned to DIR/<name>.npy (see the top of "
+                         "this file)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU solve (--impl b200)")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
@@ -547,6 +590,8 @@ def main():
         fall_back_to_nccl(why)
         iters, hist, ms_total, launches0, clocks = timed_region()
     launches = ctx.launch_count() - launches0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, u_dev, iters, hist, l0.row_offset, N, rank, world)
     ms_step = max_over_ranks(ms_total / args.steps)
     clk = clocks.summary()
     graph_info = {"vcycles_replayed_from_graph": ctx.graph_replays()}
