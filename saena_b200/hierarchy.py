@@ -368,17 +368,40 @@ def partition_hierarchy(h: Hierarchy, nprocs: int, agglomerate_below: int = 0,
                 so, sn = split_old_next, splits[l + 1]
                 level.M_coarse_old = int(so[r + 1] - so[r])
                 level.M_coarse = int(sn[r + 1] - sn[r])
-                if not np.array_equal(so, sn):
-                    # overlap of my old block with every new block (send) and vice versa (recv)
-                    for peer in range(nprocs):
-                        a, b = max(so[r], sn[peer]), min(so[r + 1], sn[peer + 1])
-                        if b > a:
-                            level.repart_send.append((peer, int(a - so[r]), int(b - a)))
-                        a, b = max(sn[r], so[peer]), min(sn[r + 1], so[peer + 1])
-                        if b > a:
-                            level.repart_recv.append((peer, int(a - sn[r]), int(b - a)))
+                level.repart_send, level.repart_recv = repart_plan(so, sn, r)
             out[r].levels.append(level)
     return out
+
+
+def repart_plan(so: Sequence[int], sn: Sequence[int], rank: int):
+    """Grid::repart_u's plan for `rank`, moving the coarse vector from partition `so` (where R writes it) to `sn`
+    (where the coarse grid lives): the overlap of my old block with every new block, (peer, offset_in_old, count)
+    to send, and of my new block with every old block, (peer, offset_in_new, count) to receive.  Empty when so == sn."""
+    send, recv = [], []
+    if not np.array_equal(so, sn):
+        for peer in range(len(so) - 1):
+            a, b = max(so[rank], sn[peer]), min(so[rank + 1], sn[peer + 1])
+            if b > a:
+                send.append((peer, int(a - so[rank]), int(b - a)))
+            a, b = max(sn[rank], so[peer]), min(sn[rank + 1], so[peer + 1])
+            if b > a:
+                recv.append((peer, int(a - sn[rank]), int(b - a)))
+    return send, recv
+
+
+def coarse_placement(nprocs: int, n_rows: int, coarsest: bool, above_on_0: bool, agglomerate_below: int,
+                     rebalance_above: float, aligned: Sequence[int], imbalance, balanced):
+    """Where coarse level l+1 of the torch-built hierarchies lives -- partition_hierarchy's rules, for builders that
+    know the level only through the arguments: `n_rows` its global rows, `aligned` the split that follows level l's
+    rows, `imbalance()` the level's split_imbalance under `aligned`, `balanced()` its nnz-balanced split.
+    `above_on_0`: level l lives on rank 0 alone.  Returns (the split R of level l writes into, the level's own split,
+    agglomerated onto rank 0?)."""
+    all_on_0 = np.concatenate(([0], np.full(nprocs, n_rows))).astype(I64)
+    agg = nprocs > 1 and (n_rows < agglomerate_below or above_on_0 or coarsest)
+    al = all_on_0 if above_on_0 else np.asarray(aligned, I64)
+    if rebalance_above > 0 and not agg and imbalance() > rebalance_above:
+        al = np.asarray(balanced(), I64)
+    return al, (all_on_0 if agg else al), agg
 
 
 # --------------------------------------------------------------------------------------

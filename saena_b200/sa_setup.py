@@ -6,8 +6,8 @@ host code (BASELINE.json north_star) and the drop-in adaptor uploads whatever
 `saena_object::setup` produced.  But the reference's setup cannot feed the bench: measured in
 this image it needs 3 s for 30^3 unknowns and 47 s for 64^3 (std::set assembly, recursive
 SpGEMM), i.e. the better part of an hour for the 256^3 workload, and its sources do not exist on
-the GPU box.  This module restates the setup's algorithm with torch tensor ops (GPU when there
-is one) so that the bench solves on a hierarchy built by the SAME rules:
+the GPU box.  This module and sa_setup_dist.py restate the setup's algorithm with torch tensor ops
+(GPU when there is one) so that the bench solves on a hierarchy built by the SAME rules:
 
   strength of connection   create_strength_matrix   src/saena_object_setup1.cpp:520-720
                            + threshold              src/strength_matrix.cpp:233-270
@@ -27,6 +27,12 @@ is one) so that the bench solves on a hierarchy built by the SAME rules:
                             reproducible run to run; here the start vector is seeded)
   precision flags          float_level              src/saena_object.cpp:241-244,277-285
 
+The steps and the level loop are written once, row-partitioned over the ranks, in sa_setup_dist.py.
+`build_device_hierarchy` runs that loop on one rank, where a rank's rows are the whole matrix and
+every exchange is empty, and keeps the global hierarchy on the device; `DeviceHierarchy.to_rank`
+cuts any rank's share out of it.  This module holds the sparse-matrix primitives both use, the
+reference layout of a rank's operator and the synthetic inputs.
+
 tests/test_sa_setup.py checks the result against the reference's own hierarchy (same
 aggregates / same operators to rounding) where oracle/_ref is available.  torch here is
 plumbing for the setup only; nothing in the solve path imports this module.
@@ -35,15 +41,14 @@ from __future__ import annotations
 
 import math
 import os
-import sys
-import time
 from dataclasses import dataclass
 from typing import List, Optional
 
 import numpy as np
 import torch
 
-from .hierarchy import F64, I32, KIND_A, KIND_P, KIND_R, Hierarchy, Level, Operator
+from .hierarchy import (KIND_A, KIND_P, KIND_R, Hierarchy, Level, Operator, balanced_split, coarse_placement,
+                        csr_from_counts, repart_plan, split_imbalance)
 
 ALMOST_ZERO = 1e-14                  # include/data_struct.h:41
 JACOBI_OMEGA = float(np.float32(2.0 / 3))   # saena_matrix.h:182 (a float, promoted)
@@ -67,11 +72,6 @@ class SetupOptions:
     seed: int = 2024
 
 
-def _sync(dev):
-    if dev.type == "cuda":
-        torch.cuda.synchronize(dev)
-
-
 class _Csr:
     """row-major sorted COO/CSR triple on one torch device"""
 
@@ -85,12 +85,6 @@ class _Csr:
     def counts(self):
         return torch.bincount(self.row, minlength=self.n_rows)
 
-    def diag(self):
-        d = torch.zeros(self.n_rows, dtype=torch.float64, device=self.val.device)
-        m = self.row == self.col
-        d[self.row[m]] = self.val[m]
-        return d
-
 
 def _coalesce(n_rows, n_cols, row, col, val) -> _Csr:
     """sort by (row, col) and add duplicates"""
@@ -103,18 +97,17 @@ def _coalesce(n_rows, n_cols, row, col, val) -> _Csr:
     return _Csr(n_rows, n_cols, uk // n_cols, uk % n_cols, out)
 
 
-# The one-process setup routes its products through the library's device SpGEMM since it passed
+# The setup on one rank routes its products through the library's device SpGEMM since it passed
 # tests/test_zzz_spgemm_gpu.py on a B200 (scipy, the reference's golden hierarchies, the live reference at 32^3, route
 # equality at 64^3) and built the 256^3 bench hierarchy end to end (profiles/r02_setup_time.json,
-# r02_bench_n1_native_spgemm.json).  The distributed setup keeps the tensor-op route until its own run with the device
+# r02_bench_n1_native_spgemm.json).  Several ranks keep the tensor-op route until their own run with the device
 # SpGEMM (SAENA_SETUP_SPGEMM=native asks for it there too).
-SPGEMM_DEFAULT = "native"
-
-
-def _native_spgemm_enabled(dev, dist: bool = False) -> bool:
+def _native_spgemm_enabled(dev, world: int) -> bool:
     """SAENA_SETUP_SPGEMM=native: the library's own SpGEMM (csrc/spgemm.cu, SURVEY 8f #3) does the products on a CUDA
-    device; =torch: the tensor-op route below (the CPU path, and the A/B)."""
-    return dev.type == "cuda" and os.environ.get("SAENA_SETUP_SPGEMM", "torch" if dist else SPGEMM_DEFAULT) != "torch"
+    device; =torch: the tensor-op route below (the CPU path, and the A/B).  The default depends on the number of
+    ranks only, so every rank takes the same route."""
+    default = "native" if world == 1 else "torch"
+    return dev.type == "cuda" and os.environ.get("SAENA_SETUP_SPGEMM", default) != "torch"
 
 
 def _spgemm_native(A: _Csr, B: _Csr) -> _Csr:
@@ -134,11 +127,11 @@ def _spgemm_native(A: _Csr, B: _Csr) -> _Csr:
     return _Csr(A.n_rows, B.n_cols, row, c_col.to(torch.int64), c_val)
 
 
-def _spgemm(A: _Csr, B: _Csr, chunk_products: int = 300_000_000, dist: bool = False) -> _Csr:
-    """C = A B: the library's device SpGEMM on CUDA; on the CPU (and for SAENA_SETUP_SPGEMM=torch) expand / sort /
-    compress with tensor ops, in row chunks bounded by the number of products"""
+def _spgemm(A: _Csr, B: _Csr, chunk_products: int, native: bool) -> _Csr:
+    """C = A B: the library's device SpGEMM if `native` (_native_spgemm_enabled); otherwise expand / sort / compress
+    with tensor ops, in row chunks bounded by the number of products"""
     dev = A.val.device
-    if _native_spgemm_enabled(dev, dist) and A.n_rows < 2 ** 31 and B.n_cols < 2 ** 31 - 1:
+    if native and A.n_rows < 2 ** 31 and B.n_cols < 2 ** 31 - 1:
         return _spgemm_native(A, B)
     b_counts = B.counts()
     b_ptr = torch.zeros(B.n_rows + 1, dtype=torch.int64, device=dev)
@@ -184,53 +177,13 @@ def _to_torch_csr(A: _Csr) -> torch.Tensor:
     return torch.sparse_csr_tensor(crow, A.col, A.val, size=(A.n_rows, A.n_cols))
 
 
-def _galerkin(R: _Csr, A: _Csr, P: _Csr, dense_budget_bytes: float = 48e9) -> _Csr:
-    """Ac = R A P.  On the deep levels of a 3D hierarchy the product is nearly dense (256^3 Poisson,
-    level 3 -> 4: rows of A P have ~20 000 entries, 8e11 scalar products) and the sparse expansion
-    drowns; there the two products are done as sparse x dense (R (A P_dense)) and the result is
-    re-sparsified.  Structural zeros stay exact zeros, so the pattern is the sparse product's
-    (barring exact cancellation)."""
-    nc = P.n_cols
-    dense_bytes = 8.0 * A.n_rows * nc
-    avg_prod_per_row = (A.nnz / max(A.n_rows, 1)) * (P.nnz / max(P.n_rows, 1))
-    if A.val.is_cuda and not _native_spgemm_enabled(A.val.device) and 2 * dense_bytes <= dense_budget_bytes \
-            and avg_prod_per_row > 4 * nc:
-        Pd = torch.zeros(P.n_rows, nc, dtype=torch.float64, device=A.val.device)
-        Pd[P.row, P.col] = P.val
-        AP = torch.sparse.mm(_to_torch_csr(A), Pd)
-        del Pd
-        Ac = torch.sparse.mm(_to_torch_csr(R), AP)
-        del AP
-        idx = torch.nonzero(Ac, as_tuple=True)
-        return _Csr(nc, nc, idx[0], idx[1], Ac[idx])
-    return _spgemm(R, _spgemm(A, P))
-
-
 def _transpose(A: _Csr) -> _Csr:
     key = A.col * A.n_rows + A.row
     key, order = torch.sort(key)
     return _Csr(A.n_cols, A.n_rows, key // A.n_rows, key % A.n_rows, A.val[order])
 
 
-def _matvec(A: _Csr, x: torch.Tensor) -> torch.Tensor:
-    y = torch.zeros(A.n_rows, dtype=torch.float64, device=x.device)
-    y.index_add_(0, A.row, A.val * x[A.col])
-    return y
-
-
 # ------------------------------------------------------------------------------------------
-def strength_graph(A: _Csr, conn_str: float):
-    """strong off-diagonal connections (row, col) -- create_strength_matrix + setup_matrix"""
-    n, dev = A.n_rows, A.val.device
-    off = A.row != A.col
-    max_per_row = torch.full((n,), -torch.finfo(torch.float64).max, dtype=torch.float64, device=dev)
-    max_per_row.scatter_reduce_(0, A.row[off], -A.val[off], reduce="amax")
-    s_row = -A.val / max_per_row[A.row]      # entry   (normalised by its row's maximum)
-    s_col = -A.val / max_per_row[A.col]      # entryT  (normalised by the column index's row maximum)
-    strong = off & ((s_row > conn_str) | (s_col > conn_str))
-    return A.row[strong], A.col[strong]
-
-
 def _expand_segments(ptr: torch.Tensor, rows: torch.Tensor):
     """entry indices of the CSR segments of `rows` and, per entry, the position of its row in `rows`"""
     dev = rows.device
@@ -243,121 +196,61 @@ def _expand_segments(ptr: torch.Tensor, rows: torch.Tensor):
     return e, seg
 
 
-def aggregate(n: int, s_row: torch.Tensor, s_col: torch.Tensor):
-    """aggregation_1_dist on one rank.  The reference sweeps every undecided node in every round;
-    a node's outcome can only change when one of its neighbours was decided in the round before,
-    so only those nodes are re-evaluated here (same rule, same synchronous updates, hence the same
-    aggregates -- tests/test_sa_setup.py compares with the reference's).  Returns (aggregate id per
-    node in coarse numbering, number of aggregates, rounds)."""
-    dev = s_row.device
-    # CSR of the strength graph by row (s_row is ascending: A is row-major sorted) and by column
-    ptr = torch.zeros(n + 1, dtype=torch.int64, device=dev)
-    ptr[1:] = torch.cumsum(torch.bincount(s_row, minlength=n), 0)
-    order = torch.argsort(s_col, stable=True)
-    t_nb = s_row[order]                      # rows that list node j as a neighbour, grouped by j
-    tptr = torch.zeros(n + 1, dtype=torch.int64, device=dev)
-    tptr[1:] = torch.cumsum(torch.bincount(s_col, minlength=n), 0)
-    del order
-    agg = torch.arange(n, dtype=torch.int64, device=dev)
-    decided = torch.zeros(n, dtype=torch.bool, device=dev)
-    is_root = torch.zeros(n, dtype=torch.bool, device=dev)
-    F = torch.arange(n, dtype=torch.int64, device=dev)   # undecided nodes to evaluate this round
-    rounds = 0
-    while F.numel():
-        rounds += 1
-        e, seg = _expand_segments(ptr, F)
-        nb = s_col[e]
-        # eligible neighbours: undecided or root; their aggregate value is their own index
-        elig = (~decided[nb]) | is_root[nb]
-        cand = torch.where(elig, nb, torch.full_like(nb, BIG))
-        m = torch.full((F.numel(),), BIG, dtype=torch.int64, device=dev)
-        m.scatter_reduce_(0, seg, cand, reduce="amin")
-        take = m < F                                     # a smaller eligible neighbour exists
-        mc = torch.where(take, m, F)
-        dec_nei = torch.where(take, decided[mc], torch.ones_like(take))
-        root_nei = take & is_root[mc]
-        new_root = dec_nei & (~take)
-        join = dec_nei & root_nei
-        newly = F[dec_nei]
-        # synchronous update: everything above read the state of the previous round
-        agg[F[join]] = mc[join]
-        is_root[F[new_root]] = True
-        decided[newly] = True
-        # next round: undecided nodes one of whose neighbours was just decided
-        te, _ = _expand_segments(tptr, newly)
-        cand_rows = t_nb[te]
-        cand_rows = cand_rows[~decided[cand_rows]]
-        F = torch.unique(cand_rows)
-    assert bool(decided.all())
-    # aggregate_index_update: coarse id = rank of the root among the sorted roots
-    coarse_of_root = torch.cumsum(is_root.to(torch.int64), 0) - 1
-    return coarse_of_root[agg], int(is_root.sum()), rounds
-
-
-def prolongator(A: _Csr, agg_c: torch.Tensor, nc: int, inv_diag: torch.Tensor) -> _Csr:
-    """SA(): P = (I - w D^-1 A) P_t with P_t(i, agg(i)) = 1"""
-    v = -JACOBI_OMEGA * inv_diag[A.row] * A.val
-    v = torch.where(A.row == A.col, v + 1.0, v)
-    P = _coalesce(A.n_rows, nc, A.row, agg_c[A.col], v)
-    keep = P.val.abs() > ALMOST_ZERO
-    return _Csr(P.n_rows, nc, P.row[keep], P.col[keep], P.val[keep])
-
-
-def filter_entries(Ac: _Csr, thre: float) -> _Csr:
-    """saena_object::filter: off-diagonal |v| <= thre is lumped into the diagonal"""
-    n, dev = Ac.n_rows, Ac.val.device
-    is_diag = Ac.row == Ac.col
-    keep = (Ac.val.abs() > thre) | is_diag
-    add = torch.zeros(n, dtype=torch.float64, device=dev)
-    add.index_add_(0, Ac.row[~keep], Ac.val[~keep])
-    row, col, val = Ac.row[keep], Ac.col[keep], Ac.val[keep].clone()
-    d = row == col
-    val[d] = val[d] + add[row[d]]
-    val[d] = torch.where(val[d].abs() < ALMOST_ZERO, torch.ones_like(val[d]), val[d])
-    has_diag = torch.zeros(n, dtype=torch.bool, device=dev)
-    has_diag[row[d]] = True
-    if not bool(has_diag.all()):
-        miss = torch.nonzero(~has_diag).flatten()
-        return _coalesce(n, n, torch.cat([row, miss]), torch.cat([col, miss]),
-                         torch.cat([val, torch.ones(miss.numel(), dtype=torch.float64, device=dev)]))
-    return _Csr(n, n, row, col, val)
-
-
-def lanczos_eig_max(A: _Csr, inv_diag: torch.Tensor, iters: int, seed: int) -> float:
-    """largest eigenvalue of D^-1/2 A D^-1/2 (find_eig: scale_matrix + find_eig_lamlan), x 1.0001"""
-    n, dev = A.n_rows, A.val.device
-    s = torch.sqrt(inv_diag.abs())
-    g = torch.Generator(device="cpu").manual_seed(seed)
-    v = torch.randn(n, dtype=torch.float64, generator=g).to(dev)
-    v /= torch.linalg.norm(v)
-    v_prev = torch.zeros_like(v)
-    alphas, betas = [], []
-    beta = 0.0
-    k = min(iters, n)
-    for _ in range(k):
-        w = s * _matvec(A, s * v) - beta * v_prev
-        alpha = float(torch.dot(w, v))
-        w = w - alpha * v
-        beta = float(torch.linalg.norm(w))
-        alphas.append(alpha)
-        if beta < 1e-14:
-            break
-        betas.append(beta)
-        v_prev, v = v, w / beta
-    T = np.diag(alphas) + np.diag(betas[:len(alphas) - 1], 1) + np.diag(betas[:len(alphas) - 1], -1)
-    return 1.0001 * float(np.linalg.eigvalsh(T)[-1])
-
-
 # ------------------------------------------------------------------------------------------
 @dataclass
 class DeviceLevel:
-    A: _Csr
+    """one level of the setup as torch tensors: this rank's rows of A, P and R (sa_setup_dist.DCsr; on one rank the
+    global matrices)"""
+    A: "DCsr"
     inv_diag: torch.Tensor
     eig_max: float
     a_use_double: bool
-    P: Optional[_Csr] = None
-    R: Optional[_Csr] = None
+    P: Optional["DCsr"] = None
+    R: Optional["DCsr"] = None
     pr_use_double: bool = True
+
+
+def rank_layout(kind, level, row, col, val, Mbig, Nbig, row_split, col_split, rank, use_double, send_side) -> Operator:
+    """One rank's Operator from its rows (`row` local ids, `col` global ids, row-major sorted), on device tensors: the
+    receive half of hierarchy.split_operator -- the local block, the remote block column-major and grouped by owner.
+    The send half is what the other ranks ask of this one, which the builders learn in different ways:
+    send_side(distinct remote columns of this rank) -> (entries sent to each rank, their local column ids)."""
+    dev = val.device
+    nprocs = len(col_split) - 1
+    r0, nrows = int(row_split[rank]), int(row_split[rank + 1] - row_split[rank])
+    c0, c1 = int(col_split[rank]), int(col_split[rank + 1])
+    local = (col >= c0) & (col < c1)
+    op = dict(kind=kind, level=level, M=nrows, Mbig=Mbig, Nbig=Nbig, row_offset=r0, col_offset=c0,
+              n_local_cols=c1 - c0, use_double=use_double, nprocs=nprocs, rank=rank)
+    op["nnzPerRow_local"] = torch.bincount(row[local], minlength=nrows).to(torch.int32).cpu().numpy()
+    op["col_local"] = col[local].to(torch.int32).cpu().numpy()
+    op["val_local"] = val[local].cpu().numpy()
+    if nprocs == 1:
+        return Operator(**op)
+    # remote part: column-major (col, then row)
+    rr, rc, rv = row[~local], col[~local], val[~local]
+    order = torch.argsort(rc * max(nrows, 1) + rr)
+    rr, rc, rv = rr[order], rc[order], rv[order]
+    distinct, counts = torch.unique_consecutive(rc, return_counts=True)
+    cs = torch.as_tensor(np.asarray(col_split, np.int64), device=dev)
+    owner_d = torch.searchsorted(cs, distinct, right=True) - 1
+    owner_e = torch.searchsorted(cs, rc, right=True) - 1
+    recv_count = torch.bincount(owner_d, minlength=nprocs).cpu().numpy().astype(np.int32)
+    nnz_per_proc = torch.bincount(owner_e, minlength=nprocs).cpu().numpy()
+    op["row_remote"] = rr.to(torch.int32).cpu().numpy()
+    op["val_remote"] = rv.cpu().numpy()
+    op["nnzPerCol_remote"] = counts.to(torch.int32).cpu().numpy()
+    op["nnzPerProcScan"] = np.concatenate(([0], np.cumsum(nnz_per_proc))).astype(np.int64)
+    op["rdispls"] = np.concatenate(([0], np.cumsum(recv_count)[:-1])).astype(np.int32)
+    op["recvProcRank"] = np.flatnonzero(recv_count).astype(np.int32)
+    op["recvProcCount"] = recv_count[recv_count != 0]
+    send_count, v_index = send_side(distinct)
+    send_count = np.asarray(send_count, np.int32)
+    op["vIndex"] = v_index.to(torch.int32).cpu().numpy()
+    op["vdispls"] = np.concatenate(([0], np.cumsum(send_count)[:-1])).astype(np.int32)
+    op["sendProcRank"] = np.flatnonzero(send_count).astype(np.int32)
+    op["sendProcCount"] = send_count[send_count != 0]
+    return Operator(**op)
 
 
 class DeviceHierarchy:
@@ -373,13 +266,12 @@ class DeviceHierarchy:
 
     # -- partitions ----------------------------------------------------------------------------
     @staticmethod
-    def _balanced_split(M: _Csr, nprocs: int) -> np.ndarray:
+    def _balanced_split(M, nprocs: int) -> np.ndarray:
         """nnz-balanced contiguous row blocks (hierarchy.balanced_split on device counts)"""
-        from .hierarchy import balanced_split, csr_from_counts
-        return balanced_split(csr_from_counts(M.counts().cpu().numpy()), nprocs)
+        return balanced_split(csr_from_counts(M.counts().cpu().numpy()), nprocs).astype(np.int64)
 
     @staticmethod
-    def _aligned_coarse_split(R: _Csr, fine_split: np.ndarray) -> np.ndarray:
+    def _aligned_coarse_split(R, fine_split: np.ndarray) -> np.ndarray:
         """hierarchy.aligned_coarse_split on device tensors"""
         dev = R.val.device
         nprocs = len(fine_split) - 1
@@ -399,72 +291,37 @@ class DeviceHierarchy:
         """(row partition of every level, partition R of the level above writes into, agglomerated?)
         -- hierarchy.partition_hierarchy's rules"""
         L = len(self.levels)
-        splits, aligned, agglomerated = [], [], []
-        for l, lv in enumerate(self.levels):
-            agg = l > 0 and (lv.A.n_rows < agglomerate_below or agglomerated[-1] or l == L - 1) and nprocs > 1
-            agglomerated.append(bool(agg))
-            all_on_0 = np.concatenate(([0], np.full(nprocs, lv.A.n_rows))).astype(np.int64)
-            if l == 0:
-                aligned.append(None)
-                splits.append(self._balanced_split(lv.A, nprocs).astype(np.int64))
-                continue
-            al = all_on_0 if agglomerated[l - 1] else self._aligned_coarse_split(self.levels[l - 1].R, splits[l - 1])
-            if rebalance_above > 0 and not agg and not agglomerated[l - 1]:
-                from .hierarchy import csr_from_counts, split_imbalance
-                indptr = csr_from_counts(lv.A.counts().cpu().numpy())
-                if split_imbalance(indptr, al) > rebalance_above:
-                    al = self._balanced_split(lv.A, nprocs).astype(np.int64)
+        splits, aligned, agglomerated = [self._balanced_split(self.levels[0].A, nprocs)], [None], [False]
+        for l in range(1, L):
+            A = self.levels[l].A
+            follow = self._aligned_coarse_split(self.levels[l - 1].R, splits[-1])
+            al, sp, agg = coarse_placement(
+                nprocs, A.n_rows, l == L - 1, agglomerated[-1], agglomerate_below, rebalance_above, follow,
+                imbalance=lambda: split_imbalance(csr_from_counts(A.counts().cpu().numpy()), follow),
+                balanced=lambda: self._balanced_split(A, nprocs))
             aligned.append(al)
-            splits.append(all_on_0 if agg else al)
+            splits.append(sp)
+            agglomerated.append(agg)
         return splits, aligned, agglomerated
 
     @staticmethod
-    def _rank_operator(kind, level, M: _Csr, row_split, col_split, rank, use_double) -> Operator:
+    def _rank_operator(kind, level, M, row_split, col_split, rank, use_double) -> Operator:
         """one rank's Operator -- hierarchy.split_operator restated on device tensors, building
         only `rank`'s arrays (the other ranks' requests are still needed for the send plan)"""
-        dev = M.val.device
         nprocs = len(row_split) - 1
-        rs = torch.as_tensor(row_split, device=dev)
-        cs = torch.as_tensor(col_split, device=dev)
         r0, r1, c0, c1 = int(row_split[rank]), int(row_split[rank + 1]), int(col_split[rank]), int(col_split[rank + 1])
         mine = (M.row >= r0) & (M.row < r1)
-        row, col, val = M.row[mine] - r0, M.col[mine], M.val[mine]
-        local = (col >= c0) & (col < c1)
-        nrows = r1 - r0
-        op = dict(kind=kind, level=level, M=nrows, Mbig=M.n_rows, Nbig=M.n_cols, row_offset=r0, col_offset=c0,
-                  n_local_cols=c1 - c0, use_double=use_double, nprocs=nprocs, rank=rank)
-        op["nnzPerRow_local"] = torch.bincount(row[local], minlength=nrows).to(torch.int32).cpu().numpy()
-        op["col_local"] = col[local].to(torch.int32).cpu().numpy()
-        op["val_local"] = val[local].cpu().numpy()
-        if nprocs == 1:
-            return Operator(**op)
-        # remote part: column-major (col, then row)
-        rr, rc, rv = row[~local], col[~local], val[~local]
-        order = torch.argsort(rc * max(nrows, 1) + rr)
-        rr, rc, rv = rr[order], rc[order], rv[order]
-        distinct, counts = torch.unique_consecutive(rc, return_counts=True)
-        owner_d = torch.searchsorted(cs, distinct, right=True) - 1
-        owner_e = torch.searchsorted(cs, rc, right=True) - 1
-        recv_count = torch.bincount(owner_d, minlength=nprocs).cpu().numpy().astype(np.int32)
-        nnz_per_proc = torch.bincount(owner_e, minlength=nprocs).cpu().numpy()
-        op["row_remote"] = rr.to(torch.int32).cpu().numpy()
-        op["val_remote"] = rv.cpu().numpy()
-        op["nnzPerCol_remote"] = counts.to(torch.int32).cpu().numpy()
-        op["nnzPerProcScan"] = np.concatenate(([0], np.cumsum(nnz_per_proc))).astype(np.int64)
-        op["rdispls"] = np.concatenate(([0], np.cumsum(recv_count)[:-1])).astype(np.int32)
-        op["recvProcRank"] = np.flatnonzero(recv_count).astype(np.int32)
-        op["recvProcCount"] = recv_count[recv_count != 0]
-        # what the others ask of me: entries whose column I own and whose row I do not
-        wanted = (M.col >= c0) & (M.col < c1) & ~mine
-        dst = torch.searchsorted(rs, M.row[wanted], right=True) - 1
-        key = torch.unique(dst * M.n_cols + M.col[wanted])
-        dst_u, col_u = key // M.n_cols, key % M.n_cols
-        send_count = torch.bincount(dst_u, minlength=nprocs).cpu().numpy().astype(np.int32)
-        op["vIndex"] = (col_u - c0).to(torch.int32).cpu().numpy()
-        op["vdispls"] = np.concatenate(([0], np.cumsum(send_count)[:-1])).astype(np.int32)
-        op["sendProcRank"] = np.flatnonzero(send_count).astype(np.int32)
-        op["sendProcCount"] = send_count[send_count != 0]
-        return Operator(**op)
+
+        def send_side(_):
+            # what the others ask of me: entries whose column I own and whose row I do not
+            rs = torch.as_tensor(row_split, device=M.val.device)
+            wanted = (M.col >= c0) & (M.col < c1) & ~mine
+            dst = torch.searchsorted(rs, M.row[wanted], right=True) - 1
+            key = torch.unique(dst * M.n_cols + M.col[wanted])
+            return torch.bincount(key // M.n_cols, minlength=nprocs).cpu().numpy(), key % M.n_cols - c0
+
+        return rank_layout(kind, level, M.row[mine] - r0, M.col[mine], M.val[mine], M.n_rows, M.n_cols, row_split,
+                           col_split, rank, use_double, send_side)
 
     def to_rank(self, rank: int = 0, nprocs: int = 1, agglomerate_below: int = 0,
                 rebalance_above: float = 0.0) -> Hierarchy:
@@ -483,14 +340,7 @@ class DeviceHierarchy:
                 out.R = self._rank_operator(KIND_R, l, lv.R, so, sp, rank, lv.pr_use_double)
                 out.M_coarse_old = int(so[rank + 1] - so[rank])
                 out.M_coarse = int(sn[rank + 1] - sn[rank])
-                if not np.array_equal(so, sn):
-                    for peer in range(nprocs):
-                        a, b = max(so[rank], sn[peer]), min(so[rank + 1], sn[peer + 1])
-                        if b > a:
-                            out.repart_send.append((peer, int(a - so[rank]), int(b - a)))
-                        a, b = max(sn[rank], so[peer]), min(sn[rank + 1], so[peer + 1])
-                        if b > a:
-                            out.repart_recv.append((peer, int(a - sn[rank]), int(b - a)))
+                out.repart_send, out.repart_recv = repart_plan(so, sn, rank)
             levels.append(out)
         last = self.levels[-1].A
         return Hierarchy(levels=levels, coarse_n=last.n_rows, coarse_row=last.row.to(torch.int32).cpu().numpy(),
@@ -500,63 +350,19 @@ class DeviceHierarchy:
 
 def build_device_hierarchy(n: int, row, col, val, opts: Optional[SetupOptions] = None, device: Optional[str] = None,
                            verbose: bool = False) -> DeviceHierarchy:
-    """Global hierarchy from a square matrix given as COO (any order, duplicates added)."""
-    opts = opts or SetupOptions()
+    """Global hierarchy from a square matrix given as COO (any order, duplicates added): the coarsening loop of
+    sa_setup_dist.py on one rank, where this rank's rows are the whole matrix."""
+    from . import sa_setup_dist as sd
     dev = torch.device(device or ("cuda" if torch.cuda.is_available() else "cpu"))
 
     def as_t(a, dt):
         return a.to(dev, dt) if isinstance(a, torch.Tensor) else torch.as_tensor(np.ascontiguousarray(a), device=dev).to(dt)
 
     A = _coalesce(n, n, as_t(row, torch.int64), as_t(col, torch.int64), as_t(val, torch.float64))
-    levels: List[DeviceLevel] = []
-    filter_thre = opts.filter_thre
-    filter_it = 0
-    l = 0
-    last_level = False
-    a_use_double = opts.float_level != 0                  # saena_object.cpp:241-244
-    while True:
-        d = A.diag()
-        if bool((d.abs() < ALMOST_ZERO).any()):
-            raise ValueError("zero diagonal element")      # inverse_diag: print + exit in the reference
-        inv_diag = 1.0 / d
-        eig = lanczos_eig_max(A, inv_diag, opts.lanczos_iters, opts.seed + l)
-        lv = DeviceLevel(A=A, inv_diag=inv_diag, eig_max=eig, a_use_double=a_use_double)
-        levels.append(lv)
-        if verbose:
-            print(f"level {l}: rows {A.n_rows} nnz {A.nnz} ({A.nnz / A.n_rows:.1f}/row) eig {eig:.4f}", file=sys.stderr, flush=True)
-        if l >= opts.max_level or last_level:
-            break
-        t_ag = time.perf_counter()
-        s_r, s_c = strength_graph(A, opts.conn_str)
-        agg_c, nc, rounds = aggregate(A.n_rows, s_r, s_c)
-        del s_r, s_c
-        if verbose:
-            _sync(dev)
-            print(f"   aggregation: {nc} aggregates in {rounds} rounds, {time.perf_counter() - t_ag:.1f}s", file=sys.stderr, flush=True)
-        t_rap = time.perf_counter()
-        # find_aggregation's dynamic-level rule: the level about to be created is the last one
-        if opts.dynamic_levels:
-            last_level = bool(nc <= opts.least_row_threshold or
-                              np.float32(nc) / np.float32(A.n_rows) > np.float32(opts.row_reduction_up_thrshld))
-        else:
-            last_level = (l + 1 == opts.max_level)
-        P = prolongator(A, agg_c, nc, inv_diag)
-        R = _transpose(P)
-        Ac = _galerkin(R, A, P)
-        filter_it += 1
-        if filter_it >= opts.filter_start:
-            filter_thre = min(filter_thre, opts.filter_max)
-            Ac = filter_entries(Ac, filter_thre)
-            filter_thre *= 10 ** opts.filter_rate
-        if verbose:
-            _sync(dev)
-            print(f"   P, R, RAP, filter: {time.perf_counter() - t_rap:.1f}s", file=sys.stderr, flush=True)
-        lv.P, lv.R = P, R
-        lv.pr_use_double = not (l >= opts.float_level)     # saena_object.cpp:277-280
-        a_use_double = not (l + 1 >= opts.float_level)     # :281-284
-        A = Ac
-        l += 1
-    return DeviceHierarchy(levels)
+    A0 = sd.DCsr(n, n, [0, n], 0, A.row, A.col, A.val)
+    del A
+    levels = sd.coarsen(sd.Comm(dev, one_rank=True), A0, opts or SetupOptions(), 0, 0.0, verbose=verbose)
+    return DeviceHierarchy([lv for lv, _, _ in levels])
 
 
 def build_hierarchy(n: int, row, col, val, opts: Optional[SetupOptions] = None, device: Optional[str] = None,

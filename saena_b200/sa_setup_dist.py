@@ -1,20 +1,22 @@
-"""sa_setup.py on several ranks: the same smoothed-aggregation setup, row-partitioned, one process per
-GPU -- ONLY to feed the benchmark with a hierarchy no single GPU can build (BASELINE.json
-configs[2]: 512^3 unknowns on 8 B200; sa_setup.py builds the global hierarchy on ONE device).
+"""The smoothed-aggregation setup of sa_setup.py (whose header cites the reference lines), row-partitioned, one
+process per GPU -- ONLY to feed the benchmark, among others with a hierarchy no single GPU can build
+(BASELINE.json configs[2]: 512^3 unknowns on 8 B200).  This is the only copy of the setup's steps and level loop:
+sa_setup.build_device_hierarchy runs them on one rank (a one-rank `Comm` even inside a process group), where the
+collectives are identities, `ColMap` has no ghosts and the aggregation refreshes no ghost states.
 
-The AMG setup is outside this package's scope (see sa_setup.py's header); like sa_setup.py this
-module is plumbing made of torch tensor ops, here with torch.distributed collectives (NCCL on GPUs,
-gloo in the CPU tests).  Nothing in the solve path imports it.
+The AMG setup is outside this package's scope (see sa_setup.py's header); this module is plumbing made of
+torch tensor ops and torch.distributed collectives (NCCL on GPUs, gloo in the CPU tests).  Nothing in the
+solve path imports it.
 
-Every step restates the step of sa_setup.py (which cites the reference lines) on a 1-D row
-partition, with the SAME rules and the same synchronous iterations:
+Every step works on a 1-D row partition, with the reference's rules and the same synchronous iterations on any
+number of ranks:
 
   * strength of connection, prolongator, filter: row-local, the values a row needs from other
     ranks (its neighbours' row maxima, aggregate ids, inverse diagonal) are fetched once;
   * aggregation: aggregation_1_dist (src/saena_object_setup1.cpp:724-995) IS a synchronous
     data-parallel iteration -- each round reads the states of the round before -- so exchanging
     the states of the ghost nodes after every round reproduces the one-rank aggregates exactly,
-    whatever the partition (tests/dist_setup_check.py compares with sa_setup.py's);
+    whatever the partition (tests/dist_setup_check.py compares N ranks with one);
   * coarse numbering: a root's coarse id is its rank among the sorted roots, so each rank's
     aggregates are a contiguous block of coarse rows -- "an aggregate lives where its root lives",
     splitNew in aggregate_index_update (src/saena_object_setup1.cpp:2124-2132);
@@ -25,10 +27,11 @@ partition, with the SAME rules and the same synchronous iterations:
   * Chebyshev bound: Lanczos on D^-1/2 A D^-1/2 from the same seeded global start vector.
 
 The partition each level ends up with is the one the solve uses (hierarchy.partition_hierarchy's
-rules): level 0 nnz-balanced, a coarse level follows the level above unless one rank would hold
-more than `rebalance_above` x the mean nnz (then it is re-split by its own nnz balance and moved),
-levels below `agglomerate_below` global rows and the coarsest live on rank 0.  The result is each
-rank's `Hierarchy` in the reference layout, ready for `saena_b200_upload_operator`.
+rules, hierarchy.coarse_placement): level 0 nnz-balanced, a coarse level follows the level above unless
+one rank would hold more than `rebalance_above` x the mean nnz (then it is re-split by its own nnz
+balance and moved), levels below `agglomerate_below` global rows and the coarsest live on rank 0.
+`coarsen` is the level loop and hands out each level's tensors; `build_distributed_hierarchy` turns
+them into each rank's `Hierarchy` in the reference layout, ready for `saena_b200_upload_operator`.
 """
 from __future__ import annotations
 
@@ -41,19 +44,20 @@ import numpy as np
 import torch
 import torch.distributed as dist
 
-from .hierarchy import F64, I64, KIND_A, KIND_P, KIND_R, Hierarchy, Level, Operator
-from .sa_setup import (ALMOST_ZERO, BIG, JACOBI_OMEGA, SetupOptions, _coalesce, _Csr, _expand_segments, _spgemm,
-                       _to_torch_csr, _transpose)
+from .hierarchy import F64, I64, KIND_A, KIND_P, KIND_R, Hierarchy, Level, Operator, coarse_placement, repart_plan
+from .sa_setup import (ALMOST_ZERO, BIG, JACOBI_OMEGA, DeviceLevel, SetupOptions, _coalesce, _Csr, _expand_segments,
+                       _native_spgemm_enabled, _spgemm, _to_torch_csr, _transpose, rank_layout)
 
 
 # ------------------------------------------------------------------------------------------
 # collectives
 # ------------------------------------------------------------------------------------------
 class Comm:
-    """the few collectives the setup needs, on whatever backend the default group runs"""
+    """the few collectives the setup needs, on whatever backend the default group runs; `one_rank`: this process
+    alone (world size 1) even where a process group runs -- the setup of sa_setup.build_device_hierarchy"""
 
-    def __init__(self, device: Optional[torch.device] = None):
-        self.on = dist.is_available() and dist.is_initialized()
+    def __init__(self, device: Optional[torch.device] = None, one_rank: bool = False):
+        self.on = not one_rank and dist.is_available() and dist.is_initialized()
         self.rank = dist.get_rank() if self.on else 0
         self.world = dist.get_world_size() if self.on else 1
         if device is None:
@@ -85,6 +89,12 @@ class Comm:
         t = torch.tensor([x], dtype=torch.int64 if isint else torch.float64, device=self.dev)
         dist.all_reduce(t)
         return int(t.item()) if isint else float(t.item())
+
+    def norm(self, x: torch.Tensor) -> float:
+        """2-norm of a row-partitioned vector"""
+        if self.world == 1:
+            return float(torch.linalg.norm(x))
+        return float(np.sqrt(self.sum(float(torch.dot(x, x)))))
 
     def sum_tensor(self, t: torch.Tensor) -> torch.Tensor:
         if self.world > 1:
@@ -151,10 +161,10 @@ class ColMap:
         self.g_lo = int((self.ghost < self.c0).sum()) if self.ghost.numel() else 0
         self.n_ext = self.m + int(self.ghost.numel())
         self.fetcher = Fetcher(comm, split, self.ghost)
-        dev = cols.device
-        self.gid = torch.cat([self.ghost[:self.g_lo], torch.arange(self.c0, self.c1, device=dev), self.ghost[self.g_lo:]])
 
     def to_ext(self, gid: torch.Tensor) -> torch.Tensor:
+        if not self.ghost.numel():          # every column is mine (one rank): no copy of the column ids at c0 = 0
+            return gid - self.c0 if self.c0 else gid
         pos = torch.searchsorted(self.ghost, gid)
         own = (gid >= self.c0) & (gid < self.c1)
         return torch.where(own, gid - self.c0 + self.g_lo, torch.where(gid < self.c0, pos, pos + self.m))
@@ -233,6 +243,8 @@ def balanced_split_dist(comm: Comm, A: DCsr) -> np.ndarray:
 def fetch_rows(comm: Comm, P: DCsr, cm: ColMap) -> _Csr:
     """rows of P for every index of cm's extended space (my own rows in the middle, the ghost rows fetched
     from their owners), as a matrix with n_ext rows"""
+    if comm.world == 1:
+        return _Csr(P.m, P.n_cols, P.row, P.col, P.val)
     dev = P.val.device
     f = cm.fetcher
     counts = P.counts()
@@ -270,13 +282,14 @@ def diag_local(A: DCsr) -> torch.Tensor:
 
 def lanczos_eig_max_dist(comm: Comm, A: DCsr, cm: ColMap, col_ext: torch.Tensor, inv_diag: torch.Tensor, iters: int,
                          seed: int) -> float:
-    """sa_setup.lanczos_eig_max with the dot products summed over ranks and the same global start vector"""
+    """largest eigenvalue of D^-1/2 A D^-1/2 (find_eig: scale_matrix + find_eig_lamlan), x 1.0001; the start vector is
+    the same global seeded vector on any number of ranks"""
     dev = A.val.device
     n = A.n_rows
     s = torch.sqrt(inv_diag.abs())
     g = torch.Generator(device="cpu").manual_seed(seed)
     v = torch.randn(n, dtype=torch.float64, generator=g)[A.r0:A.r1].to(dev)
-    v = v / np.sqrt(comm.sum(float(torch.dot(v, v))))
+    v = v / comm.norm(v)
     v_prev = torch.zeros_like(v)
     alphas, betas = [], []
     beta = 0.0
@@ -287,7 +300,7 @@ def lanczos_eig_max_dist(comm: Comm, A: DCsr, cm: ColMap, col_ext: torch.Tensor,
         w = s * w - beta * v_prev
         alpha = comm.sum(float(torch.dot(w, v)))
         w = w - alpha * v
-        beta = float(np.sqrt(comm.sum(float(torch.dot(w, w)))))
+        beta = comm.norm(w)
         alphas.append(alpha)
         if beta < 1e-14:
             break
@@ -299,27 +312,32 @@ def lanczos_eig_max_dist(comm: Comm, A: DCsr, cm: ColMap, col_ext: torch.Tensor,
 
 
 def strength_graph_dist(A: DCsr, cm: ColMap, col_ext: torch.Tensor, conn_str: float):
-    """sa_setup.strength_graph; returns the strong connections in cm's extended numbering"""
+    """strong off-diagonal connections (row, col) -- create_strength_matrix + setup_matrix -- in cm's extended
+    numbering"""
     dev = A.val.device
     off = (A.row + A.r0) != A.col
     max_per_row = torch.full((A.m,), -torch.finfo(torch.float64).max, dtype=torch.float64, device=dev)
     max_per_row.scatter_reduce_(0, A.row[off], -A.val[off], reduce="amax")
     mpr_ext = cm.extend(max_per_row)
-    s_row = -A.val / max_per_row[A.row]
-    s_col = -A.val / mpr_ext[col_ext]
+    s_row = -A.val / max_per_row[A.row]      # entry   (normalised by its row's maximum)
+    s_col = -A.val / mpr_ext[col_ext]        # entryT  (normalised by the column index's row maximum)
     strong = off & ((s_row > conn_str) | (s_col > conn_str))
     return A.row[strong] + cm.g_lo, col_ext[strong]
 
 
 def aggregate_dist(comm: Comm, cm: ColMap, s_row: torch.Tensor, s_col: torch.Tensor):
-    """sa_setup.aggregate on a partition: the states of the ghost nodes are refreshed after every round.
-    Returns (coarse id of every node of the extended space, number of aggregates, coarse split, rounds)."""
+    """aggregation_1_dist.  The reference sweeps every undecided node in every round; a node's outcome can only change
+    when one of its neighbours was decided in the round before, so only those nodes are re-evaluated here (same rule,
+    same synchronous updates, hence the same aggregates -- tests/test_sa_setup.py compares with the reference's).  On
+    several ranks the states of the ghost nodes are refreshed after every round.  Returns (coarse id of every node of
+    the extended space, number of aggregates, coarse split, rounds)."""
     dev = s_row.device
     E, m, lo = cm.n_ext, cm.m, cm.g_lo
+    # CSR of the strength graph by row (s_row is ascending: A is row-major sorted) and by column
     ptr = torch.zeros(E + 1, dtype=torch.int64, device=dev)
     ptr[1:] = torch.cumsum(torch.bincount(s_row, minlength=E), 0)
     order = torch.argsort(s_col, stable=True)
-    t_nb = s_row[order]
+    t_nb = s_row[order]                      # rows that list node j as a neighbour, grouped by j
     tptr = torch.zeros(E + 1, dtype=torch.int64, device=dev)
     tptr[1:] = torch.cumsum(torch.bincount(s_col, minlength=E), 0)
     del order
@@ -327,23 +345,25 @@ def aggregate_dist(comm: Comm, cm: ColMap, s_row: torch.Tensor, s_col: torch.Ten
     decided = torch.zeros(E, dtype=torch.bool, device=dev)
     is_root = torch.zeros(E, dtype=torch.bool, device=dev)
     ghost_idx = cm.ghost_ext_index()
-    F = torch.arange(lo, lo + m, dtype=torch.int64, device=dev)
+    F = torch.arange(lo, lo + m, dtype=torch.int64, device=dev)   # undecided nodes to evaluate this round
     rounds = 0
     while comm.sum(int(F.numel())) > 0:
         rounds += 1
         e, seg = _expand_segments(ptr, F)
         nb = s_col[e]
+        # eligible neighbours: undecided or root; their aggregate value is their own index
         elig = (~decided[nb]) | is_root[nb]
         cand = torch.where(elig, nb, torch.full_like(nb, BIG))
         mn = torch.full((F.numel(),), BIG, dtype=torch.int64, device=dev)
         mn.scatter_reduce_(0, seg, cand, reduce="amin")
-        take = mn < F
+        take = mn < F                                    # a smaller eligible neighbour exists
         mc = torch.where(take, mn, F)
         dec_nei = torch.where(take, decided[mc], torch.ones_like(take))
         root_nei = take & is_root[mc]
         new_root = dec_nei & (~take)
         join = dec_nei & root_nei
         newly = F[dec_nei]
+        # synchronous update: everything above read the state of the previous round
         agg[F[join]] = mc[join]
         is_root[F[new_root]] = True
         decided[newly] = True
@@ -356,6 +376,7 @@ def aggregate_dist(comm: Comm, cm: ColMap, s_row: torch.Tensor, s_col: torch.Ten
             decided[ghost_idx] = g_dec
             is_root[ghost_idx] = (g & 2).bool()
             newly = torch.cat([newly, changed])
+        # next round: undecided nodes one of whose neighbours was just decided
         te, _ = _expand_segments(tptr, newly)
         cand_rows = t_nb[te]
         cand_rows = cand_rows[~decided[cand_rows]]
@@ -372,7 +393,7 @@ def aggregate_dist(comm: Comm, cm: ColMap, s_row: torch.Tensor, s_col: torch.Ten
 
 
 def prolongator_dist(A: DCsr, col_ext: torch.Tensor, agg_c_ext: torch.Tensor, nc: int, inv_diag: torch.Tensor) -> DCsr:
-    """sa_setup.prolongator on my rows"""
+    """SA(): P = (I - w D^-1 A) P_t with P_t(i, agg(i)) = 1, on my rows"""
     v = -JACOBI_OMEGA * inv_diag[A.row] * A.val
     v = torch.where((A.row + A.r0) == A.col, v + 1.0, v)
     P = _coalesce(max(A.m, 1), nc, A.row, agg_c_ext[col_ext], v)
@@ -391,6 +412,8 @@ def transpose_dist(comm: Comm, P: DCsr, coarse_split: np.ndarray) -> DCsr:
 
 def _add_partial_rows(comm: Comm, nc: int, coarse_split: np.ndarray, grow, gcol, val) -> DCsr:
     """partial coarse rows (global ids) -> their owners, duplicates added"""
+    if comm.world == 1:                  # whole rows, already sorted and without duplicates
+        return DCsr(nc, nc, coarse_split, 0, grow, gcol, val)
     grow, gcol, val = _route_rows(comm, coarse_split, grow, gcol, val)
     c0 = int(coarse_split[comm.rank])
     mc = int(coarse_split[comm.rank + 1]) - c0
@@ -398,7 +421,7 @@ def _add_partial_rows(comm: Comm, nc: int, coarse_split: np.ndarray, grow, gcol,
     return DCsr(nc, nc, coarse_split, comm.rank, C.row, C.col, C.val)
 
 
-# measured on one B200 at 256^3 (gpurun_out/run7.log, sa_setup.py): level 3 -> 4 through sparse x dense products,
+# measured on one B200 at 256^3: level 3 -> 4 through sparse x dense products,
 # 167 M stored entries x 21 466 columns in 2.5 s ~ 1.4e12 multiply-adds/s; the expand / sort / compress route
 # does a few 1e9 scalar products per second (level 2 -> 3: 7.4 s)
 _SPMM_FMA_PER_S = 1.4e12
@@ -406,13 +429,13 @@ _ESC_PRODUCTS_PER_S = 5e9
 
 
 def _prefer_dense(comm: Comm, A: DCsr, A_x: _Csr, P: DCsr, P_ext: _Csr, nc: int) -> bool:
-    """Which of the two routes of galerkin_dist is cheaper for the slowest rank.  On the CPU (tests) only
-    sa_setup._galerkin's rule on small levels, so that both routes stay exercised."""
+    """Which of the two tensor-op routes of galerkin_dist is cheaper for the slowest rank.  On the CPU: expand / sort /
+    compress on one rank (the hierarchies the goldens and the CPU suite compare against), and on several ranks
+    sparse x dense on small nearly dense levels, so that the gloo tests exercise both routes."""
     dev = A.val.device
-    from . import sa_setup
-    if sa_setup._native_spgemm_enabled(dev, dist=True):
-        return False          # the library's device SpGEMM takes every level (same environment on every rank)
     if dev.type != "cuda":
+        if comm.world == 1:
+            return False
         a_nnz, p_nnz = comm.sum(A.nnz), comm.sum(P.nnz)
         return (a_nnz / max(A.n_rows, 1)) * (p_nnz / max(P.n_rows, 1)) > 4 * nc and A.n_rows <= 20000
     prod_ap = int(P_ext.counts()[A_x.col].sum()) if A.nnz else 0          # scalar products of A P on my rows
@@ -428,8 +451,11 @@ def _prefer_dense(comm: Comm, A: DCsr, A_x: _Csr, P: DCsr, P_ext: _Csr, nc: int)
 
 def galerkin_dist(comm: Comm, A: DCsr, cm: ColMap, col_ext: torch.Tensor, P: DCsr, coarse_split: np.ndarray,
                   dense: Optional[bool] = None, dense_budget_bytes: float = 24e9, verbose: bool = False) -> DCsr:
-    """Ac = P^T A P.  `dense` None: sa_setup._galerkin's rule on the global sizes (nearly dense deep levels go
-    through sparse x dense products, column block by column block; everything else expand / sort / compress)."""
+    """Ac = P^T A P.  On the deep levels of a 3D hierarchy the product is nearly dense (256^3 Poisson, level 3 -> 4:
+    rows of A P have ~20 000 entries, 8e11 scalar products) and the sparse expansion drowns; there the products are
+    done as sparse x dense, column block by column block, and the result is re-sparsified (structural zeros stay
+    exact zeros, so the pattern is the sparse product's barring exact cancellation).  `dense` None: the library's
+    device SpGEMM where _native_spgemm_enabled, else _prefer_dense decides."""
     dev = A.val.device
     nc = P.n_cols
     # tests shrink both work sizes so that several column blocks / product chunks are exercised on small inputs
@@ -437,13 +463,15 @@ def galerkin_dist(comm: Comm, A: DCsr, cm: ColMap, col_ext: torch.Tensor, P: DCs
     chunk = int(os.environ.get("SAENA_SETUP_CHUNK_PRODUCTS", 300_000_000))
     P_ext = fetch_rows(comm, P, cm)
     A_x = _Csr(A.m, cm.n_ext, A.row, col_ext, A.val)
+    native = _native_spgemm_enabled(dev, comm.world)
     if dense is None:
-        dense = _prefer_dense(comm, A, A_x, P, P_ext, nc)
+        dense = not native and _prefer_dense(comm, A, A_x, P, P_ext, nc)
     uc, inv = torch.unique(P.col, return_inverse=True)                 # coarse rows my P rows reach
     Pt = _transpose(_Csr(A.m, max(int(uc.numel()), 1), P.row, inv, P.val))        # compact coarse rows x my fine rows
+    del inv
     if not dense:
-        AP = _spgemm(A_x, P_ext, chunk, dist=True)
-        C = _spgemm(Pt, AP, chunk, dist=True)
+        AP = _spgemm(A_x, P_ext, chunk, native)
+        C = _spgemm(Pt, AP, chunk, native)
         del AP
         return _add_partial_rows(comm, nc, coarse_split, uc[C.row] if C.nnz else C.row, C.col, C.val)
     # dense column blocks: AP[:, c0:c1] = A_x P_ext[:, c0:c1]; partial coarse rows P_local^T AP summed over ranks
@@ -481,7 +509,8 @@ def galerkin_dist(comm: Comm, A: DCsr, cm: ColMap, col_ext: torch.Tensor, P: DCs
 
 
 def filter_entries_dist(Ac: DCsr, thre: float) -> DCsr:
-    """sa_setup.filter_entries on my rows (a row's diagonal lives in the row)"""
+    """saena_object::filter on my rows: off-diagonal |v| <= thre is lumped into the diagonal (a row's diagonal lives in
+    the row)"""
     n, dev = Ac.m, Ac.val.device
     grow = Ac.row + Ac.r0
     is_diag = grow == Ac.col
@@ -506,103 +535,56 @@ def filter_entries_dist(Ac: DCsr, thre: float) -> DCsr:
 # a rank's share in the reference layout
 # ------------------------------------------------------------------------------------------
 def rank_operator(comm: Comm, kind: int, level: int, M: DCsr, col_split: np.ndarray, use_double: bool) -> Operator:
-    """sa_setup.DeviceHierarchy._rank_operator where every rank holds only its own rows: what the others ask of
-    me arrives through the request lists (recvCount -> MPI_Alltoall -> sendCount in set_off_on_diagonal,
-    src/saena_matrix_setup.cpp:904-1072)"""
-    dev = M.val.device
-    nprocs, rank = comm.world, comm.rank
-    col_split = np.asarray(col_split, I64)
-    cs = torch.as_tensor(col_split, device=dev)
-    c0, c1 = int(col_split[rank]), int(col_split[rank + 1])
-    row, col, val = M.row, M.col, M.val
-    local = (col >= c0) & (col < c1)
-    nrows = M.m
-    op = dict(kind=kind, level=level, M=nrows, Mbig=M.n_rows, Nbig=M.n_cols, row_offset=M.r0, col_offset=c0,
-              n_local_cols=c1 - c0, use_double=use_double, nprocs=nprocs, rank=rank)
-    op["nnzPerRow_local"] = torch.bincount(row[local], minlength=nrows).to(torch.int32).cpu().numpy()
-    op["col_local"] = col[local].to(torch.int32).cpu().numpy()
-    op["val_local"] = val[local].cpu().numpy()
-    if nprocs == 1:
-        return Operator(**op)
-    rr, rc, rv = row[~local], col[~local], val[~local]
-    order = torch.argsort(rc * max(nrows, 1) + rr)
-    rr, rc, rv = rr[order], rc[order], rv[order]
-    distinct, counts = torch.unique_consecutive(rc, return_counts=True)
-    owner_d = _owner(cs, distinct)
-    owner_e = _owner(cs, rc)
-    recv_count = torch.bincount(owner_d, minlength=nprocs).cpu().numpy().astype(np.int32)
-    nnz_per_proc = torch.bincount(owner_e, minlength=nprocs).cpu().numpy()
-    op["row_remote"] = rr.to(torch.int32).cpu().numpy()
-    op["val_remote"] = rv.cpu().numpy()
-    op["nnzPerCol_remote"] = counts.to(torch.int32).cpu().numpy()
-    op["nnzPerProcScan"] = np.concatenate(([0], np.cumsum(nnz_per_proc))).astype(np.int64)
-    op["rdispls"] = np.concatenate(([0], np.cumsum(recv_count)[:-1])).astype(np.int32)
-    op["recvProcRank"] = np.flatnonzero(recv_count).astype(np.int32)
-    op["recvProcCount"] = recv_count[recv_count != 0]
-    f = Fetcher(comm, col_split, distinct)
-    send_count = np.asarray(f.serve_counts, np.int32)
-    op["vIndex"] = f.serve_idx.to(torch.int32).cpu().numpy()
-    op["vdispls"] = np.concatenate(([0], np.cumsum(send_count)[:-1])).astype(np.int32)
-    op["sendProcRank"] = np.flatnonzero(send_count).astype(np.int32)
-    op["sendProcCount"] = send_count[send_count != 0]
-    return Operator(**op)
+    """sa_setup.rank_layout where every rank holds only its own rows: what the others ask of me arrives through the
+    request lists (recvCount -> MPI_Alltoall -> sendCount in set_off_on_diagonal, src/saena_matrix_setup.cpp:904-1072)"""
+    def send_side(distinct):
+        f = Fetcher(comm, col_split, distinct)
+        return f.serve_counts, f.serve_idx
+
+    return rank_layout(kind, level, M.row, M.col, M.val, M.n_rows, M.n_cols, M.split, col_split, comm.rank, use_double,
+                       send_side)
 
 
-def _repart_plan(so: np.ndarray, sn: np.ndarray, rank: int):
-    send, recv = [], []
-    if not np.array_equal(so, sn):
-        for peer in range(len(so) - 1):
-            a, b = max(so[rank], sn[peer]), min(so[rank + 1], sn[peer + 1])
-            if b > a:
-                send.append((peer, int(a - so[rank]), int(b - a)))
-            a, b = max(sn[rank], so[peer]), min(sn[rank + 1], so[peer + 1])
-            if b > a:
-                recv.append((peer, int(a - sn[rank]), int(b - a)))
-    return send, recv
-
-
-def build_distributed_hierarchy(A0: DCsr, opts: Optional[SetupOptions] = None, agglomerate_below: int = 10_000,
-                                rebalance_above: float = 1.10, verbose: bool = False, dense: Optional[bool] = None,
-                                comm: Optional[Comm] = None):
-    """Collective.  A0: my rows of the fine matrix (any row partition; it is moved to the nnz-balanced one).
-    Returns (this rank's Hierarchy, summary lines of the global hierarchy)."""
-    opts = opts or SetupOptions()
-    comm = comm or Comm(A0.val.device)
+# ------------------------------------------------------------------------------------------
+# the level loop
+# ------------------------------------------------------------------------------------------
+def coarsen(comm: Comm, A0: DCsr, opts: SetupOptions, agglomerate_below: int, rebalance_above: float,
+            dense: Optional[bool] = None, verbose: bool = False):
+    """Collective generator.  A0: my rows of the fine matrix (any row partition; it is moved to the nnz-balanced one).
+    Yields every level, finest first, as (DeviceLevel with my rows of A, P and R, so, sn): `so` is the partition R
+    writes the coarse vector into (P's column partition), `sn` the one the coarse level lives on; the coarsest level
+    comes last, with P, R, so and sn None.  Where a coarse level lives follows hierarchy.partition_hierarchy's rules
+    (hierarchy.coarse_placement).  The generator drops its references to a level's tensors once it is resumed."""
     rank, nprocs = comm.rank, comm.world
     say = (lambda s: print(s, file=sys.stderr, flush=True)) if (verbose and rank == 0) else (lambda s: None)
 
     A = repartition(comm, A0, balanced_split_dist(comm, A0))
-    levels: List[Level] = []
-    summary = []
     filter_thre, filter_it = opts.filter_thre, 0
     l, last_level = 0, False
-    a_use_double = opts.float_level != 0
-    all_on_0 = lambda n: np.concatenate(([0], np.full(nprocs, n))).astype(I64)   # noqa: E731
+    a_use_double = opts.float_level != 0                  # saena_object.cpp:241-244
     while True:
         t_lv = time.perf_counter()
         cm = ColMap(comm, A.split, A.col)
         col_ext = cm.to_ext(A.col)
         d = diag_local(A)
         if comm.sum(int((d.abs() < ALMOST_ZERO).sum())) > 0:
-            raise ValueError("zero diagonal element")
+            raise ValueError("zero diagonal element")      # inverse_diag: print + exit in the reference
         inv_diag = 1.0 / d
         eig = lanczos_eig_max_dist(comm, A, cm, col_ext, inv_diag, opts.lanczos_iters, opts.seed + l)
         g_nnz = comm.sum(A.nnz)
-        line = f"L{l}: M={A.n_rows} nnz={g_nnz} ({g_nnz / A.n_rows:.1f}/row) eig={eig:.4f}"
         say(f"level {l}: rows {A.n_rows} nnz {g_nnz} ({g_nnz / A.n_rows:.1f}/row) eig {eig:.4f} "
             f"[rows per rank {comm.gather_ints(A.m).tolist()}]")
-        lv = Level(level=l, A=rank_operator(comm, KIND_A, l, A, A.split, a_use_double),
-                   inv_diag=inv_diag.cpu().numpy(), eig_max=eig, active=A.m > 0)
-        levels.append(lv)
+        lv = DeviceLevel(A=A, inv_diag=inv_diag, eig_max=eig, a_use_double=a_use_double)
         if l >= opts.max_level or last_level:
-            summary.append(line)
-            break
+            yield lv, None, None
+            return
         t_ag = time.perf_counter()
         s_r, s_c = strength_graph_dist(A, cm, col_ext, opts.conn_str)
         agg_c_ext, nc, so, rounds = aggregate_dist(comm, cm, s_r, s_c)
         del s_r, s_c
         say(f"   aggregation: {nc} aggregates in {rounds} rounds, {time.perf_counter() - t_ag:.1f}s")
         t_rap = time.perf_counter()
+        # find_aggregation's dynamic-level rule: the level about to be created is the last one
         if opts.dynamic_levels:
             last_level = bool(nc <= opts.least_row_threshold or
                               np.float32(nc) / np.float32(A.n_rows) > np.float32(opts.row_reduction_up_thrshld))
@@ -617,39 +599,65 @@ def build_distributed_hierarchy(A0: DCsr, opts: Optional[SetupOptions] = None, a
             filter_thre = min(filter_thre, opts.filter_max)
             Ac = filter_entries_dist(Ac, filter_thre)
             filter_thre *= 10 ** opts.filter_rate
-        # where the coarse level lives (hierarchy.partition_hierarchy's rules)
-        agglomerate = nprocs > 1 and (nc < agglomerate_below or last_level or
-                                      l + 1 >= opts.max_level or bool(np.array_equal(A.split, all_on_0(A.n_rows))))
-        sn = so
-        if agglomerate:
-            sn = all_on_0(nc)
-        elif nprocs > 1 and rebalance_above > 0:
+
+        def imbalance():                 # Ac lives on the aligned split `so`
             per = comm.gather_ints(Ac.nnz)
-            if per.max() * nprocs / max(int(per.sum()), 1) > rebalance_above:
-                sn = so = balanced_split_dist(comm, Ac)      # R and P are partitioned by the new split too
-        R = transpose_dist(comm, P, so)
-        pr_use_double = not (l >= opts.float_level)
-        lv.P = rank_operator(comm, KIND_P, l, P, so, pr_use_double)
-        lv.R = rank_operator(comm, KIND_R, l, R, A.split, pr_use_double)
-        lv.M_coarse_old = int(so[rank + 1] - so[rank])
-        lv.M_coarse = int(sn[rank + 1] - sn[rank])
-        lv.repart_send, lv.repart_recv = _repart_plan(so, sn, rank)
-        summary.append(line + f" | P nnz={comm.sum(P.nnz)}")
-        del P, R
+            return per.max() * nprocs / max(int(per.sum()), 1)
+
+        # a level whose split leaves every row on rank 0 takes its coarse level along; R and P are partitioned by a
+        # re-balanced split too
+        so, sn, _ = coarse_placement(nprocs, nc, last_level or l + 1 >= opts.max_level, bool(A.split[1] == A.n_rows),
+                                     agglomerate_below, rebalance_above, so, imbalance,
+                                     lambda: balanced_split_dist(comm, Ac))
+        lv.P, lv.R = P, transpose_dist(comm, P, so)
+        lv.pr_use_double = not (l >= opts.float_level)     # saena_object.cpp:277-280
+        del P
+        yield lv, so, sn
+        del lv
         A = repartition(comm, Ac, sn)
         del Ac
         say(f"   P, R, RAP, filter, operators: {time.perf_counter() - t_rap:.1f}s (level {time.perf_counter() - t_lv:.1f}s)")
-        a_use_double = not (l + 1 >= opts.float_level)
+        a_use_double = not (l + 1 >= opts.float_level)     # :281-284
         l += 1
-    # the coarsest operator as global COO on every rank (tiny)
-    own = A.m > 0 or nprocs == 1
-    src = int(np.flatnonzero(np.diff(A.split) > 0)[0]) if A.n_rows else 0
-    crow = comm.bcast_tensor((A.row + A.r0) if own else None, torch.int64, src)
-    ccol = comm.bcast_tensor(A.col if own else None, torch.int64, src)
-    cval = comm.bcast_tensor(A.val if own else None, torch.float64, src)
-    h = Hierarchy(levels=levels, coarse_n=A.n_rows, coarse_row=crow.to(torch.int32).cpu().numpy(),
-                  coarse_col=ccol.to(torch.int32).cpu().numpy(), coarse_val=cval.cpu().numpy(), nprocs=nprocs, rank=rank)
-    return h, summary
+
+
+def build_distributed_hierarchy(A0: DCsr, opts: Optional[SetupOptions] = None, agglomerate_below: int = 10_000,
+                                rebalance_above: float = 1.10, verbose: bool = False, dense: Optional[bool] = None,
+                                comm: Optional[Comm] = None):
+    """Collective.  A0: my rows of the fine matrix (any row partition; it is moved to the nnz-balanced one).
+    Returns (this rank's Hierarchy, summary lines of the global hierarchy).  Each level is turned into this rank's
+    Operators as soon as it is coarsened and its device tensors are dropped, so the setup holds one level at a time."""
+    comm = comm or Comm(A0.val.device)
+    rank, nprocs = comm.rank, comm.world
+    levels: List[Level] = []
+    summary = []
+    for l, (lv, so, sn) in enumerate(coarsen(comm, A0, opts or SetupOptions(), agglomerate_below, rebalance_above,
+                                             dense, verbose)):
+        A = lv.A
+        g_nnz = comm.sum(A.nnz)
+        line = f"L{l}: M={A.n_rows} nnz={g_nnz} ({g_nnz / A.n_rows:.1f}/row) eig={lv.eig_max:.4f}"
+        out = Level(level=l, A=rank_operator(comm, KIND_A, l, A, A.split, lv.a_use_double),
+                    inv_diag=lv.inv_diag.cpu().numpy(), eig_max=lv.eig_max, active=A.m > 0)
+        if lv.P is not None:
+            out.P = rank_operator(comm, KIND_P, l, lv.P, so, lv.pr_use_double)
+            out.R = rank_operator(comm, KIND_R, l, lv.R, A.split, lv.pr_use_double)
+            out.M_coarse_old = int(so[rank + 1] - so[rank])
+            out.M_coarse = int(sn[rank + 1] - sn[rank])
+            out.repart_send, out.repart_recv = repart_plan(so, sn, rank)
+            line += f" | P nnz={comm.sum(lv.P.nnz)}"
+        else:
+            # the coarsest operator as global COO on every rank (tiny)
+            own = A.m > 0 or nprocs == 1
+            src = int(np.flatnonzero(np.diff(A.split) > 0)[0]) if A.n_rows else 0
+            crow = comm.bcast_tensor((A.row + A.r0) if own else None, torch.int64, src)
+            ccol = comm.bcast_tensor(A.col if own else None, torch.int64, src)
+            cval = comm.bcast_tensor(A.val if own else None, torch.float64, src)
+            coarse = dict(coarse_n=A.n_rows, coarse_row=crow.to(torch.int32).cpu().numpy(),
+                          coarse_col=ccol.to(torch.int32).cpu().numpy(), coarse_val=cval.cpu().numpy())
+        levels.append(out)
+        summary.append(line)
+        del lv, A
+    return Hierarchy(levels=levels, nprocs=nprocs, rank=rank, **coarse), summary
 
 
 # ------------------------------------------------------------------------------------------

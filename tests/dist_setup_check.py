@@ -1,12 +1,12 @@
-"""Run under torchrun with N CPU processes (gloo): the distributed setup (saena_b200/sa_setup_dist.py)
-against the one-process setup (saena_b200/sa_setup.py) on the same matrix.
+"""Run under torchrun with N CPU processes (gloo): the row-partitioned setup (saena_b200/sa_setup_dist.py) on N
+ranks against the same setup on one rank (sa_setup.build_device_hierarchy, the global hierarchy) on the same matrix.
 
 Every rank builds its share; rank 0 gathers the shares, re-assembles the global operators of every
 level from the per-rank reference layout (local block + remote block) and compares them with the
-one-process hierarchy: same level count, same aggregates (identical P patterns), same sparsity patterns,
+one-rank hierarchy: same level count, same aggregates (identical P patterns), same sparsity patterns,
 values to summation order, same Chebyshev bounds.  Then the multi-rank oracle solves on the gathered
 shares (halo plan, repartition plan and agglomeration included) and must reproduce the one-rank
-oracle's PCG run on the one-process hierarchy.
+oracle's PCG run on the one-rank hierarchy.
 
 With DSC_GPU=1 (one process per GPU, NCCL; tests/test_multigpu.py) the setup runs on the GPUs and every rank
 also uploads its share and solves with the CUDA library: same iteration count and residual history as the
@@ -90,7 +90,7 @@ def main():
     shares = [None] * world
     dist.gather_object(h, shares if rank == 0 else None, dst=0)
     if rank == 0 and "nocompare" in sys.argv[3:]:
-        # sizes the one-process setup is too slow for on the CPU: the shares must still be a working hierarchy
+        # sizes the one-rank setup is too slow for on the CPU: the shares must still be a working hierarchy
         from oracle.oracle import Oracle
         on = Oracle(shares)
         parts = [rhs[s.levels[0].A.row_offset:s.levels[0].A.row_offset + s.levels[0].A.M] for s in shares]
@@ -130,7 +130,7 @@ def main():
         for l in spread:
             per = np.array([s.levels[l].A.nnz for s in shares], float)
             assert per.max() * world / per.sum() < 1.6, (l, per)
-        # the solve: multi-rank oracle on the shares vs one-rank oracle on the one-process hierarchy
+        # the solve: multi-rank oracle on the shares vs one-rank oracle on the one-rank hierarchy
         from oracle.oracle import Oracle
         o1 = Oracle(ref.to_rank(0, 1))
         u1, it1, h1 = o1.solve_pcg(rhs)

@@ -1,5 +1,5 @@
-"""The distributed setup that feeds the multi-GPU bench (saena_b200/sa_setup_dist.py) on N CPU processes over
-gloo, against the one-process setup -- tests/dist_setup_check.py does the comparing."""
+"""The row-partitioned setup (saena_b200/sa_setup_dist.py) on N CPU processes over gloo, against the same setup on
+one rank (sa_setup.build_device_hierarchy) -- tests/dist_setup_check.py does the comparing."""
 import os
 import subprocess
 import sys
@@ -32,7 +32,9 @@ def test_distributed_setup_equals_the_one_process_setup(world, args, env):
 
 
 def test_one_rank_distributed_setup_is_the_one_process_setup():
-    """no process group: the distributed code path on a single rank gives the one-process hierarchy, array by array"""
+    """no process group: on a single rank the two layout paths -- each rank's operators from its own rows
+    (build_distributed_hierarchy, rank_operator) and from the global matrices (build_hierarchy, to_rank) -- give the
+    same hierarchy, array by array and bit for bit"""
     import numpy as np
     from saena_b200 import sa_setup, sa_setup_dist as sd
     from saena_b200.hierarchy import hierarchy_to_arrays
@@ -44,10 +46,7 @@ def test_one_rank_distributed_setup_is_the_one_process_setup():
     a, b = hierarchy_to_arrays(h), hierarchy_to_arrays(ref)
     assert a.keys() == b.keys() and len(summary) == len(ref.levels)
     for k in a:
-        if a[k].dtype.kind == "f":
-            assert a[k].shape == b[k].shape and np.allclose(a[k], b[k], rtol=1e-12, atol=1e-300), k
-        else:
-            assert np.array_equal(a[k], b[k]), k
+        assert a[k].dtype == b[k].dtype and a[k].shape == b[k].shape and np.array_equal(a[k], b[k]), k
 
 
 @pytest.mark.parametrize("world", [2, 4])
