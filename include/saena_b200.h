@@ -255,13 +255,14 @@ int saena_b200_dot(saena_b200_ctx *ctx, const double *a, const double *b, int n,
 /* ---- measurement ---------------------------------------------------------------------------
  * Device-resident timing loops for bench.py: `reps` applications of one operator / smoother
  * sweep, each launch bracketed by CUDA events on the launching stream; returns the median
- * milliseconds per launch. */
+ * milliseconds per launch.  KIND_A of a level on the route (saena_b200_set_level_route) times the route. */
 int saena_b200_time_matvec(saena_b200_ctx *ctx, int level, int kind, int reps, int flush_l2, float *ms_out);
 int saena_b200_time_smooth_sweep(saena_b200_ctx *ctx, int level, int smoother, int reps, int flush_l2,
                                  float *ms_out);
 /* N > 1 (collective): the same operator application timed three ways -- complete (exchange
  * overlapped with the interior rows), local kernels alone, pack + exchange alone -- so that
- * hidden = 1 - (full - local) / halo can be reported. */
+ * hidden = 1 - (full - local) / halo can be reported.  Like saena_b200_time_matvec, KIND_A times what the solve
+ * applies: the route on a level that takes it (saena_b200_set_level_route). */
 int saena_b200_time_matvec_parts(saena_b200_ctx *ctx, int level, int kind, int reps, float *full_ms,
                                  float *local_ms, float *halo_ms);
 /* CUDA-event stopwatch on the context's compute stream (the stream every kernel of this library
@@ -306,10 +307,26 @@ int saena_b200_sellp_layout(int M, const int64_t *rowptr, int32_t *perm, long lo
  * neighbouring mappings (1/8 .. 8x the threads per row; the sorted sliced layout where it applies) with `reps`
  * applications each and keeps the fastest where it wins by more than min_gain (e.g. 0.03).  Collective on several
  * ranks (same candidates everywhere, decision on the slowest rank's time, one mapping per operator on all ranks);
- * call after finalize -- and after p2p_import, so that the exchange timed is the one the solve will use. */
+ * call after finalize -- and after p2p_import, so that the exchange timed is the one the solve will use.  On one rank
+ * it then puts each level on the route (saena_b200_set_level_route) where the three operators stream fewer bytes than
+ * the stored one and a Chebyshev sweep through them measures faster by more than min_gain. */
 int saena_b200_autotune_mapping(saena_b200_ctx *ctx, int reps, double min_gain, int *changed_out);
 /* the mapping in use (same codes) */
 int saena_b200_get_mapping(const saena_b200_ctx *ctx, int level, int kind);
+/* Level route: level `level`'s operator applied as R_{l-1} (A_{l-1} (P_{l-1} x)), three SpMVs over the operators of the
+ * level above, instead of streaming the stored Galerkin product A_l -- fewer bytes where A_l's rows are much longer than
+ * the fine level's (level 1 of a 7-point Poisson hierarchy).  Every application of A_l in the solve, the per-operator
+ * hooks and the timing loops then take the route, and saena_b200_operator_bytes(level, KIND_A) reports the three
+ * operators' bytes; the eigenvalue estimate keeps the stored operator.  One rank, no scaled hierarchy, level >= 1 with
+ * no repartition below the level above, no operator with a halo or on the dense path; and R A P must agree with the
+ * stored A_l to 1e-12 (relative 2-norm on two seeded random vectors), so that a hierarchy whose A_l is not the product
+ * of the operators next to it keeps its own.  saena_b200_autotune_mapping picks the route per level by measurement on
+ * one rank; this setter (tests, A/B runs) fails where the conditions or the check do not hold.  finalize resets every
+ * level to its stored operator.  get: 1 on the route, 0 not, -1 no such level; ms_stored / ms_route (optional) receive
+ * the autotune's median ms of a Chebyshev sweep on the stored operator and on the route (0 where it did not time the
+ * level: not eligible, not fewer bytes, or the check failed). */
+int saena_b200_set_level_route(saena_b200_ctx *ctx, int level, int on);
+int saena_b200_get_level_route(const saena_b200_ctx *ctx, int level, float *ms_stored, float *ms_route);
 /* algorithmic bytes of one application of an operator (SURVEY.md 8d formula), for the roofline */
 int64_t saena_b200_operator_bytes(const saena_b200_ctx *ctx, int level, int kind);
 

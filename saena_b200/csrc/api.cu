@@ -123,6 +123,7 @@ int saena_b200_destroy(saena_b200_ctx *ctx) {
     for (int i = 0; i < 4; ++i) cudaFree(ctx->stage[i]);
     cudaFree(ctx->flush_buf);
     cudaFree(ctx->tune_dev);
+    cudaFree(ctx->route_t); cudaFree(ctx->route_s);
     sb_nccl_destroy(ctx);
     cudaEventDestroy(ctx->ev_packed); cudaEventDestroy(ctx->ev_halo);
     cudaEventDestroy(ctx->ev_t0); cudaEventDestroy(ctx->ev_t1);
@@ -259,12 +260,35 @@ static int alloc_d(saena_b200_ctx *ctx, double **p, size_t n) {
     return 0;
 }
 
+// the two fine-level intermediates of the level route (sb_apply_level_A)
+static void route_free(saena_b200_ctx *ctx) {
+    cudaFree(ctx->route_t); cudaFree(ctx->route_s);
+    ctx->route_t = ctx->route_s = nullptr;
+    ctx->route_cap = 0;
+}
+
+static int route_alloc(saena_b200_ctx *ctx, int n) {
+    if (ctx->route_cap >= n) return 0;
+    route_free(ctx);
+    SB_TRY(alloc_d(ctx, &ctx->route_t, n));
+    SB_TRY(alloc_d(ctx, &ctx->route_s, n));
+    ctx->route_cap = n;
+    return 0;
+}
+
 int saena_b200_finalize(saena_b200_ctx *ctx) {
     if (!ctx) return 1;
     SB_CUDA(cudaSetDevice(ctx->device));
     const int L = (int)ctx->levels.size();
     if (L == 0) SB_FAIL("finalize: no level uploaded");
     sb_invalidate_graphs(ctx);
+    // the operators may have been replaced: every level starts on its stored A (the route is chosen again by
+    // saena_b200_autotune_mapping or saena_b200_set_level_route)
+    for (DevLevel &lv : ctx->levels) {
+        lv.route = false;
+        lv.route_ms[0] = lv.route_ms[1] = 0.f;
+    }
+    route_free(ctx);
     SB_TRY(sb_arena_build(ctx));  // ghost buffers of every operator, one allocation (p2p_halo.cu)
     for (int l = 0; l < L; ++l) {
         DevLevel &lv = ctx->levels[l];
@@ -452,6 +476,12 @@ static DevOperator *get_op(saena_b200_ctx *ctx, int level, int kind) {
     DevLevel &lv = ctx->levels[level];
     DevOperator *op = kind == SAENA_B200_KIND_A ? &lv.A : (kind == SAENA_B200_KIND_P ? &lv.P : &lv.R);
     return op->present ? op : nullptr;
+}
+
+// what the solve applies for (level, kind): A through sb_apply_level_A (the route on a route level)
+static int apply_kind(saena_b200_ctx *ctx, int level, int kind, const double *x, int epi, const EpiArgs &e) {
+    if (kind == SAENA_B200_KIND_A) return sb_apply_level_A(ctx, level, x, epi, e);
+    return sb_apply(ctx, *get_op(ctx, level, kind), x, epi, e);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -679,7 +709,7 @@ int saena_b200_matvec(saena_b200_ctx *ctx, int level, int kind, const double *v,
     SB_TRY(h2d(ctx, ctx->stage[0], v, op->n_local_cols));
     EpiArgs e{};
     e.out = ctx->stage[1];
-    SB_TRY(sb_apply(ctx, *op, ctx->stage[0], EPI_PLAIN, e));
+    SB_TRY(apply_kind(ctx, level, kind, ctx->stage[0], EPI_PLAIN, e));
     SB_TRY(d2h(ctx, w, ctx->stage[1], op->M));
     return 0;
 }
@@ -694,7 +724,7 @@ int saena_b200_residual(saena_b200_ctx *ctx, int level, const double *u, const d
     EpiArgs e{};
     e.rhs = ctx->stage[1];
     e.out = ctx->stage[2];
-    SB_TRY(sb_apply(ctx, *op, ctx->stage[0], EPI_RESIDUAL, e));
+    SB_TRY(sb_apply_level_A(ctx, level, ctx->stage[0], EPI_RESIDUAL, e));
     SB_TRY(d2h(ctx, res, ctx->stage[2], op->M));
     return 0;
 }
@@ -783,7 +813,7 @@ int saena_b200_time_matvec(saena_b200_ctx *ctx, int level, int kind, int reps, i
     for (int it = 0; it < reps; ++it) {
         if (do_flush) SB_TRY(flush_l2(ctx));
         SB_CUDA(cudaEventRecord(ctx->ev_t0, ctx->stream));
-        SB_TRY(sb_apply(ctx, *op, ctx->stage[0], EPI_PLAIN, e));
+        SB_TRY(apply_kind(ctx, level, kind, ctx->stage[0], EPI_PLAIN, e));
         SB_CUDA(cudaEventRecord(ctx->ev_t1, ctx->stream));
         SB_TRY(sb_sync_stream(ctx, ctx->stream));
         float ms = 0.f;
@@ -848,6 +878,167 @@ int saena_b200_autotune_halo(saena_b200_ctx *ctx, int reps) {
     return sb_agree_fault(ctx);
 }
 
+}  // extern "C"
+
+// median ms of `reps` calls of apply() (two untimed first), each bracketed by CUDA events
+template <typename F>
+static int time_median(saena_b200_ctx *ctx, int reps, bool flush, F apply, float *ms_out) {
+    std::vector<float> t;
+    for (int it = -2; it < reps; ++it) {
+        if (flush) SB_TRY(flush_l2(ctx));
+        SB_CUDA(cudaEventRecord(ctx->ev_t0, ctx->stream));
+        SB_TRY(apply());
+        SB_CUDA(cudaEventRecord(ctx->ev_t1, ctx->stream));
+        SB_TRY(sb_sync_stream(ctx, ctx->stream));
+        float ms = 0.f;
+        SB_CUDA(cudaEventElapsedTime(&ms, ctx->ev_t0, ctx->ev_t1));
+        if (it >= 0) t.push_back(ms);
+    }
+    *ms_out = median_of(t);
+    return 0;
+}
+
+extern "C" {
+
+static int time_apply_median(saena_b200_ctx *ctx, DevOperator *op, int reps, bool flush, float *ms_out) {
+    EpiArgs e{};
+    e.out = ctx->stage[1];
+    return time_median(ctx, reps, flush, [&]() { return sb_apply(ctx, *op, ctx->stage[0], EPI_PLAIN, e); }, ms_out);
+}
+
+// ---------------------------------------------------------------------------------------------
+// Level route (sb_apply_level_A): level l's operator applied as R_{l-1} A_{l-1} P_{l-1}.
+// ---------------------------------------------------------------------------------------------
+// nullptr when level l may take the route, else why not.  One rank only: on several ranks each of the three operators
+// would need its own halo exchange.  The scaled path and the repartitioned levels store an A_l that is not R A P of the
+// operators next to it; a dense level rounds its input through float.
+static const char *route_refusal(const saena_b200_ctx *ctx, int l) {
+    if (ctx->nranks != 1) return "one rank only";
+    if (ctx->scale) return "not on a scaled hierarchy";
+    if (l < 1 || l >= (int)ctx->levels.size()) return "no level above this one";
+    const DevLevel &lv = ctx->levels[l], &fl = ctx->levels[l - 1];
+    if (!fl.repart.identity()) return "the level above repartitions its coarse vector";
+    for (const DevOperator *op : {&lv.A, &fl.A, &fl.P, &fl.R}) {
+        if (!op->present) return "an operator of the route is missing";
+        if (!op->sends.empty() || !op->recvs.empty() || op->nnz_remote > 0 || op->merged) return "an operator has a halo";
+        if (op->use_dense) return "an operator is on the dense path";
+    }
+    return nullptr;
+}
+
+// the intermediates are kept only while some level is on the route
+static void route_release_if_unused(saena_b200_ctx *ctx) {
+    for (const DevLevel &lv : ctx->levels)
+        if (lv.route) return;
+    route_free(ctx);
+}
+
+// Largest ||route x - A_l x|| / ||A_l x|| over two seeded random x.  The difference comes out of the route's last
+// SpMV directly (residual epilogue against the stored product), so no digits are lost to cancellation.
+static const double ROUTE_PROBE_TOL = 1e-12;
+
+static int route_probe(saena_b200_ctx *ctx, int l, double *rel_out) {
+    DevLevel &lv = ctx->levels[l];
+    const int n = lv.M;
+    for (int i = 0; i < 3; ++i) SB_TRY(stage_buf(ctx, i, n));
+    SB_TRY(route_alloc(ctx, ctx->levels[l - 1].M));
+    const bool was = lv.route;
+    double worst = 0.0;
+    for (unsigned long long seed = 1; seed <= 2; ++seed) {
+        SB_TRY(sb_fill_random(ctx, n, 0, 0x5EEDull + seed, ctx->stage[0]));
+        EpiArgs e{};
+        e.out = ctx->stage[1];
+        lv.route = false;
+        SB_TRY(sb_apply_level_A(ctx, l, ctx->stage[0], EPI_PLAIN, e));   // stored A_l x
+        e.rhs = ctx->stage[1];
+        e.out = ctx->stage[2];
+        lv.route = true;
+        const int rc = sb_apply_level_A(ctx, l, ctx->stage[0], EPI_RESIDUAL, e);   // route x - A_l x
+        lv.route = was;
+        SB_TRY(rc);
+        SB_TRY(sb_dot(ctx, ctx->stage[2], ctx->stage[2], n, S_TMP));
+        SB_TRY(sb_dot(ctx, ctx->stage[1], ctx->stage[1], n, S_TMP + 1));
+        SB_TRY(sb_read_scalars(ctx));
+        const double num = ctx->scalars_host[S_TMP], den = ctx->scalars_host[S_TMP + 1];
+        const double r = den > 0.0 ? sqrt(num / den) : (num > 0.0 ? INFINITY : 0.0);
+        if (!(r <= worst)) worst = r;   // NaN stays
+    }
+    *rel_out = worst;
+    return 0;
+}
+
+int saena_b200_set_level_route(saena_b200_ctx *ctx, int level, int on) {
+    SB_ENTER();
+    if (level < 0 || level >= (int)ctx->levels.size()) SB_FAIL("set_level_route: no such level");
+    DevLevel &lv = ctx->levels[level];
+    sb_invalidate_graphs(ctx);
+    if (!on) {
+        lv.route = false;
+        route_release_if_unused(ctx);
+        return 0;
+    }
+    if (const char *why = route_refusal(ctx, level)) SB_FAIL(std::string("set_level_route: ") + why);
+    double rel = 0.0;
+    const int rc = route_probe(ctx, level, &rel);
+    if (rc || !(rel <= ROUTE_PROBE_TOL)) {
+        route_release_if_unused(ctx);
+        if (rc) return rc;
+        SB_FAIL("set_level_route: R A P of the level above differs from the stored operator by " + std::to_string(rel) +
+                " relative (more than 1e-12)");
+    }
+    lv.route = true;
+    return 0;
+}
+
+int saena_b200_get_level_route(const saena_b200_ctx *ctx, int level, float *ms_stored, float *ms_route) {
+    if (!ctx || level < 0 || level >= (int)ctx->levels.size()) return -1;
+    const DevLevel &lv = ctx->levels[level];
+    if (ms_stored) *ms_stored = lv.route_ms[0];
+    if (ms_route) *ms_route = lv.route_ms[1];
+    return lv.route ? 1 : 0;
+}
+
+// Setup-time choice of the route, after the mappings are settled: for every level it may take, the stored operator and
+// the route are each timed as the V-cycle's most frequent application, a Chebyshev sweep after the first, and the route
+// is kept where it is faster by more than min_gain.  Tried only where the three operators together stream fewer bytes
+// than the stored one and pass the probe check.  The coarsest level is left alone: the V-cycle never applies its A.
+static int autotune_route(saena_b200_ctx *ctx, int reps, double min_gain) {
+    for (int l = 1; l + 1 < (int)ctx->levels.size(); ++l) {
+        DevLevel &lv = ctx->levels[l], &fl = ctx->levels[l - 1];
+        lv.route = false;
+        lv.route_ms[0] = lv.route_ms[1] = 0.f;
+        if (route_refusal(ctx, l) || lv.M == 0) continue;
+        const int64_t stored = sb_operator_bytes(lv.A);
+        if (sb_operator_bytes(fl.P) + sb_operator_bytes(fl.A) + sb_operator_bytes(fl.R) >= stored) continue;
+        double rel = 0.0;
+        SB_TRY(route_probe(ctx, l, &rel));
+        if (!(rel <= ROUTE_PROBE_TOL)) continue;
+        // stage[0]: iterate and rhs (zeros), stage[1]: new iterate, stage[2]: direction (in place, as in the solve)
+        SB_CUDA(cudaMemsetAsync(ctx->stage[0], 0, sizeof(double) * lv.M, ctx->stream));
+        SB_CUDA(cudaMemsetAsync(ctx->stage[2], 0, sizeof(double) * lv.M, ctx->stream));
+        EpiArgs e{};
+        e.rhs = ctx->stage[0];
+        e.inv_diag = lv.inv_diag;
+        e.d_in = e.d_out = ctx->stage[2];
+        e.u_in = ctx->stage[0];
+        e.out = ctx->stage[1];
+        e.c1 = 0.5;
+        e.c2 = 0.5;
+        const bool flush = stored < (int64_t)300e6;
+        float ms[2] = {0.f, 0.f};
+        for (int r = 0; r < 2; ++r) {
+            lv.route = r == 1;
+            SB_TRY(time_median(ctx, reps, flush, [&]() { return sb_apply_level_A(ctx, l, ctx->stage[0], EPI_CHEB_NEXT, e); },
+                               &ms[r]));
+        }
+        lv.route_ms[0] = ms[0];
+        lv.route_ms[1] = ms[1];
+        lv.route = ms[1] < (1.0 - min_gain) * ms[0];
+    }
+    route_release_if_unused(ctx);
+    return 0;
+}
+
 // ---------------------------------------------------------------------------------------------
 // Setup-time choice of every operator's row mapping BY MEASUREMENT (north_star: "warp-per-row or row-block mapping
 // chosen per level by nnz/row"): sb_choose_mapping's nnz/row rule gives the starting point, this walks the
@@ -860,26 +1051,9 @@ int saena_b200_autotune_halo(saena_b200_ctx *ctx, int reps) {
 // exchange all ranks take part in, and the decision is taken on the slowest rank's median time (all-reduce MAX) --
 // one mapping per operator on all ranks.  Sliced operators (mapping 100) stay: where the rule picks the sliced
 // layout it measured fastest on every shape tried (profiles/r01_mapping_sweep.md).
-// changed_out (optional): number of operators whose mapping changed on this rank.
+// changed_out (optional): number of operators whose mapping changed on this rank.  On one rank the level route is
+// chosen afterwards, on the settled mappings (autotune_route).
 // ---------------------------------------------------------------------------------------------
-static int time_apply_median(saena_b200_ctx *ctx, DevOperator *op, int reps, bool flush, float *ms_out) {
-    EpiArgs e{};
-    e.out = ctx->stage[1];
-    std::vector<float> t;
-    for (int it = -2; it < reps; ++it) {
-        if (flush) SB_TRY(flush_l2(ctx));
-        SB_CUDA(cudaEventRecord(ctx->ev_t0, ctx->stream));
-        SB_TRY(sb_apply(ctx, *op, ctx->stage[0], EPI_PLAIN, e));
-        SB_CUDA(cudaEventRecord(ctx->ev_t1, ctx->stream));
-        SB_TRY(sb_sync_stream(ctx, ctx->stream));
-        float ms = 0.f;
-        SB_CUDA(cudaEventElapsedTime(&ms, ctx->ev_t0, ctx->ev_t1));
-        if (it >= 0) t.push_back(ms);
-    }
-    *ms_out = median_of(t);
-    return 0;
-}
-
 int saena_b200_autotune_mapping(saena_b200_ctx *ctx, int reps, double min_gain, int *changed_out) {
     SB_ENTER();
     if (reps < 3) reps = 10;
@@ -950,7 +1124,8 @@ int saena_b200_autotune_mapping(saena_b200_ctx *ctx, int reps, double min_gain, 
         }
     }
     if (changed_out) *changed_out = changed;
-    return multi ? sb_agree_fault(ctx) : 0;
+    if (multi) return sb_agree_fault(ctx);
+    return ctx->nranks == 1 ? autotune_route(ctx, reps, min_gain) : 0;
 }
 
 // 1: fused kernel, 0: separate launches / NCCL, -1: no such operator; ms[2] = this rank's autotune timings
@@ -1157,7 +1332,8 @@ int64_t saena_b200_operator_bytes(const saena_b200_ctx *ctx, int level, int kind
     if (!ctx || level < 0 || level >= (int)ctx->levels.size()) return -1;
     const DevLevel &lv = ctx->levels[level];
     const DevOperator &op = kind == SAENA_B200_KIND_A ? lv.A : (kind == SAENA_B200_KIND_P ? lv.P : lv.R);
-    return op.present ? sb_operator_bytes(op) : -1;
+    if (!op.present) return -1;
+    return kind == SAENA_B200_KIND_A ? sb_level_A_bytes(ctx, level) : sb_operator_bytes(op);
 }
 
 }  // extern "C"

@@ -199,6 +199,10 @@ struct DevLevel {
     int M_coarse = 0;      // Ac.M
     RepartPlan repart;
     bool aux_set = false;
+    // A is applied as R_{l-1} (A_{l-1} (P_{l-1} x)) instead of streaming the stored Galerkin product
+    // (sb_apply_level_A; chosen by saena_b200_autotune_mapping or saena_b200_set_level_route, reset by finalize)
+    bool route = false;
+    float route_ms[2] = {0.f, 0.f};  // autotune: median ms of a Chebyshev sweep on the stored A / on the route (0: not timed)
 
     // work vectors (Grid::allocate_mem + the smoother's temp1/temp2)
     double *u[2] = {nullptr, nullptr};  // ping-pong iterate; u[cur] is current
@@ -293,6 +297,11 @@ struct saena_b200_ctx {
 
     double *tune_dev = nullptr;   // [32] scratch of the collective mapping autotune (all-reduce MAX of candidate times)
 
+    // the two fine-level intermediates of a route level (P_{l-1} x, A_{l-1} P_{l-1} x); allocated while a level is
+    // on the route or being timed for it
+    double *route_t = nullptr, *route_s = nullptr;
+    int route_cap = 0;
+
     // L2 flush buffer for the timing loops
     void *flush_buf = nullptr;
     size_t flush_bytes = 0;
@@ -383,10 +392,15 @@ int sb_coarsest_cg(saena_b200_ctx *ctx, const double *rhs, double *u);  // u: in
 int sb_read_scalars(saena_b200_ctx *ctx);  // device scalars -> scalars_host (synchronises the stream)
 
 // ---- lanczos.cu
+// out = uniform(-1, 1) from a counter-based generator on the global row index (row_offset + i)
+int sb_fill_random(saena_b200_ctx *ctx, int n, long long row_offset, unsigned long long seed, double *out);
 int sb_find_eig(saena_b200_ctx *ctx, int level, int max_iter, const double *start_dev, unsigned long long seed,
                 double *eig_out, int *iters_out);
 
 // ---- solve.cu
+// level l's operator with a fused epilogue: the stored A_l, or on a route level R_{l-1} A_{l-1} P_{l-1}
+int sb_apply_level_A(saena_b200_ctx *ctx, int l, const double *x, int epi, const EpiArgs &args);
+int64_t sb_level_A_bytes(const saena_b200_ctx *ctx, int l);  // algorithmic bytes of what sb_apply_level_A streams
 int sb_smooth(saena_b200_ctx *ctx, int l, int smoother, int iters, const double *rhs, bool u_is_zero);
 int sb_vcycle(saena_b200_ctx *ctx, int l, int smoother, int pre, int post, const double *rhs, bool u_is_zero);
 // level-0 V-cycle from a zero iterate, replayed from a CUDA graph when nothing in it needs the host

@@ -88,6 +88,14 @@ double largest_tridiag_eig(const std::vector<double> &a, const std::vector<doubl
 
 }  // namespace
 
+int sb_fill_random(saena_b200_ctx *ctx, int n, long long row_offset, unsigned long long seed, double *out) {
+    if (n <= 0) return 0;
+    ++ctx->launches;
+    lz_random_kernel<<<(n + 255) / 256, 256, 0, ctx->stream>>>(n, row_offset, seed, out);
+    SB_CUDA(cudaGetLastError());
+    return 0;
+}
+
 // eig_out = 1.0001 * lambda_max(D^-1/2 A D^-1/2) of level `level`; start_dev: optional start vector
 // (device, this rank's rows), else the seeded generator.  Collective over the ranks.
 int sb_find_eig(saena_b200_ctx *ctx, int level, int max_iter, const double *start_dev, unsigned long long seed,
@@ -125,8 +133,8 @@ int sb_find_eig(saena_b200_ctx *ctx, int level, int max_iter, const double *star
     LZ_TRY(sb_fill_zero(ctx, u[0], n));
     if (start_dev) {
         if (n) cudaMemcpyAsync(u[1], start_dev, sizeof(double) * n, cudaMemcpyDeviceToDevice, s);
-    } else if (n) {
-        lz_random_kernel<<<blocks, 256, 0, s>>>(n, (long long)lv.A.col_offset, seed, u[1]);
+    } else {
+        LZ_TRY(sb_fill_random(ctx, n, (long long)lv.A.col_offset, seed, u[1]));
     }
     LZ_TRY(sb_dot(ctx, u[1], u[1], n, S_TMP));
     LZ_TRY(sb_read_scalars(ctx));

@@ -16,6 +16,32 @@
 
 #include "common.h"
 
+// Level l's operator.  Pairwise aggregation halves the rows of the fine level, but the Galerkin product A_l = R A P
+// of a short-row operator has far longer rows: on the 256^3 Poisson hierarchy A_1 has 68 entries a row and five times
+// A_0's bytes, while P_0, A_0 and R_0 together stream 0.66 of A_1's bytes.  On a route level (DevLevel::route) the product
+// is therefore applied as three SpMVs, each operator on its own mapping, through two fine-level intermediates; R's
+// rows are level l's rows, so the epilogue (residual, smoother update) fuses into the last one unchanged.  A_{l-1} is
+// always the stored operator.
+int sb_apply_level_A(saena_b200_ctx *ctx, int l, const double *x, int epi, const EpiArgs &args) {
+    DevLevel &lv = ctx->levels[l];
+    if (!lv.route) return sb_apply(ctx, lv.A, x, epi, args);
+    DevLevel &fl = ctx->levels[l - 1];
+    if (ctx->route_cap < fl.M) SB_FAIL("apply: route level without its intermediate vectors");
+    EpiArgs e{};
+    e.out = ctx->route_t;
+    SB_TRY(sb_apply(ctx, fl.P, x, EPI_PLAIN, e));
+    e.out = ctx->route_s;
+    SB_TRY(sb_apply(ctx, fl.A, ctx->route_t, EPI_PLAIN, e));
+    return sb_apply(ctx, fl.R, ctx->route_s, epi, args);
+}
+
+int64_t sb_level_A_bytes(const saena_b200_ctx *ctx, int l) {
+    const DevLevel &lv = ctx->levels[l];
+    if (!lv.route) return sb_operator_bytes(lv.A);
+    const DevLevel &fl = ctx->levels[l - 1];
+    return sb_operator_bytes(fl.P) + sb_operator_bytes(fl.A) + sb_operator_bytes(fl.R);
+}
+
 int sb_smooth(saena_b200_ctx *ctx, int l, int smoother, int iters, const double *rhs, bool u_is_zero) {
     DevLevel &lv = ctx->levels[l];
     if (iters <= 0 || lv.M == 0) {
@@ -37,7 +63,7 @@ int sb_smooth(saena_b200_ctx *ctx, int l, int smoother, int iters, const double 
         for (; j < iters; ++j) {
             e.u_in = lv.u[lv.cur];
             e.out = lv.u[lv.cur ^ 1];
-            SB_TRY(sb_apply(ctx, lv.A, lv.u[lv.cur], EPI_JACOBI, e));
+            SB_TRY(sb_apply_level_A(ctx, l, lv.u[lv.cur], EPI_JACOBI, e));
             lv.cur ^= 1;
         }
         return 0;
@@ -61,7 +87,7 @@ int sb_smooth(saena_b200_ctx *ctx, int l, int smoother, int iters, const double 
         e.c1 = 1.0 / theta;
         e.u_in = lv.u[lv.cur];
         e.out = lv.u[lv.cur ^ 1];
-        SB_TRY(sb_apply(ctx, lv.A, lv.u[lv.cur], EPI_CHEB_FIRST, e));
+        SB_TRY(sb_apply_level_A(ctx, l, lv.u[lv.cur], EPI_CHEB_FIRST, e));
         lv.cur ^= 1;
     }
     for (int i = 1; i < iters; ++i) {
@@ -74,7 +100,7 @@ int sb_smooth(saena_b200_ctx *ctx, int l, int smoother, int iters, const double 
         e.c2 = d2;
         e.u_in = lv.u[lv.cur];
         e.out = lv.u[lv.cur ^ 1];
-        SB_TRY(sb_apply(ctx, lv.A, lv.u[lv.cur], EPI_CHEB_NEXT, e));
+        SB_TRY(sb_apply_level_A(ctx, l, lv.u[lv.cur], EPI_CHEB_NEXT, e));
         lv.cur ^= 1;
     }
     return 0;
@@ -106,9 +132,10 @@ int sb_vcycle(saena_b200_ctx *ctx, int l, int smoother, int pre, int post, const
     //    partition if they differ.  Opt-in (saena_b200_set_fused_restrict): both as ONE pass over A that scatters every
     //    fine residual through its row of P and never writes res (fused_restrict.cu; measured in
     //    profiles/r02_fused_restrict.md: -8 % on level 0, +3 % / +37 % on levels 1 / 2 -- off by default, and FP64
-    //    atomics make the coarse vector's last bits depend on the run).
+    //    atomics make the coarse vector's last bits depend on the run).  Not on a route level: the fused kernel
+    //    walks the stored A.
     bool fused_rr = false;
-    if (!(pre == 0 && u_is_zero) && ctx->fused_restrict_levels > l) {
+    if (!(pre == 0 && u_is_zero) && ctx->fused_restrict_levels > l && !lv.route) {
         const bool ident = lv.repart.identity();
         const int rc = sb_residual_restrict_fused(ctx, l, lv.u[lv.cur], rhs, ident ? cl.rhs : lv.xfer_old);
         if (rc < 0) SB_FAIL("vcycle: fused residual + restriction failed to launch");
@@ -124,7 +151,7 @@ int sb_vcycle(saena_b200_ctx *ctx, int l, int smoother, int pre, int post, const
         EpiArgs e{};
         e.rhs = rhs;
         e.out = lv.res;
-        SB_TRY(sb_apply(ctx, lv.A, lv.u[lv.cur], EPI_RESIDUAL, e));
+        SB_TRY(sb_apply_level_A(ctx, l, lv.u[lv.cur], EPI_RESIDUAL, e));
     }
     if (!fused_rr) {
         SbRange rg(ctx, "Rtransfer", l);

@@ -112,6 +112,8 @@ def load_library(path: Optional[str] = None):
     L.saena_b200_autotune_mapping.argtypes = [vp, i, ctypes.c_double, ip]
     L.saena_b200_set_mapping_deferred.argtypes = [vp, i, i, i]
     L.saena_b200_get_mapping.argtypes = [vp, i, i]
+    L.saena_b200_set_level_route.argtypes = [vp, i, i]
+    L.saena_b200_get_level_route.argtypes = [vp, i, ctypes.POINTER(ctypes.c_float), ctypes.POINTER(ctypes.c_float)]
     L.saena_b200_operator_bytes.restype = ctypes.c_int64
     L.saena_b200_operator_bytes.argtypes = [vp, i, i]
     _lib = L
@@ -127,7 +129,7 @@ EXPORTED_SYMBOLS = [
     "saena_b200_solve_pcg_dev", "saena_b200_matvec", "saena_b200_residual", "saena_b200_smooth",
     "saena_b200_vcycle", "saena_b200_coarsest_solve", "saena_b200_dot", "saena_b200_time_matvec",
     "saena_b200_time_smooth_sweep", "saena_b200_time_matvec_parts", "saena_b200_time_vcycle", "saena_b200_timer_start", "saena_b200_timer_stop", "saena_b200_launch_count", "saena_b200_graph_replays", "saena_b200_set_mapping", "saena_b200_set_fused_restrict", "saena_b200_spgemm_symbolic", "saena_b200_spgemm_numeric", "saena_b200_time_residual_restrict", "saena_b200_autotune_mapping", "saena_b200_set_mapping_deferred", "saena_b200_get_mapping",
-    "saena_b200_operator_bytes",
+    "saena_b200_set_level_route", "saena_b200_get_level_route", "saena_b200_operator_bytes",
 ]
 
 
@@ -502,6 +504,21 @@ class Context:
 
     def get_mapping(self, level, kind) -> int:
         return int(self._L.saena_b200_get_mapping(self._h, level, kind))
+
+    def set_level_route(self, level: int, on: bool):
+        """apply level `level`'s operator as R A P of the level above (True) or stream its stored A (False); raises
+        where the route is not allowed or R A P differs from the stored operator by more than 1e-12"""
+        self._ck(self._L.saena_b200_set_level_route(self._h, int(level), int(on)))
+
+    def get_level_route(self, level: int) -> bool:
+        return self.level_route_choice(level)[0] == 1
+
+    def level_route_choice(self, level: int):
+        """-> (choice, ms_stored, ms_route); choice 1 on the route, 0 not, -1 no such level; the two times are the
+        autotune's medians of a Chebyshev sweep each way (0: the level was not timed)"""
+        a, b = ctypes.c_float(0), ctypes.c_float(0)
+        c = int(self._L.saena_b200_get_level_route(self._h, int(level), ctypes.byref(a), ctypes.byref(b)))
+        return c, a.value, b.value
 
     def set_fused_restrict(self, levels: int):
         """levels [0, levels) of the V-cycle: residual + restriction as one scatter kernel where eligible (0: off)"""
