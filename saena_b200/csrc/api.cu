@@ -473,8 +473,7 @@ static int d2h(saena_b200_ctx *ctx, double *dst, const double *src, size_t n) {
 
 static DevOperator *get_op(saena_b200_ctx *ctx, int level, int kind) {
     if (level < 0 || level >= (int)ctx->levels.size()) return nullptr;
-    DevLevel &lv = ctx->levels[level];
-    DevOperator *op = kind == SAENA_B200_KIND_A ? &lv.A : (kind == SAENA_B200_KIND_P ? &lv.P : &lv.R);
+    DevOperator *op = &ctx->levels[level].op(kind);
     return op->present ? op : nullptr;
 }
 
@@ -1068,7 +1067,7 @@ int saena_b200_autotune_mapping(saena_b200_ctx *ctx, int reps, double min_gain, 
             DevOperator *op = ops[kind];
             // ---- what this rank holds
             const bool mine = op->present && op->M > 0 && op->nnz_local + op->nnz_remote > 0;
-            const int cur = !mine ? 0 : (op->use_sell ? SB_MAPPING_SELL : (op->use_sellp ? SB_MAPPING_SELLP : (op->use_stream ? -op->lanes : op->lanes)));
+            const int cur = mine ? op->mapping : 0;
             const bool has_halo = mine && (!op->sends.empty() || !op->recvs.empty() || op->nnz_remote > 0 || op->merged);
             // ---- agree: [largest threads-per-row starting point, somebody is sliced / streaming / pinned]
             double agree[2] = {(cur >= 1 && cur <= 256) ? (double)cur : 0.0,
@@ -1131,8 +1130,7 @@ int saena_b200_autotune_mapping(saena_b200_ctx *ctx, int reps, double min_gain, 
 // 1: fused kernel, 0: separate launches / NCCL, -1: no such operator; ms[2] = this rank's autotune timings
 int saena_b200_halo_choice(const saena_b200_ctx *ctx, int level, int kind, float *ms_fused, float *ms_unfused) {
     if (!ctx || level < 0 || level >= (int)ctx->levels.size()) return -1;
-    const DevLevel &lv = ctx->levels[level];
-    const DevOperator &op = kind == SAENA_B200_KIND_A ? lv.A : (kind == SAENA_B200_KIND_P ? lv.P : lv.R);
+    const DevOperator &op = ctx->levels[level].op(kind);
     if (!op.present) return -1;
     if (ms_fused) *ms_fused = op.tune_ms[0];
     if (ms_unfused) *ms_unfused = op.tune_ms[1];
@@ -1321,17 +1319,13 @@ int saena_b200_sellp_layout(int M, const int64_t *rowptr, int32_t *perm, long lo
 
 int saena_b200_get_mapping(const saena_b200_ctx *ctx, int level, int kind) {
     if (!ctx || level < 0 || level >= (int)ctx->levels.size()) return 0;
-    const DevLevel &lv = ctx->levels[level];
-    const DevOperator &op = kind == SAENA_B200_KIND_A ? lv.A : (kind == SAENA_B200_KIND_P ? lv.P : lv.R);
-    if (!op.present) return 0;
-    if (op.use_sellp) return SB_MAPPING_SELLP;
-    return op.use_sell ? SB_MAPPING_SELL : (op.use_stream ? -op.lanes : op.lanes);
+    const DevOperator &op = ctx->levels[level].op(kind);
+    return op.present ? op.mapping : 0;
 }
 
 int64_t saena_b200_operator_bytes(const saena_b200_ctx *ctx, int level, int kind) {
     if (!ctx || level < 0 || level >= (int)ctx->levels.size()) return -1;
-    const DevLevel &lv = ctx->levels[level];
-    const DevOperator &op = kind == SAENA_B200_KIND_A ? lv.A : (kind == SAENA_B200_KIND_P ? lv.P : lv.R);
+    const DevOperator &op = ctx->levels[level].op(kind);
     if (!op.present) return -1;
     return kind == SAENA_B200_KIND_A ? sb_level_A_bytes(ctx, level) : sb_operator_bytes(op);
 }

@@ -92,6 +92,15 @@ struct HaloSyncDev {
     unsigned long long **signal_consumed = nullptr;  // [recvs.size()] the senders' arenas
 };
 
+// sliced layout (32-slot slices, column-major inside a slice, padded per slice to its longest row), built on the
+// device from the CSR arrays.  perm: slot -> row (-1: no row) of the sorted layout; nullptr: slot = row.
+struct SlicedLayout {
+    long long *ptr = nullptr;  // [n_slices+1] element offsets
+    int *perm = nullptr;
+    int *col = nullptr;
+    double *val = nullptr;
+};
+
 struct DevOperator {
     bool present = false;
     int kind = 0, level = 0;
@@ -113,24 +122,16 @@ struct DevOperator {
     int *blk_row = nullptr;
     int n_blk = 0;
 
-    // sliced layout (32-row slices, column-major, padded per slice) for short regular rows
-    long long *sell_ptr = nullptr;  // [n_slices+1] element offsets
-    int *sell_col = nullptr;
-    double *sell_val = nullptr;
-    int64_t sell_padded = 0;        // stored entries incl. padding
-    int64_t sell_padded_est = 0;    // what the padding would be (computed at upload)
+    // sliced layout in row order (mapping 100) for short regular rows
+    SlicedLayout sell;
+    int64_t sell_padded_est = 0;    // stored entries incl. padding the sliced layout would have (computed at upload)
     bool sell_only = false;         // the CSR col/val were released once the sliced copy existed (no other mapping)
 
     // sliced layout over a row permutation (mapping 101): inside every window of 256 consecutive rows (one CTA) the
     // rows are sorted by length, longest first, so that the 32 rows of a slice have nearly the same length and the
-    // padding of irregular operators (unstructured matrices, smoothed prolongators) all but disappears.  slot -> row
-    // in sellp_perm (-1: no row); operators without a halo only.  Never chosen by the heuristic: set_mapping / autotune.
-    long long *sellp_ptr = nullptr;
-    int *sellp_perm = nullptr;
-    int *sellp_col = nullptr;
-    double *sellp_val = nullptr;
-    int64_t sellp_padded = 0;
-    bool use_sellp = false;
+    // padding of irregular operators (unstructured matrices, smoothed prolongators) all but disappears.  Operators
+    // without a halo only.  Never chosen by the heuristic: set_mapping / autotune.
+    SlicedLayout sellp;
 
     // remote block re-sorted by row at upload: boundary rows only
     // interior rows = the contiguous range [int_lo, int_hi) (multiples of 32) that holds no row with
@@ -175,11 +176,11 @@ struct DevOperator {
     int op_id = 0;                                // level * 3 + kind (fault reports)
     HaloSyncDev hs;
 
-    // kernel mapping
-    int lanes = 0;            // lanes per row (vec) / lanes per row in the reduce phase (stream)
-    bool use_stream = false;
-    bool use_sell = false;
-    int forced_mapping = 0;   // see saena_b200_set_mapping
+    // kernel mapping: the canonical code of saena_b200_set_mapping that sb_choose_mapping settled on (1..16 lanes
+    // per row, 32..256 threads per row, -1..-32 streaming row blocks with -mapping lanes per row in the reduce
+    // phase, SB_MAPPING_SELL, SB_MAPPING_SELLP; 0 until the operator is prepared)
+    int mapping = 0;
+    int forced_mapping = 0;   // the code requested by set_mapping / the autotune (0: the nnz/row rule)
 
     double avg_nnz_row() const { return M ? double(nnz_local + nnz_remote) / M : 0.0; }
 };
@@ -191,6 +192,9 @@ struct RepartPlan {
 
 struct DevLevel {
     DevOperator A, P, R;
+    // the operator of an ABI kind (SAENA_B200_KIND_*); any kind other than A or P is R
+    DevOperator &op(int kind) { return kind == SAENA_B200_KIND_A ? A : (kind == SAENA_B200_KIND_P ? P : R); }
+    const DevOperator &op(int kind) const { return const_cast<DevLevel *>(this)->op(kind); }
     double *inv_diag = nullptr;
     double *inv_sq_diag = nullptr;  // inv_sq_diag_orig, only for scale=true hierarchies
     double eig_max = 0.0;

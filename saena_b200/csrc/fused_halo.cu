@@ -28,6 +28,9 @@
 //                                source by column index -- no x_ext copy, no widen pass.
 //   last CTA of each role        raises the flags of the hand-shake and advances the role's counter
 //
+// The kernel's MAP is the operator's mapping code (DevOperator::mapping), dispatched by the same
+// sb_dispatch_mapping as the stand-alone launches and with the same grid rule, sb_mapping_blocks.
+//
 // The hand-shake (halo_sync.cuh) is shared with the separate-launch form (p2p_halo.cu): monotonic
 // counters in device memory, two landing buffers selected by the application's parity, every wait
 // bounded by a globaltimer deadline.  A launch carries no host-side state: the kernel replays from
@@ -245,48 +248,35 @@ fused_halo_spmv_kernel(const __grid_constant__ FusedArgs a) {
     if (a.do_sync) sb_halo_release_cta(a.h, a.n_wait, done);
 }
 
-static int main_blocks(const DevOperator &op, int nrows) {
-    if (nrows <= 0) return 0;
-    if (op.use_sell || op.lanes < 32) return (nrows + 255) / 256;
-    const int rows_per_block = 256 / op.lanes;
-    return (nrows + rows_per_block - 1) / rows_per_block;
-}
-
 // The fused kernel covers the 32-bit-offset CSR / sliced mappings; anything else (64-bit row offsets, the
 // streaming mapping) takes the separate launches, which speak the same hand-shake -- the choice is local.
 bool sb_fused_eligible(const DevOperator &op) {
-    return op.p2p && op.fused && !op.wide_offsets && !op.use_stream && !op.use_sellp &&
+    return op.p2p && op.fused && !op.wide_offsets && op.mapping > 0 && op.mapping != SB_MAPPING_SELLP &&
            (!op.sends.empty() || !op.recvs.empty());
 }
 
 template <int EPI, bool MERGED>
 static int launch_fused(saena_b200_ctx *ctx, const DevOperator &op, const FusedArgs &a, int grid) {
-    cudaStream_t s = ctx->stream;
-#define SB_FUSED_CASE(MAP)                                                                          \
-    case MAP: fused_halo_spmv_kernel<MAP, EPI, MERGED><<<grid, 256, 0, s>>>(a); break;
-    switch (op.use_sell ? SB_MAPPING_SELL : op.lanes) {
-        SB_FUSED_CASE(100) SB_FUSED_CASE(1) SB_FUSED_CASE(2) SB_FUSED_CASE(4) SB_FUSED_CASE(8) SB_FUSED_CASE(16)
-        SB_FUSED_CASE(32) SB_FUSED_CASE(64) SB_FUSED_CASE(128) SB_FUSED_CASE(256)
-        default: SB_FAIL("fused apply: unknown mapping");
-    }
-#undef SB_FUSED_CASE
+    const bool known = sb_dispatch_mapping(op.mapping, [&](auto map) {
+        fused_halo_spmv_kernel<decltype(map)::value, EPI, MERGED><<<grid, 256, 0, ctx->stream>>>(a);
+    });
+    if (!known) SB_FAIL("fused apply: unknown mapping");
     SB_CUDA(cudaGetLastError());
     return 0;
 }
 
 template <int EPI>
 static int apply_fused_epi(saena_b200_ctx *ctx, DevOperator &op, const double *x, const EpiArgs &e) {
-    static_assert(SB_MAPPING_SELL == 100, "mapping code");
     const int mode = ctx->apply_mode;  // 0 full, 1 compute only (stale ghosts), 2 exchange only
     FusedArgs a{};
     a.rowptr = (const int *)op.rowptr; a.col = op.col; a.val = op.val;
-    a.sell_ptr = op.sell_ptr; a.sell_col = op.sell_col; a.sell_val = op.sell_val;
+    a.sell_ptr = op.sell.ptr; a.sell_col = op.sell.col; a.sell_val = op.sell.val;
     a.M = op.M; a.int_lo = op.int_lo; a.int_hi = op.int_hi; a.n_local = op.n_local_cols;
     a.n_brows = op.n_brows; a.bnd_wide = op.avg_nnz_row() >= 48.0;
     a.brow = op.brow; a.brow_ptr = op.brow_ptr; a.bcol = op.bcol; a.bval = op.bval;
     a.x = x; a.ghost = op.ghost_d; a.recvSize = op.recvSize; a.e = e;
     a.rowmid = op.rowmid; a.partial = op.partial;
-    a.split = mode == 0 && op.merged && !op.use_sell && op.rowmid && op.partial && ctx->merged_split;
+    a.split = mode == 0 && op.merged && op.mapping != SB_MAPPING_SELL && op.rowmid && op.partial && ctx->merged_split;
     a.do_sync = mode != 1;
     a.do_compute = mode != 2;
     a.vIndexSize = op.vIndexSize; a.vIndex = op.vIndex;
@@ -295,9 +285,9 @@ static int apply_fused_epi(saena_b200_ctx *ctx, DevOperator &op, const double *x
     a.n_pack = mode == 1 ? 0 : (op.vIndexSize + SB_PACK_PER_CTA - 1) / SB_PACK_PER_CTA;
     if (op.merged) {
         a.n_int = 0;
-        a.n_wait_blocks = main_blocks(op, op.M);
+        a.n_wait_blocks = sb_mapping_blocks(op.mapping, op.M);
     } else {
-        a.n_int = main_blocks(op, op.int_hi - op.int_lo);
+        a.n_int = sb_mapping_blocks(op.mapping, op.int_hi - op.int_lo);
         const int rows_per_block = 256 / (a.bnd_wide ? 32 : 8);
         a.n_wait_blocks = (op.n_brows + rows_per_block - 1) / rows_per_block;
     }

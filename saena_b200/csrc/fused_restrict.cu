@@ -58,12 +58,12 @@ int sb_residual_restrict_fused(saena_b200_ctx *ctx, int l, const double *u, cons
     DevLevel &lv = ctx->levels[l];
     DevOperator &A = lv.A, &P = lv.P, &R = lv.R;
     if (l >= ctx->fused_restrict_levels) return 0;
-    if (!A.use_sell || !A.sell_ptr || !P.present || P.wide_offsets || !P.col || !P.val || P.merged || R.merged) return 0;
+    if (A.mapping != SB_MAPPING_SELL || !A.sell.ptr || !P.present || P.wide_offsets || !P.col || !P.val || P.merged || R.merged) return 0;
     if (!A.sends.empty() || !A.recvs.empty() || !P.sends.empty() || !P.recvs.empty() || !R.sends.empty() || !R.recvs.empty()) return 0;
     if (A.nnz_remote || P.nnz_remote || R.nnz_remote || lv.M == 0) return 0;
     if (cudaMemsetAsync(res_coarse, 0, sizeof(double) * (size_t)std::max(R.M, 1), ctx->stream) != cudaSuccess) return -1;
     ctx->launches += 1;
-    residual_restrict_sell_kernel<<<(lv.M + 255) / 256, 256, 0, ctx->stream>>>(lv.M, A.sell_ptr, A.sell_col, A.sell_val, u, rhs,
+    residual_restrict_sell_kernel<<<(lv.M + 255) / 256, 256, 0, ctx->stream>>>(lv.M, A.sell.ptr, A.sell.col, A.sell.val, u, rhs,
                                                                           (const int *)P.rowptr, P.col, P.val, res_coarse);
     return cudaGetLastError() == cudaSuccess ? 1 : -1;
 }
@@ -84,7 +84,7 @@ extern "C" int saena_b200_time_residual_restrict(saena_b200_ctx *ctx, int level,
     if (level < 0 || level + 1 >= (int)ctx->levels.size()) SB_FAIL("time_residual_restrict: no such level");
     DevLevel &lv = ctx->levels[level];
     DevOperator &A = lv.A, &P = lv.P, &R = lv.R;
-    if (!A.use_sell || !A.sell_ptr) SB_FAIL("time_residual_restrict: A of this level is not on the sliced layout");
+    if (A.mapping != SB_MAPPING_SELL || !A.sell.ptr) SB_FAIL("time_residual_restrict: A of this level is not on the sliced layout");
     if (!P.present || P.wide_offsets || !P.col || !P.val) SB_FAIL("time_residual_restrict: P needs 32-bit CSR arrays");
     if (reps < 3) reps = 10;
     const int M = lv.M, Mc = R.M;
@@ -117,7 +117,7 @@ extern "C" int saena_b200_time_residual_restrict(saena_b200_ctx *ctx, int level,
         // ---- fused: zero-fill of the coarse vector + one kernel that never writes res
         cudaEventRecord(ctx->ev_t0, s);
         cudaMemsetAsync(out2, 0, sizeof(double) * std::max(Mc, 1), s);
-        residual_restrict_sell_kernel<<<(M + 255) / 256, 256, 0, s>>>(M, A.sell_ptr, A.sell_col, A.sell_val, u, rhs,
+        residual_restrict_sell_kernel<<<(M + 255) / 256, 256, 0, s>>>(M, A.sell.ptr, A.sell.col, A.sell.val, u, rhs,
                                                                     (const int *)P.rowptr, P.col, P.val, out2);
         cudaEventRecord(ctx->ev_t1, s);
         cudaEventSynchronize(ctx->ev_t1);

@@ -30,6 +30,51 @@ static int dev_upload(saena_b200_ctx *ctx, T **dst, const T *src, size_t n) {
     return 0;
 }
 
+// host row offsets -> the operator's rowptr, 64-bit with wide_offsets, else 32-bit
+static int upload_rowptr(saena_b200_ctx *ctx, DevOperator &op, const std::vector<int64_t> &rp) {
+    if (op.wide_offsets) {
+        int64_t *p = nullptr;
+        SB_TRY(dev_upload(ctx, &p, rp.data(), rp.size()));
+        op.rowptr = p;
+    } else {
+        std::vector<int> rp32(rp.begin(), rp.end());
+        int *p = nullptr;
+        SB_TRY(dev_upload(ctx, &p, rp32.data(), rp32.size()));
+        op.rowptr = p;
+    }
+    return 0;
+}
+
+// the operator's row offsets back on the host, widened to 64 bits
+static int read_rowptr(saena_b200_ctx *ctx, const DevOperator &op, std::vector<int64_t> &rp) {
+    rp.assign((size_t)op.M + 1, 0);
+    if (op.wide_offsets) {
+        SB_CUDA(cudaMemcpy(rp.data(), op.rowptr, sizeof(int64_t) * rp.size(), cudaMemcpyDeviceToHost));
+    } else {
+        std::vector<int> rp32(rp.size());
+        SB_CUDA(cudaMemcpy(rp32.data(), op.rowptr, sizeof(int) * rp32.size(), cudaMemcpyDeviceToHost));
+        std::copy(rp32.begin(), rp32.end(), rp.begin());
+    }
+    return 0;
+}
+
+// stored entries of the sliced layout over these rows: every 32-row slice padded to its longest row
+static int64_t sliced_padded_est(const std::vector<int64_t> &rp) {
+    const int M = (int)rp.size() - 1;
+    int64_t padded = 0;
+    for (int s0 = 0; s0 < M; s0 += 32) {
+        int64_t mx = 0;
+        for (int i = s0; i < std::min(M, s0 + 32); ++i) mx = std::max(mx, rp[i + 1] - rp[i]);
+        padded += mx * 32;
+    }
+    return padded;
+}
+
+static void free_sliced(SlicedLayout &s) {
+    cudaFree(s.ptr); cudaFree(s.perm); cudaFree(s.col); cudaFree(s.val);
+    s = SlicedLayout();
+}
+
 void sb_free_operator(DevOperator &op) {
     cudaFree(op.rowptr); cudaFree(op.col); cudaFree(op.val); cudaFree(op.blk_row);
     cudaFree(op.brow); cudaFree(op.brow_ptr); cudaFree(op.bcol); cudaFree(op.bval); cudaFree(op.brow_mask);
@@ -37,8 +82,8 @@ void sb_free_operator(DevOperator &op) {
     cudaFree(op.hs.epoch); cudaFree(op.hs.tickets); cudaFree(op.hs.segs);
     cudaFree(op.hs.wait_consumed); cudaFree(op.hs.wait_arrived); cudaFree(op.hs.signal_consumed);
     // ghost_buf / x_ext belong to the context's halo arena
-    cudaFree(op.sell_ptr); cudaFree(op.sell_col); cudaFree(op.sell_val);
-    cudaFree(op.sellp_ptr); cudaFree(op.sellp_perm); cudaFree(op.sellp_col); cudaFree(op.sellp_val);
+    free_sliced(op.sell);
+    free_sliced(op.sellp);
     cudaFree(op.x_round);
     cudaFree(op.rowmid); cudaFree(op.partial);
     op = DevOperator();
@@ -50,7 +95,7 @@ int sb_upload_operator(saena_b200_ctx *ctx, const saena_b200_operator_desc *d) {
     if (d->M < 0 || d->nnz_local < 0 || d->nnz_remote < 0) SB_FAIL("upload_operator: negative size");
     if ((int)ctx->levels.size() <= d->level) ctx->levels.resize(d->level + 1);
     DevLevel &lv = ctx->levels[d->level];
-    DevOperator &op = d->kind == SAENA_B200_KIND_A ? lv.A : (d->kind == SAENA_B200_KIND_P ? lv.P : lv.R);
+    DevOperator &op = lv.op(d->kind);
     if (ctx->arena) sb_arena_free(ctx);  // ghost areas are re-carved at the next finalize
     if (op.present) sb_free_operator(op);
     op.present = true;
@@ -129,25 +174,13 @@ int sb_upload_operator(saena_b200_ctx *ctx, const saena_b200_operator_desc *d) {
         op.nnz_local = nt;   // the kernels see one block
         op.nnz_remote = 0;
         op.wide_offsets = nt >= (int64_t)INT32_MAX;
-        op.sell_padded_est = 0;
-        for (int s0 = 0; s0 < M; s0 += 32) {
-            int64_t mx = 0;
-            for (int i = s0; i < std::min(M, s0 + 32); ++i) mx = std::max(mx, rp[i + 1] - rp[i]);
-            op.sell_padded_est += mx * 32;
-        }
-        if (op.wide_offsets) {
-            int64_t *p = nullptr;
-            SB_TRY(dev_upload(ctx, &p, rp.data(), rp.size()));
-            op.rowptr = p;
-        } else {
-            std::vector<int> rp32(rp.begin(), rp.end());
-            int *p = nullptr;
-            SB_TRY(dev_upload(ctx, &p, rp32.data(), rp32.size()));
-            op.rowptr = p;
+        op.sell_padded_est = sliced_padded_est(rp);
+        SB_TRY(upload_rowptr(ctx, op, rp));
+        if (!op.wide_offsets) {
             // rows are stored [local columns | ghost columns]: the split point of each row, and the scratch that keeps
             // the local sums across the fused kernel's wait
             std::vector<int> mid((size_t)std::max(M, 1));
-            for (int i = 0; i < M; ++i) mid[i] = rp32[i] + d->nnzPerRow_local[i];
+            for (int i = 0; i < M; ++i) mid[i] = (int)rp[i] + d->nnzPerRow_local[i];
             SB_TRY(dev_upload(ctx, &op.rowmid, mid.data(), (size_t)M));
             SB_CUDA(cudaMalloc((void **)&op.partial, sizeof(double) * (size_t)std::max(M, 1)));
         }
@@ -161,22 +194,8 @@ int sb_upload_operator(saena_b200_ctx *ctx, const saena_b200_operator_desc *d) {
         std::vector<int64_t> rp(M + 1, 0);
         for (int i = 0; i < M; ++i) rp[i + 1] = rp[i] + d->nnzPerRow_local[i];
         if (rp[M] != d->nnz_local) SB_FAIL("upload_operator: sum(nnzPerRow_local) != nnz_local");
-        op.sell_padded_est = 0;
-        for (int s0 = 0; s0 < M; s0 += 32) {
-            int mx = 0;
-            for (int i = s0; i < std::min(M, s0 + 32); ++i) mx = std::max(mx, d->nnzPerRow_local[i]);
-            op.sell_padded_est += (int64_t)mx * 32;
-        }
-        if (op.wide_offsets) {
-            int64_t *p = nullptr;
-            SB_TRY(dev_upload(ctx, &p, rp.data(), rp.size()));
-            op.rowptr = p;
-        } else {
-            std::vector<int> rp32(rp.begin(), rp.end());
-            int *p = nullptr;
-            SB_TRY(dev_upload(ctx, &p, rp32.data(), rp32.size()));
-            op.rowptr = p;
-        }
+        op.sell_padded_est = sliced_padded_est(rp);
+        SB_TRY(upload_rowptr(ctx, op, rp));
         // columns arrive as GLOBAL ids; make them local on the device and range-check there
         SB_TRY(dev_upload(ctx, &op.col, d->col_local, (size_t)d->nnz_local));
         if (d->nnz_local) {
@@ -356,9 +375,10 @@ int sb_upload_band_operator(saena_b200_ctx *ctx, int level, int n, int half_band
 // mapping heuristic: lanes per row from nnz/row; short rows stream.  (north_star: "warp-per-row
 // or row-block mapping chosen per level by nnz/row".)  Measured crossovers are in DESIGN.md.
 // ---------------------------------------------------------------------------------------------
-static int pow2_at_most(double v) {
+// the largest power of two <= v, at least 1 and at most cap
+static int pow2_at_most(double v, int cap) {
     int p = 1;
-    while (p * 2 <= v && p < 32) p *= 2;
+    while (p * 2 <= v && p < cap) p *= 2;
     return p;
 }
 
@@ -381,8 +401,7 @@ void sb_choose_mapping(saena_b200_ctx *ctx, DevOperator &op) {
         if (regular && enough_rows) m = SB_MAPPING_SELL;
         else {
             // ~4+ elements per lane; rows of hundreds..thousands of entries get 32..256 threads
-            m = 1;
-            while (m * 2 <= (avg + 1.0) / 4.0 && m < 256) m *= 2;
+            m = pow2_at_most((avg + 1.0) / 4.0, 256);
             // few rows: the sub-warp mapping walks its 32 rows in `lanes` dependent steps (2 rows at a
             // time at 16 lanes), and with fewer than ~32 warps per SM nothing hides that chain --
             // measured on the unstructured 2-D hierarchy (profiles/r01_unstructured.md): levels of
@@ -392,33 +411,16 @@ void sb_choose_mapping(saena_b200_ctx *ctx, DevOperator &op) {
             if (m < 32 && op.M <= 32 * 32 * ctx->sm_count) m = 32;
         }
     }
-    op.use_stream = op.use_sell = op.use_sellp = false;
-    if (m == SB_MAPPING_SELL) {
-        op.use_sell = true;
-        op.lanes = 1;
-    } else if (m == SB_MAPPING_SELLP) {
-        op.use_sellp = true;
-        op.lanes = 1;
-    } else if (m < 0) {
-        op.use_stream = true;
-        op.lanes = std::min(32, std::max(1, pow2_at_most(-m)));
-    } else {
-        int l = 1;
-        while (l * 2 <= m && l < 256) l *= 2;
-        op.lanes = l;
-    }
+    // the one place a code is made canonical: threads per row 1..256 and streaming lanes 1..32, powers of two
+    if (m == SB_MAPPING_SELL || m == SB_MAPPING_SELLP) op.mapping = m;
+    else if (m < 0) op.mapping = -pow2_at_most(-m, 32);
+    else op.mapping = pow2_at_most(m, 256);
 }
 
 // rows [blk_row[b], blk_row[b+1]) : at most `rows_per_block` rows and STREAM_TILE nnz
 static int build_row_blocks(saena_b200_ctx *ctx, DevOperator &op, int rows_per_block) {
-    std::vector<int64_t> rp(op.M + 1);
-    if (op.wide_offsets) {
-        SB_CUDA(cudaMemcpy(rp.data(), op.rowptr, sizeof(int64_t) * (op.M + 1), cudaMemcpyDeviceToHost));
-    } else {
-        std::vector<int> rp32(op.M + 1);
-        SB_CUDA(cudaMemcpy(rp32.data(), op.rowptr, sizeof(int) * (op.M + 1), cudaMemcpyDeviceToHost));
-        std::copy(rp32.begin(), rp32.end(), rp.begin());
-    }
+    std::vector<int64_t> rp;
+    SB_TRY(read_rowptr(ctx, op, rp));
     std::vector<int> blk(1, 0);
     int r = 0;
     while (r < op.M) {
@@ -437,8 +439,8 @@ static int build_row_blocks(saena_b200_ctx *ctx, DevOperator &op, int rows_per_b
 }
 
 // ---------------------------------------------------------------------------------------------
-// sliced layout, built on the device from the CSR arrays (one-time, at finalize):
-// 32-row slices, column-major inside a slice, padded to the slice's longest row
+// sliced layouts, built on the device from the CSR arrays (one-time, at finalize):
+// 32-slot slices, column-major inside a slice, padded to the slice's longest row
 // ---------------------------------------------------------------------------------------------
 template <typename OffT>
 __global__ void sell_slice_len_kernel(int M, const OffT *__restrict__ rowptr, int *__restrict__ slice_len) {
@@ -449,17 +451,20 @@ __global__ void sell_slice_len_kernel(int M, const OffT *__restrict__ rowptr, in
     if ((threadIdx.x & 31) == 0 && (row >> 5) < (M + 31) / 32) slice_len[row >> 5] = len;
 }
 
+// slot -> row through perm (sorted layout) or slot = row; a slot past the last row holds padding only
 template <typename OffT>
-__global__ void sell_fill_kernel(int M, const OffT *__restrict__ rowptr, const int *__restrict__ col,
-                                 const double *__restrict__ val, const long long *__restrict__ slice_ptr,
-                                 int *__restrict__ scol, double *__restrict__ sval) {
-    const int row = blockIdx.x * blockDim.x + threadIdx.x;
-    const int slice = row >> 5, lane = row & 31;
-    if ((slice << 5) >= M) return;
+__global__ void sliced_fill_kernel(int n_slots, int M, const int *__restrict__ perm, const OffT *__restrict__ rowptr,
+                                   const int *__restrict__ col, const double *__restrict__ val,
+                                   const long long *__restrict__ slice_ptr, int *__restrict__ scol,
+                                   double *__restrict__ sval) {
+    const int slot = blockIdx.x * blockDim.x + threadIdx.x;
+    if (slot >= n_slots) return;
+    const int slice = slot >> 5, lane = slot & 31;
     const long long base = slice_ptr[slice];
     const int len = (int)((slice_ptr[slice + 1] - base) >> 5);
+    const int row = perm ? perm[slot] : (slot < M ? slot : -1);
     OffT a = 0, b = 0;
-    if (row < M) { a = rowptr[row]; b = rowptr[row + 1]; }
+    if (row >= 0) { a = rowptr[row]; b = rowptr[row + 1]; }
     const int pad_col = (b > a) ? col[b - 1] : 0;  // padding: val 0.0, a column the row already touches
     for (int j = 0; j < len; ++j) {
         const long long dst = base + (long long)j * 32 + lane;
@@ -473,8 +478,33 @@ __global__ void sell_fill_kernel(int M, const OffT *__restrict__ rowptr, const i
     }
 }
 
+// fills s from the operator's CSR arrays: sp = element offsets of the 32-slot slices, perm = slot -> row or nullptr
+static int build_sliced(saena_b200_ctx *ctx, DevOperator &op, SlicedLayout &s, const std::vector<long long> &sp,
+                        const std::vector<int> *perm) {
+    const int n_slots = (int)(sp.size() - 1) * 32;
+    const int64_t padded = sp.back();
+    SB_TRY(dev_upload(ctx, &s.ptr, sp.data(), sp.size()));
+    if (perm) SB_TRY(dev_upload(ctx, &s.perm, perm->data(), perm->size()));
+    SB_CUDA(cudaMalloc((void **)&s.col, sizeof(int) * std::max<int64_t>(padded, 1)));
+    SB_CUDA(cudaMalloc((void **)&s.val, sizeof(double) * std::max<int64_t>(padded, 1)));
+    if (n_slots) {
+        const int blocks = (n_slots + 255) / 256;
+        if (op.wide_offsets)
+            sliced_fill_kernel<int64_t><<<blocks, 256, 0, ctx->stream>>>(n_slots, op.M, s.perm, (const int64_t *)op.rowptr,
+                                                                         op.col, op.val, s.ptr, s.col, s.val);
+        else
+            sliced_fill_kernel<int><<<blocks, 256, 0, ctx->stream>>>(n_slots, op.M, s.perm, (const int *)op.rowptr,
+                                                                     op.col, op.val, s.ptr, s.col, s.val);
+    }
+    SB_CUDA(cudaGetLastError());
+    SB_CUDA(cudaStreamSynchronize(ctx->stream));
+    return 0;
+}
+
+// the slice lengths come from the row offsets on the device: the row offsets of a device-generated band operator
+// (50 M rows) are never read back
 static int build_sell(saena_b200_ctx *ctx, DevOperator &op) {
-    if (op.sell_ptr) return 0;
+    if (op.sell.ptr) return 0;
     const int M = op.M;
     const int ns = (M + 31) / 32;
     int *d_len = nullptr;
@@ -492,21 +522,7 @@ static int build_sell(saena_b200_ctx *ctx, DevOperator &op) {
     cudaFree(d_len);
     std::vector<long long> sp(ns + 1, 0);
     for (int s0 = 0; s0 < ns; ++s0) sp[s0 + 1] = sp[s0] + (long long)len[s0] * 32;
-    const int64_t padded = sp[ns];
-    op.sell_padded = padded;
-    SB_TRY(dev_upload(ctx, &op.sell_ptr, sp.data(), sp.size()));
-    SB_CUDA(cudaMalloc((void **)&op.sell_col, sizeof(int) * std::max<int64_t>(padded, 1)));
-    SB_CUDA(cudaMalloc((void **)&op.sell_val, sizeof(double) * std::max<int64_t>(padded, 1)));
-    if (ns) {
-        if (op.wide_offsets)
-            sell_fill_kernel<int64_t><<<blocks, 256, 0, ctx->stream>>>(M, (const int64_t *)op.rowptr, op.col, op.val,
-                                                                       op.sell_ptr, op.sell_col, op.sell_val);
-        else
-            sell_fill_kernel<int><<<blocks, 256, 0, ctx->stream>>>(M, (const int *)op.rowptr, op.col, op.val,
-                                                                   op.sell_ptr, op.sell_col, op.sell_val);
-    }
-    SB_CUDA(cudaGetLastError());
-    SB_CUDA(cudaStreamSynchronize(ctx->stream));
+    SB_TRY(build_sliced(ctx, op, op.sell, sp, nullptr));
     if (op.sell_only) {
         // the sliced copy is the operator from here on: give the CSR entries back (half the footprint)
         cudaFree(op.col);
@@ -522,32 +538,6 @@ static int build_sell(saena_b200_ctx *ctx, DevOperator &op) {
 // consecutive rows; the permutation is made on the host from the row offsets, the entries are moved on the device
 // ---------------------------------------------------------------------------------------------
 constexpr int SELLP_WINDOW = 256;  // = the CTA size of spmv_sellp_kernel
-
-template <typename OffT>
-__global__ void sellp_fill_kernel(int n_slots, const int *__restrict__ perm, const OffT *__restrict__ rowptr,
-                                  const int *__restrict__ col, const double *__restrict__ val,
-                                  const long long *__restrict__ slice_ptr, int *__restrict__ scol,
-                                  double *__restrict__ sval) {
-    const int slot = blockIdx.x * blockDim.x + threadIdx.x;
-    if (slot >= n_slots) return;
-    const int slice = slot >> 5, lane = slot & 31;
-    const long long base = slice_ptr[slice];
-    const int len = (int)((slice_ptr[slice + 1] - base) >> 5);
-    const int row = perm[slot];
-    OffT a = 0, b = 0;
-    if (row >= 0) { a = rowptr[row]; b = rowptr[row + 1]; }
-    const int pad_col = (b > a) ? col[b - 1] : 0;  // padding: val 0.0, a column the row already touches
-    for (int j = 0; j < len; ++j) {
-        const long long dst = base + (long long)j * 32 + lane;
-        if (a + j < b) {
-            scol[dst] = col[a + j];
-            sval[dst] = val[a + j];
-        } else {
-            scol[dst] = pad_col;
-            sval[dst] = 0.0;
-        }
-    }
-}
 
 // host only: slot -> row (rows of each SELLP_WINDOW-row window sorted by length, longest first, stable; -1 where the
 // last window runs past M) and the element offset of every 32-slot slice (its longest row's length x 32).
@@ -570,64 +560,29 @@ void sb_sellp_layout(int M, const int64_t *rp, int *perm, long long *sp) {
 }
 
 static int build_sellp(saena_b200_ctx *ctx, DevOperator &op) {
-    if (op.sellp_ptr) return 0;
+    if (op.sellp.ptr) return 0;
     if (!op.col || !op.val) SB_FAIL("sorted sliced layout: the CSR entries of this operator were released");
-    const int M = op.M;
-    const int n_win = (M + SELLP_WINDOW - 1) / SELLP_WINDOW;
-    const int n_slots = n_win * SELLP_WINDOW;
-    const int ns = n_slots / 32;
-    // row lengths from the row offsets
-    std::vector<int64_t> rp((size_t)M + 1, 0);
-    if (op.wide_offsets) {
-        SB_CUDA(cudaMemcpy(rp.data(), op.rowptr, sizeof(int64_t) * ((size_t)M + 1), cudaMemcpyDeviceToHost));
-    } else {
-        std::vector<int> rp32((size_t)M + 1, 0);
-        SB_CUDA(cudaMemcpy(rp32.data(), op.rowptr, sizeof(int) * ((size_t)M + 1), cudaMemcpyDeviceToHost));
-        for (int i = 0; i <= M; ++i) rp[i] = rp32[i];
-    }
+    const int n_slots = (op.M + SELLP_WINDOW - 1) / SELLP_WINDOW * SELLP_WINDOW;
+    std::vector<int64_t> rp;
+    SB_TRY(read_rowptr(ctx, op, rp));
     std::vector<int> perm((size_t)std::max(n_slots, 1), -1);
-    std::vector<long long> sp((size_t)ns + 1, 0);
-    sb_sellp_layout(M, rp.data(), perm.data(), sp.data());
-    const int64_t padded = sp[ns];
-    op.sellp_padded = padded;
-    SB_TRY(dev_upload(ctx, &op.sellp_ptr, sp.data(), sp.size()));
-    SB_TRY(dev_upload(ctx, &op.sellp_perm, perm.data(), perm.size()));
-    SB_CUDA(cudaMalloc((void **)&op.sellp_col, sizeof(int) * std::max<int64_t>(padded, 1)));
-    SB_CUDA(cudaMalloc((void **)&op.sellp_val, sizeof(double) * std::max<int64_t>(padded, 1)));
-    if (n_slots) {
-        const int blocks = n_slots / 256;
-        if (op.wide_offsets)
-            sellp_fill_kernel<int64_t><<<blocks, 256, 0, ctx->stream>>>(n_slots, op.sellp_perm, (const int64_t *)op.rowptr,
-                                                                        op.col, op.val, op.sellp_ptr, op.sellp_col, op.sellp_val);
-        else
-            sellp_fill_kernel<int><<<blocks, 256, 0, ctx->stream>>>(n_slots, op.sellp_perm, (const int *)op.rowptr, op.col,
-                                                                    op.val, op.sellp_ptr, op.sellp_col, op.sellp_val);
-    }
-    SB_CUDA(cudaGetLastError());
-    SB_CUDA(cudaStreamSynchronize(ctx->stream));
-    return 0;
+    std::vector<long long> sp((size_t)n_slots / 32 + 1, 0);
+    sb_sellp_layout(op.M, rp.data(), perm.data(), sp.data());
+    return build_sliced(ctx, op, op.sellp, sp, &perm);
 }
 
 // copies of the entries in layouts the operator no longer uses (a mapping walk builds them to time them)
 void sb_drop_unused_layouts(DevOperator &op) {
-    if (!op.use_sellp && op.sellp_ptr) {
-        cudaFree(op.sellp_ptr); cudaFree(op.sellp_perm); cudaFree(op.sellp_col); cudaFree(op.sellp_val);
-        op.sellp_ptr = nullptr; op.sellp_perm = nullptr; op.sellp_col = nullptr; op.sellp_val = nullptr;
-        op.sellp_padded = 0;
-    }
-    if (!op.use_sell && !op.sell_only && op.sell_ptr) {
-        cudaFree(op.sell_ptr); cudaFree(op.sell_col); cudaFree(op.sell_val);
-        op.sell_ptr = nullptr; op.sell_col = nullptr; op.sell_val = nullptr;
-        op.sell_padded = 0;
-    }
+    if (op.mapping != SB_MAPPING_SELLP) free_sliced(op.sellp);
+    if (op.mapping != SB_MAPPING_SELL && !op.sell_only) free_sliced(op.sell);
 }
 
 int sb_prepare_operator(saena_b200_ctx *ctx, DevOperator &op) {
     if (!op.present) return 0;
     sb_choose_mapping(ctx, op);
-    if (op.use_stream) SB_TRY(build_row_blocks(ctx, op, STREAM_THREADS / op.lanes));
-    if (op.use_sell) SB_TRY(build_sell(ctx, op));
-    if (op.use_sellp) SB_TRY(build_sellp(ctx, op));
+    if (op.mapping < 0) SB_TRY(build_row_blocks(ctx, op, STREAM_THREADS / -op.mapping));
+    if (op.mapping == SB_MAPPING_SELL) SB_TRY(build_sell(ctx, op));
+    if (op.mapping == SB_MAPPING_SELLP) SB_TRY(build_sellp(ctx, op));
     return 0;
 }
 
@@ -635,23 +590,23 @@ int sb_prepare_operator(saena_b200_ctx *ctx, DevOperator &op) {
 // launchers
 // ---------------------------------------------------------------------------------------------
 template <int EPI, typename OffT>
-static void launch_local(saena_b200_ctx *ctx, DevOperator &op, const double *x, const EpiArgs &e) {
+static int launch_local(saena_b200_ctx *ctx, DevOperator &op, const double *x, const EpiArgs &e) {
     const OffT *rp = (const OffT *)op.rowptr;
     cudaStream_t s = ctx->stream;
+    const bool stream = op.mapping < 0;
     // rows [lo, hi): everything when there is no halo, else the interior range
-    const int lo = op.use_stream ? 0 : op.int_lo, hi = op.use_stream ? op.M : op.int_hi;
+    const int lo = stream ? 0 : op.int_lo, hi = stream ? op.M : op.int_hi;
     const int nrows = hi - lo;
-    if (nrows <= 0) return;
+    if (nrows <= 0) return 0;
     ++ctx->launches;
-    if (op.use_sellp) {
+    if (op.mapping == SB_MAPPING_SELLP) {
         // whole operator (no halo, see sb_choose_mapping): one CTA per 256-row window
-        spmv_sellp_kernel<EPI><<<(op.M + 255) / 256, 256, 0, s>>>(op.M, op.sellp_ptr, op.sellp_perm, op.sellp_col,
-                                                                   op.sellp_val, x, e);
-    } else if (op.use_sell) {
-        const int blocks = (nrows + 255) / 256;
-        spmv_sell_kernel<EPI><<<blocks, 256, 0, s>>>(lo, hi, op.sell_ptr, op.sell_col, op.sell_val, x, e, nullptr);
-    } else if (op.use_stream) {
-        switch (op.lanes) {
+        spmv_sellp_kernel<EPI><<<(op.M + 255) / 256, 256, 0, s>>>(op.M, op.sellp.ptr, op.sellp.perm, op.sellp.col,
+                                                                   op.sellp.val, x, e);
+        return 0;
+    }
+    if (stream) {
+        switch (-op.mapping) {
 #define SB_STREAM_CASE(L)                                                                          \
     case L:                                                                                        \
         spmv_stream_kernel<L, EPI, OffT><<<op.n_blk, STREAM_THREADS, 0, s>>>(                      \
@@ -661,28 +616,20 @@ static void launch_local(saena_b200_ctx *ctx, DevOperator &op, const double *x, 
             SB_STREAM_CASE(16) SB_STREAM_CASE(32)
 #undef SB_STREAM_CASE
         }
-    } else if (op.lanes >= 32) {
-        switch (op.lanes) {
-#define SB_RG_CASE(T)                                                                              \
-    case T:                                                                                        \
-        spmv_rowgroup_kernel<T, EPI, OffT><<<(nrows + 256 / T - 1) / (256 / T), 256, 0, s>>>(      \
-            lo, hi, rp, op.col, op.val, x, e, nullptr);                                            \
-        break;
-            SB_RG_CASE(32) SB_RG_CASE(64) SB_RG_CASE(128) SB_RG_CASE(256)
-#undef SB_RG_CASE
-        }
-    } else {
-        const int blocks = (nrows + 255) / 256;  // 8 warps x 32 rows
-        switch (op.lanes) {
-#define SB_VEC_CASE(L)                                                                             \
-    case L:                                                                                        \
-        spmv_vec_kernel<L, EPI, OffT><<<blocks, 256, 0, s>>>(lo, hi, rp, op.col, op.val, x, e,     \
-                                                             nullptr);                             \
-        break;
-            SB_VEC_CASE(1) SB_VEC_CASE(2) SB_VEC_CASE(4) SB_VEC_CASE(8) SB_VEC_CASE(16)
-#undef SB_VEC_CASE
-        }
+        return 0;
     }
+    const int blocks = sb_mapping_blocks(op.mapping, nrows);
+    const bool known = sb_dispatch_mapping(op.mapping, [&](auto map) {
+        constexpr int MAP = decltype(map)::value;
+        if constexpr (MAP == SB_MAPPING_SELL)
+            spmv_sell_kernel<EPI><<<blocks, 256, 0, s>>>(lo, hi, op.sell.ptr, op.sell.col, op.sell.val, x, e, nullptr);
+        else if constexpr (MAP >= 32)
+            spmv_rowgroup_kernel<MAP, EPI, OffT><<<blocks, 256, 0, s>>>(lo, hi, rp, op.col, op.val, x, e, nullptr);
+        else
+            spmv_vec_kernel<MAP, EPI, OffT><<<blocks, 256, 0, s>>>(lo, hi, rp, op.col, op.val, x, e, nullptr);
+    });
+    if (!known) SB_FAIL("apply: unknown mapping");
+    return 0;
 }
 
 template <int EPI, typename OffT>
@@ -763,16 +710,16 @@ static int apply_epi(saena_b200_ctx *ctx, DevOperator &op, const double *x, cons
                 widen_ghost_kernel<<<(op.recvSize + 255) / 256, 256, 0, ctx->stream>>>(
                     op.recvSize, (const float *)op.ghost_buf, op.x_ext + op.n_local_cols);
             }
-            if (op.wide_offsets) launch_local<EPI, int64_t>(ctx, op, op.x_ext, e);
-            else launch_local<EPI, int>(ctx, op, op.x_ext, e);
+            if (op.wide_offsets) SB_TRY((launch_local<EPI, int64_t>(ctx, op, op.x_ext, e)));
+            else SB_TRY((launch_local<EPI, int>(ctx, op, op.x_ext, e)));
         }
         if (halo && op.p2p) SB_TRY(sb_p2p_release(ctx, op, ctx->stream));
         SB_CUDA(cudaGetLastError());
         return 0;
     }
     if (compute) {
-        if (op.wide_offsets) launch_local<EPI, int64_t>(ctx, op, x, e);
-        else launch_local<EPI, int>(ctx, op, x, e);
+        if (op.wide_offsets) SB_TRY((launch_local<EPI, int64_t>(ctx, op, x, e)));
+        else SB_TRY((launch_local<EPI, int>(ctx, op, x, e)));
     }
     if (halo) SB_TRY(wait_halo(ctx, op));
     if (has_halo && compute) {

@@ -20,6 +20,8 @@
 //                      (7-point level 0) where a per-row mapping wastes lanes.
 #pragma once
 
+#include <type_traits>
+
 #include "common.h"
 
 template <int EPI>
@@ -452,4 +454,29 @@ __global__ void halo_pack_kernel(int n, const int *__restrict__ vIndex, const do
                                  SendT *__restrict__ out) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) out[i] = (SendT)v[vIndex[i]];
+}
+
+// ---------------------------------------------------------------------------------------------
+// host side: the mappings with one body per row range -- spmv_vec (1..16), spmv_rowgroup (32..256) and the sliced
+// layout -- launched alone (operator.cu) or inside the fused halo kernel (fused_halo.cu).  The streaming row blocks
+// and the sorted sliced layout have launches of their own.
+// ---------------------------------------------------------------------------------------------
+// calls f(std::integral_constant<int, MAP>{}) with MAP = mapping; false (nothing called) for any other code
+template <typename F>
+bool sb_dispatch_mapping(int mapping, F &&f) {
+    switch (mapping) {
+#define SB_MAP_CASE(MAP)                                                                           \
+    case MAP: f(std::integral_constant<int, MAP>{}); return true;
+        SB_MAP_CASE(1) SB_MAP_CASE(2) SB_MAP_CASE(4) SB_MAP_CASE(8) SB_MAP_CASE(16)
+        SB_MAP_CASE(32) SB_MAP_CASE(64) SB_MAP_CASE(128) SB_MAP_CASE(256) SB_MAP_CASE(SB_MAPPING_SELL)
+#undef SB_MAP_CASE
+    }
+    return false;
+}
+
+// 256-thread CTAs over nrows rows: 8 warps x 32 rows (sub-warp, sliced), 256 / mapping rows (row groups)
+inline int sb_mapping_blocks(int mapping, int nrows) {
+    if (nrows <= 0) return 0;
+    const int rows_per_block = (mapping == SB_MAPPING_SELL || mapping < 32) ? 256 : 256 / mapping;
+    return (nrows + rows_per_block - 1) / rows_per_block;
 }

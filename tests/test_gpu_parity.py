@@ -200,6 +200,28 @@ def test_every_kernel_mapping_gives_the_same_answer(golden_ctx):
                     ctx.set_mapping(l, k, 0)
 
 
+def test_mapping_codes_are_canonical(golden_ctx):
+    """set_mapping normalises a requested code to one of the codes get_mapping reports: threads per row rounded down
+    to a power of two up to 256, streaming lanes to a power of two up to 32, the two sliced layouts as they are; 0
+    gives back the rule's choice"""
+    g, ctx = golden_ctx
+    kept = [1, 16, 32, 256, -1, -32, 100, 101]
+    rounded = {3: 2, 17: 16, 31: 16, 33: 32, 99: 64, 102: 64, 255: 128, 300: 256, -3: -2, -64: -32}
+    for l, lv in enumerate(g.hier.levels):
+        for k in (KIND_A, KIND_P, KIND_R) if lv.P is not None else (KIND_A,):
+            at_upload = ctx.get_mapping(l, k)
+            try:
+                for m in kept:
+                    ctx.set_mapping(l, k, m)
+                    assert ctx.get_mapping(l, k) == m, (l, k, m)
+                for m, want in rounded.items():
+                    ctx.set_mapping(l, k, m)
+                    assert ctx.get_mapping(l, k) == want, (l, k, m)
+            finally:
+                ctx.set_mapping(l, k, 0)
+            assert ctx.get_mapping(l, k) == at_upload, (l, k)
+
+
 def test_other_solvers_and_option_sets_against_oracle(golden_ctx):
     g, ctx = golden_ctx
     o = Oracle(g.hier)

@@ -1,6 +1,6 @@
 """Mapping 101 (sliced layout over rows sorted by length inside 256-row windows), the half that needs no GPU:
 saena_b200_sellp_layout -- the function the device build calls -- gives the permutation and the slice offsets; the
-fill kernel and the product kernel (csrc/operator.cu:sellp_fill_kernel, csrc/spmv_kernels.cuh:spmv_sellp_body) are
+fill kernel and the product kernel (csrc/operator.cu:sliced_fill_kernel, csrc/spmv_kernels.cuh:spmv_sellp_body) are
 restated in numpy on top of it, index for index, and must reproduce the CSR product.  The kernels themselves are
 tested on the GPU (tests/test_zz_dense_levels_gpu.py::test_sorted_sliced_layout_mapping_101)."""
 import numpy as np
@@ -11,13 +11,13 @@ from tests.util import GOLDEN_EXTRA, Golden
 
 
 def _emulate(rowptr, col, val, x):
-    """sellp_fill_kernel + spmv_sellp_body, slot by slot"""
+    """sliced_fill_kernel + spmv_sellp_body, slot by slot"""
     M = len(rowptr) - 1
     perm, sp = sellp_layout(rowptr)
     n_slots = len(perm)
     scol = np.zeros(max(int(sp[-1]), 1), np.int64)
     sval = np.zeros(max(int(sp[-1]), 1))
-    for slot in range(n_slots):                       # sellp_fill_kernel
+    for slot in range(n_slots):                       # sliced_fill_kernel
         sl, lane = slot >> 5, slot & 31
         base, ln = int(sp[sl]), int(sp[sl + 1] - sp[sl]) >> 5
         row = int(perm[slot])
