@@ -206,6 +206,37 @@ int saena_b200_halo_choice(const saena_b200_ctx *ctx, int level, int kind, float
 int saena_b200_find_eig(saena_b200_ctx *ctx, int level, int max_iter, const double *start, uint64_t seed, int store,
                         double *eig_out, int *iters_out);
 
+/* ---- next to the solve path (SURVEY.md 8f #4): new values on the same pattern, without a new setup ----------------
+ * For a user who solves many systems with one matrix pattern (time steps, Newton steps, coefficient sweeps).  One rank.
+ * val_local: new values of level 0's A in the UPLOADED order -- row-major, the nnzPerRow_local / col_local given at
+ * upload, nnz_local entries.  The aggregates, P, R, every stored pattern, the kernel mappings, row blocks and the
+ * autotune's choices are kept; the values are recomputed:
+ *   1. level 0's A takes the values;
+ *   2. for l = 0 .. L-1, C = R_l (A_l P_l) on the device (the SpGEMM below) is mapped onto A_{l+1}'s stored pattern with
+ *      the setup's filter rule (saena_object::filter): a stored entry takes C's value, an off-diagonal entry of C
+ *      outside the pattern is lumped into its row's diagonal, a diagonal below 1e-14 in magnitude (or one C lacks) is 1;
+ *      a stored off-diagonal entry that C lacks is an error ("not a Galerkin product of the level above").  With the
+ *      uploaded values this reproduces the setup's own A_{l+1};
+ *   3. every level's inv_diag = 1 / diag(A_l) and eig_max = find_eig(l, max_eig_iter, NULL, seed, store = 1);
+ *   4. the sliced copies of the operators' entries (mappings 100 / 101) and the coarsest dense factor are rebuilt;
+ *   5. captured V-cycles are dropped, and a level on the route (saena_b200_set_level_route) stays there only if
+ *      R A P still matches its stored operator to the route's tolerance (saena_b200_get_level_route reports it).
+ * dropped_out (optional, dropped_cap entries): per level, the lumped entries' share ||C - C|pattern||_F / ||C||_F --
+ * how far the frozen pattern has drifted from what a new setup would keep; dropped_out[0] = 0.
+ * Refused, with the hierarchy untouched: several ranks (the coarse product of a row-partitioned level needs the other
+ * ranks' rows of P), a scaled hierarchy, a context that is not finalized, nnz_local != level 0's, an operator uploaded
+ * sliced_only (its CSR values were released), a new level-0 diagonal that is missing or below 1e-14 in magnitude.
+ * A failure after writing has begun (a coarse pattern that is not a Galerkin product, a CUDA error) leaves the
+ * context un-finalized: every solver and hook refuses until the hierarchy is uploaded again.
+ * The _dev variant takes the values in device memory (complete before the call).
+ * saena_b200_update_values_times: host-clock ms of the last update's phases -- products, pattern map (with the
+ * diagonals), sliced layouts, eigenvalue bounds, coarsest factor (cap <= 5 entries). */
+int saena_b200_update_values(saena_b200_ctx *ctx, const double *val_local, int64_t nnz_local, int max_eig_iter,
+                             uint64_t seed, double *dropped_out, int dropped_cap);
+int saena_b200_update_values_dev(saena_b200_ctx *ctx, const double *val_local_dev, int64_t nnz_local,
+                                 int max_eig_iter, uint64_t seed, double *dropped_out, int dropped_cap);
+int saena_b200_update_values_times(const saena_b200_ctx *ctx, double *ms_out, int cap);
+
 /* ---- next to the solve path (SURVEY.md 8f #3): the Galerkin product's SpGEMM on the device ----------
  * C = A B for CSR operands (64-bit row offsets, int32 columns, FP64 values), all pointers DEVICE pointers, work on
  * the default stream.  What saena_object::triple_mat_mult (src/saena_object_setup2.cpp:361) computes as R (A P)

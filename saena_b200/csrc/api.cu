@@ -187,25 +187,18 @@ int saena_b200_upload_level_scale(saena_b200_ctx *ctx, int level, const double *
     return 0;
 }
 
+}  // extern "C"
+
 // Dense LU with partial pivoting on the host, then the explicit inverse; the device applies
 // Ainv with one refinement step against A (vector_ops.cu).  Stands in for SuperLU_DIST's
-// factor + pdgssvx solve (saena_object_solve.cpp:117-419, :793-958).
-int saena_b200_upload_coarsest(saena_b200_ctx *ctx, int n, int64_t nnz, const int32_t *row, const int32_t *col,
-                               const double *val) {
-    if (!ctx) return 1;
-    SB_CUDA(cudaSetDevice(ctx->device));
-    sb_invalidate_graphs(ctx);  // a captured V-cycle's coarsest_kernel node points at the buffers released below
-    ctx->finalized = false;
-    cudaFree(ctx->coarse_A); cudaFree(ctx->coarse_Ainv); cudaFree(ctx->coarse_tmp);
-    ctx->coarse_A = ctx->coarse_Ainv = ctx->coarse_tmp = nullptr;
-    ctx->coarse_n = 0;
-    if (n == 0) return 0;
+// factor + pdgssvx solve (saena_object_solve.cpp:117-419, :793-958).  Used by the upload and by
+// saena_b200_update_values; the factor's old buffers are released once the new one is computed.
+int sb_coarsest_factor(saena_b200_ctx *ctx, int n, int64_t nnz, const int32_t *row, const int32_t *col, const double *val) {
     // coarsest_kernel keeps one n-vector in dynamic shared memory: 4096 doubles = 32 KB, inside the 48 KB default
-    if (n < 0 || n > 4096) SB_FAIL("upload_coarsest: coarsest level must have 1..4096 rows");
-    ctx->coarse_n = n;
+    if (n < 1 || n > 4096) SB_FAIL("coarsest factor: coarsest level must have 1..4096 rows");
     std::vector<double> A((size_t)n * n, 0.0);
     for (int64_t k = 0; k < nnz; ++k) {
-        if (row[k] < 0 || row[k] >= n || col[k] < 0 || col[k] >= n) SB_FAIL("upload_coarsest: index out of range");
+        if (row[k] < 0 || row[k] >= n || col[k] < 0 || col[k] >= n) SB_FAIL("coarsest factor: index out of range");
         A[(size_t)row[k] * n + col[k]] += val[k];
     }
     std::vector<double> LU(A), inv((size_t)n * n, 0.0);
@@ -215,7 +208,7 @@ int saena_b200_upload_coarsest(saena_b200_ctx *ctx, int n, int64_t nnz, const in
         double best = fabs(LU[(size_t)k * n + k]);
         for (int i = k + 1; i < n; ++i)
             if (fabs(LU[(size_t)i * n + k]) > best) { best = fabs(LU[(size_t)i * n + k]); p = i; }
-        if (best == 0.0) SB_FAIL("upload_coarsest: coarsest operator is singular");
+        if (best == 0.0) SB_FAIL("coarsest factor: coarsest operator is singular");
         piv[k] = p;
         if (p != k)
             for (int j = 0; j < n; ++j) std::swap(LU[(size_t)k * n + j], LU[(size_t)p * n + j]);
@@ -245,12 +238,31 @@ int saena_b200_upload_coarsest(saena_b200_ctx *ctx, int n, int64_t nnz, const in
         }
         for (int i = 0; i < n; ++i) inv[(size_t)i * n + e] = c[i];
     }
+    cudaFree(ctx->coarse_A); cudaFree(ctx->coarse_Ainv); cudaFree(ctx->coarse_tmp);
+    ctx->coarse_A = ctx->coarse_Ainv = ctx->coarse_tmp = nullptr;
+    ctx->coarse_n = 0;
     SB_CUDA(cudaMalloc((void **)&ctx->coarse_A, sizeof(double) * n * n));
     SB_CUDA(cudaMalloc((void **)&ctx->coarse_Ainv, sizeof(double) * n * n));
     SB_CUDA(cudaMalloc((void **)&ctx->coarse_tmp, sizeof(double) * 2 * n));
     SB_CUDA(cudaMemcpy(ctx->coarse_A, A.data(), sizeof(double) * n * n, cudaMemcpyHostToDevice));
     SB_CUDA(cudaMemcpy(ctx->coarse_Ainv, inv.data(), sizeof(double) * n * n, cudaMemcpyHostToDevice));
+    ctx->coarse_n = n;
     return 0;
+}
+
+extern "C" {
+
+int saena_b200_upload_coarsest(saena_b200_ctx *ctx, int n, int64_t nnz, const int32_t *row, const int32_t *col,
+                               const double *val) {
+    if (!ctx) return 1;
+    SB_CUDA(cudaSetDevice(ctx->device));
+    sb_invalidate_graphs(ctx);  // a captured V-cycle's coarsest_kernel node points at the buffers released below
+    ctx->finalized = false;
+    cudaFree(ctx->coarse_A); cudaFree(ctx->coarse_Ainv); cudaFree(ctx->coarse_tmp);
+    ctx->coarse_A = ctx->coarse_Ainv = ctx->coarse_tmp = nullptr;
+    ctx->coarse_n = 0;
+    if (n == 0) return 0;
+    return sb_coarsest_factor(ctx, n, nnz, row, col, val);
 }
 
 static int alloc_d(saena_b200_ctx *ctx, double **p, size_t n) {
@@ -1159,6 +1171,32 @@ int saena_b200_find_eig(saena_b200_ctx *ctx, int level, int max_iter, const doub
     return 0;
 }
 
+// Next to find_eig: new values for level 0's A, every coarse level recomputed on its stored pattern (refresh.cu).
+// The host variant stages the values in stage[3], which no other entry point uses.
+int saena_b200_update_values(saena_b200_ctx *ctx, const double *val_local, int64_t nnz_local, int max_eig_iter,
+                             uint64_t seed, double *dropped_out, int dropped_cap) {
+    SB_ENTER();
+    if (nnz_local < 0 || (nnz_local && !val_local)) SB_FAIL("update_values: no values");
+    SB_TRY(stage_buf(ctx, 3, (size_t)nnz_local));   // the caller's array holds nnz_local values; checked next
+    SB_TRY(h2d(ctx, ctx->stage[3], val_local, (size_t)nnz_local));
+    return sb_update_values(ctx, ctx->stage[3], nnz_local, max_eig_iter, (unsigned long long)seed, dropped_out,
+                            dropped_cap);
+}
+
+int saena_b200_update_values_dev(saena_b200_ctx *ctx, const double *val_local_dev, int64_t nnz_local, int max_eig_iter,
+                                 uint64_t seed, double *dropped_out, int dropped_cap) {
+    SB_ENTER();
+    if (nnz_local < 0 || (nnz_local && !val_local_dev)) SB_FAIL("update_values: no values");
+    return sb_update_values(ctx, val_local_dev, nnz_local, max_eig_iter, (unsigned long long)seed, dropped_out,
+                            dropped_cap);
+}
+
+int saena_b200_update_values_times(const saena_b200_ctx *ctx, double *ms_out, int cap) {
+    if (!ctx || !ms_out) return 1;
+    for (int i = 0; i < cap && i < 5; ++i) ms_out[i] = ctx->update_ms[i];
+    return 0;
+}
+
 // compute side only (apply_mode 1: no pack, no flags, no exchange; ghost values as they lie) of one
 // operator, through the fused kernel (fused != 0) or the separate interior + boundary kernels.  The one
 // timing hook a detached context (saena_b200_init_detached) supports; also valid on a live one.
@@ -1331,3 +1369,17 @@ int64_t saena_b200_operator_bytes(const saena_b200_ctx *ctx, int level, int kind
 }
 
 }  // extern "C"
+
+// After the operators' values changed (saena_b200_update_values): a level stays on the route only while R A P of the
+// level above still matches its stored operator to the probe's tolerance.
+int sb_recheck_routes(saena_b200_ctx *ctx) {
+    for (int l = 1; l < (int)ctx->levels.size(); ++l) {
+        DevLevel &lv = ctx->levels[l];
+        if (!lv.route) continue;
+        double rel = 0.0;
+        SB_TRY(route_probe(ctx, l, &rel));
+        if (!(rel <= ROUTE_PROBE_TOL)) lv.route = false;
+    }
+    route_release_if_unused(ctx);
+    return 0;
+}

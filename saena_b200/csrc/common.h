@@ -309,6 +309,9 @@ struct saena_b200_ctx {
     // L2 flush buffer for the timing loops
     void *flush_buf = nullptr;
     size_t flush_bytes = 0;
+
+    // host-clock ms of the last saena_b200_update_values, by phase (refresh.cu: UPDATE_PHASES)
+    double update_ms[5] = {0.0, 0.0, 0.0, 0.0, 0.0};
 };
 
 // scalar slots
@@ -343,6 +346,8 @@ void sb_choose_mapping(saena_b200_ctx *ctx, DevOperator &op);
 int sb_prepare_operator(saena_b200_ctx *ctx, DevOperator &op);
 void sb_drop_unused_layouts(DevOperator &op);
 void sb_sellp_layout(int M, const int64_t *rowptr, int *perm, long long *slice_ptr);
+// (re)writes the entries of an existing sliced layout of op from its CSR arrays (slice offsets and perm in place)
+int sb_fill_sliced(saena_b200_ctx *ctx, const DevOperator &op, SlicedLayout &s);
 // w-style application of an operator with a fused epilogue; x is the local input vector.
 int sb_apply(saena_b200_ctx *ctx, DevOperator &op, const double *x, int epi, const EpiArgs &args);
 int64_t sb_operator_bytes(const DevOperator &op);
@@ -377,6 +382,15 @@ int sb_check_fault(saena_b200_ctx *ctx);                   // non-zero (and ctx-
 // collective end of a solver call: all ranks return the same status (one all-reduce of the fault flags), so no rank
 // leaves the sequence of collective calls while the others go on
 int sb_agree_fault(saena_b200_ctx *ctx);
+// the coarsest level's dense factor from its global COO (host LU + inverse, kept on the device); n in 1..4096
+int sb_coarsest_factor(saena_b200_ctx *ctx, int n, int64_t nnz, const int32_t *row, const int32_t *col, const double *val);
+// probes every level on the route again and takes off the route each one whose stored A_l no longer matches R A P
+int sb_recheck_routes(saena_b200_ctx *ctx);
+
+// ---- refresh.cu
+// saena_b200_update_values on values already on the device (checks first, then writes)
+int sb_update_values(saena_b200_ctx *ctx, const double *val_dev, int64_t nnz, int max_eig_iter, unsigned long long seed,
+                     double *dropped_out, int dropped_cap);
 
 // ---- fused_restrict.cu
 int sb_residual_restrict_fused(saena_b200_ctx *ctx, int l, const double *u, const double *rhs, double *res_coarse);

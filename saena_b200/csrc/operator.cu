@@ -478,15 +478,13 @@ __global__ void sliced_fill_kernel(int n_slots, int M, const int *__restrict__ p
     }
 }
 
-// fills s from the operator's CSR arrays: sp = element offsets of the 32-slot slices, perm = slot -> row or nullptr
-static int build_sliced(saena_b200_ctx *ctx, DevOperator &op, SlicedLayout &s, const std::vector<long long> &sp,
-                        const std::vector<int> *perm) {
-    const int n_slots = (int)(sp.size() - 1) * 32;
-    const int64_t padded = sp.back();
-    SB_TRY(dev_upload(ctx, &s.ptr, sp.data(), sp.size()));
-    if (perm) SB_TRY(dev_upload(ctx, &s.perm, perm->data(), perm->size()));
-    SB_CUDA(cudaMalloc((void **)&s.col, sizeof(int) * std::max<int64_t>(padded, 1)));
-    SB_CUDA(cudaMalloc((void **)&s.val, sizeof(double) * std::max<int64_t>(padded, 1)));
+constexpr int SELLP_WINDOW = 256;  // = the CTA size of spmv_sellp_kernel (mapping 101, below)
+
+// The entries of an existing layout from the operator's CSR arrays: at build time, and again when the values change
+// on the same pattern (saena_b200_update_values).  One slot per row, rounded up to whole slices (32 rows) in row
+// order, to whole SELLP_WINDOW-row windows over a permutation.
+int sb_fill_sliced(saena_b200_ctx *ctx, const DevOperator &op, SlicedLayout &s) {
+    const int n_slots = s.perm ? (op.M + SELLP_WINDOW - 1) / SELLP_WINDOW * SELLP_WINDOW : (op.M + 31) / 32 * 32;
     if (n_slots) {
         const int blocks = (n_slots + 255) / 256;
         if (op.wide_offsets)
@@ -499,6 +497,18 @@ static int build_sliced(saena_b200_ctx *ctx, DevOperator &op, SlicedLayout &s, c
     SB_CUDA(cudaGetLastError());
     SB_CUDA(cudaStreamSynchronize(ctx->stream));
     return 0;
+}
+
+// allocates s and fills it from the operator's CSR arrays: sp = element offsets of the 32-slot slices, perm = slot ->
+// row or nullptr
+static int build_sliced(saena_b200_ctx *ctx, DevOperator &op, SlicedLayout &s, const std::vector<long long> &sp,
+                        const std::vector<int> *perm) {
+    const int64_t padded = sp.back();
+    SB_TRY(dev_upload(ctx, &s.ptr, sp.data(), sp.size()));
+    if (perm) SB_TRY(dev_upload(ctx, &s.perm, perm->data(), perm->size()));
+    SB_CUDA(cudaMalloc((void **)&s.col, sizeof(int) * std::max<int64_t>(padded, 1)));
+    SB_CUDA(cudaMalloc((void **)&s.val, sizeof(double) * std::max<int64_t>(padded, 1)));
+    return sb_fill_sliced(ctx, op, s);
 }
 
 // the slice lengths come from the row offsets on the device: the row offsets of a device-generated band operator
@@ -537,8 +547,6 @@ static int build_sell(saena_b200_ctx *ctx, DevOperator &op) {
 // sorted sliced layout (mapping 101): rows sorted by length, longest first, inside windows of SELLP_WINDOW
 // consecutive rows; the permutation is made on the host from the row offsets, the entries are moved on the device
 // ---------------------------------------------------------------------------------------------
-constexpr int SELLP_WINDOW = 256;  // = the CTA size of spmv_sellp_kernel
-
 // host only: slot -> row (rows of each SELLP_WINDOW-row window sorted by length, longest first, stable; -1 where the
 // last window runs past M) and the element offset of every 32-slot slice (its longest row's length x 32).
 // perm[ceil(M / 256) * 256], slice_ptr[ceil(M / 256) * 8 + 1].

@@ -74,6 +74,9 @@ def load_library(path: Optional[str] = None):
     L.saena_b200_p2p_import.argtypes = [vp, vp, ctypes.c_int64]
     L.saena_b200_find_eig.argtypes = [vp, i, i, vp, ctypes.c_uint64, i, ctypes.POINTER(ctypes.c_double),
                                       ctypes.POINTER(ctypes.c_int)]
+    L.saena_b200_update_values.argtypes = [vp, vp, ctypes.c_int64, i, ctypes.c_uint64, dp, i]
+    L.saena_b200_update_values_dev.argtypes = [vp, vp, ctypes.c_int64, i, ctypes.c_uint64, dp, i]
+    L.saena_b200_update_values_times.argtypes = [vp, dp, i]
     L.saena_b200_p2p_enable.argtypes = [vp, i]
     L.saena_b200_fault_status.argtypes = [vp]
     L.saena_b200_clear_fault.argtypes = [vp]
@@ -125,7 +128,7 @@ EXPORTED_SYMBOLS = [
     "saena_b200_upload_operator", "saena_b200_upload_band_operator", "saena_b200_upload_level_aux", "saena_b200_upload_level_scale",
     "saena_b200_upload_coarsest",
     "saena_b200_set_coarsest_solver", "saena_b200_set_operator_dense", "saena_b200_sellp_layout", "saena_b200_set_graphs", "saena_b200_finalize",
-    "saena_b200_p2p_export", "saena_b200_p2p_import", "saena_b200_find_eig", "saena_b200_p2p_enable", "saena_b200_fault_status", "saena_b200_clear_fault", "saena_b200_set_timeouts", "saena_b200_autotune_halo", "saena_b200_halo_choice", "saena_b200_solve_pcg", "saena_b200_solve_vcycle", "saena_b200_solve_smoother", "saena_b200_solve_cg",
+    "saena_b200_p2p_export", "saena_b200_p2p_import", "saena_b200_find_eig", "saena_b200_update_values", "saena_b200_update_values_dev", "saena_b200_update_values_times", "saena_b200_p2p_enable", "saena_b200_fault_status", "saena_b200_clear_fault", "saena_b200_set_timeouts", "saena_b200_autotune_halo", "saena_b200_halo_choice", "saena_b200_solve_pcg", "saena_b200_solve_vcycle", "saena_b200_solve_smoother", "saena_b200_solve_cg",
     "saena_b200_solve_pcg_dev", "saena_b200_matvec", "saena_b200_residual", "saena_b200_smooth",
     "saena_b200_vcycle", "saena_b200_coarsest_solve", "saena_b200_dot", "saena_b200_time_matvec",
     "saena_b200_time_smooth_sweep", "saena_b200_time_matvec_parts", "saena_b200_time_vcycle", "saena_b200_timer_start", "saena_b200_timer_stop", "saena_b200_launch_count", "saena_b200_graph_replays", "saena_b200_set_mapping", "saena_b200_set_fused_restrict", "saena_b200_spgemm_symbolic", "saena_b200_spgemm_numeric", "saena_b200_time_residual_restrict", "saena_b200_autotune_mapping", "saena_b200_set_mapping_deferred", "saena_b200_get_mapping",
@@ -365,6 +368,35 @@ class Context:
         self._ck(self._L.saena_b200_find_eig(self._h, level, int(max_iter), _vp(arr), int(seed), int(store),
                                              ctypes.byref(eig), ctypes.byref(it)))
         return eig.value, it.value
+
+    def update_values(self, val_local, max_eig_iter: int = 20, seed: int = 0) -> np.ndarray:
+        """New values for level 0's A on its uploaded pattern (saena_b200_update_values): val_local in the uploaded
+        order (row-major, the nnzPerRow_local / col_local given at upload), a numpy array or a CUDA torch tensor (float64,
+        contiguous; it goes to the device-pointer entry).  Every coarse level is recomputed as R A P on its stored
+        pattern, with inv_diag, the Chebyshev bounds (find_eig with max_eig_iter and seed), the sliced layouts and the
+        coarsest factor.  Returns, per level, the share ||C - C|pattern||_F / ||C||_F of R A P lumped into the
+        diagonal (entry 0 is 0).  `self.hier` keeps the uploaded host arrays: it does not follow the update."""
+        out = np.zeros(len(self.level_rows), F64)
+        if hasattr(val_local, "is_cuda") and val_local.is_cuda:
+            import torch
+            if val_local.dtype != torch.float64 or not val_local.is_contiguous():
+                raise ValueError("update_values: a device tensor must be contiguous float64")
+            with torch.cuda.device(val_local.device):
+                torch.cuda.current_stream().synchronize()   # the values are complete before the library reads them
+            self._ck(self._L.saena_b200_update_values_dev(self._h, ctypes.c_void_p(val_local.data_ptr()),
+                                                          int(val_local.numel()), int(max_eig_iter), int(seed),
+                                                          _f64p(out), len(out)))
+        else:
+            v = np.ascontiguousarray(val_local, F64)
+            self._ck(self._L.saena_b200_update_values(self._h, _vp(v), len(v), int(max_eig_iter), int(seed), _f64p(out),
+                                                      len(out)))
+        return out
+
+    def update_values_times(self) -> dict:
+        """host-clock ms of the last update_values, by phase"""
+        ms = np.zeros(5, F64)
+        self._ck(self._L.saena_b200_update_values_times(self._h, _f64p(ms), 5))
+        return dict(zip(("products", "pattern_map", "layouts", "eig", "coarsest"), ms.tolist()))
 
     def set_graphs(self, on: bool):
         self._ck(self._L.saena_b200_set_graphs(self._h, int(on)))
