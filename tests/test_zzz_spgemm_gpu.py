@@ -1,11 +1,17 @@
-"""The device SpGEMM of the Galerkin product (csrc/spgemm.cu, SURVEY 8f #3) against scipy on shapes that hit every
-accumulator (per-warp / per-CTA hash tables, dense accumulators in shared and in global memory, the bitmask symbolic
-passes), and the hierarchy it builds against the REFERENCE's own coarse operators: the golden files hold A_l, P_l, R_l
-of every level as saena_object::setup left them (Ac = R A P through the reference's matmat + MKL product shim), and
-where oracle/_ref travelled, the live reference at 32^3."""
+"""The device SpGEMM of the Galerkin product (csrc/spgemm.cu, SURVEY 8f #3) against an exact reference, and the
+hierarchy it builds against the REFERENCE's own coarse operators: the golden files hold A_l, P_l, R_l of every level as
+saena_object::setup left them (Ac = R A P through the reference's matmat + MKL product shim), and where oracle/_ref
+travelled, the live reference at 32^3.
+
+The products are checked by one checker against tests/spgemm_cases.py's reference: pattern and row offsets exactly,
+values bit for bit where the operands make every sum exact, else within the per-entry rounding bound.  The cases
+there reach every bin of both passes at and across its edges, hash tables whose probes wrap around, CTAs of the
+grid-stride kernels that handle more than one row, thousands of scan blocks, degenerate shapes and entries that cancel
+to exactly 0; each case's claim is re-checked against the SM count and shared memory of the card that runs it."""
 import numpy as np
 import pytest
 
+from tests import spgemm_cases
 from tests.util import GOLDEN, Golden
 
 pytestmark = pytest.mark.gpu
@@ -31,7 +37,36 @@ def _device_product(A, B):
     return rp.cpu().numpy(), col.cpu().numpy(), val.cpu().numpy()
 
 
-# (rows of A, inner size, columns of B, nnz per row of A, nnz per row of B): what each case is there for
+def _first(mask, rp):
+    i = int(np.argmax(mask))
+    return f"first at entry {i} (row {int(np.searchsorted(rp, i, side='right')) - 1})"
+
+
+def _check_product(A, B):
+    """C = A B on the device: row offsets, nnz and columns equal the structural reference, columns strictly ascend in
+    each row, a second call gives the same structure bit for bit, and values equal the reference bit for bit where the
+    operands make every sum exact (spgemm_cases.values_are_exact), else lie within its per-entry bound"""
+    ref = spgemm_cases.reference(A, B)
+    rp, col, val = _device_product(A, B)
+    bad_rows = np.flatnonzero(np.diff(rp) != np.diff(ref.indptr)) if len(rp) == len(ref.indptr) else []
+    assert np.array_equal(rp, ref.indptr), f"row offsets differ: {len(bad_rows)} rows with a wrong count, first {bad_rows[:5]}"
+    assert len(col) == len(val) == rp[-1], "nnz differs from rowptr[M]"
+    first_of_row = np.zeros(len(col), bool)
+    first_of_row[rp[:-1][rp[:-1] < len(col)]] = True
+    assert np.all(np.diff(col)[~first_of_row[1:]] > 0), "columns do not strictly ascend inside a row"
+    assert np.array_equal(col, ref.indices), "columns differ: " + _first(col != ref.indices, rp)
+    rp2, col2, _ = _device_product(A, B)
+    assert np.array_equal(rp2, rp) and np.array_equal(col2, col), "a second call gives another structure"
+    got = val.astype(np.longdouble)
+    if spgemm_cases.values_are_exact(A, B, ref.count):
+        wrong = got != ref.value
+        assert not wrong.any(), f"{int(wrong.sum())} values differ from the exact reference, " + _first(wrong, rp)
+    else:
+        wrong = np.abs(got - ref.value) > ref.bound
+        assert not wrong.any(), f"{int(wrong.sum())} values outside (k + 1) 2^-53 (|A||B|)_ij, " + _first(wrong, rp)
+
+
+# (rows of A, inner size, columns of B, nnz per row of A, nnz per row of B): random values in [-1, 1]
 CASES = [
     (3000, 2500, 4000, (0, 1, 3, 7), (0, 2, 5)),                  # empty rows, tiny rows: the 32-entry warp tables
     (1200, 900, 5000, (5, 9, 14), (6, 9, 12)),                    # <= 128 / <= 512 entries: the larger warp tables
@@ -48,14 +83,17 @@ def test_device_spgemm_matches_scipy(m, k, n, a_nnz, b_nnz):
     rng = np.random.default_rng(m + k + n)
     A = _rand_csr(rng, m, k, rng.choice(a_nnz, m))
     B = _rand_csr(rng, k, n, rng.choice(b_nnz, k))
-    rp, col, val = _device_product(A, B)
-    C = (A @ B).tocsr()
-    C.sort_indices()
-    # scipy drops nothing structurally in csr @ csr either: same pattern (exact cancellation has probability 0 here)
-    assert np.array_equal(rp, C.indptr.astype(np.int64)), "row offsets differ"
-    assert np.array_equal(col, C.indices.astype(np.int32)), "columns differ (or are not ascending inside a row)"
-    scale = np.max(np.abs(C.data)) if C.nnz else 1.0
-    assert np.max(np.abs(val - C.data)) <= 1e-13 * scale if C.nnz else True
+    _check_product(A, B)
+
+
+@pytest.mark.parametrize("name", spgemm_cases.NAMES)
+def test_device_spgemm_at_every_dispatch_edge(name):
+    import torch
+    case = spgemm_cases.build(name)
+    props = torch.cuda.get_device_properties(0)
+    unmet = spgemm_cases.unmet_claims(case, props.multi_processor_count, props.shared_memory_per_block_optin)
+    assert unmet == [], f"on {props.name} the case does not cover what it claims: {unmet}"
+    _check_product(case.A, case.B)
 
 
 def _same_operator(a, b, tol=1e-13):
