@@ -1060,8 +1060,9 @@ static int autotune_route(saena_b200_ctx *ctx, int reps, double min_gain) {
 // Collective on several ranks: every rank walks the same operators and the same candidates (derived from the
 // all-reduced maximum of the ranks' starting points), every timed application of an operator with a halo is an
 // exchange all ranks take part in, and the decision is taken on the slowest rank's median time (all-reduce MAX) --
-// one mapping per operator on all ranks.  Sliced operators (mapping 100) stay: where the rule picks the sliced
-// layout it measured fastest on every shape tried (profiles/r01_mapping_sweep.md).
+// one mapping per operator on all ranks.  Sliced operators (mapping 100) keep a sliced layout: where the rule picks it,
+// it measured fastest on every shape tried (profiles/r01_mapping_sweep.md); on one rank they are timed against the
+// sorted sliced layout (101).
 // changed_out (optional): number of operators whose mapping changed on this rank.  On one rank the level route is
 // chosen afterwards, on the settled mappings (autotune_route).
 // ---------------------------------------------------------------------------------------------
@@ -1081,6 +1082,29 @@ int saena_b200_autotune_mapping(saena_b200_ctx *ctx, int reps, double min_gain, 
             const bool mine = op->present && op->M > 0 && op->nnz_local + op->nnz_remote > 0;
             const int cur = mine ? op->mapping : 0;
             const bool has_halo = mine && (!op->sends.empty() || !op->recvs.empty() || op->nnz_remote > 0 || op->merged);
+            // ---- one rank, sliced, no halo: the same layout over rows sorted by length (101) against it.  One lane
+            //      sums a row in column order in both (same result, bit for bit); the sorted layout streams less
+            //      padding where the rows of a 32-row slice differ in length (the 267-entry rows of level 2 of the
+            //      256^3 hierarchy), at the price of a permutation and a pass through shared memory.
+            if (!multi && mine && cur == SB_MAPPING_SELL && !op->sell_only && !has_halo) {
+                SB_TRY(stage_buf(ctx, 0, op->n_local_cols));
+                SB_TRY(stage_buf(ctx, 1, op->M));
+                SB_CUDA(cudaMemsetAsync(ctx->stage[0], 0, sizeof(double) * op->n_local_cols, ctx->stream));
+                const bool flush = sb_operator_bytes(*op) < (int64_t)300e6;
+                const int cands[2] = {SB_MAPPING_SELL, SB_MAPPING_SELLP};
+                float t[2] = {0.f, 0.f};
+                for (int k = 0; k < 2; ++k) {
+                    op->forced_mapping = cands[k];
+                    SB_TRY(sb_prepare_operator(ctx, *op));
+                    SB_TRY(time_apply_median(ctx, op, reps, flush, &t[k]));
+                }
+                op->forced_mapping = t[1] < (1.0 - min_gain) * t[0] ? SB_MAPPING_SELLP : SB_MAPPING_SELL;
+                SB_TRY(sb_prepare_operator(ctx, *op));
+                SB_CUDA(cudaStreamSynchronize(ctx->stream));
+                sb_drop_unused_layouts(*op);
+                if (op->mapping != cur) ++changed;
+                continue;
+            }
             // ---- agree: [largest threads-per-row starting point, somebody is sliced / streaming / pinned]
             double agree[2] = {(cur >= 1 && cur <= 256) ? (double)cur : 0.0,
                                (mine && (cur <= 0 || cur == SB_MAPPING_SELL || cur == SB_MAPPING_SELLP || op->sell_only)) ? 1.0 : 0.0};

@@ -84,7 +84,7 @@ struct FusedArgs {
 template <int MAP, int EPI, typename XS>
 __device__ __forceinline__ void fused_rows(int vb, int lo, int hi, const FusedArgs &a, const XS xs) {
     if constexpr (MAP == SB_MAPPING_SELL)
-        spmv_sell_body<EPI>(vb, lo, hi, a.sell_ptr, a.sell_col, a.sell_val, xs, a.e, nullptr);
+        spmv_sell_body<EPI, XS, 4>(vb, lo, hi, a.sell_ptr, a.sell_col, a.sell_val, xs, a.e, nullptr);
     else if constexpr (MAP >= 32)
         spmv_rowgroup_body<MAP, EPI, int>(vb, lo, hi, a.rowptr, a.col, a.val, xs, a.e, nullptr);
     else

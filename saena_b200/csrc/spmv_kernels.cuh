@@ -24,6 +24,9 @@
 
 #include "common.h"
 
+// Every input of row i is read before the first store: the pointers are not restrict-qualified, so a load written after
+// a store is issued only once the values the store depends on have arrived -- a second memory round trip per thread.
+// (No caller passes u_in aliasing d_out; out may be u_in, d_out may be d_in: same element, read first either way.)
 template <int EPI>
 __device__ __forceinline__ void sb_epilogue(int i, double ax, const EpiArgs &e) {
     if (EPI == EPI_PLAIN) {
@@ -31,14 +34,16 @@ __device__ __forceinline__ void sb_epilogue(int i, double ax, const EpiArgs &e) 
     } else if (EPI == EPI_RESIDUAL) {
         e.out[i] = ax - e.rhs[i];
     } else if (EPI == EPI_CHEB_FIRST) {
+        const double u = e.u_in[i];
         const double d = e.c1 * e.inv_diag[i] * (e.rhs[i] - ax);
         e.d_out[i] = d;
-        e.out[i] = e.u_in[i] + d;
+        e.out[i] = u + d;
     } else if (EPI == EPI_CHEB_NEXT) {
+        const double u = e.u_in[i];
         const double res = e.c2 * e.inv_diag[i] * (e.rhs[i] - ax);
         const double d = (e.c1 * e.d_in[i]) + res;
         e.d_out[i] = d;
-        e.out[i] = e.u_in[i] + d;
+        e.out[i] = u + d;
     } else if (EPI == EPI_JACOBI) {
         const double t = (ax - e.rhs[i]) * (e.inv_diag[i] * e.c1);
         e.out[i] = e.u_in[i] - t;
@@ -297,7 +302,34 @@ spmv_stream_kernel(int M, const OffT *__restrict__ rowptr, const int *__restrict
 // stencil the x gather is coalesced too (neighbour j of 32 consecutive rows = 32 consecutive x).
 // No shuffles, no shared memory; the epilogue streams are coalesced by construction.
 // ---------------------------------------------------------------------------------------------
-template <int EPI, typename XS>
+// One lane's row of a slice of `len` entries (cp, vp: the lane's first entry), summed in column order.  Each trip
+// covers DEPTH entries, its loads predicated on the slice's length -- the same for all 32 lanes, so nothing diverges.
+// A short row (7 entries on the 7-point level, 6-8 on its prolongator's slices) is one trip with its loads
+// overlapped, where a 4-deep trip followed by one dependent col -> x chain per remaining entry waited on memory once
+// per entry (256^3 Poisson on a B200: level-0 SpMV 0.292 -> 0.259 ms, profiles/r04_sliced_depth.md).
+constexpr int SELL_UNROLL = 8;
+
+template <int DEPTH, typename XS>
+__device__ __forceinline__ double sb_sliced_row_sum(const int *cp, const double *vp, int len, const XS &xs) {
+    double sum = 0.0;
+    for (int j = 0; j < len; j += DEPTH) {
+        int c[DEPTH];
+        double a[DEPTH];
+#pragma unroll
+        for (int q = 0; q < DEPTH; ++q) {
+            const bool in = j + q < len;
+            c[q] = in ? sb_ld_stream(cp + (j + q) * 32) : 0;
+            a[q] = in ? sb_ld_stream(vp + (j + q) * 32) : 0.0;
+        }
+#pragma unroll
+        for (int q = 0; q < DEPTH; ++q)
+            if (j + q < len) sum += a[q] * xs.ld(c[q]);
+    }
+    return sum;
+}
+
+// DEPTH: SELL_UNROLL, or 4 in the fused halo kernel, which runs 8 CTAs an SM (32 registers) and would spill at 8
+template <int EPI, typename XS, int DEPTH = SELL_UNROLL>
 __device__ __forceinline__ void
 spmv_sell_body(int vb, int row_begin, int M, const long long *__restrict__ slice_ptr, const int *__restrict__ col,
                const double *__restrict__ val, const XS xs, const EpiArgs &e,
@@ -308,22 +340,7 @@ spmv_sell_body(int vb, int row_begin, int M, const long long *__restrict__ slice
     if ((slice << 5) >= M) return;
     const long long base = slice_ptr[slice];
     const int len = (int)((slice_ptr[slice + 1] - base) >> 5);
-    const int *cp = col + base + lane;
-    const double *vp = val + base + lane;
-    double sum = 0.0;
-    int j = 0;
-    for (; j + 4 <= len; j += 4) {
-        int c[4];
-        double a[4];
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-            c[q] = sb_ld_stream(cp + (j + q) * 32);
-            a[q] = sb_ld_stream(vp + (j + q) * 32);
-        }
-#pragma unroll
-        for (int q = 0; q < 4; ++q) sum += a[q] * xs.ld(c[q]);
-    }
-    for (; j < len; ++j) sum += sb_ld_stream(vp + j * 32) * xs.ld(sb_ld_stream(cp + j * 32));
+    const double sum = sb_sliced_row_sum<DEPTH>(col + base + lane, val + base + lane, len, xs);
     if (row < M && !sb_row_skipped(skip_mask, row)) sb_epilogue<EPI>(row, sum, e);
 }
 
@@ -353,22 +370,7 @@ spmv_sellp_body(int vb, int M, const long long *__restrict__ slice_ptr, const in
     const int slice = slot >> 5;
     const long long base = slice_ptr[slice];
     const int len = (int)((slice_ptr[slice + 1] - base) >> 5);
-    const int *cp = col + base + lane;
-    const double *vp = val + base + lane;
-    double sum = 0.0;
-    int j = 0;
-    for (; j + 4 <= len; j += 4) {
-        int c[4];
-        double a[4];
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-            c[q] = sb_ld_stream(cp + (j + q) * 32);
-            a[q] = sb_ld_stream(vp + (j + q) * 32);
-        }
-#pragma unroll
-        for (int q = 0; q < 4; ++q) sum += a[q] * xs.ld(c[q]);
-    }
-    for (; j < len; ++j) sum += sb_ld_stream(vp + j * 32) * xs.ld(sb_ld_stream(cp + j * 32));
+    const double sum = sb_sliced_row_sum<SELL_UNROLL>(col + base + lane, val + base + lane, len, xs);
     // back to row order through shared memory: the window's rows are the 256 consecutive rows from vb * 256, each in
     // exactly one slot, so thread t finishes row vb * 256 + t and the epilogue's vector streams stay coalesced
     const int wbase = vb * 256;
