@@ -324,7 +324,11 @@ int64_t saena_b200_launch_count(const saena_b200_ctx *ctx);
  * per thread group; -1..-32 = streaming row blocks with that many lanes per row in the reduce
  * phase; 100 = sliced layout (32-row slices, column-major, one lane per row); 101 = the sliced
  * layout over rows sorted by length inside 256-row windows (irregular rows: the slices' padding all
- * but disappears; operators without a halo only, otherwise the heuristic's choice is kept). */
+ * but disappears; operators without a halo only, otherwise the heuristic's choice is kept); 103 = symmetric
+ * diagonals (an exactly symmetric square operator on at most 32 diagonals, one rank, no halo: diagonal 0 and the
+ * positive offsets as dense arrays, no column ids; the heuristic picks it for such an operator with at most 4 stored
+ * diagonals and at least the sliced layout's row count; on an operator that is not eligible the heuristic's choice is
+ * kept). */
 int saena_b200_set_mapping(saena_b200_ctx *ctx, int level, int kind, int mapping);
 /* The same, taking effect at the next saena_b200_finalize (no layout is built for the mapping that
  * is being replaced: matters for an operator that fills half the HBM). */
@@ -334,6 +338,14 @@ int saena_b200_set_mapping_deferred(saena_b200_ctx *ctx, int level, int kind, in
  * stable; -1 where the last window runs past M) and slice_ptr[ceil(M / 256) * 8 + 1], the element offset of every
  * 32-slot slice (32 x its longest row). */
 int saena_b200_sellp_layout(int M, const int64_t *rowptr, int32_t *perm, long long *slice_ptr);
+/* Host only: the rule behind mapping 103 (symmetric diagonals).  For an operator of M rows and nnz entries whose
+ * distinct offsets col - row are offsets[n_offsets] and whose sliced layout would store padded_est entries: the number
+ * of stored diagonals, written to stored[] (offset 0, then the positive offsets ascending; at most 16), or 0 when the
+ * layout does not apply -- more than 32 offsets, an offset without its mirror, more than 16 stored diagonals, or
+ * 8 * stored * M > 0.75 * 12 * padded_est bytes.  -1 on bad arguments.  (The device build also requires the values to
+ * be exactly symmetric and the columns of every row to ascend.) */
+int saena_b200_symdiag_plan(int M, int n_offsets, const int32_t *offsets, int64_t nnz, int64_t padded_est,
+                            int32_t *stored);
 /* Setup-time choice of every operator's row mapping by measurement: starting from the nnz/row rule, times the
  * neighbouring mappings (1/8 .. 8x the threads per row; the sorted sliced layout where it applies) with `reps`
  * applications each and keeps the fastest where it wins by more than min_gain (e.g. 0.03).  Collective on several

@@ -1085,20 +1085,27 @@ int saena_b200_autotune_mapping(saena_b200_ctx *ctx, int reps, double min_gain, 
             // ---- one rank, sliced, no halo: the same layout over rows sorted by length (101) against it.  One lane
             //      sums a row in column order in both (same result, bit for bit); the sorted layout streams less
             //      padding where the rows of a 32-row slice differ in length (the 267-entry rows of level 2 of the
-            //      256^3 hierarchy), at the price of a permutation and a pass through shared memory.
-            if (!multi && mine && cur == SB_MAPPING_SELL && !op->sell_only && !has_halo) {
+            //      256^3 hierarchy), at the price of a permutation and a pass through shared memory.  An eligible symmetric
+            //      operator (the rule put it on 103) is timed on the symmetric diagonals against both.
+            if (!multi && mine && (cur == SB_MAPPING_SELL || cur == SB_MAPPING_SYMDIAG) && !op->sell_only && !has_halo) {
                 SB_TRY(stage_buf(ctx, 0, op->n_local_cols));
                 SB_TRY(stage_buf(ctx, 1, op->M));
                 SB_CUDA(cudaMemsetAsync(ctx->stage[0], 0, sizeof(double) * op->n_local_cols, ctx->stream));
                 const bool flush = sb_operator_bytes(*op) < (int64_t)300e6;
-                const int cands[2] = {SB_MAPPING_SELL, SB_MAPPING_SELLP};
-                float t[2] = {0.f, 0.f};
-                for (int k = 0; k < 2; ++k) {
+                // the symmetric diagonals (103) where the operator is eligible; the rule's choice is the base
+                std::vector<int> cands = {SB_MAPPING_SELL, SB_MAPPING_SELLP};
+                if (op->sdiag_n > 0) cands.push_back(SB_MAPPING_SYMDIAG);
+                std::vector<float> t(cands.size(), 0.f);
+                size_t best = 0, base = 0;
+                for (size_t k = 0; k < cands.size(); ++k) {
                     op->forced_mapping = cands[k];
                     SB_TRY(sb_prepare_operator(ctx, *op));
                     SB_TRY(time_apply_median(ctx, op, reps, flush, &t[k]));
+                    if (cands[k] == cur) base = k;
+                    if (t[k] < t[best]) best = k;
                 }
-                op->forced_mapping = t[1] < (1.0 - min_gain) * t[0] ? SB_MAPPING_SELLP : SB_MAPPING_SELL;
+                if (!(t[best] < (1.0 - min_gain) * t[base])) best = base;
+                op->forced_mapping = cands[best];
                 SB_TRY(sb_prepare_operator(ctx, *op));
                 SB_CUDA(cudaStreamSynchronize(ctx->stream));
                 sb_drop_unused_layouts(*op);
@@ -1107,7 +1114,7 @@ int saena_b200_autotune_mapping(saena_b200_ctx *ctx, int reps, double min_gain, 
             }
             // ---- agree: [largest threads-per-row starting point, somebody is sliced / streaming / pinned]
             double agree[2] = {(cur >= 1 && cur <= 256) ? (double)cur : 0.0,
-                               (mine && (cur <= 0 || cur == SB_MAPPING_SELL || cur == SB_MAPPING_SELLP || op->sell_only)) ? 1.0 : 0.0};
+                               (mine && (cur <= 0 || cur >= SB_MAPPING_SELL || op->sell_only)) ? 1.0 : 0.0};
             if (multi) {
                 SB_CUDA(cudaMemcpyAsync(ctx->tune_dev, agree, sizeof(agree), cudaMemcpyHostToDevice, ctx->stream));
                 SB_TRY(sb_allreduce_max(ctx, ctx->tune_dev, 2, ctx->stream));
@@ -1377,6 +1384,12 @@ int saena_b200_sellp_layout(int M, const int64_t *rowptr, int32_t *perm, long lo
     if (M < 0 || !rowptr || !perm || !slice_ptr) return 1;
     sb_sellp_layout(M, rowptr, perm, slice_ptr);
     return 0;
+}
+
+int saena_b200_symdiag_plan(int M, int n_offsets, const int32_t *offsets, int64_t nnz, int64_t padded_est,
+                            int32_t *stored) {
+    if (n_offsets < 0 || (n_offsets && !offsets) || !stored) return -1;
+    return sb_symdiag_plan(M, n_offsets, offsets, nnz, padded_est, stored);
 }
 
 int saena_b200_get_mapping(const saena_b200_ctx *ctx, int level, int kind) {

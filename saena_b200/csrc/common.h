@@ -101,6 +101,14 @@ struct SlicedLayout {
     double *val = nullptr;
 };
 
+// the stored diagonals of mapping 103: off[0] = 0, then the positive offsets ascending (kernel argument, by value)
+static const int SYMDIAG_MAX = 16;
+static const int SYMDIAG_RULE_MAX = 4;   // the most stored diagonals sb_choose_mapping picks mapping 103 for
+struct SymDiagOffsets {
+    int nd = 0;
+    int off[SYMDIAG_MAX] = {};
+};
+
 struct DevOperator {
     bool present = false;
     int kind = 0, level = 0;
@@ -132,6 +140,14 @@ struct DevOperator {
     // padding of irregular operators (unstructured matrices, smoothed prolongators) all but disappears.  Operators
     // without a halo only.  Never chosen by the heuristic: set_mapping / autotune.
     SlicedLayout sellp;
+
+    // symmetric diagonals (mapping 103): an exactly symmetric square operator whose entries lie on a few diagonals,
+    // stored as dense double[sdiag.nd][M] arrays of diagonal 0 and the positive offsets only -- no column ids.  Row i
+    // reads its lower entry a_{i,i-k} as d_k[i-k] (= a_{i-k,i}, same bits).  One rank, no halo, not merged.
+    // sdiag_n: -1 not probed yet, 0 not eligible, > 0 the stored diagonals (sdiag.off).  sdiag_val: null unless built.
+    SymDiagOffsets sdiag;
+    int sdiag_n = -1;
+    double *sdiag_val = nullptr;
 
     // remote block re-sorted by row at upload: boundary rows only
     // interior rows = the contiguous range [int_lo, int_hi) (multiples of 32) that holds no row with
@@ -323,6 +339,7 @@ enum { S_RHO_RES = 0, S_PDOTH = 1, S_RR = 2, S_BETA_NUM = 3, S_TMP = 4,
 
 static const int SB_MAPPING_SELL = 100;   // forced_mapping / set_mapping code of the sliced layout
 static const int SB_MAPPING_SELLP = 101;  // ... of the sliced layout with rows sorted by length inside 256-row windows
+static const int SB_MAPPING_SYMDIAG = 103;  // ... of the symmetric diagonals (DevOperator::sdiag)
 static const int STREAM_TILE = 2048;      // nnz per row block of the streaming kernel (16 KB of products)
 static const int STREAM_THREADS = 256;
 static const int RED_MAX_BLOCKS = 1184;   // 148 SMs x 8
@@ -348,6 +365,12 @@ void sb_drop_unused_layouts(DevOperator &op);
 void sb_sellp_layout(int M, const int64_t *rowptr, int *perm, long long *slice_ptr);
 // (re)writes the entries of an existing sliced layout of op from its CSR arrays (slice offsets and perm in place)
 int sb_fill_sliced(saena_b200_ctx *ctx, const DevOperator &op, SlicedLayout &s);
+// host only: the stored diagonals of mapping 103 for an operator of M rows, nnz entries, `padded_est` sliced entries
+// and these distinct offsets col - row; 0 when the layout does not apply (stored: SYMDIAG_MAX ints)
+int sb_symdiag_plan(int M, int n_offsets, const int *offsets, int64_t nnz, int64_t padded_est, int *stored);
+// after new values on the same pattern (saena_b200_update_values): an operator on mapping 103 gets its diagonals
+// filled again; when the new values are not symmetric it moves to the sliced layout
+int sb_refresh_symdiag(saena_b200_ctx *ctx, DevOperator &op);
 // w-style application of an operator with a fused epilogue; x is the local input vector.
 int sb_apply(saena_b200_ctx *ctx, DevOperator &op, const double *x, int epi, const EpiArgs &args);
 int64_t sb_operator_bytes(const DevOperator &op);

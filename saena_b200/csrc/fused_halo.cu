@@ -252,6 +252,7 @@ fused_halo_spmv_kernel(const __grid_constant__ FusedArgs a) {
 // streaming mapping) takes the separate launches, which speak the same hand-shake -- the choice is local.
 bool sb_fused_eligible(const DevOperator &op) {
     return op.p2p && op.fused && !op.wide_offsets && op.mapping > 0 && op.mapping != SB_MAPPING_SELLP &&
+           op.mapping != SB_MAPPING_SYMDIAG &&
            (!op.sends.empty() || !op.recvs.empty());
 }
 

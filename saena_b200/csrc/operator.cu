@@ -9,6 +9,7 @@
 //                   (no atomics in the remote kernel), column = index into the ghost buffer
 //   halo plan    -> vIndex + per-peer (offset,count) slices of the packed send / ghost buffers
 #include <algorithm>
+#include <climits>
 #include <numeric>
 
 #include "spmv_kernels.cuh"
@@ -84,6 +85,7 @@ void sb_free_operator(DevOperator &op) {
     // ghost_buf / x_ext belong to the context's halo arena
     free_sliced(op.sell);
     free_sliced(op.sellp);
+    cudaFree(op.sdiag_val);
     cudaFree(op.x_round);
     cudaFree(op.rowmid); cudaFree(op.partial);
     op = DevOperator();
@@ -388,6 +390,8 @@ void sb_choose_mapping(saena_b200_ctx *ctx, DevOperator &op) {
     // the sorted sliced layout permutes rows inside 256-row windows: no interior / boundary row ranges, so only for
     // operators without a halo (one rank, or a block that happens to have no remote part)
     if (m == SB_MAPPING_SELLP && (!op.sends.empty() || !op.recvs.empty() || op.merged || op.nnz_remote > 0)) m = 0;
+    // the symmetric diagonals only where sb_prepare_operator found the operator eligible
+    if (m == SB_MAPPING_SYMDIAG && op.sdiag_n <= 0) m = 0;
     if (m == 0) {
         // short and regular rows: sliced layout (padding <= 15 %); otherwise a sub-warp per row
         // with ~4+ elements per lane.  Crossovers measured on B200, see DESIGN.md.
@@ -398,7 +402,11 @@ void sb_choose_mapping(saena_b200_ctx *ctx, DevOperator &op) {
         //  profiles/r01_bench_levels.md)
         const bool regular = op.nnz_local > 0 && double(op.sell_padded_est) <= 1.20 * double(op.nnz_local);
         const bool enough_rows = op.M >= 2 * 2048 * ctx->sm_count / 4;  // 151 552 rows on B200
-        if (regular && enough_rows) m = SB_MAPPING_SELL;
+        // an eligible symmetric operator streams its stored diagonals (<= 0.75 of the sliced layout's bytes) instead;
+        // the rule takes it where it was measured, up to 4 stored diagonals (the 7-point stencil, 40 registers).  More
+        // diagonals (74-78 / 128 registers at 8 / 16) only through set_mapping or the mapping walk, which times them
+        if (op.sdiag_n > 0 && op.sdiag.nd <= SYMDIAG_RULE_MAX && enough_rows) m = SB_MAPPING_SYMDIAG;
+        else if (regular && enough_rows) m = SB_MAPPING_SELL;
         else {
             // ~4+ elements per lane; rows of hundreds..thousands of entries get 32..256 threads
             m = pow2_at_most((avg + 1.0) / 4.0, 256);
@@ -412,7 +420,7 @@ void sb_choose_mapping(saena_b200_ctx *ctx, DevOperator &op) {
         }
     }
     // the one place a code is made canonical: threads per row 1..256 and streaming lanes 1..32, powers of two
-    if (m == SB_MAPPING_SELL || m == SB_MAPPING_SELLP) op.mapping = m;
+    if (m == SB_MAPPING_SELL || m == SB_MAPPING_SELLP || m == SB_MAPPING_SYMDIAG) op.mapping = m;
     else if (m < 0) op.mapping = -pow2_at_most(-m, 32);
     else op.mapping = pow2_at_most(m, 256);
 }
@@ -579,15 +587,239 @@ static int build_sellp(saena_b200_ctx *ctx, DevOperator &op) {
     return build_sliced(ctx, op, op.sellp, sp, &perm);
 }
 
+// ---------------------------------------------------------------------------------------------
+// symmetric diagonals (mapping 103): eligibility from the distinct offsets col - row (one device pass, bounded table)
+// and a host rule; the diagonals filled from the CSR and checked for exact symmetry on the device
+// ---------------------------------------------------------------------------------------------
+constexpr int SD_TABLE = 32;           // distinct offsets collected before the operator is given up
+constexpr int SD_EMPTY = INT_MIN;      // free table slot (no offset of a square operator is INT_MIN)
+enum { SD_OVERFLOW = 1, SD_UNSORTED = 2, SD_ASYMMETRIC = 4 };
+
+// offset -> its slot in the table (inserted if new); false when the table is full
+__device__ __forceinline__ bool sd_insert(int *t, int off) {
+    for (int j = 0; j < SD_TABLE; ++j) {
+        int v = *(volatile int *)(t + j);
+        if (v == SD_EMPTY) v = atomicCAS(t + j, SD_EMPTY, off);
+        if (v == SD_EMPTY || v == off) return true;
+    }
+    return false;
+}
+
+// the distinct offsets of the operator into table[SD_TABLE] (per CTA in shared memory, then merged); flags: more than
+// SD_TABLE offsets, or a row whose columns do not strictly ascend (the kernel's sum order is the CSR's column order)
+template <typename OffT>
+__global__ void sd_offsets_kernel(int M, const OffT *__restrict__ rowptr, const int *__restrict__ col, int *table,
+                                  int *flags) {
+    __shared__ int s[SD_TABLE];
+    if (threadIdx.x < SD_TABLE) s[threadIdx.x] = SD_EMPTY;
+    __syncthreads();
+    int f = 0;
+    for (int row = blockIdx.x * blockDim.x + threadIdx.x; row < M; row += gridDim.x * blockDim.x) {
+        // more than SD_TABLE offsets anywhere: the operator is given up, nothing more to scan
+        if (*(volatile int *)flags & SD_OVERFLOW) break;
+        int prev = INT_MIN;
+        for (OffT k = rowptr[row]; k < rowptr[row + 1]; ++k) {
+            const int c = col[k];
+            if (c <= prev) f |= SD_UNSORTED;
+            prev = c;
+            if (!sd_insert(s, c - row)) {
+                atomicOr(flags, SD_OVERFLOW);
+                break;
+            }
+        }
+    }
+    if (f) atomicOr(flags, f);
+    __syncthreads();
+    if (threadIdx.x < SD_TABLE && s[threadIdx.x] != SD_EMPTY && !sd_insert(table, s[threadIdx.x])) atomicOr(flags, SD_OVERFLOW);
+}
+
+__device__ __forceinline__ int sd_index(const SymDiagOffsets &s, int k) {
+    for (int q = 0; q < s.nd; ++q)
+        if (s.off[q] == k) return q;
+    return -1;
+}
+
+// upper entries (col >= row) into d_q[row]: each slot written once (columns strictly ascend)
+template <typename OffT>
+__global__ void sd_fill_kernel(int M, const OffT *__restrict__ rowptr, const int *__restrict__ col,
+                               const double *__restrict__ val, const SymDiagOffsets s, double *__restrict__ d,
+                               int *flags) {
+    const int row = blockIdx.x * blockDim.x + threadIdx.x;
+    if (row >= M) return;
+    for (OffT k = rowptr[row]; k < rowptr[row + 1]; ++k) {
+        const int c = col[k];
+        if (c < row) continue;
+        const int q = sd_index(s, c - row);
+        if (q < 0) { atomicOr(flags, SD_ASYMMETRIC); continue; }
+        d[(size_t)q * (size_t)M + row] = val[k];
+    }
+}
+
+// every lower entry a_{row,c} (c < row): row c holds column `row`, and a_{row,c} has the bits of d_{row-c}[c] (that
+// entry); balance += lower - upper off-diagonal entries, 0 when the pattern is symmetric
+template <typename OffT>
+__global__ void sd_check_kernel(int M, const OffT *__restrict__ rowptr, const int *__restrict__ col,
+                                const double *__restrict__ val, const SymDiagOffsets s, const double *__restrict__ d,
+                                int *flags, unsigned long long *balance) {
+    const int row = blockIdx.x * blockDim.x + threadIdx.x;
+    long long bal = 0;
+    bool bad = false;
+    if (row < M) {
+        for (OffT k = rowptr[row]; k < rowptr[row + 1]; ++k) {
+            const int c = col[k];
+            if (c > row) --bal;
+            if (c >= row) continue;
+            ++bal;
+            const int q = sd_index(s, row - c);
+            OffT lo = rowptr[c], hi = rowptr[c + 1];   // row c's columns ascend: binary search for `row`
+            while (lo < hi) {
+                const OffT mid = lo + (hi - lo) / 2;
+                if (col[mid] < row) lo = mid + 1; else hi = mid;
+            }
+            if (q < 0 || lo == rowptr[c + 1] || col[lo] != row ||
+                __double_as_longlong(val[k]) != __double_as_longlong(d[(size_t)q * (size_t)M + c]))
+                bad = true;
+        }
+    }
+    if (bad) atomicOr(flags, SD_ASYMMETRIC);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) bal += __shfl_xor_sync(0xffffffffu, bal, o);
+    if ((threadIdx.x & 31) == 0 && bal) atomicAdd(balance, (unsigned long long)bal);
+}
+
+int sb_symdiag_plan(int M, int n_offsets, const int *offsets, int64_t nnz, int64_t padded_est, int *stored) {
+    if (M <= 0 || nnz <= 0 || n_offsets < 0 || n_offsets > SD_TABLE) return 0;
+    std::vector<int> off(offsets, offsets + n_offsets);
+    std::sort(off.begin(), off.end());
+    off.erase(std::unique(off.begin(), off.end()), off.end());
+    std::vector<int> pos;
+    for (int k : off) {
+        if (k <= -M || k >= M) return 0;
+        if (!std::binary_search(off.begin(), off.end(), -k)) return 0;   // every offset has its mirror
+        if (k > 0) pos.push_back(k);
+    }
+    const int nd = 1 + (int)pos.size();
+    if (nd > SYMDIAG_MAX) return 0;
+    // clearly fewer bytes than the sliced layout: values of the stored diagonals against values + column ids
+    if (8.0 * nd * (double)M > 0.75 * 12.0 * (double)padded_est) return 0;
+    stored[0] = 0;
+    std::copy(pos.begin(), pos.end(), stored + 1);
+    return nd;
+}
+
+// one rank, no halo, square, CSR entries kept
+static bool symdiag_candidate(const saena_b200_ctx *ctx, const DevOperator &op) {
+    return ctx->nranks == 1 && !op.merged && !op.sell_only && op.nnz_remote == 0 && op.sends.empty() &&
+           op.recvs.empty() && op.M > 0 && op.M == op.n_local_cols && op.nnz_local > 0 && op.col && op.val;
+}
+
+// op.sdiag_n from the operator's offsets and the host rule (pattern only; the values are checked at every fill)
+static int probe_symdiag(saena_b200_ctx *ctx, DevOperator &op) {
+    cudaFree(op.sdiag_val);   // filled from values that may have changed since
+    op.sdiag_val = nullptr;
+    op.sdiag_n = 0;
+    if (!symdiag_candidate(ctx, op)) return 0;
+    int *dev = nullptr;   // [SD_TABLE] offsets, [1] flags
+    SB_CUDA(cudaMalloc((void **)&dev, sizeof(int) * (SD_TABLE + 1)));
+    std::vector<int> h(SD_TABLE + 1, SD_EMPTY);
+    h[SD_TABLE] = 0;
+    SB_CUDA(cudaMemcpyAsync(dev, h.data(), sizeof(int) * h.size(), cudaMemcpyHostToDevice, ctx->stream));
+    const int blocks = std::min((op.M + 255) / 256, 8 * ctx->sm_count);
+    if (op.wide_offsets)
+        sd_offsets_kernel<int64_t><<<blocks, 256, 0, ctx->stream>>>(op.M, (const int64_t *)op.rowptr, op.col, dev, dev + SD_TABLE);
+    else
+        sd_offsets_kernel<int><<<blocks, 256, 0, ctx->stream>>>(op.M, (const int *)op.rowptr, op.col, dev, dev + SD_TABLE);
+    SB_CUDA(cudaGetLastError());
+    SB_CUDA(cudaMemcpyAsync(h.data(), dev, sizeof(int) * h.size(), cudaMemcpyDeviceToHost, ctx->stream));
+    SB_CUDA(cudaStreamSynchronize(ctx->stream));
+    cudaFree(dev);
+    if (h[SD_TABLE]) return 0;
+    std::vector<int> off;
+    for (int j = 0; j < SD_TABLE; ++j)
+        if (h[j] != SD_EMPTY) off.push_back(h[j]);
+    SymDiagOffsets s;
+    s.nd = sb_symdiag_plan(op.M, (int)off.size(), off.data(), op.nnz_local, op.sell_padded_est, s.off);
+    op.sdiag = s;
+    op.sdiag_n = s.nd;
+    return 0;
+}
+
+// The diagonals from the operator's CSR arrays, then the symmetry check: at build time, and again when the values
+// change on the same pattern (saena_b200_update_values).  *symmetric false: the values are not exactly symmetric.
+static int fill_symdiag(saena_b200_ctx *ctx, DevOperator &op, bool *symmetric) {
+    const int M = op.M, blocks = (M + 255) / 256;
+    const SymDiagOffsets &s = op.sdiag;
+    int *flags = nullptr;   // [0] flags, then (8-byte aligned) the balance
+    SB_CUDA(cudaMalloc((void **)&flags, 2 * sizeof(unsigned long long)));
+    unsigned long long *balance = (unsigned long long *)flags + 1;
+    SB_CUDA(cudaMemsetAsync(flags, 0, 2 * sizeof(unsigned long long), ctx->stream));
+    SB_CUDA(cudaMemsetAsync(op.sdiag_val, 0, sizeof(double) * (size_t)s.nd * (size_t)M, ctx->stream));
+    if (op.wide_offsets) {
+        const int64_t *rp = (const int64_t *)op.rowptr;
+        sd_fill_kernel<int64_t><<<blocks, 256, 0, ctx->stream>>>(M, rp, op.col, op.val, s, op.sdiag_val, flags);
+        sd_check_kernel<int64_t><<<blocks, 256, 0, ctx->stream>>>(M, rp, op.col, op.val, s, op.sdiag_val, flags, balance);
+    } else {
+        const int *rp = (const int *)op.rowptr;
+        sd_fill_kernel<int><<<blocks, 256, 0, ctx->stream>>>(M, rp, op.col, op.val, s, op.sdiag_val, flags);
+        sd_check_kernel<int><<<blocks, 256, 0, ctx->stream>>>(M, rp, op.col, op.val, s, op.sdiag_val, flags, balance);
+    }
+    SB_CUDA(cudaGetLastError());
+    unsigned long long h[2] = {0ull, 0ull};   // the int flags are the low half of h[0]
+    SB_CUDA(cudaMemcpyAsync(h, flags, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
+    SB_CUDA(cudaStreamSynchronize(ctx->stream));
+    cudaFree(flags);
+    *symmetric = h[0] == 0ull && h[1] == 0ull;
+    return 0;
+}
+
+// allocates and fills the diagonals; an operator whose values are not symmetric loses its eligibility (freed)
+static int build_symdiag(saena_b200_ctx *ctx, DevOperator &op, bool *ok) {
+    *ok = true;
+    if (op.sdiag_val) return 0;
+    SB_CUDA(cudaMalloc((void **)&op.sdiag_val, sizeof(double) * (size_t)op.sdiag.nd * (size_t)op.M));
+    SB_TRY(fill_symdiag(ctx, op, ok));
+    if (!*ok) {
+        cudaFree(op.sdiag_val);
+        op.sdiag_val = nullptr;
+        op.sdiag_n = 0;
+    }
+    return 0;
+}
+
+int sb_refresh_symdiag(saena_b200_ctx *ctx, DevOperator &op) {
+    if (op.mapping != SB_MAPPING_SYMDIAG) {
+        op.sdiag_n = -1;   // probed again (and a stale copy freed) the next time the operator is prepared
+        return 0;
+    }
+    bool ok = false;
+    SB_TRY(fill_symdiag(ctx, op, &ok));
+    if (ok) return 0;
+    cudaFree(op.sdiag_val);
+    op.sdiag_val = nullptr;
+    op.sdiag_n = 0;
+    op.forced_mapping = SB_MAPPING_SELL;
+    return sb_prepare_operator(ctx, op);
+}
+
 // copies of the entries in layouts the operator no longer uses (a mapping walk builds them to time them)
 void sb_drop_unused_layouts(DevOperator &op) {
     if (op.mapping != SB_MAPPING_SELLP) free_sliced(op.sellp);
     if (op.mapping != SB_MAPPING_SELL && !op.sell_only) free_sliced(op.sell);
+    if (op.mapping != SB_MAPPING_SYMDIAG) {
+        cudaFree(op.sdiag_val);
+        op.sdiag_val = nullptr;
+    }
 }
 
 int sb_prepare_operator(saena_b200_ctx *ctx, DevOperator &op) {
     if (!op.present) return 0;
+    if (op.sdiag_n < 0) SB_TRY(probe_symdiag(ctx, op));
     sb_choose_mapping(ctx, op);
+    if (op.mapping == SB_MAPPING_SYMDIAG) {
+        bool ok = false;
+        SB_TRY(build_symdiag(ctx, op, &ok));
+        if (!ok) sb_choose_mapping(ctx, op);   // not symmetric after all: the rule's choice (or the forced one)
+    }
     if (op.mapping < 0) SB_TRY(build_row_blocks(ctx, op, STREAM_THREADS / -op.mapping));
     if (op.mapping == SB_MAPPING_SELL) SB_TRY(build_sell(ctx, op));
     if (op.mapping == SB_MAPPING_SELLP) SB_TRY(build_sellp(ctx, op));
@@ -607,6 +839,15 @@ static int launch_local(saena_b200_ctx *ctx, DevOperator &op, const double *x, c
     const int nrows = hi - lo;
     if (nrows <= 0) return 0;
     ++ctx->launches;
+    if (op.mapping == SB_MAPPING_SYMDIAG) {
+        // whole operator (no halo): one thread per row
+        const int blocks = (op.M + 255) / 256;
+        const double *d = op.sdiag_val;
+        if (op.sdiag.nd <= 4) spmv_symdiag_kernel<4, EPI><<<blocks, 256, 0, s>>>(op.M, d, op.sdiag, x, e);
+        else if (op.sdiag.nd <= 8) spmv_symdiag_kernel<8, EPI><<<blocks, 256, 0, s>>>(op.M, d, op.sdiag, x, e);
+        else spmv_symdiag_kernel<SYMDIAG_MAX, EPI><<<blocks, 256, 0, s>>>(op.M, d, op.sdiag, x, e);
+        return 0;
+    }
     if (op.mapping == SB_MAPPING_SELLP) {
         // whole operator (no halo, see sb_choose_mapping): one CTA per 256-row window
         spmv_sellp_kernel<EPI><<<(op.M + 255) / 256, 256, 0, s>>>(op.M, op.sellp.ptr, op.sellp.perm, op.sellp.col,
@@ -766,8 +1007,10 @@ int sb_apply(saena_b200_ctx *ctx, DevOperator &op, const double *x, int epi, con
     SB_FAIL("apply: unknown epilogue");
 }
 
-// algorithmic bytes of w = Op v (SURVEY.md 8d): nnz*(8+4) + M*p (row offsets) + N*8 (x once) + M*8 (w)
+// algorithmic bytes of w = Op v (SURVEY.md 8d): nnz*(8+4) + M*p (row offsets) + N*8 (x once) + M*8 (w); on the
+// symmetric diagonals each stored diagonal once (its second, lagging read is expected from L2) + x + w
 int64_t sb_operator_bytes(const DevOperator &op) {
+    if (op.mapping == SB_MAPPING_SYMDIAG) return 8 * (int64_t)op.sdiag.nd * op.M + (int64_t)op.n_local_cols * 8 + (int64_t)op.M * 8;
     const int64_t p = op.wide_offsets ? 8 : 4;
     return (op.nnz_local + op.nnz_remote) * 12 + (int64_t)op.M * p + (int64_t)op.n_local_cols * 8 +
            (int64_t)op.M * 8;

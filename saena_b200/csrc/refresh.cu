@@ -339,9 +339,12 @@ int update_body(saena_b200_ctx *ctx, const double *val_dev, int64_t nnz, int max
     for (int l = 0; l + 1 < L; ++l) SB_TRY(refresh_level(ctx, l, flags_dev, norms_dev, &dropped[l + 1], ms));
     // the sliced copies of the entries (the eigenvalue estimate and the route probe apply the operators through them)
     auto t1 = clk::now();
+    // the symmetric diagonals are filled and checked again; an operator whose new values are not symmetric moves to the
+    // sliced layout here, before anything applies it
     for (DevLevel &lv : ctx->levels) {
         if (lv.A.sell.ptr) SB_TRY(sb_fill_sliced(ctx, lv.A, lv.A.sell));
         if (lv.A.sellp.ptr) SB_TRY(sb_fill_sliced(ctx, lv.A, lv.A.sellp));
+        SB_TRY(sb_refresh_symdiag(ctx, lv.A));
     }
     auto t2 = clk::now();
     for (int l = 0; l < L; ++l) {   // find_eig(store = 1) on every level

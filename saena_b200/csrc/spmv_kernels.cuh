@@ -10,6 +10,8 @@
 // Three row mappings, chosen per operator from nnz/row and row-length regularity (sb_choose_mapping):
 //   spmv_sell          32-row slices stored column-major (padded per slice): lane = row, every load
 //                      coalesced and independent.  Short regular rows (the 7-point level 0).
+//   spmv_symdiag<ND>   an exactly symmetric operator on a few diagonals: diagonal 0 and the positive
+//                      offsets as dense arrays, no column ids.  The 7-point level 0 on one rank.
 //   spmv_rowgroup<TPR> 32..256 threads per row: the deep coarse levels (thousands of nnz per row)
 //   spmv_vec<LANES>    LANES (1..16) lanes cooperate on a row, a warp owns 32 consecutive rows
 //                      and results are transposed so lane j finishes row j: the epilogue's
@@ -386,6 +388,50 @@ __global__ void __launch_bounds__(256)
 spmv_sellp_kernel(int M, const long long *__restrict__ slice_ptr, const int *__restrict__ perm,
                   const int *__restrict__ col, const double *__restrict__ val, const double *__restrict__ x, EpiArgs e) {
     spmv_sellp_body<EPI>(blockIdx.x, M, slice_ptr, perm, col, val, XLocal{x}, e);
+}
+
+// ---------------------------------------------------------------------------------------------
+// spmv_symdiag: symmetric diagonals (mapping 103), one thread per row.  d holds diagonal 0 and the positive offsets
+// k of an exactly symmetric operator as dense arrays d_q[M] (q = index of k in s.off); row i's lower entry a_{i,i-k} is
+// d_q[i-k].  Row i sums its terms in ascending column order -- lower terms for k descending, d_0[i] x[i], upper terms
+// for k ascending -- with the `sum += a * x` chain of sb_sliced_row_sum, so a row sum has the bits of the sliced and
+// CSR kernels (a slot the pattern leaves empty holds 0.0 and adds a zero).  Terms outside [0, M) are skipped.
+// Loads: d_q[i] is the first touch of its line and stays cached in L2 (.cg) until d_q[i-k], k rows later, reads it
+// again as the last use (.cs, evict first).  ND: the kernel's bucket (4, 8, 16 diagonals), s.nd <= ND of them stored.
+// ---------------------------------------------------------------------------------------------
+template <int ND, int EPI>
+__global__ void __launch_bounds__(256)
+spmv_symdiag_kernel(int M, const double *__restrict__ d, const SymDiagOffsets s, const double *__restrict__ x,
+                    EpiArgs e) {
+    const int i = blockIdx.x * 256 + threadIdx.x;
+    if (i >= M) return;
+    const size_t m = (size_t)M;
+    // every load of the row in flight before the first use
+    double la[ND], lx[ND], ua[ND], ux[ND];
+    // (in the reverse of the order the terms are summed: the first multiply-add needs the last load issued, so the
+    // compiler has no partial sum to start before every load is in flight)
+#pragma unroll
+    for (int q = ND - 1; q >= 1; --q) {
+        const bool up = q < s.nd && i < M - s.off[q];
+        ua[q] = up ? __ldcg(d + q * m + i) : 0.0;
+        ux[q] = up ? __ldg(x + (i + s.off[q])) : 0.0;
+    }
+    const double a0 = __ldcg(d + i), x0 = __ldg(x + i);
+#pragma unroll
+    for (int q = 1; q < ND; ++q) {
+        const bool lo = q < s.nd && i >= s.off[q];
+        la[q] = lo ? __ldcs(d + q * m + (i - s.off[q])) : 0.0;
+        lx[q] = lo ? __ldg(x + (i - s.off[q])) : 0.0;
+    }
+    // a skipped term is 0.0 * 0.0: adding +0 leaves a non-zero sum as it is, and keeps the chain free of branches
+    // (with a branch per term the compiler issues the upper loads only after the lower terms are summed)
+    double sum = 0.0;
+#pragma unroll
+    for (int q = ND - 1; q >= 1; --q) sum += la[q] * lx[q];
+    sum += a0 * x0;
+#pragma unroll
+    for (int q = 1; q < ND; ++q) sum += ua[q] * ux[q];
+    sb_epilogue<EPI>(i, sum, e);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -68,6 +68,7 @@ def load_library(path: Optional[str] = None):
     L.saena_b200_set_coarsest_solver.argtypes = [vp, i]
     L.saena_b200_set_operator_dense.argtypes = [vp, i, i, i]
     L.saena_b200_sellp_layout.argtypes = [i, vp, vp, vp]
+    L.saena_b200_symdiag_plan.argtypes = [i, i, vp, ctypes.c_int64, ctypes.c_int64, vp]
     L.saena_b200_set_graphs.argtypes = [vp, i]
     L.saena_b200_finalize.argtypes = [vp]
     L.saena_b200_p2p_export.argtypes = [vp, vp, ctypes.c_int64, ctypes.POINTER(ctypes.c_int64)]
@@ -127,7 +128,7 @@ EXPORTED_SYMBOLS = [
     "saena_b200_nccl_unique_id", "saena_b200_init", "saena_b200_init_detached", "saena_b200_time_matvec_compute_only", "saena_b200_destroy", "saena_b200_last_error",
     "saena_b200_upload_operator", "saena_b200_upload_band_operator", "saena_b200_upload_level_aux", "saena_b200_upload_level_scale",
     "saena_b200_upload_coarsest",
-    "saena_b200_set_coarsest_solver", "saena_b200_set_operator_dense", "saena_b200_sellp_layout", "saena_b200_set_graphs", "saena_b200_finalize",
+    "saena_b200_set_coarsest_solver", "saena_b200_set_operator_dense", "saena_b200_sellp_layout", "saena_b200_symdiag_plan", "saena_b200_set_graphs", "saena_b200_finalize",
     "saena_b200_p2p_export", "saena_b200_p2p_import", "saena_b200_find_eig", "saena_b200_update_values", "saena_b200_update_values_dev", "saena_b200_update_values_times", "saena_b200_p2p_enable", "saena_b200_fault_status", "saena_b200_clear_fault", "saena_b200_set_timeouts", "saena_b200_autotune_halo", "saena_b200_halo_choice", "saena_b200_solve_pcg", "saena_b200_solve_vcycle", "saena_b200_solve_smoother", "saena_b200_solve_cg",
     "saena_b200_solve_pcg_dev", "saena_b200_matvec", "saena_b200_residual", "saena_b200_smooth",
     "saena_b200_vcycle", "saena_b200_coarsest_solve", "saena_b200_dot", "saena_b200_time_matvec",
@@ -181,6 +182,18 @@ def sellp_layout(rowptr: np.ndarray):
     if L.saena_b200_sellp_layout(M, _vp(rp), _vp(perm), _vp(sp)):
         raise RuntimeError("saena_b200_sellp_layout failed")
     return perm[:n_slots], sp
+
+
+def symdiag_plan(M: int, offsets, nnz: int, padded_est: int):
+    """host-only rule of mapping 103 (saena_b200_symdiag_plan): the stored diagonals (0, then the positive offsets
+    ascending) for an operator with these distinct offsets col - row, or None where the layout does not apply"""
+    off = np.ascontiguousarray(offsets, I32)
+    stored = np.zeros(16, I32)
+    L = load_library()
+    nd = L.saena_b200_symdiag_plan(int(M), len(off), _vp(off), int(nnz), int(padded_est), _vp(stored))
+    if nd < 0:
+        raise RuntimeError("saena_b200_symdiag_plan: bad arguments")
+    return stored[:nd].tolist() if nd else None
 
 
 def spgemm_csr(M: int, K: int, N: int, a_rowptr, a_col, a_val, b_rowptr, b_col, b_val):
@@ -531,7 +544,8 @@ class Context:
 
     def set_mapping(self, level, kind, mapping: int):
         """mapping > 0: that many lanes per row (sub-warp mapping); < 0: streaming row blocks with
-        -mapping lanes per row in the reduce phase; 0: heuristic from nnz/row."""
+        -mapping lanes per row in the reduce phase; 100 / 101: the sliced layouts; 103: symmetric diagonals (where
+        the operator is eligible, else the heuristic's choice); 0: heuristic from nnz/row."""
         self._ck(self._L.saena_b200_set_mapping(self._h, level, kind, int(mapping)))
 
     def get_mapping(self, level, kind) -> int:

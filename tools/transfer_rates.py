@@ -27,7 +27,7 @@ from saena_b200 import native  # noqa: E402
 from saena_b200.hierarchy import KIND_A, KIND_P, KIND_R  # noqa: E402
 from saena_b200.sa_setup import build_device_hierarchy, poisson3d_coo  # noqa: E402
 
-SELL, SELLP = 100, 101
+SELL, SELLP, SYMDIAG = 100, 101, 103
 REPS = 20
 L2_BYTES = 300e6   # below this an operator's stream could stay in the 126 MB L2 between launches: flush
 
@@ -37,6 +37,8 @@ def mapping_name(m: int) -> str:
         return "sliced"
     if m == SELLP:
         return "sorted sliced"
+    if m == SYMDIAG:
+        return "symmetric diagonals"
     if m < 0:
         return f"stream/{-m}"
     return f"{m} lanes/row" if m < 32 else f"{m} thr/row"
