@@ -283,6 +283,32 @@ int saena_b200_vcycle(saena_b200_ctx *ctx, int level, int smoother, int pre, int
 int saena_b200_coarsest_solve(saena_b200_ctx *ctx, const double *rhs, double *u);
 int saena_b200_dot(saena_b200_ctx *ctx, const double *a, const double *b, int n, double *out);
 
+/* ---- block solve: 1 <= k <= 8 right-hand sides on one hierarchy, one rank --------------------------------------------
+ * Every vector argument is a block of k ordinary vectors back to back (column-major): column j starts at
+ * base + j * ld, ld = the level's rows (grids[0].A->M for the solve), or the operator's local columns for an operator's
+ * input.  Each operator is streamed once for all k columns.  Column j gives exactly -- to the bit -- what the single
+ * call gives for column j: for the solve the same iteration count, residual history and u; columns are independent (a
+ * zero or NaN column changes no other column).  Every call returns non-zero, and leaves the hierarchy as it was, for
+ * k outside 1..8, a context of several ranks (a detached share included) or one not finalized.  The work vectors for k
+ * columns (about 2 x the single solve's per column) are allocated at the first call with a larger k than before; an
+ * allocation that fails returns non-zero and the context stays usable for single solves. */
+/* saena_b200_solve_pcg on k columns: iters[k], hist[k * hist_cap] (column j's history at hist + j * hist_cap),
+ * hist_len[k] */
+int saena_b200_solve_pcg_block(saena_b200_ctx *ctx, int k, const double *rhs, double *u, int max_iter, double tol,
+                               int smoother, int pre, int post, int *iters, double *hist, int hist_cap,
+                               int *hist_len);
+/* the same with rhs / u in device memory */
+int saena_b200_solve_pcg_block_dev(saena_b200_ctx *ctx, int k, const double *rhs_dev, double *u_dev, int max_iter,
+                                   double tol, int smoother, int pre, int post, int *iters, double *hist,
+                                   int hist_cap, int *hist_len);
+/* saena_b200_matvec / _residual / _smooth / _vcycle on k columns */
+int saena_b200_matvec_block(saena_b200_ctx *ctx, int level, int kind, int k, const double *v, double *w);
+int saena_b200_residual_block(saena_b200_ctx *ctx, int level, int k, const double *u, const double *rhs, double *res);
+int saena_b200_smooth_block(saena_b200_ctx *ctx, int level, int smoother, int iters, int k, double *u,
+                            const double *rhs);
+int saena_b200_vcycle_block(saena_b200_ctx *ctx, int level, int smoother, int pre, int post, int k, double *u,
+                            const double *rhs);
+
 /* ---- measurement ---------------------------------------------------------------------------
  * Device-resident timing loops for bench.py: `reps` applications of one operator / smoother
  * sweep, each launch bracketed by CUDA events on the launching stream; returns the median

@@ -124,6 +124,7 @@ int saena_b200_destroy(saena_b200_ctx *ctx) {
     cudaFree(ctx->flush_buf);
     cudaFree(ctx->tune_dev);
     cudaFree(ctx->route_t); cudaFree(ctx->route_s);
+    sb_block_free(ctx);
     sb_nccl_destroy(ctx);
     cudaEventDestroy(ctx->ev_packed); cudaEventDestroy(ctx->ev_halo);
     cudaEventDestroy(ctx->ev_t0); cudaEventDestroy(ctx->ev_t1);
@@ -288,6 +289,89 @@ static int route_alloc(saena_b200_ctx *ctx, int n) {
     return 0;
 }
 
+}  // extern "C"
+
+// ---------------------------------------------------------------------------------------------
+// block solve buffers
+// ---------------------------------------------------------------------------------------------
+static void drop_block_graphs(saena_b200_ctx *ctx) {
+    for (size_t i = 0; i < ctx->graphs.size(); ++i)
+        if (ctx->graphs[i].k) {
+            if (ctx->graphs[i].exec) cudaGraphExecDestroy(ctx->graphs[i].exec);
+            ctx->graphs.erase(ctx->graphs.begin() + i);
+            --i;
+        }
+}
+
+void sb_block_free(saena_b200_ctx *ctx) {
+    drop_block_graphs(ctx);
+    for (DevLevel &lv : ctx->levels) {
+        cudaFree(lv.bu[0]); cudaFree(lv.bu[1]); cudaFree(lv.bd); cudaFree(lv.bres); cudaFree(lv.brhs);
+        cudaFree(lv.bxfer_old);
+        lv.bu[0] = lv.bu[1] = lv.bd = lv.bres = lv.brhs = lv.bxfer_old = nullptr;
+        lv.bcur = 0;
+    }
+    double **vecs[] = {&ctx->blk_r, &ctx->blk_p, &ctx->blk_h, &ctx->blk_u, &ctx->blk_rhs, &ctx->blk_route_t,
+                       &ctx->blk_route_s, &ctx->blk_partials, &ctx->blk_scal};
+    for (double **v : vecs) { cudaFree(*v); *v = nullptr; }
+    cudaFree(ctx->blk_counter); ctx->blk_counter = nullptr;
+    cudaFree(ctx->blk_active); ctx->blk_active = nullptr;
+    cudaFreeHost(ctx->blk_scal_host); ctx->blk_scal_host = nullptr;
+    cudaFreeHost(ctx->blk_active_host); ctx->blk_active_host = nullptr;
+    ctx->blk_cap = 0;
+    ctx->blk_route_cap = 0;
+}
+
+int sb_block_reserve(saena_b200_ctx *ctx, int k) {
+    size_t route_rows = 0;   // the largest fine level under a level on the route
+    for (size_t l = 1; l < ctx->levels.size(); ++l)
+        if (ctx->levels[l].route) route_rows = std::max(route_rows, (size_t)ctx->levels[l - 1].M);
+    if (k <= ctx->blk_cap && route_rows * ctx->blk_cap <= ctx->blk_route_cap) return 0;
+    const int cap = std::max(k, ctx->blk_cap);
+    sb_block_free(ctx);   // also drops every block graph: they point into the buffers being replaced
+    const int L = (int)ctx->levels.size();
+    bool ok = true;
+    auto grab = [&](double **p, size_t n) {
+        if (!ok) return;
+        ok = cudaMalloc((void **)p, sizeof(double) * std::max<size_t>(n, 1)) == cudaSuccess &&
+             cudaMemsetAsync(*p, 0, sizeof(double) * std::max<size_t>(n, 1), ctx->stream) == cudaSuccess;
+    };
+    for (int l = 0; l < L; ++l) {
+        DevLevel &lv = ctx->levels[l];
+        const size_t n = (size_t)cap * lv.M;
+        grab(&lv.bu[0], n);
+        grab(&lv.bu[1], n);
+        grab(&lv.bd, n);
+        grab(&lv.bres, n);
+        if (l > 0) grab(&lv.brhs, n);
+        if (l < L - 1 && !lv.repart.identity()) grab(&lv.bxfer_old, (size_t)cap * lv.M_coarse_old);
+    }
+    const size_t n0 = (size_t)cap * ctx->levels[0].M;
+    for (double **v : {&ctx->blk_r, &ctx->blk_p, &ctx->blk_h, &ctx->blk_u, &ctx->blk_rhs}) grab(v, n0);
+    if (route_rows) {
+        grab(&ctx->blk_route_t, route_rows * cap);
+        grab(&ctx->blk_route_s, route_rows * cap);
+    }
+    grab(&ctx->blk_partials, (size_t)SB_BLOCK_MAX * RED_MAX_BLOCKS);
+    grab(&ctx->blk_scal, (size_t)S_COUNT * SB_BLOCK_MAX);
+    ok = ok && cudaMalloc((void **)&ctx->blk_counter, sizeof(unsigned int) * SB_BLOCK_MAX) == cudaSuccess &&
+         cudaMemsetAsync(ctx->blk_counter, 0, sizeof(unsigned int) * SB_BLOCK_MAX, ctx->stream) == cudaSuccess;
+    ok = ok && cudaMalloc((void **)&ctx->blk_active, sizeof(int) * SB_BLOCK_MAX) == cudaSuccess;
+    ok = ok && cudaMallocHost((void **)&ctx->blk_scal_host, sizeof(double) * S_COUNT * SB_BLOCK_MAX) == cudaSuccess;
+    ok = ok && cudaMallocHost((void **)&ctx->blk_active_host, sizeof(int) * SB_BLOCK_MAX) == cudaSuccess;
+    if (!ok) {
+        cudaGetLastError();   // an out-of-memory status is not sticky: clear it, the single path is unaffected
+        sb_block_free(ctx);
+        SB_FAIL("block solve: not enough device memory for the work vectors of " + std::to_string(cap) +
+                " right-hand sides");
+    }
+    ctx->blk_cap = cap;
+    ctx->blk_route_cap = route_rows * cap;
+    return 0;
+}
+
+extern "C" {
+
 int saena_b200_finalize(saena_b200_ctx *ctx) {
     if (!ctx) return 1;
     SB_CUDA(cudaSetDevice(ctx->device));
@@ -301,6 +385,7 @@ int saena_b200_finalize(saena_b200_ctx *ctx) {
         lv.route_ms[0] = lv.route_ms[1] = 0.f;
     }
     route_free(ctx);
+    sb_block_free(ctx);
     SB_TRY(sb_arena_build(ctx));  // ghost buffers of every operator, one allocation (p2p_halo.cu)
     for (int l = 0; l < L; ++l) {
         DevLevel &lv = ctx->levels[l];
@@ -788,6 +873,175 @@ int saena_b200_dot(saena_b200_ctx *ctx, const double *a, const double *b, int n,
     SB_TRY(sb_read_scalars(ctx));
     *out = ctx->scalars_host[S_TMP];
     return sb_check_fault(ctx);
+}
+
+// ---------------------------------------------------------------------------------------------
+// block solve: k <= SB_BLOCK_MAX right-hand sides on one hierarchy, every operator streamed once for all of them.
+// Column j gives what saena_b200_solve_pcg gives for right-hand side j: each column has its own alpha, beta, init_dot
+// and stop test, and once it has stopped its u, r and p are left as they are (the PCG updates skip it) while the
+// others go on; it still rides through the V-cycle and the SpMV, whose results it never reads.
+// ---------------------------------------------------------------------------------------------
+static int block_enter(saena_b200_ctx *ctx, int k) {
+    if (k < 1 || k > SB_BLOCK_MAX) SB_FAIL("block call: k must be in 1..8");
+    if (ctx->nranks > 1) SB_FAIL("block call: one rank only (the halo exchange has no block form)");
+    return sb_block_reserve(ctx, k);
+}
+
+#define SB_ENTER_BLOCK(k)                                                 \
+    SB_ENTER();                                                           \
+    SB_TRY(block_enter(ctx, k))
+
+static int upload_active(saena_b200_ctx *ctx, int k) {
+    SB_CUDA(cudaMemcpyAsync(ctx->blk_active, ctx->blk_active_host, sizeof(int) * k, cudaMemcpyHostToDevice,
+                            ctx->stream));
+    return 0;
+}
+
+static int pcg_block_device(saena_b200_ctx *ctx, int k, const double *rhs, double *u, int max_iter, double tol,
+                            int smoother, int pre, int post, int *iters, double *hist, int hist_cap, int *hist_len) {
+    DevLevel &l0 = ctx->levels[0];
+    const int n = l0.M;
+    const long long ld = n;
+    if (ctx->levels.size() == 1) {
+        // direct solver only (pcg_device :2507-2521): nothing to share, one column after the other
+        for (int j = 0; j < k; ++j)
+            SB_TRY(pcg_device(ctx, rhs + j * ld, u + j * ld, max_iter, tol, smoother, pre, post, iters + j,
+                              hist ? hist + (long long)j * hist_cap : nullptr, hist_cap, hist_len + j));
+        return 0;
+    }
+    double *r = ctx->blk_r, *p = ctx->blk_p, *h = ctx->blk_h;
+    const double *sc = ctx->blk_scal_host;
+    auto rr_of = [&](int j) { return sc[S_RR * SB_BLOCK_MAX + j]; };
+    auto push = [&](int j, double v) { push_hist(v, hist ? hist + (long long)j * hist_cap : nullptr, hist_cap, hist_len[j]); };
+    double thr[SB_BLOCK_MAX];
+    int *active = ctx->blk_active_host;
+    SB_TRY(sb_fill_zero(ctx, u, (size_t)k * n));
+    SB_TRY(sb_negate_copy_block(ctx, n, k, rhs, r));
+    SB_TRY(sb_dot_block(ctx, r, r, n, k, S_RR));
+    SB_TRY(sb_read_block_scalars(ctx));
+    for (int j = 0; j < k; ++j) {
+        hist_len[j] = 0;
+        iters[j] = max_iter;   // a column that never stops ends at max_iter (pcg_device :2673-2682)
+        active[j] = 1;
+        thr[j] = rr_of(j) * tol * tol;
+        push(j, rr_of(j));
+    }
+    SB_TRY(upload_active(ctx, k));
+    double *rho = nullptr;
+    SB_TRY(sb_vcycle_block_from_zero(ctx, k, smoother, pre, post, r));
+    rho = l0.bu[l0.bcur];
+    if (n) SB_CUDA(cudaMemcpyAsync(p, rho, sizeof(double) * k * ld, cudaMemcpyDeviceToDevice, ctx->stream));
+    SB_TRY(sb_dot_block(ctx, r, rho, n, k, S_RHO_RES));
+    int n_active = k;
+    for (int i = 0; i < max_iter && n_active; i++) {
+        EpiArgs e{};
+        e.out = h;
+        SB_TRY(sb_apply_block(ctx, l0.A, k, p, EPI_PLAIN, e));
+        SB_TRY(sb_dot_block(ctx, p, h, n, k, S_PDOTH));
+        SB_TRY(sb_pcg_update_block(ctx, n, k, u, r, p, h));
+        SB_TRY(sb_read_block_scalars(ctx));
+        bool changed = false;
+        for (int j = 0; j < k; ++j) {
+            if (!active[j]) continue;
+            push(j, rr_of(j));
+            if (!(rr_of(j) >= thr[j])) {   // NaN also stops
+                active[j] = 0;
+                iters[j] = i + 1;
+                --n_active;
+                changed = true;
+            }
+        }
+        if (!n_active) break;
+        if (changed) SB_TRY(upload_active(ctx, k));
+        SB_TRY(sb_vcycle_block_from_zero(ctx, k, smoother, pre, post, r));
+        rho = l0.bu[l0.bcur];
+        SB_TRY(sb_dot_block(ctx, r, rho, n, k, S_BETA_NUM));
+        SB_TRY(sb_pcg_p_update_block(ctx, n, k, p, rho));
+    }
+    if (ctx->scale) SB_TRY(sb_scale_vector_block(ctx, n, k, u, l0.inv_sq_diag));
+    return 0;
+}
+
+int saena_b200_solve_pcg_block_dev(saena_b200_ctx *ctx, int k, const double *rhs_dev, double *u_dev, int max_iter,
+                                   double tol, int smoother, int pre, int post, int *iters, double *hist,
+                                   int hist_cap, int *hist_len) {
+    SB_ENTER_BLOCK(k);
+    if (!iters || !hist_len || !rhs_dev || !u_dev) SB_FAIL("solve_pcg_block: null argument");
+    SB_TRY(pcg_block_device(ctx, k, rhs_dev, u_dev, max_iter, tol, smoother, pre, post, iters, hist, hist_cap,
+                            hist_len));
+    SB_TRY(sb_sync_stream(ctx, ctx->stream));
+    return sb_agree_fault(ctx);
+}
+
+int saena_b200_solve_pcg_block(saena_b200_ctx *ctx, int k, const double *rhs, double *u, int max_iter, double tol,
+                               int smoother, int pre, int post, int *iters, double *hist, int hist_cap,
+                               int *hist_len) {
+    SB_ENTER_BLOCK(k);
+    if (!iters || !hist_len || !rhs || !u) SB_FAIL("solve_pcg_block: null argument");
+    const size_t n = (size_t)k * ctx->levels[0].M;
+    SB_TRY(h2d(ctx, ctx->blk_rhs, rhs, n));
+    SB_TRY(pcg_block_device(ctx, k, ctx->blk_rhs, ctx->blk_u, max_iter, tol, smoother, pre, post, iters, hist,
+                            hist_cap, hist_len));
+    SB_TRY(sb_agree_fault(ctx));
+    return d2h(ctx, u, ctx->blk_u, n);
+}
+
+int saena_b200_matvec_block(saena_b200_ctx *ctx, int level, int kind, int k, const double *v, double *w) {
+    SB_ENTER_BLOCK(k);
+    DevOperator *op = get_op(ctx, level, kind);
+    if (!op) SB_FAIL("matvec_block: no such operator");
+    const size_t nx = (size_t)k * op->n_local_cols, nw = (size_t)k * op->M;
+    SB_TRY(stage_buf(ctx, 0, nx));
+    SB_TRY(stage_buf(ctx, 1, nw));
+    SB_TRY(h2d(ctx, ctx->stage[0], v, nx));
+    EpiArgs e{};
+    e.out = ctx->stage[1];
+    if (kind == SAENA_B200_KIND_A) SB_TRY(sb_apply_level_A_block(ctx, level, k, ctx->stage[0], EPI_PLAIN, e));
+    else SB_TRY(sb_apply_block(ctx, *op, k, ctx->stage[0], EPI_PLAIN, e));
+    return d2h(ctx, w, ctx->stage[1], nw);
+}
+
+int saena_b200_residual_block(saena_b200_ctx *ctx, int level, int k, const double *u, const double *rhs, double *res) {
+    SB_ENTER_BLOCK(k);
+    DevOperator *op = get_op(ctx, level, SAENA_B200_KIND_A);
+    if (!op) SB_FAIL("residual_block: no such level");
+    const size_t n = (size_t)k * op->M;
+    for (int i = 0; i < 3; ++i) SB_TRY(stage_buf(ctx, i, n));
+    SB_TRY(h2d(ctx, ctx->stage[0], u, n));
+    SB_TRY(h2d(ctx, ctx->stage[1], rhs, n));
+    EpiArgs e{};
+    e.rhs = ctx->stage[1];
+    e.out = ctx->stage[2];
+    SB_TRY(sb_apply_level_A_block(ctx, level, k, ctx->stage[0], EPI_RESIDUAL, e));
+    return d2h(ctx, res, ctx->stage[2], n);
+}
+
+int saena_b200_smooth_block(saena_b200_ctx *ctx, int level, int smoother, int iters, int k, double *u,
+                            const double *rhs) {
+    SB_ENTER_BLOCK(k);
+    if (level < 0 || level >= (int)ctx->levels.size()) SB_FAIL("smooth_block: no such level");
+    DevLevel &lv = ctx->levels[level];
+    const size_t n = (size_t)k * lv.M;
+    SB_TRY(stage_buf(ctx, 1, n));
+    lv.bcur = 0;
+    SB_TRY(h2d(ctx, lv.bu[0], u, n));
+    SB_TRY(h2d(ctx, ctx->stage[1], rhs, n));
+    SB_TRY(sb_smooth_block(ctx, level, k, smoother, iters, ctx->stage[1], false));
+    return d2h(ctx, u, lv.bu[lv.bcur], n);
+}
+
+int saena_b200_vcycle_block(saena_b200_ctx *ctx, int level, int smoother, int pre, int post, int k, double *u,
+                            const double *rhs) {
+    SB_ENTER_BLOCK(k);
+    if (level < 0 || level >= (int)ctx->levels.size()) SB_FAIL("vcycle_block: no such level");
+    DevLevel &lv = ctx->levels[level];
+    const size_t n = (size_t)k * lv.M;
+    SB_TRY(stage_buf(ctx, 1, n));
+    lv.bcur = 0;
+    SB_TRY(h2d(ctx, lv.bu[0], u, n));
+    SB_TRY(h2d(ctx, ctx->stage[1], rhs, n));
+    SB_TRY(sb_vcycle_block(ctx, level, k, smoother, pre, post, ctx->stage[1], false));
+    return d2h(ctx, u, lv.bu[lv.bcur], n);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -231,6 +231,12 @@ struct DevLevel {
     double *res = nullptr;       // residual (Grid::res)
     double *rhs = nullptr;       // this level's right-hand side (parent's res_coarse after repart); level 0: external
     double *xfer_old = nullptr;  // coarse vector in the old partition (Ac.M_old), used when repart is not identity
+
+    // the same work vectors for a block of up to ctx->blk_cap columns, column-major (column j at + j * M, xfer_old's
+    // at + j * M_coarse_old); allocated by sb_block_reserve on the first block call, bcur is their ping-pong parity
+    double *bu[2] = {nullptr, nullptr};
+    int bcur = 0;
+    double *bd = nullptr, *bres = nullptr, *brhs = nullptr, *bxfer_old = nullptr;
 };
 
 // A V-cycle from a zero iterate is the same launch sequence every time (same buffers, same
@@ -242,6 +248,7 @@ struct VcycleGraph {
     cudaGraphExec_t exec;
     int64_t launches;
     std::vector<int> cur_after;  // each level's ping-pong parity when the V-cycle ends
+    int k = 0;                   // 0: the single V-cycle; 1..SB_BLOCK_MAX: the block V-cycle on k columns
     // exec == nullptr: a multi-rank configuration that has run eagerly once and is captured at its next use
 };
 
@@ -328,6 +335,20 @@ struct saena_b200_ctx {
 
     // host-clock ms of the last saena_b200_update_values, by phase (refresh.cu: UPDATE_PHASES)
     double update_ms[5] = {0.0, 0.0, 0.0, 0.0, 0.0};
+
+    // block solve (sb_block_reserve): work vectors for up to blk_cap columns -- the levels' (DevLevel::bu ...), the
+    // PCG's and the route's -- and reduction state of its own: per column a row of RED_MAX_BLOCKS partials and a
+    // counter, and the scalars as blk_scal[slot * SB_BLOCK_MAX + column] (slots as ctx->scalars', S_COUNT of them)
+    int blk_cap = 0;
+    size_t blk_route_cap = 0;  // elements of each route intermediate (columns x the routed fine level's rows)
+    double *blk_r = nullptr, *blk_p = nullptr, *blk_h = nullptr, *blk_u = nullptr, *blk_rhs = nullptr;
+    double *blk_route_t = nullptr, *blk_route_s = nullptr;
+    double *blk_partials = nullptr;   // [SB_BLOCK_MAX * RED_MAX_BLOCKS]
+    unsigned int *blk_counter = nullptr;  // [SB_BLOCK_MAX]
+    double *blk_scal = nullptr;       // [S_COUNT * SB_BLOCK_MAX]
+    double *blk_scal_host = nullptr;  // pinned mirror
+    int *blk_active = nullptr;        // [SB_BLOCK_MAX] 1: the column still iterates (the PCG updates skip the others)
+    int *blk_active_host = nullptr;   // pinned mirror
 };
 
 // scalar slots
@@ -343,6 +364,7 @@ static const int SB_MAPPING_SYMDIAG = 103;  // ... of the symmetric diagonals (D
 static const int STREAM_TILE = 2048;      // nnz per row block of the streaming kernel (16 KB of products)
 static const int STREAM_THREADS = 256;
 static const int RED_MAX_BLOCKS = 1184;   // 148 SMs x 8
+static const int SB_BLOCK_MAX = 8;        // right-hand sides of one block solve
 
 // ---------------------------------------------------------------------------------------------
 // NVTX ranges (SAENA_B200_NVTX=1): the stages the reference's PROFILE_PCG / PROFILE_VCYCLE builds time
@@ -373,6 +395,9 @@ int sb_symdiag_plan(int M, int n_offsets, const int *offsets, int64_t nnz, int64
 int sb_refresh_symdiag(saena_b200_ctx *ctx, DevOperator &op);
 // w-style application of an operator with a fused epilogue; x is the local input vector.
 int sb_apply(saena_b200_ctx *ctx, DevOperator &op, const double *x, int epi, const EpiArgs &args);
+// ---- spmv_block.cu
+// sb_apply on k column-major vectors: x's column j at x + j * n_local_cols, the epilogue's at + j * M (inv_diag shared)
+int sb_apply_block(saena_b200_ctx *ctx, DevOperator &op, int k, const double *x, int epi, const EpiArgs &args);
 int64_t sb_operator_bytes(const DevOperator &op);
 
 // ---- nccl_comm.cu
@@ -431,6 +456,18 @@ int sb_scale_vector(saena_b200_ctx *ctx, int n, double *v, const double *w);    
 int sb_coarsest_apply(saena_b200_ctx *ctx, const double *rhs, double *u);
 int sb_coarsest_cg(saena_b200_ctx *ctx, const double *rhs, double *u);  // u: initial guess in, solution out
 int sb_read_scalars(saena_b200_ctx *ctx);  // device scalars -> scalars_host (synchronises the stream)
+// Block forms on k column-major columns of n rows (column j at + j * n).  Each column goes through the single kernel's
+// arithmetic: the reductions use the same CTA count and summation tree per column, with the block's own partials and
+// counters, and write blk_scal[slot * SB_BLOCK_MAX + j].  The PCG updates take per-column alpha / beta from blk_scal
+// and leave the columns whose blk_active entry is 0 as they are.
+int sb_dot_block(saena_b200_ctx *ctx, const double *a, const double *b, int n, int k, int slot);
+int sb_pcg_update_block(saena_b200_ctx *ctx, int n, int k, double *u, double *r, const double *p, const double *h);
+int sb_pcg_p_update_block(saena_b200_ctx *ctx, int n, int k, double *p, const double *rho);
+int sb_cheb_first_zero_block(saena_b200_ctx *ctx, int n, int k, const double *rhs, const double *inv_diag, double c,
+                             double *d, double *u);
+int sb_negate_copy_block(saena_b200_ctx *ctx, int n, int k, const double *src, double *dst);
+int sb_scale_vector_block(saena_b200_ctx *ctx, int n, int k, double *v, const double *w);
+int sb_read_block_scalars(saena_b200_ctx *ctx);  // blk_scal -> blk_scal_host (synchronises the stream)
 
 // ---- lanczos.cu
 // out = uniform(-1, 1) from a counter-based generator on the global row index (row_offset + i)
@@ -447,3 +484,16 @@ int sb_vcycle(saena_b200_ctx *ctx, int l, int smoother, int pre, int post, const
 // level-0 V-cycle from a zero iterate, replayed from a CUDA graph when nothing in it needs the host
 int sb_vcycle_from_zero(saena_b200_ctx *ctx, int smoother, int pre, int post, const double *rhs);
 void sb_invalidate_graphs(saena_b200_ctx *ctx);
+// the block forms on k columns of the levels' block buffers (DevLevel::bu[bcur] is the iterate)
+int sb_apply_level_A_block(saena_b200_ctx *ctx, int l, int k, const double *x, int epi, const EpiArgs &args);
+int sb_smooth_block(saena_b200_ctx *ctx, int l, int k, int smoother, int iters, const double *rhs, bool u_is_zero);
+int sb_vcycle_block(saena_b200_ctx *ctx, int l, int k, int smoother, int pre, int post, const double *rhs,
+                    bool u_is_zero);
+// the level-0 block V-cycle from a zero iterate, replayed from a CUDA graph like sb_vcycle_from_zero's
+int sb_vcycle_block_from_zero(saena_b200_ctx *ctx, int k, int smoother, int pre, int post, const double *rhs);
+
+// ---- api.cu (block solve)
+// block buffers for k columns (grown to the largest k so far, and to the routed levels; growing drops every captured
+// block V-cycle); a failed allocation leaves no block buffer and the context usable for single solves
+int sb_block_reserve(saena_b200_ctx *ctx, int k);
+void sb_block_free(saena_b200_ctx *ctx);

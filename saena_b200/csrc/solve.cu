@@ -214,7 +214,7 @@ int sb_vcycle_from_zero(saena_b200_ctx *ctx, int smoother, int pre, int post, co
     if (!capturable) return sb_vcycle(ctx, 0, smoother, pre, post, rhs, true);
     VcycleGraph *known = nullptr;
     for (VcycleGraph &g : ctx->graphs)
-        if (g.rhs == rhs && g.smoother == smoother && g.pre == pre && g.post == post) known = &g;
+        if (g.k == 0 && g.rhs == rhs && g.smoother == smoother && g.pre == pre && g.post == post) known = &g;
     if (known && known->exec) {
         SB_CUDA(cudaGraphLaunch(known->exec, ctx->stream));
         ctx->launches += known->launches;
@@ -263,6 +263,177 @@ int sb_vcycle_from_zero(saena_b200_ctx *ctx, int smoother, int pre, int post, co
     }
     for (DevLevel &lv : ctx->levels) g.cur_after.push_back(lv.cur);
     drop_pending();
+    ctx->graphs.push_back(g);
+    SB_CUDA(cudaGraphLaunch(g.exec, ctx->stream));
+    ++ctx->graph_replays;
+    return 0;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Block forms: k column-major right-hand sides on the levels' block buffers (DevLevel::bu, bd, bres, brhs,
+// bxfer_old; column j of a level-l vector at + j * M_l).  Step for step the single code path above -- zero-iterate
+// shortcuts, route, repartition, scaling -- with every operator applied once for the k columns (sb_apply_block) and the
+// coarsest level solved column by column: column j of every result has the bits of the single path on column j.
+// ---------------------------------------------------------------------------------------------
+int sb_apply_level_A_block(saena_b200_ctx *ctx, int l, int k, const double *x, int epi, const EpiArgs &args) {
+    DevLevel &lv = ctx->levels[l];
+    if (!lv.route) return sb_apply_block(ctx, lv.A, k, x, epi, args);
+    DevLevel &fl = ctx->levels[l - 1];
+    if (ctx->blk_route_cap < (size_t)k * fl.M) SB_FAIL("apply_block: route level without its intermediate vectors");
+    EpiArgs e{};
+    e.out = ctx->blk_route_t;
+    SB_TRY(sb_apply_block(ctx, fl.P, k, x, EPI_PLAIN, e));
+    e.out = ctx->blk_route_s;
+    SB_TRY(sb_apply_block(ctx, fl.A, k, ctx->blk_route_t, EPI_PLAIN, e));
+    return sb_apply_block(ctx, fl.R, k, ctx->blk_route_s, epi, args);
+}
+
+int sb_smooth_block(saena_b200_ctx *ctx, int l, int k, int smoother, int iters, const double *rhs, bool u_is_zero) {
+    DevLevel &lv = ctx->levels[l];
+    if (iters <= 0 || lv.M == 0) return 0;
+    EpiArgs e{};
+    e.rhs = rhs;
+    e.inv_diag = lv.inv_diag;
+    if (smoother == SAENA_B200_JACOBI) {
+        e.c1 = (double)(float)(2.0 / 3);
+        int j = 0;
+        if (u_is_zero) {
+            SB_TRY(sb_cheb_first_zero_block(ctx, lv.M, k, rhs, lv.inv_diag, e.c1, lv.bd, lv.bu[lv.bcur]));
+            j = 1;
+        }
+        for (; j < iters; ++j) {
+            e.u_in = lv.bu[lv.bcur];
+            e.out = lv.bu[lv.bcur ^ 1];
+            SB_TRY(sb_apply_level_A_block(ctx, l, k, lv.bu[lv.bcur], EPI_JACOBI, e));
+            lv.bcur ^= 1;
+        }
+        return 0;
+    }
+    if (smoother != SAENA_B200_CHEBYSHEV) SB_FAIL("smooth: unknown smoother");
+    const double eig = lv.eig_max;
+    const double alpha = 0.13 * eig;
+    const double beta = eig;
+    const double delta = (beta - alpha) / 2.0;
+    const double theta = (beta + alpha) / 2.0;
+    const double s1 = theta / delta;
+    const double twos1 = 2.0 * s1;
+    double rhok = 1.0 / s1;
+    e.d_in = lv.bd;
+    e.d_out = lv.bd;
+    if (u_is_zero) {
+        SB_TRY(sb_cheb_first_zero_block(ctx, lv.M, k, rhs, lv.inv_diag, 1.0 / theta, lv.bd, lv.bu[lv.bcur]));
+    } else {
+        e.c1 = 1.0 / theta;
+        e.u_in = lv.bu[lv.bcur];
+        e.out = lv.bu[lv.bcur ^ 1];
+        SB_TRY(sb_apply_level_A_block(ctx, l, k, lv.bu[lv.bcur], EPI_CHEB_FIRST, e));
+        lv.bcur ^= 1;
+    }
+    for (int i = 1; i < iters; ++i) {
+        const double rhokp1 = 1.0 / (twos1 - rhok);
+        const double two_rhokp1 = 2.0 * rhokp1;
+        const double d1 = rhokp1 * rhok;
+        const double d2 = two_rhokp1 / delta;
+        rhok = rhokp1;
+        e.c1 = d1;
+        e.c2 = d2;
+        e.u_in = lv.bu[lv.bcur];
+        e.out = lv.bu[lv.bcur ^ 1];
+        SB_TRY(sb_apply_level_A_block(ctx, l, k, lv.bu[lv.bcur], EPI_CHEB_NEXT, e));
+        lv.bcur ^= 1;
+    }
+    return 0;
+}
+
+int sb_vcycle_block(saena_b200_ctx *ctx, int l, int k, int smoother, int pre, int post, const double *rhs,
+                    bool u_is_zero) {
+    const int max_level = (int)ctx->levels.size() - 1;
+    DevLevel &lv = ctx->levels[l];
+    const long long M = lv.M;
+    if (l == max_level) {
+        if (lv.M > 0 && ctx->coarsest_cg) {
+            if (u_is_zero) SB_TRY(sb_fill_zero(ctx, lv.bu[lv.bcur], (size_t)k * M));
+            for (int j = 0; j < k; ++j) SB_TRY(sb_coarsest_cg(ctx, rhs + j * M, lv.bu[lv.bcur] + j * M));
+        } else if (lv.M > 0) {
+            if (ctx->coarse_n != lv.M) SB_FAIL("vcycle: no coarsest factor was uploaded for the coarsest level");
+            for (int j = 0; j < k; ++j) SB_TRY(sb_coarsest_apply(ctx, rhs + j * M, lv.bu[lv.bcur] + j * M));
+        }
+        return 0;
+    }
+    DevLevel &cl = ctx->levels[l + 1];
+    const long long Mc = cl.M, Mo = lv.M_coarse_old;
+    const bool ident = lv.repart.identity();
+    if (pre) SB_TRY(sb_smooth_block(ctx, l, k, smoother, pre, rhs, u_is_zero));
+    else if (u_is_zero) SB_TRY(sb_fill_zero(ctx, lv.bu[lv.bcur], (size_t)k * M));
+    if (pre == 0 && u_is_zero) {
+        SB_TRY(sb_negate_copy_block(ctx, lv.M, k, rhs, lv.bres));
+    } else {
+        EpiArgs e{};
+        e.rhs = rhs;
+        e.out = lv.bres;
+        SB_TRY(sb_apply_level_A_block(ctx, l, k, lv.bu[lv.bcur], EPI_RESIDUAL, e));
+    }
+    {
+        EpiArgs e{};
+        e.out = ident ? cl.brhs : lv.bxfer_old;
+        SB_TRY(sb_apply_block(ctx, lv.R, k, lv.bres, EPI_PLAIN, e));
+        if (!ident)
+            for (int j = 0; j < k; ++j)
+                SB_TRY(sb_repart(ctx, lv.repart, false, lv.bxfer_old + j * Mo, cl.brhs + j * Mc, ctx->stream));
+    }
+    if (ctx->scale) SB_TRY(sb_scale_vector_block(ctx, cl.M, k, cl.brhs, cl.inv_sq_diag));
+    SB_TRY(sb_vcycle_block(ctx, l + 1, k, smoother, pre, post, cl.brhs, true));
+    if (ctx->scale) SB_TRY(sb_scale_vector_block(ctx, cl.M, k, cl.bu[cl.bcur], cl.inv_sq_diag));
+    {
+        const double *ec = cl.bu[cl.bcur];
+        if (!ident) {
+            for (int j = 0; j < k; ++j)
+                SB_TRY(sb_repart(ctx, lv.repart, true, ec + j * Mc, lv.bxfer_old + j * Mo, ctx->stream));
+            ec = lv.bxfer_old;
+        }
+        EpiArgs e{};
+        e.u_in = lv.bu[lv.bcur];
+        e.out = lv.bu[lv.bcur];
+        SB_TRY(sb_apply_block(ctx, lv.P, k, ec, EPI_SUB, e));
+    }
+    if (post) SB_TRY(sb_smooth_block(ctx, l, k, smoother, post, rhs, false));
+    return 0;
+}
+
+// One rank only (the block calls refuse several), so the first use of a configuration is captured at once.  The key
+// is (rhs, smoother, pre, post, k): the block buffers a graph points into stay put until they grow, and growing them
+// drops every block graph (sb_block_reserve).
+int sb_vcycle_block_from_zero(saena_b200_ctx *ctx, int k, int smoother, int pre, int post, const double *rhs) {
+    for (DevLevel &lv : ctx->levels) lv.bcur = 0;
+    if (!ctx->use_graphs || ctx->coarsest_cg) return sb_vcycle_block(ctx, 0, k, smoother, pre, post, rhs, true);
+    for (VcycleGraph &g : ctx->graphs)
+        if (g.k == k && g.rhs == rhs && g.smoother == smoother && g.pre == pre && g.post == post) {
+            SB_CUDA(cudaGraphLaunch(g.exec, ctx->stream));
+            ctx->launches += g.launches;
+            ++ctx->graph_replays;
+            for (size_t l = 0; l < ctx->levels.size(); ++l) ctx->levels[l].bcur = g.cur_after[l];
+            return 0;
+        }
+    const int64_t before = ctx->launches;
+    cudaGraph_t graph = nullptr;
+    SB_CUDA(cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal));
+    const int rc = sb_vcycle_block(ctx, 0, k, smoother, pre, post, rhs, true);
+    const cudaError_t ce = cudaStreamEndCapture(ctx->stream, &graph);
+    cudaGraphExec_t exec = nullptr;
+    const cudaError_t ie = (rc || ce != cudaSuccess || !graph) ? cudaErrorUnknown : cudaGraphInstantiate(&exec, graph, 0);
+    if (graph) cudaGraphDestroy(graph);
+    if (ie != cudaSuccess) {
+        // the capture executed nothing: run eagerly (a failed capture of the block V-cycle leaves the single one's
+        // graphs as they are)
+        cudaGetLastError();
+        ctx->launches = before;
+        for (DevLevel &lv : ctx->levels) lv.bcur = 0;
+        if (rc) return rc;
+        ctx->error.clear();
+        return sb_vcycle_block(ctx, 0, k, smoother, pre, post, rhs, true);
+    }
+    VcycleGraph g{rhs, smoother, pre, post, exec, ctx->launches - before, {}, k};
+    for (DevLevel &lv : ctx->levels) g.cur_after.push_back(lv.bcur);
     ctx->graphs.push_back(g);
     SB_CUDA(cudaGraphLaunch(g.exec, ctx->stream));
     ++ctx->graph_replays;

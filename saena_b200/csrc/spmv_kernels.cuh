@@ -29,29 +29,36 @@
 // Every input of row i is read before the first store: the pointers are not restrict-qualified, so a load written after
 // a store is issued only once the values the store depends on have arrived -- a second memory round trip per thread.
 // (No caller passes u_in aliasing d_out; out may be u_in, d_out may be d_in: same element, read first either way.)
+// Row i of the operator; o: where row i's entries of the epilogue's vectors are (i, or i + j * ld in column j of a
+// block: inv_diag, one per row, is shared by the columns).
+template <int EPI, typename IdxT>
+__device__ __forceinline__ void sb_epilogue_at(int i, IdxT o, double ax, const EpiArgs &e) {
+    if (EPI == EPI_PLAIN) {
+        e.out[o] = ax;
+    } else if (EPI == EPI_RESIDUAL) {
+        e.out[o] = ax - e.rhs[o];
+    } else if (EPI == EPI_CHEB_FIRST) {
+        const double u = e.u_in[o];
+        const double d = e.c1 * e.inv_diag[i] * (e.rhs[o] - ax);
+        e.d_out[o] = d;
+        e.out[o] = u + d;
+    } else if (EPI == EPI_CHEB_NEXT) {
+        const double u = e.u_in[o];
+        const double res = e.c2 * e.inv_diag[i] * (e.rhs[o] - ax);
+        const double d = (e.c1 * e.d_in[o]) + res;
+        e.d_out[o] = d;
+        e.out[o] = u + d;
+    } else if (EPI == EPI_JACOBI) {
+        const double t = (ax - e.rhs[o]) * (e.inv_diag[i] * e.c1);
+        e.out[o] = e.u_in[o] - t;
+    } else if (EPI == EPI_SUB) {
+        e.out[o] = e.u_in[o] - ax;
+    }
+}
+
 template <int EPI>
 __device__ __forceinline__ void sb_epilogue(int i, double ax, const EpiArgs &e) {
-    if (EPI == EPI_PLAIN) {
-        e.out[i] = ax;
-    } else if (EPI == EPI_RESIDUAL) {
-        e.out[i] = ax - e.rhs[i];
-    } else if (EPI == EPI_CHEB_FIRST) {
-        const double u = e.u_in[i];
-        const double d = e.c1 * e.inv_diag[i] * (e.rhs[i] - ax);
-        e.d_out[i] = d;
-        e.out[i] = u + d;
-    } else if (EPI == EPI_CHEB_NEXT) {
-        const double u = e.u_in[i];
-        const double res = e.c2 * e.inv_diag[i] * (e.rhs[i] - ax);
-        const double d = (e.c1 * e.d_in[i]) + res;
-        e.d_out[i] = d;
-        e.out[i] = u + d;
-    } else if (EPI == EPI_JACOBI) {
-        const double t = (ax - e.rhs[i]) * (e.inv_diag[i] * e.c1);
-        e.out[i] = e.u_in[i] - t;
-    } else if (EPI == EPI_SUB) {
-        e.out[i] = e.u_in[i] - ax;
-    }
+    sb_epilogue_at<EPI>(i, i, ax, e);
 }
 
 // (Fetching the epilogue's vector inputs before the row loop was tried in round 1: +3 % on the
@@ -502,6 +509,249 @@ __global__ void halo_pack_kernel(int n, const int *__restrict__ vIndex, const do
                                  SendT *__restrict__ out) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) out[i] = (SendT)v[vIndex[i]];
+}
+
+// ---------------------------------------------------------------------------------------------
+// Block SpMV: one pass over the operator for k <= K right-hand sides (saena_b200_solve_pcg_block).  The block is k
+// ordinary vectors back to back, column-major: x's column j starts at x + j * ldx (ldx = n_local_cols), every epilogue
+// vector's at + j * ld (ld = M).  Each entry's value, column id and row offset is loaded once and applied to the k
+// gathered x values; columns j >= k are predicated off, nothing is padded in memory.  Per column every row is summed
+// in the order, with the multiply-adds and the epilogue arithmetic, of the single kernel of the same mapping: column j
+// of a block application has the bits of the single application to column j.
+// ---------------------------------------------------------------------------------------------
+template <int EPI, int K>
+__device__ __forceinline__ void sb_epilogue_block(int i, long long ld, int k, const double (&ax)[K], const EpiArgs &e) {
+#pragma unroll
+    for (int j = 0; j < K; ++j)
+        if (j < k) sb_epilogue_at<EPI>(i, (long long)i + j * ld, ax[j], e);
+}
+
+// sb_sliced_row_sum for K columns: the same trips, loads and per-column `sum += a * x` chain
+template <int DEPTH, int K>
+__device__ __forceinline__ void sb_sliced_row_sums(const int *cp, const double *vp, int len, const double *x,
+                                                   long long ldx, int k, double (&sum)[K]) {
+#pragma unroll
+    for (int j = 0; j < K; ++j) sum[j] = 0.0;
+    for (int t = 0; t < len; t += DEPTH) {
+        int c[DEPTH];
+        double a[DEPTH];
+#pragma unroll
+        for (int q = 0; q < DEPTH; ++q) {
+            const bool in = t + q < len;
+            c[q] = in ? sb_ld_stream(cp + (t + q) * 32) : 0;
+            a[q] = in ? sb_ld_stream(vp + (t + q) * 32) : 0.0;
+        }
+#pragma unroll
+        for (int q = 0; q < DEPTH; ++q)
+            if (t + q < len) {
+#pragma unroll
+                for (int j = 0; j < K; ++j)
+                    if (j < k) sum[j] += a[q] * __ldg(x + (c[q] + j * ldx));
+            }
+    }
+}
+
+template <int EPI, int K>
+__global__ void __launch_bounds__(256)
+spmv_sell_block_kernel(int row_begin, int M, int k, const long long *__restrict__ slice_ptr, const int *__restrict__ col,
+                       const double *__restrict__ val, const double *__restrict__ x, long long ldx, EpiArgs e,
+                       long long ld) {
+    const int row = row_begin + blockIdx.x * blockDim.x + threadIdx.x;
+    const int lane = threadIdx.x & 31;
+    const int slice = row >> 5;
+    if ((slice << 5) >= M) return;
+    const long long base = slice_ptr[slice];
+    const int len = (int)((slice_ptr[slice + 1] - base) >> 5);
+    double sum[K];
+    sb_sliced_row_sums<SELL_UNROLL, K>(col + base + lane, val + base + lane, len, x, ldx, k, sum);
+    if (row < M) sb_epilogue_block<EPI, K>(row, ld, k, sum, e);
+}
+
+template <int EPI, int K>
+__global__ void __launch_bounds__(256)
+spmv_sellp_block_kernel(int M, int k, const long long *__restrict__ slice_ptr, const int *__restrict__ perm,
+                        const int *__restrict__ col, const double *__restrict__ val, const double *__restrict__ x,
+                        long long ldx, EpiArgs e, long long ld) {
+    __shared__ double s_sum[K][256];
+    const int slot = blockIdx.x * 256 + threadIdx.x;
+    const int lane = threadIdx.x & 31;
+    const int slice = slot >> 5;
+    const long long base = slice_ptr[slice];
+    const int len = (int)((slice_ptr[slice + 1] - base) >> 5);
+    double sum[K];
+    sb_sliced_row_sums<SELL_UNROLL, K>(col + base + lane, val + base + lane, len, x, ldx, k, sum);
+    const int wbase = blockIdx.x * 256;
+    const int row = perm[slot];
+    if (row >= 0) {
+#pragma unroll
+        for (int j = 0; j < K; ++j) s_sum[j][row - wbase] = sum[j];
+    }
+    __syncthreads();
+    const int mine = wbase + threadIdx.x;
+    if (mine >= M) return;
+#pragma unroll
+    for (int j = 0; j < K; ++j) sum[j] = s_sum[j][threadIdx.x];
+    sb_epilogue_block<EPI, K>(mine, ld, k, sum, e);
+}
+
+// spmv_symdiag_kernel for K columns: the row's stored values are loaded once, then every column is summed with the
+// single kernel's chain (skipped terms add 0.0 * 0.0 as there)
+template <int ND, int EPI, int K>
+__global__ void __launch_bounds__(256)
+spmv_symdiag_block_kernel(int M, int k, const double *__restrict__ d, const SymDiagOffsets s,
+                          const double *__restrict__ x, long long ldx, EpiArgs e, long long ld) {
+    const int i = blockIdx.x * 256 + threadIdx.x;
+    if (i >= M) return;
+    const size_t m = (size_t)M;
+    double la[ND], ua[ND];
+#pragma unroll
+    for (int q = ND - 1; q >= 1; --q) {
+        const bool up = q < s.nd && i < M - s.off[q];
+        ua[q] = up ? __ldcg(d + q * m + i) : 0.0;
+    }
+    const double a0 = __ldcg(d + i);
+#pragma unroll
+    for (int q = 1; q < ND; ++q) {
+        const bool lo = q < s.nd && i >= s.off[q];
+        la[q] = lo ? __ldcs(d + q * m + (i - s.off[q])) : 0.0;
+    }
+#pragma unroll
+    for (int j = 0; j < K; ++j) {
+        if (j >= k) break;
+        const double *xj = x + j * ldx;
+        double lx[ND], ux[ND];
+#pragma unroll
+        for (int q = ND - 1; q >= 1; --q) ux[q] = (q < s.nd && i < M - s.off[q]) ? __ldg(xj + (i + s.off[q])) : 0.0;
+        const double x0 = __ldg(xj + i);
+#pragma unroll
+        for (int q = 1; q < ND; ++q) lx[q] = (q < s.nd && i >= s.off[q]) ? __ldg(xj + (i - s.off[q])) : 0.0;
+        double sum = 0.0;
+#pragma unroll
+        for (int q = ND - 1; q >= 1; --q) sum += la[q] * lx[q];
+        sum += a0 * x0;
+#pragma unroll
+        for (int q = 1; q < ND; ++q) sum += ua[q] * ux[q];
+        sb_epilogue_at<EPI>(i, (long long)i + j * ld, sum, e);
+    }
+}
+
+// spmv_vec_body for K columns
+template <int LANES, int EPI, int K, typename OffT>
+__global__ void __launch_bounds__(256)
+spmv_vec_block_kernel(int row_begin, int M, int k, const OffT *__restrict__ rowptr, const int *__restrict__ col,
+                      const double *__restrict__ val, const double *__restrict__ x, long long ldx, EpiArgs e,
+                      long long ld) {
+    constexpr int G = 32 / LANES;
+    const int lane = threadIdx.x & 31;
+    const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int row0 = row_begin + warp * 32;
+    if (row0 >= M) return;
+    const int my_row = row0 + lane;
+    OffT my_start = 0, my_end = 0;
+    if (my_row < M) {
+        my_start = rowptr[my_row];
+        my_end = rowptr[my_row + 1];
+    }
+    double mine[K];
+#pragma unroll
+    for (int j = 0; j < K; ++j) mine[j] = 0.0;
+    const int g = lane / LANES;
+    const int sub = lane % LANES;
+    // (not unrolled, unlike the single kernel: K sums per step, unrolled LANES times, would spill)
+#pragma unroll 1
+    for (int t = 0; t < LANES; ++t) {
+        const int src = t * G + g;
+        const OffT start = __shfl_sync(0xffffffffu, my_start, src);
+        const OffT end = __shfl_sync(0xffffffffu, my_end, src);
+        double sum[K];
+#pragma unroll
+        for (int j = 0; j < K; ++j) sum[j] = 0.0;
+        for (OffT kk0 = start + sub; kk0 < end; kk0 += LANES * VEC_UNROLL) {
+            int c[VEC_UNROLL];
+            double a[VEC_UNROLL];
+#pragma unroll
+            for (int q = 0; q < VEC_UNROLL; ++q) {
+                const OffT kk = kk0 + q * LANES;
+                const bool in = kk < end;
+                c[q] = in ? sb_ld_stream(col + kk) : 0;
+                a[q] = in ? sb_ld_stream(val + kk) : 0.0;
+            }
+#pragma unroll
+            for (int q = 0; q < VEC_UNROLL; ++q) {
+#pragma unroll
+                for (int j = 0; j < K; ++j)
+                    if (j < k) sum[j] += a[q] * __ldg(x + (c[q] + j * ldx));
+            }
+        }
+#pragma unroll
+        for (int j = 0; j < K; ++j) {
+#pragma unroll
+            for (int o = LANES / 2; o > 0; o >>= 1) sum[j] += __shfl_xor_sync(0xffffffffu, sum[j], o);
+            const double v = __shfl_sync(0xffffffffu, sum[j], (lane % G) * LANES);
+            if (lane / G == t) mine[j] = v;
+        }
+    }
+    if (my_row < M) sb_epilogue_block<EPI, K>(my_row, ld, k, mine, e);
+}
+
+// spmv_rowgroup_body for K columns
+template <int TPR, int EPI, int K, typename OffT>
+__global__ void __launch_bounds__(256)
+spmv_rowgroup_block_kernel(int row_begin, int M, int k, const OffT *__restrict__ rowptr, const int *__restrict__ col,
+                           const double *__restrict__ val, const double *__restrict__ x, long long ldx, EpiArgs e,
+                           long long ld) {
+    constexpr int ROWS = 256 / TPR;
+    constexpr int WPR = TPR / 32;
+    __shared__ double s_part[K][8];
+    const int g = threadIdx.x / TPR, sub = threadIdx.x % TPR;
+    const int row = row_begin + blockIdx.x * ROWS + g;
+    double sum[K];
+#pragma unroll
+    for (int j = 0; j < K; ++j) sum[j] = 0.0;
+    if (row < M) {
+        const OffT start = rowptr[row], end = rowptr[row + 1];
+        for (OffT kk0 = start + sub; kk0 < end; kk0 += TPR * VEC_UNROLL) {
+            int c[VEC_UNROLL];
+            double a[VEC_UNROLL];
+#pragma unroll
+            for (int q = 0; q < VEC_UNROLL; ++q) {
+                const OffT kk = kk0 + q * TPR;
+                const bool in = kk < end;
+                c[q] = in ? sb_ld_stream(col + kk) : 0;
+                a[q] = in ? sb_ld_stream(val + kk) : 0.0;
+            }
+#pragma unroll
+            for (int q = 0; q < VEC_UNROLL; ++q) {
+#pragma unroll
+                for (int j = 0; j < K; ++j)
+                    if (j < k) sum[j] += a[q] * __ldg(x + (c[q] + j * ldx));
+            }
+        }
+    }
+#pragma unroll
+    for (int j = 0; j < K; ++j) {
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) sum[j] += __shfl_xor_sync(0xffffffffu, sum[j], o);
+    }
+    if (WPR == 1) {
+        if (sub == 0 && row < M) sb_epilogue_block<EPI, K>(row, ld, k, sum, e);
+    } else {
+        if ((threadIdx.x & 31) == 0) {
+#pragma unroll
+            for (int j = 0; j < K; ++j) s_part[j][threadIdx.x >> 5] = sum[j];
+        }
+        __syncthreads();
+        if (sub == 0 && row < M) {
+            double tot[K];
+#pragma unroll
+            for (int j = 0; j < K; ++j) {
+                tot[j] = 0.0;
+#pragma unroll
+                for (int w = 0; w < WPR; ++w) tot[j] += s_part[j][g * WPR + w];
+            }
+            sb_epilogue_block<EPI, K>(row, ld, k, tot, e);
+        }
+    }
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -7,6 +7,10 @@
 // Reductions are deterministic: every CTA writes one partial, the last CTA to finish (atomic
 // ticket) adds the partials in index order.  The scalars of the Krylov recurrences live in
 // device memory (ctx->scalars) so alpha/beta never round-trip through the host.
+//
+// Block forms (saena_b200_solve_pcg_block): the same kernels on a grid with one row of CTAs per column (grid.y =
+// column j, vectors at + j * ld); each column has its own partials, counter and scalars (stride sstride) and so the
+// single call's CTA count, reduction tree and bits.  A single call is the grid with one row.
 #include <nvtx3/nvToolsExt.h>
 #include <stdio.h>
 
@@ -58,9 +62,15 @@ __device__ __forceinline__ void finalize_sum(double block_total, double *partial
 }
 
 __global__ void __launch_bounds__(256)
-dot_kernel(int n, const double *__restrict__ a, const double *__restrict__ b, double *partials,
+dot_kernel(int n, long long ld, const double *__restrict__ a, const double *__restrict__ b, double *partials,
            unsigned int *counter, double *out) {
     __shared__ double s_w[8];
+    const long long o = blockIdx.y * ld;
+    a += o;
+    b += o;
+    partials += blockIdx.y * RED_MAX_BLOCKS;
+    counter += blockIdx.y;
+    out += blockIdx.y;
     double acc = 0.0;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) acc += a[i] * b[i];
     const double t = block_sum_256(acc, s_w);
@@ -69,11 +79,21 @@ dot_kernel(int n, const double *__restrict__ a, const double *__restrict__ b, do
 
 // u -= alpha p ; r -= alpha h ; <r,r>       alpha = rho_res / pdoth   (solve.cpp:2588-2603)
 __global__ void __launch_bounds__(256)
-pcg_update_kernel(int n, double *__restrict__ u, double *__restrict__ r, const double *__restrict__ p,
-                  const double *__restrict__ h, const double *__restrict__ scal, double *partials,
-                  unsigned int *counter, double *out_rr) {
+pcg_update_kernel(int n, long long ld, double *__restrict__ u, double *__restrict__ r, const double *__restrict__ p,
+                  const double *__restrict__ h, const double *__restrict__ scal, int sstride,
+                  const int *__restrict__ active, double *partials, unsigned int *counter, double *out_rr) {
     __shared__ double s_w[8];
-    const double alpha = scal[S_RHO_RES] / scal[S_PDOTH];
+    const int j = blockIdx.y;
+    if (active && !active[j]) return;   // a column that has stopped: every CTA of its row leaves, nothing is reduced
+    const long long o = j * ld;
+    u += o;
+    r += o;
+    p += o;
+    h += o;
+    partials += j * RED_MAX_BLOCKS;
+    counter += j;
+    out_rr += j;
+    const double alpha = scal[S_RHO_RES * sstride + j] / scal[S_PDOTH * sstride + j];
     double acc = 0.0;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
         u[i] -= alpha * p[i];
@@ -89,8 +109,13 @@ pcg_update_kernel(int n, double *__restrict__ u, double *__restrict__ r, const d
 // (solve.cpp:2655-2667; the next iteration's <r,rho> at :2580 is the same number, r and rho
 // being untouched in between, so it is carried over instead of recomputed)
 __global__ void __launch_bounds__(256)
-pcg_p_update_kernel(int n, double *__restrict__ p, const double *__restrict__ rho, const double *__restrict__ scal) {
-    const double beta = scal[S_BETA_NUM] / scal[S_RHO_RES];
+pcg_p_update_kernel(int n, long long ld, double *__restrict__ p, const double *__restrict__ rho,
+                    const double *__restrict__ scal, int sstride, const int *__restrict__ active) {
+    const int j = blockIdx.y;
+    if (active && !active[j]) return;
+    p += j * ld;
+    rho += j * ld;
+    const double beta = scal[S_BETA_NUM * sstride + j] / scal[S_RHO_RES * sstride + j];
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
         p[i] = rho[i] + beta * p[i];
 }
@@ -127,8 +152,12 @@ ccg_update_kernel(int n, double *__restrict__ u, double *__restrict__ res, const
 // first Chebyshev sweep from a zero iterate: A*0 = 0, so d = (1/theta) D^-1 rhs and u = d
 // (saena_matrix.cpp:1099-1109 with u == 0; bit-identical to running the SpMV on zeros)
 __global__ void __launch_bounds__(256)
-cheb_first_zero_kernel(int n, const double *__restrict__ rhs, const double *__restrict__ inv_diag, double c,
-                       double *__restrict__ d, double *__restrict__ u) {
+cheb_first_zero_kernel(int n, long long ld, const double *__restrict__ rhs, const double *__restrict__ inv_diag,
+                       double c, double *__restrict__ d, double *__restrict__ u) {
+    const long long o = blockIdx.y * ld;
+    rhs += o;
+    d += o;
+    u += o;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
         const double v = c * inv_diag[i] * rhs[i];
         d[i] = v;
@@ -138,12 +167,15 @@ cheb_first_zero_kernel(int n, const double *__restrict__ rhs, const double *__re
 
 // saena_object::scale_vector (src/saena_object.cpp:563-569)
 __global__ void __launch_bounds__(256)
-scale_vector_kernel(int n, double *__restrict__ v, const double *__restrict__ w) {
+scale_vector_kernel(int n, long long ld, double *__restrict__ v, const double *__restrict__ w) {
+    v += blockIdx.y * ld;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) v[i] *= w[i];
 }
 
 __global__ void __launch_bounds__(256)
-negate_copy_kernel(int n, const double *__restrict__ src, double *__restrict__ dst) {
+negate_copy_kernel(int n, long long ld, const double *__restrict__ src, double *__restrict__ dst) {
+    src += blockIdx.y * ld;
+    dst += blockIdx.y * ld;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) dst[i] = -src[i];
 }
 
@@ -193,7 +225,7 @@ coarsest_kernel(int n, const double *__restrict__ A, const double *__restrict__ 
 // ---------------------------------------------------------------------------------------------
 int sb_dot(saena_b200_ctx *ctx, const double *a, const double *b, int n, int slot) {
     ++ctx->launches;
-    dot_kernel<<<red_blocks(ctx, n), 256, 0, ctx->stream>>>(n, a, b, ctx->red_partials, ctx->red_counter,
+    dot_kernel<<<red_blocks(ctx, n), 256, 0, ctx->stream>>>(n, 0, a, b, ctx->red_partials, ctx->red_counter,
                                                            ctx->scalars + slot);
     SB_CUDA(cudaGetLastError());
     if (ctx->nranks > 1) SB_TRY(sb_allreduce_sum(ctx, ctx->scalars + slot, 1, ctx->stream));
@@ -202,8 +234,9 @@ int sb_dot(saena_b200_ctx *ctx, const double *a, const double *b, int n, int slo
 
 int sb_pcg_update(saena_b200_ctx *ctx, int n, double *u, double *r, const double *p, const double *h) {
     ++ctx->launches;
-    pcg_update_kernel<<<red_blocks(ctx, n), 256, 0, ctx->stream>>>(n, u, r, p, h, ctx->scalars, ctx->red_partials,
-                                                                  ctx->red_counter, ctx->scalars + S_RR);
+    pcg_update_kernel<<<red_blocks(ctx, n), 256, 0, ctx->stream>>>(n, 0, u, r, p, h, ctx->scalars, 1, nullptr,
+                                                                  ctx->red_partials, ctx->red_counter,
+                                                                  ctx->scalars + S_RR);
     SB_CUDA(cudaGetLastError());
     if (ctx->nranks > 1) SB_TRY(sb_allreduce_sum(ctx, ctx->scalars + S_RR, 1, ctx->stream));
     return 0;
@@ -211,7 +244,7 @@ int sb_pcg_update(saena_b200_ctx *ctx, int n, double *u, double *r, const double
 
 int sb_pcg_p_update(saena_b200_ctx *ctx, int n, double *p, const double *rho) {
     ctx->launches += 2;
-    pcg_p_update_kernel<<<red_blocks(ctx, n), 256, 0, ctx->stream>>>(n, p, rho, ctx->scalars);
+    pcg_p_update_kernel<<<red_blocks(ctx, n), 256, 0, ctx->stream>>>(n, 0, p, rho, ctx->scalars, 1, nullptr);
     carry_scalar_kernel<<<1, 1, 0, ctx->stream>>>(ctx->scalars, S_RHO_RES, S_BETA_NUM);
     SB_CUDA(cudaGetLastError());
     return 0;
@@ -228,7 +261,7 @@ int sb_cheb_first_zero(saena_b200_ctx *ctx, int n, const double *rhs, const doub
                        double *u) {
     if (n == 0) return 0;
     ++ctx->launches;
-    cheb_first_zero_kernel<<<red_blocks(ctx, n), 256, 0, ctx->stream>>>(n, rhs, inv_diag, c, d, u);
+    cheb_first_zero_kernel<<<red_blocks(ctx, n), 256, 0, ctx->stream>>>(n, 0, rhs, inv_diag, c, d, u);
     SB_CUDA(cudaGetLastError());
     return 0;
 }
@@ -236,7 +269,7 @@ int sb_cheb_first_zero(saena_b200_ctx *ctx, int n, const double *rhs, const doub
 int sb_negate_copy(saena_b200_ctx *ctx, int n, const double *src, double *dst) {
     if (n == 0) return 0;
     ++ctx->launches;
-    negate_copy_kernel<<<red_blocks(ctx, n), 256, 0, ctx->stream>>>(n, src, dst);
+    negate_copy_kernel<<<red_blocks(ctx, n), 256, 0, ctx->stream>>>(n, 0, src, dst);
     SB_CUDA(cudaGetLastError());
     return 0;
 }
@@ -245,7 +278,7 @@ int sb_scale_vector(saena_b200_ctx *ctx, int n, double *v, const double *w) {
     if (n == 0) return 0;
     if (!w) SB_FAIL("scale=true but a level has no inv_sq_diag_orig (saena_b200_upload_level_scale)");
     ++ctx->launches;
-    scale_vector_kernel<<<red_blocks(ctx, n), 256, 0, ctx->stream>>>(n, v, w);
+    scale_vector_kernel<<<red_blocks(ctx, n), 256, 0, ctx->stream>>>(n, 0, v, w);
     SB_CUDA(cudaGetLastError());
     return 0;
 }
@@ -310,6 +343,70 @@ int sb_coarsest_cg(saena_b200_ctx *ctx, const double *rhs, double *u) {
         i++;
     }
     return 0;
+}
+
+// ---- block forms: grid.y = column
+static dim3 block_grid(const saena_b200_ctx *ctx, int n, int k) { return dim3(red_blocks(ctx, n), k); }
+
+int sb_dot_block(saena_b200_ctx *ctx, const double *a, const double *b, int n, int k, int slot) {
+    ++ctx->launches;
+    dot_kernel<<<block_grid(ctx, n, k), 256, 0, ctx->stream>>>(n, n, a, b, ctx->blk_partials, ctx->blk_counter,
+                                                              ctx->blk_scal + slot * SB_BLOCK_MAX);
+    SB_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int sb_pcg_update_block(saena_b200_ctx *ctx, int n, int k, double *u, double *r, const double *p, const double *h) {
+    ++ctx->launches;
+    pcg_update_kernel<<<block_grid(ctx, n, k), 256, 0, ctx->stream>>>(n, n, u, r, p, h, ctx->blk_scal, SB_BLOCK_MAX,
+                                                                     ctx->blk_active, ctx->blk_partials,
+                                                                     ctx->blk_counter,
+                                                                     ctx->blk_scal + S_RR * SB_BLOCK_MAX);
+    SB_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int sb_pcg_p_update_block(saena_b200_ctx *ctx, int n, int k, double *p, const double *rho) {
+    ++ctx->launches;
+    pcg_p_update_kernel<<<block_grid(ctx, n, k), 256, 0, ctx->stream>>>(n, n, p, rho, ctx->blk_scal, SB_BLOCK_MAX,
+                                                                       ctx->blk_active);
+    SB_CUDA(cudaGetLastError());
+    // rho_res <- <r,rho>_new for every column (a stopped column's are never read again)
+    SB_CUDA(cudaMemcpyAsync(ctx->blk_scal + S_RHO_RES * SB_BLOCK_MAX, ctx->blk_scal + S_BETA_NUM * SB_BLOCK_MAX,
+                            sizeof(double) * k, cudaMemcpyDeviceToDevice, ctx->stream));
+    return 0;
+}
+
+int sb_cheb_first_zero_block(saena_b200_ctx *ctx, int n, int k, const double *rhs, const double *inv_diag, double c,
+                             double *d, double *u) {
+    if (n == 0) return 0;
+    ++ctx->launches;
+    cheb_first_zero_kernel<<<block_grid(ctx, n, k), 256, 0, ctx->stream>>>(n, n, rhs, inv_diag, c, d, u);
+    SB_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int sb_negate_copy_block(saena_b200_ctx *ctx, int n, int k, const double *src, double *dst) {
+    if (n == 0) return 0;
+    ++ctx->launches;
+    negate_copy_kernel<<<block_grid(ctx, n, k), 256, 0, ctx->stream>>>(n, n, src, dst);
+    SB_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int sb_scale_vector_block(saena_b200_ctx *ctx, int n, int k, double *v, const double *w) {
+    if (n == 0) return 0;
+    if (!w) SB_FAIL("scale=true but a level has no inv_sq_diag_orig (saena_b200_upload_level_scale)");
+    ++ctx->launches;
+    scale_vector_kernel<<<block_grid(ctx, n, k), 256, 0, ctx->stream>>>(n, n, v, w);
+    SB_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int sb_read_block_scalars(saena_b200_ctx *ctx) {
+    SB_CUDA(cudaMemcpyAsync(ctx->blk_scal_host, ctx->blk_scal, sizeof(double) * S_COUNT * SB_BLOCK_MAX,
+                            cudaMemcpyDeviceToHost, ctx->stream));
+    return sb_sync_stream(ctx, ctx->stream);
 }
 
 int sb_read_scalars(saena_b200_ctx *ctx) {

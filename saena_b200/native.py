@@ -96,6 +96,13 @@ def load_library(path: Optional[str] = None):
     L.saena_b200_vcycle.argtypes = [vp, i, i, i, i, vp, vp]
     L.saena_b200_coarsest_solve.argtypes = [vp, vp, vp]
     L.saena_b200_dot.argtypes = [vp, vp, vp, i, dp]
+    block_solve_args = [vp, i, vp, vp, i, d, i, i, i, ip, dp, i, ip]
+    L.saena_b200_solve_pcg_block.argtypes = block_solve_args
+    L.saena_b200_solve_pcg_block_dev.argtypes = block_solve_args
+    L.saena_b200_matvec_block.argtypes = [vp, i, i, i, vp, vp]
+    L.saena_b200_residual_block.argtypes = [vp, i, i, vp, vp, vp]
+    L.saena_b200_smooth_block.argtypes = [vp, i, i, i, i, vp, vp]
+    L.saena_b200_vcycle_block.argtypes = [vp, i, i, i, i, i, vp, vp]
     L.saena_b200_time_matvec.argtypes = [vp, i, i, i, i, ctypes.POINTER(ctypes.c_float)]
     L.saena_b200_time_smooth_sweep.argtypes = [vp, i, i, i, i, ctypes.POINTER(ctypes.c_float)]
     L.saena_b200_time_matvec_parts.argtypes = [vp, i, i, i] + [ctypes.POINTER(ctypes.c_float)] * 3
@@ -134,6 +141,8 @@ EXPORTED_SYMBOLS = [
     "saena_b200_vcycle", "saena_b200_coarsest_solve", "saena_b200_dot", "saena_b200_time_matvec",
     "saena_b200_time_smooth_sweep", "saena_b200_time_matvec_parts", "saena_b200_time_vcycle", "saena_b200_timer_start", "saena_b200_timer_stop", "saena_b200_launch_count", "saena_b200_graph_replays", "saena_b200_set_mapping", "saena_b200_set_fused_restrict", "saena_b200_spgemm_symbolic", "saena_b200_spgemm_numeric", "saena_b200_time_residual_restrict", "saena_b200_autotune_mapping", "saena_b200_set_mapping_deferred", "saena_b200_get_mapping",
     "saena_b200_set_level_route", "saena_b200_get_level_route", "saena_b200_operator_bytes",
+    "saena_b200_solve_pcg_block", "saena_b200_solve_pcg_block_dev", "saena_b200_matvec_block",
+    "saena_b200_residual_block", "saena_b200_smooth_block", "saena_b200_vcycle_block",
 ]
 
 
@@ -453,6 +462,68 @@ class Context:
         self._ck(self._L.saena_b200_solve_cg(self._h, _vp(rhs), _vp(u), int(max_iter), float(tol),
                                              ctypes.byref(iters), _f64p(hist), len(hist), ctypes.byref(n)))
         return u, iters.value, hist[:n.value]
+
+    # ---- block solve: k = 1..8 right-hand sides as (k, n) arrays (row j = column j of the C ABI's block) ----
+    @staticmethod
+    def _block(a, n: int) -> np.ndarray:
+        a = np.ascontiguousarray(a, F64)
+        if a.ndim != 2 or a.shape[1] != n:
+            raise ValueError(f"expected a (k, {n}) array, got shape {a.shape}")
+        return a
+
+    def solve_pcg_block(self, rhs, max_iter=50, tol=1e-8, smoother="chebyshev", pre=3, post=3):
+        """saena_b200_solve_pcg_block: rhs (k, n) -> (u (k, n), iters [k], [history of each column]); column j is
+        bit for bit what solve_pcg(rhs[j]) gives.  rhs may be a CUDA torch tensor (float64, contiguous): it then goes
+        to the device-pointer entry and u comes back as a torch tensor on the same device."""
+        n = self.level_rows[0]
+        dev = hasattr(rhs, "is_cuda") and rhs.is_cuda
+        if dev:
+            import torch
+            if rhs.dtype != torch.float64 or not rhs.is_contiguous() or rhs.dim() != 2 or rhs.shape[1] != n:
+                raise ValueError(f"solve_pcg_block: a device tensor must be contiguous float64 of shape (k, {n})")
+            u = torch.zeros_like(rhs)
+            with torch.cuda.device(rhs.device):
+                torch.cuda.current_stream().synchronize()   # rhs and u are complete before the library reads them
+            fn, a, b = self._L.saena_b200_solve_pcg_block_dev, ctypes.c_void_p(rhs.data_ptr()), ctypes.c_void_p(u.data_ptr())
+        else:
+            rhs = self._block(rhs, n)
+            u = np.zeros_like(rhs)
+            fn, a, b = self._L.saena_b200_solve_pcg_block, _vp(rhs), _vp(u)
+        k = int(rhs.shape[0])
+        iters, lens = np.zeros(max(k, 1), np.int32), np.zeros(max(k, 1), np.int32)
+        cap = max_iter + 2
+        hist = np.zeros((max(k, 1), cap), F64)
+        self._ck(fn(self._h, k, a, b, int(max_iter), float(tol), smoother_id(smoother), int(pre), int(post),
+                    _i32p(iters), _f64p(hist), cap, _i32p(lens)))
+        return u, iters[:k].tolist(), [hist[j, :lens[j]] for j in range(k)]
+
+    def matvec_block(self, level: int, kind: int, v) -> np.ndarray:
+        op = self._op(level, kind)
+        v = self._block(v, op.n_local_cols)
+        w = np.zeros((v.shape[0], op.M), F64)
+        self._ck(self._L.saena_b200_matvec_block(self._h, level, kind, v.shape[0], _vp(v), _vp(w)))
+        return w
+
+    def residual_block(self, level, u, rhs) -> np.ndarray:
+        n = self.level_rows[level]
+        u, rhs = self._block(u, n), self._block(rhs, n)
+        res = np.zeros_like(u)
+        self._ck(self._L.saena_b200_residual_block(self._h, level, u.shape[0], _vp(u), _vp(rhs), _vp(res)))
+        return res
+
+    def smooth_block(self, level, smoother, iters, u, rhs) -> np.ndarray:
+        n = self.level_rows[level]
+        u, rhs = self._block(u, n).copy(), self._block(rhs, n)
+        self._ck(self._L.saena_b200_smooth_block(self._h, level, smoother_id(smoother), int(iters), u.shape[0], _vp(u),
+                                                 _vp(rhs)))
+        return u
+
+    def vcycle_block(self, level, u, rhs, pre=3, post=3, smoother="chebyshev") -> np.ndarray:
+        n = self.level_rows[level]
+        u, rhs = self._block(u, n).copy(), self._block(rhs, n)
+        self._ck(self._L.saena_b200_vcycle_block(self._h, level, smoother_id(smoother), int(pre), int(post),
+                                                 u.shape[0], _vp(u), _vp(rhs)))
+        return u
 
     # ---- hooks ----
     def _op(self, level, kind) -> Operator:
