@@ -312,7 +312,8 @@ int saena_b200_vcycle_block(saena_b200_ctx *ctx, int level, int smoother, int pr
 /* ---- measurement ---------------------------------------------------------------------------
  * Device-resident timing loops for bench.py: `reps` applications of one operator / smoother
  * sweep, each launch bracketed by CUDA events on the launching stream; returns the median
- * milliseconds per launch.  KIND_A of a level on the route (saena_b200_set_level_route) times the route. */
+ * milliseconds per launch.  KIND_A of a level on the route (saena_b200_set_level_route) times the route.  While the
+ * preconditioner precision is 32 (saena_b200_set_precond_precision) both time the FP32 kernels the V-cycle runs. */
 int saena_b200_time_matvec(saena_b200_ctx *ctx, int level, int kind, int reps, int flush_l2, float *ms_out);
 int saena_b200_time_smooth_sweep(saena_b200_ctx *ctx, int level, int smoother, int reps, int flush_l2,
                                  float *ms_out);
@@ -340,7 +341,8 @@ int saena_b200_time_residual_restrict(saena_b200_ctx *ctx, int level, const doub
 int saena_b200_set_fused_restrict(saena_b200_ctx *ctx, int levels);
 int saena_b200_timer_start(saena_b200_ctx *ctx);
 /* ms per V-cycle entered at `level` from a zero iterate (reps back-to-back, eager, collective over
- * the ranks); the difference between consecutive levels is one level's cost inside a solve */
+ * the ranks); the difference between consecutive levels is one level's cost inside a solve.  While the preconditioner
+ * precision is 32 (saena_b200_set_precond_precision) it times the FP32 V-cycle, which is what the solve runs. */
 int saena_b200_time_vcycle(saena_b200_ctx *ctx, int level, int smoother, int pre, int post, int reps, float *ms_out);
 int saena_b200_timer_stop(saena_b200_ctx *ctx, float *ms_out);
 /* kernels launched by this context since init (bench.py's gpu_launches) */
@@ -396,8 +398,30 @@ int saena_b200_get_mapping(const saena_b200_ctx *ctx, int level, int kind);
  * level: not eligible, not fewer bytes, or the check failed). */
 int saena_b200_set_level_route(saena_b200_ctx *ctx, int level, int on);
 int saena_b200_get_level_route(const saena_b200_ctx *ctx, int level, float *ms_stored, float *ms_route);
-/* algorithmic bytes of one application of an operator (SURVEY.md 8d formula), for the roofline */
+/* algorithmic bytes of one application of an operator (SURVEY.md 8d formula), for the roofline.  While the
+ * preconditioner precision is 32: the FP32 V-cycle's bytes, 4-byte values and vector elements (column ids and row
+ * offsets unchanged). */
 int64_t saena_b200_operator_bytes(const saena_b200_ctx *ctx, int level, int kind);
+
+/* FP32 preconditioner.  bits = 64 (default) or 32.  At 32, saena_b200_solve_pcg and _pcg_dev apply the preconditioner
+ * as an FP32 V-cycle: r is rounded to float, the V-cycle runs from a zero iterate on float vectors and FP32 copies of the
+ * operators' values (same smoother, constants, route and graphs; the coarsest level's FP64 solve between two
+ * conversions), and its iterate is widened to double.  The Krylov loop stays FP64: the residual recurrence, alpha, beta,
+ * the dots, the stop test and u.  solve_vcycle, solve_cg and solve_smoother ignore the switch.  The FP32 copies follow
+ * every later update_values, set_mapping, autotune_mapping, set_level_route, set_operator_dense and
+ * set_coarsest_solver: they are rebuilt before the next FP32 use.  Refused (non-zero, the switch stays at 64, the
+ * reason in last_error): bits other than 32 / 64; several ranks or a detached share; a context not finalized; a scaled
+ * hierarchy; a repartitioning level; an operator with a halo, in the merged layout or on streaming row blocks (negative
+ * mapping codes); a failed allocation.  finalize resets the switch to 64.  While it is 32 the block solve and its hooks
+ * refuse. */
+int saena_b200_set_precond_precision(saena_b200_ctx *ctx, int bits);
+int saena_b200_get_precond_precision(const saena_b200_ctx *ctx);
+/* The per-operator hooks on the FP32 path (float vectors on the host; refused unless the precision is 32):
+ * w = Op v, res = A u - rhs, `iters` smoother sweeps on u in place, one FP32 V-cycle on u in place. */
+int saena_b200_matvec_f32(saena_b200_ctx *ctx, int level, int kind, const float *v, float *w);
+int saena_b200_residual_f32(saena_b200_ctx *ctx, int level, const float *u, const float *rhs, float *res);
+int saena_b200_smooth_f32(saena_b200_ctx *ctx, int level, int smoother, int iters, float *u, const float *rhs);
+int saena_b200_vcycle_f32(saena_b200_ctx *ctx, int level, int smoother, int pre, int post, float *u, const float *rhs);
 
 #ifdef __cplusplus
 }

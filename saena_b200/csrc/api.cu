@@ -108,6 +108,7 @@ int saena_b200_destroy(saena_b200_ctx *ctx) {
     sb_sync_stream(ctx, ctx->comm_stream);
     sb_invalidate_graphs(ctx);
     sb_arena_free(ctx);
+    sb_f32_free(ctx);
     for (size_t l = 0; l < ctx->levels.size(); ++l) {
         DevLevel &lv = ctx->levels[l];
         sb_free_operator(lv.A); sb_free_operator(lv.P); sb_free_operator(lv.R);
@@ -370,7 +371,132 @@ int sb_block_reserve(saena_b200_ctx *ctx, int k) {
     return 0;
 }
 
+// ---------------------------------------------------------------------------------------------
+// FP32 preconditioner state (saena_b200_set_precond_precision)
+// ---------------------------------------------------------------------------------------------
+void sb_f32_free(saena_b200_ctx *ctx) {
+    for (size_t i = 0; i < ctx->graphs.size(); ++i)
+        if (ctx->graphs[i].bits == 32) {
+            if (ctx->graphs[i].exec) cudaGraphExecDestroy(ctx->graphs[i].exec);
+            ctx->graphs.erase(ctx->graphs.begin() + i);
+            --i;
+        }
+    for (DevLevel &lv : ctx->levels) {
+        float **vecs[] = {&lv.u32[0], &lv.u32[1], &lv.d32, &lv.res32, &lv.rhs32, &lv.inv_diag32};
+        for (float **v : vecs) { cudaFree(*v); *v = nullptr; }
+        for (DevOperator *op : {&lv.A, &lv.P, &lv.R}) {
+            float **vals[] = {&op->val32, &op->sell.val32, &op->sellp.val32, &op->sdiag_val32};
+            for (float **v : vals) { cudaFree(*v); *v = nullptr; }
+        }
+    }
+    cudaFree(ctx->route32_t); cudaFree(ctx->route32_s);
+    ctx->route32_t = ctx->route32_s = nullptr;
+}
+
+// nullptr when the hierarchy can run the FP32 preconditioner, else why not: every operator needs an FP32 body
+// (spmv_f32.cu) and the V-cycle no FP64-only step
+static const char *f32_refusal(const saena_b200_ctx *ctx) {
+    if (ctx->nranks != 1 || ctx->detached) return "one rank only";
+    if (!ctx->finalized) return "call saena_b200_finalize first";
+    if (ctx->scale) return "not on a scaled hierarchy";
+    const size_t L = ctx->levels.size();
+    for (size_t l = 0; l < L; ++l) {
+        const DevLevel &lv = ctx->levels[l];
+        if (l + 1 < L && !lv.repart.identity()) return "a level repartitions its coarse vector";
+        for (const DevOperator *op : {&lv.A, &lv.P, &lv.R}) {
+            if (!op->present) continue;
+            if (!op->sends.empty() || !op->recvs.empty() || op->nnz_remote > 0 || op->merged)
+                return "an operator has a halo or is in the merged layout";
+            if (op->mapping < 0) return "an operator is on streaming row blocks";
+        }
+    }
+    return nullptr;
+}
+
+// stored entries of a sliced layout: the last slice offset
+static int sliced_entries(saena_b200_ctx *ctx, const SlicedLayout &s, int n_slices, long long *out) {
+    SB_CUDA(cudaMemcpy(out, s.ptr + n_slices, sizeof(long long), cudaMemcpyDeviceToHost));
+    return 0;
+}
+
+static int f32_build(saena_b200_ctx *ctx) {
+    bool ok = true;
+    auto grab = [&](float **p, size_t n) {
+        if (!ok) return;
+        ok = cudaMalloc((void **)p, sizeof(float) * std::max<size_t>(n, 1)) == cudaSuccess &&
+             cudaMemsetAsync(*p, 0, sizeof(float) * std::max<size_t>(n, 1), ctx->stream) == cudaSuccess;
+    };
+    // FP32 copy of `n` FP64 values
+    auto copy = [&](float **p, const double *src, size_t n) -> int {
+        grab(p, n);
+        if (ok && n) SB_TRY(sb_convert(ctx, n, src, *p));
+        return 0;
+    };
+    for (DevLevel &lv : ctx->levels) {
+        // every work vector sized from the level's rows, as its FP64 twin
+        for (float **v : {&lv.u32[0], &lv.u32[1], &lv.d32, &lv.res32, &lv.rhs32}) grab(v, lv.M);
+        SB_TRY(copy(&lv.inv_diag32, lv.inv_diag, lv.M));
+        for (DevOperator *op : {&lv.A, &lv.P, &lv.R}) {
+            if (!op->present || !ok) continue;
+            long long n = 0;
+            if (op->mapping == SB_MAPPING_SELL) {
+                SB_TRY(sliced_entries(ctx, op->sell, (op->M + 31) / 32, &n));
+                SB_TRY(copy(&op->sell.val32, op->sell.val, n));
+            } else if (op->mapping == SB_MAPPING_SELLP) {
+                SB_TRY(sliced_entries(ctx, op->sellp, (op->M + 255) / 256 * 8, &n));
+                SB_TRY(copy(&op->sellp.val32, op->sellp.val, n));
+            } else if (op->mapping == SB_MAPPING_SYMDIAG) {
+                SB_TRY(copy(&op->sdiag_val32, op->sdiag_val, (size_t)op->sdiag.nd * op->M));
+            } else {
+                SB_TRY(copy(&op->val32, op->val, op->nnz_local));
+            }
+        }
+    }
+    if (ctx->route_cap > 0) {
+        grab(&ctx->route32_t, ctx->route_cap);
+        grab(&ctx->route32_s, ctx->route_cap);
+    }
+    if (!ok) {
+        cudaGetLastError();   // an out-of-memory status is not sticky
+        SB_FAIL("set_precond_precision: not enough device memory for the FP32 copies");
+    }
+    return sb_sync_stream(ctx, ctx->stream);
+}
+
+int sb_f32_sync(saena_b200_ctx *ctx) {
+    if (ctx->precond_bits != 32 || !ctx->f32_stale) return 0;
+    sb_f32_free(ctx);   // the copies of layouts no longer in use, and every captured FP32 V-cycle
+    const char *why = f32_refusal(ctx);
+    const int rc = why ? 1 : f32_build(ctx);
+    if (rc) {
+        sb_f32_free(ctx);
+        ctx->precond_bits = 64;
+        if (why) SB_FAIL(std::string("precision 32: ") + why + "; the preconditioner stays FP64");
+        return rc;
+    }
+    ctx->f32_stale = false;
+    return 0;
+}
+
 extern "C" {
+
+int saena_b200_set_precond_precision(saena_b200_ctx *ctx, int bits) {
+    if (!ctx) return 1;
+    SB_CUDA(cudaSetDevice(ctx->device));
+    if (bits != 32 && bits != 64) SB_FAIL("set_precond_precision: bits must be 32 or 64");
+    if (bits == 64) {
+        sb_f32_free(ctx);
+        ctx->precond_bits = 64;
+        return 0;
+    }
+    if (ctx->precond_bits != 32) {
+        ctx->precond_bits = 32;
+        ctx->f32_stale = true;
+    }
+    return sb_f32_sync(ctx);
+}
+
+int saena_b200_get_precond_precision(const saena_b200_ctx *ctx) { return ctx ? ctx->precond_bits : 0; }
 
 int saena_b200_finalize(saena_b200_ctx *ctx) {
     if (!ctx) return 1;
@@ -386,6 +512,8 @@ int saena_b200_finalize(saena_b200_ctx *ctx) {
     }
     route_free(ctx);
     sb_block_free(ctx);
+    sb_f32_free(ctx);
+    ctx->precond_bits = 64;
     SB_TRY(sb_arena_build(ctx));  // ghost buffers of every operator, one allocation (p2p_halo.cu)
     for (int l = 0; l < L; ++l) {
         DevLevel &lv = ctx->levels[l];
@@ -558,12 +686,15 @@ static int stage_buf(saena_b200_ctx *ctx, int i, size_t n) {
     }
     return 0;
 }
-static int h2d(saena_b200_ctx *ctx, double *dst, const double *src, size_t n) {
-    if (n) SB_CUDA(cudaMemcpyAsync(dst, src, n * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+extern "C++" {   // templates, inside the extern "C" block of the entry points
+template <typename T>
+static int h2d(saena_b200_ctx *ctx, T *dst, const T *src, size_t n) {
+    if (n) SB_CUDA(cudaMemcpyAsync(dst, src, n * sizeof(T), cudaMemcpyHostToDevice, ctx->stream));
     return 0;
 }
-static int d2h(saena_b200_ctx *ctx, double *dst, const double *src, size_t n) {
-    if (n) SB_CUDA(cudaMemcpyAsync(dst, src, n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+template <typename T>
+static int d2h(saena_b200_ctx *ctx, T *dst, const T *src, size_t n) {
+    if (n) SB_CUDA(cudaMemcpyAsync(dst, src, n * sizeof(T), cudaMemcpyDeviceToHost, ctx->stream));
     SB_TRY(sb_sync_stream(ctx, ctx->stream));
     return sb_check_fault(ctx);   // every host-buffer entry point ends here: a timed-out exchange is an error status
 }
@@ -575,10 +706,12 @@ static DevOperator *get_op(saena_b200_ctx *ctx, int level, int kind) {
 }
 
 // what the solve applies for (level, kind): A through sb_apply_level_A (the route on a route level)
-static int apply_kind(saena_b200_ctx *ctx, int level, int kind, const double *x, int epi, const EpiArgs &e) {
+template <typename V>
+static int apply_kind(saena_b200_ctx *ctx, int level, int kind, const V *x, int epi, const EpiArgsT<V> &e) {
     if (kind == SAENA_B200_KIND_A) return sb_apply_level_A(ctx, level, x, epi, e);
     return sb_apply(ctx, *get_op(ctx, level, kind), x, epi, e);
 }
+}  // extern "C++"
 
 // ---------------------------------------------------------------------------------------------
 // Krylov drivers (device-resident vectors; one host read of <r,r> per iteration for the stop test)
@@ -586,6 +719,19 @@ static int apply_kind(saena_b200_ctx *ctx, int level, int kind, const double *x,
 static void push_hist(double v, double *hist, int cap, int &n) {
     if (hist && n < cap) hist[n] = sqrt(v);
     ++n;
+}
+
+// rho = M^-1 r from a zero iterate into level 0's u[cur].  Precision 32: r rounded into level 0's FP32 rhs, the FP32
+// V-cycle, its iterate widened into u[0] (cur = 0); the Krylov loop around it stays FP64.
+static int precondition(saena_b200_ctx *ctx, int smoother, int pre, int post, const double *r) {
+    if (ctx->precond_bits != 32) return sb_vcycle_from_zero(ctx, smoother, pre, post, r);
+    SB_TRY(sb_f32_sync(ctx));
+    DevLevel &l0 = ctx->levels[0];
+    SB_TRY(sb_convert(ctx, l0.M, r, l0.rhs32));
+    SB_TRY(sb_vcycle_from_zero(ctx, smoother, pre, post, (const float *)l0.rhs32));
+    SB_TRY(sb_convert(ctx, l0.M, l0.u32[l0.cur], l0.u[0]));
+    l0.cur = 0;
+    return 0;
 }
 
 static int pcg_device(saena_b200_ctx *ctx, const double *rhs, double *u, int max_iter, double tol, int smoother,
@@ -622,7 +768,7 @@ static int pcg_device(saena_b200_ctx *ctx, const double *rhs, double *u, int max
         return 0;
     }
     // rho = 0; vcycle(rho, r) (:2535-2537); rho lives in level 0's iterate buffers
-    SB_TRY(sb_vcycle_from_zero(ctx, smoother, pre, post, r));
+    SB_TRY(precondition(ctx, smoother, pre, post, r));
     // p = rho (:2554)
     if (n) SB_CUDA(cudaMemcpyAsync(p, l0.u[l0.cur], sizeof(double) * n, cudaMemcpyDeviceToDevice, ctx->stream));
     const double THRSHLD = init_dot * tol * tol;  // :2558
@@ -638,7 +784,7 @@ static int pcg_device(saena_b200_ctx *ctx, const double *rhs, double *u, int max
         current_dot = ctx->scalars_host[S_RR];
         push_hist(current_dot, hist, hist_cap, nh);
         if (!(current_dot >= THRSHLD)) break;          // :2620 (NaN also stops)
-        { SbRange rg(ctx, "vcycle_pCG"); SB_TRY(sb_vcycle_from_zero(ctx, smoother, pre, post, r)); }  // :2640-2641
+        { SbRange rg(ctx, "vcycle_pCG"); SB_TRY(precondition(ctx, smoother, pre, post, r)); }  // :2640-2641
         SB_TRY(sb_dot(ctx, r, l0.u[l0.cur], n, S_BETA_NUM));      // :2655
         SB_TRY(sb_pcg_p_update(ctx, n, p, l0.u[l0.cur]));          // :2662-2667
     }
@@ -876,6 +1022,68 @@ int saena_b200_dot(saena_b200_ctx *ctx, const double *a, const double *b, int n,
 }
 
 // ---------------------------------------------------------------------------------------------
+// FP32 hooks: the per-operator hooks above on the FP32 copies and vectors (precision 32 only); staged through the
+// same buffers, which hold n floats where they hold n doubles
+// ---------------------------------------------------------------------------------------------
+#define SB_ENTER_F32(name)                                                                       \
+    SB_ENTER();                                                                                  \
+    if (ctx->precond_bits != 32) SB_FAIL(name ": call saena_b200_set_precond_precision(ctx, 32) first"); \
+    SB_TRY(sb_f32_sync(ctx))
+
+static float *stage32(saena_b200_ctx *ctx, int i) { return (float *)ctx->stage[i]; }
+
+int saena_b200_matvec_f32(saena_b200_ctx *ctx, int level, int kind, const float *v, float *w) {
+    SB_ENTER_F32("matvec_f32");
+    DevOperator *op = get_op(ctx, level, kind);
+    if (!op) SB_FAIL("matvec_f32: no such operator");
+    SB_TRY(stage_buf(ctx, 0, op->n_local_cols));
+    SB_TRY(stage_buf(ctx, 1, op->M));
+    SB_TRY(h2d(ctx, stage32(ctx, 0), v, op->n_local_cols));
+    EpiArgs32 e{};
+    e.out = stage32(ctx, 1);
+    SB_TRY(apply_kind(ctx, level, kind, (const float *)stage32(ctx, 0), EPI_PLAIN, e));
+    return d2h(ctx, w, stage32(ctx, 1), op->M);
+}
+
+int saena_b200_residual_f32(saena_b200_ctx *ctx, int level, const float *u, const float *rhs, float *res) {
+    SB_ENTER_F32("residual_f32");
+    DevOperator *op = get_op(ctx, level, SAENA_B200_KIND_A);
+    if (!op) SB_FAIL("residual_f32: no such level");
+    for (int i = 0; i < 3; ++i) SB_TRY(stage_buf(ctx, i, op->M));
+    SB_TRY(h2d(ctx, stage32(ctx, 0), u, op->M));
+    SB_TRY(h2d(ctx, stage32(ctx, 1), rhs, op->M));
+    EpiArgs32 e{};
+    e.rhs = stage32(ctx, 1);
+    e.out = stage32(ctx, 2);
+    SB_TRY(sb_apply_level_A(ctx, level, (const float *)stage32(ctx, 0), EPI_RESIDUAL, e));
+    return d2h(ctx, res, stage32(ctx, 2), op->M);
+}
+
+int saena_b200_smooth_f32(saena_b200_ctx *ctx, int level, int smoother, int iters, float *u, const float *rhs) {
+    SB_ENTER_F32("smooth_f32");
+    if (level < 0 || level >= (int)ctx->levels.size()) SB_FAIL("smooth_f32: no such level");
+    DevLevel &lv = ctx->levels[level];
+    SB_TRY(stage_buf(ctx, 1, lv.M));
+    lv.cur = 0;
+    SB_TRY(h2d(ctx, lv.u32[0], u, lv.M));
+    SB_TRY(h2d(ctx, stage32(ctx, 1), rhs, lv.M));
+    SB_TRY(sb_smooth(ctx, level, smoother, iters, (const float *)stage32(ctx, 1), false));
+    return d2h(ctx, u, lv.u32[lv.cur], lv.M);
+}
+
+int saena_b200_vcycle_f32(saena_b200_ctx *ctx, int level, int smoother, int pre, int post, float *u, const float *rhs) {
+    SB_ENTER_F32("vcycle_f32");
+    if (level < 0 || level >= (int)ctx->levels.size()) SB_FAIL("vcycle_f32: no such level");
+    DevLevel &lv = ctx->levels[level];
+    SB_TRY(stage_buf(ctx, 1, lv.M));
+    lv.cur = 0;
+    SB_TRY(h2d(ctx, lv.u32[0], u, lv.M));
+    SB_TRY(h2d(ctx, stage32(ctx, 1), rhs, lv.M));
+    SB_TRY(sb_vcycle(ctx, level, smoother, pre, post, (const float *)stage32(ctx, 1), false));
+    return d2h(ctx, u, lv.u32[lv.cur], lv.M);
+}
+
+// ---------------------------------------------------------------------------------------------
 // block solve: k <= SB_BLOCK_MAX right-hand sides on one hierarchy, every operator streamed once for all of them.
 // Column j gives what saena_b200_solve_pcg gives for right-hand side j: each column has its own alpha, beta, init_dot
 // and stop test, and once it has stopped its u, r and p are left as they are (the PCG updates skip it) while the
@@ -883,6 +1091,8 @@ int saena_b200_dot(saena_b200_ctx *ctx, const double *a, const double *b, int n,
 // ---------------------------------------------------------------------------------------------
 static int block_enter(saena_b200_ctx *ctx, int k) {
     if (k < 1 || k > SB_BLOCK_MAX) SB_FAIL("block call: k must be in 1..8");
+    // column j is the single solve's bits: with the FP32 preconditioner that would be an FP32 block V-cycle
+    if (ctx->precond_bits == 32) SB_FAIL("block call: not while the preconditioner precision is 32");
     if (ctx->nranks > 1) SB_FAIL("block call: one rank only (the halo exchange has no block form)");
     return sb_block_reserve(ctx, k);
 }
@@ -1069,16 +1279,21 @@ int saena_b200_time_matvec(saena_b200_ctx *ctx, int level, int kind, int reps, i
     SB_ENTER();
     DevOperator *op = get_op(ctx, level, kind);
     if (!op) SB_FAIL("time_matvec: no such operator");
+    const bool f32 = ctx->precond_bits == 32;
+    if (f32) SB_TRY(sb_f32_sync(ctx));
     SB_TRY(stage_buf(ctx, 0, op->n_local_cols));
     SB_TRY(stage_buf(ctx, 1, op->M));
     SB_CUDA(cudaMemsetAsync(ctx->stage[0], 0, sizeof(double) * op->n_local_cols, ctx->stream));
     EpiArgs e{};
     e.out = ctx->stage[1];
+    EpiArgs32 e32{};
+    e32.out = stage32(ctx, 1);
     std::vector<float> t;
     for (int it = 0; it < reps; ++it) {
         if (do_flush) SB_TRY(flush_l2(ctx));
         SB_CUDA(cudaEventRecord(ctx->ev_t0, ctx->stream));
-        SB_TRY(apply_kind(ctx, level, kind, ctx->stage[0], EPI_PLAIN, e));
+        if (f32) SB_TRY(apply_kind(ctx, level, kind, (const float *)stage32(ctx, 0), EPI_PLAIN, e32));
+        else SB_TRY(apply_kind(ctx, level, kind, (const double *)ctx->stage[0], EPI_PLAIN, e));
         SB_CUDA(cudaEventRecord(ctx->ev_t1, ctx->stream));
         SB_TRY(sb_sync_stream(ctx, ctx->stream));
         float ms = 0.f;
@@ -1522,13 +1737,16 @@ int saena_b200_time_smooth_sweep(saena_b200_ctx *ctx, int level, int smoother, i
     SB_ENTER();
     if (level < 0 || level >= (int)ctx->levels.size()) SB_FAIL("time_smooth_sweep: no such level");
     DevLevel &lv = ctx->levels[level];
+    const bool f32 = ctx->precond_bits == 32;
+    if (f32) SB_TRY(sb_f32_sync(ctx));
     SB_TRY(stage_buf(ctx, 1, lv.M));
     SB_CUDA(cudaMemsetAsync(ctx->stage[1], 0, sizeof(double) * lv.M, ctx->stream));
     std::vector<float> t;
     for (int it = 0; it < reps; ++it) {
         if (do_flush) SB_TRY(flush_l2(ctx));
         SB_CUDA(cudaEventRecord(ctx->ev_t0, ctx->stream));
-        SB_TRY(sb_smooth(ctx, level, smoother, 1, ctx->stage[1], false));
+        if (f32) SB_TRY(sb_smooth(ctx, level, smoother, 1, (const float *)stage32(ctx, 1), false));
+        else SB_TRY(sb_smooth(ctx, level, smoother, 1, (const double *)ctx->stage[1], false));
         SB_CUDA(cudaEventRecord(ctx->ev_t1, ctx->stream));
         SB_TRY(sb_sync_stream(ctx, ctx->stream));
         float ms = 0.f;
@@ -1546,11 +1764,14 @@ int saena_b200_time_vcycle(saena_b200_ctx *ctx, int level, int smoother, int pre
     SB_ENTER();
     if (level < 0 || level >= (int)ctx->levels.size() || reps < 1) SB_FAIL("time_vcycle: no such level");
     DevLevel &lv = ctx->levels[level];
+    const bool f32 = ctx->precond_bits == 32;
+    if (f32) SB_TRY(sb_f32_sync(ctx));
     const double *rhs = level == 0 ? ctx->pcg_r : lv.rhs;
     for (int it = -1; it < reps; ++it) {   // one untimed pass first
         if (it == 0) SB_CUDA(cudaEventRecord(ctx->ev_t0, ctx->stream));
         for (size_t l = level; l < ctx->levels.size(); ++l) ctx->levels[l].cur = 0;
-        SB_TRY(sb_vcycle(ctx, level, smoother, pre, post, rhs, true));
+        if (f32) SB_TRY(sb_vcycle(ctx, level, smoother, pre, post, (const float *)lv.rhs32, true));
+        else SB_TRY(sb_vcycle(ctx, level, smoother, pre, post, rhs, true));
     }
     SB_CUDA(cudaEventRecord(ctx->ev_t1, ctx->stream));
     SB_TRY(sb_sync_stream(ctx, ctx->stream));
@@ -1656,7 +1877,8 @@ int64_t saena_b200_operator_bytes(const saena_b200_ctx *ctx, int level, int kind
     if (!ctx || level < 0 || level >= (int)ctx->levels.size()) return -1;
     const DevOperator &op = ctx->levels[level].op(kind);
     if (!op.present) return -1;
-    return kind == SAENA_B200_KIND_A ? sb_level_A_bytes(ctx, level) : sb_operator_bytes(op);
+    const int vb = ctx->precond_bits == 32 ? 4 : 8;   // what the V-cycle streams
+    return kind == SAENA_B200_KIND_A ? sb_level_A_bytes(ctx, level, vb) : sb_operator_bytes(op, vb);
 }
 
 }  // extern "C"

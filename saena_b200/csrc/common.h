@@ -51,15 +51,20 @@ enum EpiKind {
     EPI_COUNT = 6
 };
 
-struct EpiArgs {
-    const double *rhs;
-    const double *inv_diag;
-    const double *d_in;
-    double *d_out;
-    const double *u_in;
-    double *out;
-    double c1, c2;
+template <typename V>
+struct EpiArgsT {
+    const V *rhs;
+    const V *inv_diag;
+    const V *d_in;
+    V *d_out;
+    const V *u_in;
+    V *out;
+    V c1, c2;
 };
+using EpiArgs = EpiArgsT<double>;
+// the FP32 preconditioner's (saena_b200_set_precond_precision): float vectors, the constants computed in double on the
+// host and rounded to float at launch
+using EpiArgs32 = EpiArgsT<float>;
 
 // ---------------------------------------------------------------------------------------------
 // device-side operator
@@ -99,6 +104,7 @@ struct SlicedLayout {
     int *perm = nullptr;
     int *col = nullptr;
     double *val = nullptr;
+    float *val32 = nullptr;  // FP32 copy of val (FP32 preconditioner, sb_f32_sync); shares ptr, perm and col
 };
 
 // the stored diagonals of mapping 103: off[0] = 0, then the positive offsets ascending (kernel argument, by value)
@@ -125,6 +131,7 @@ struct DevOperator {
     void *rowptr = nullptr;  // int32[M+1] or int64[M+1]
     int *col = nullptr;
     double *val = nullptr;
+    float *val32 = nullptr;  // FP32 copy of val while a mapping 1..256 is in use at precision 32 (sb_f32_sync)
 
     // row blocks of the streaming kernel: rows [blk_row[b], blk_row[b+1]) hold <= STREAM_TILE nnz
     int *blk_row = nullptr;
@@ -148,6 +155,7 @@ struct DevOperator {
     SymDiagOffsets sdiag;
     int sdiag_n = -1;
     double *sdiag_val = nullptr;
+    float *sdiag_val32 = nullptr;  // FP32 copy of sdiag_val (sb_f32_sync)
 
     // remote block re-sorted by row at upload: boundary rows only
     // interior rows = the contiguous range [int_lo, int_hi) (multiples of 32) that holds no row with
@@ -237,18 +245,36 @@ struct DevLevel {
     double *bu[2] = {nullptr, nullptr};
     int bcur = 0;
     double *bd = nullptr, *bres = nullptr, *brhs = nullptr, *bxfer_old = nullptr;
+
+    // FP32 preconditioner (precision 32, sb_f32_sync): the work vectors above in float, with the same ping-pong parity
+    // cur; level 0's rhs32 is the converted PCG residual.  inv_diag32: inv_diag rounded to float.
+    float *u32[2] = {nullptr, nullptr};
+    float *d32 = nullptr, *res32 = nullptr, *rhs32 = nullptr, *inv_diag32 = nullptr;
 };
+
+// a level's work vectors in one precision: what the templated smoother and V-cycle of solve.cu run on
+template <typename V>
+struct LevelVecs {
+    V **u;
+    V *d, *res, *rhs;
+    const V *inv_diag;
+};
+inline LevelVecs<double> sb_level_vecs(DevLevel &lv, double) { return {lv.u, lv.d, lv.res, lv.rhs, lv.inv_diag}; }
+inline LevelVecs<float> sb_level_vecs(DevLevel &lv, float) {
+    return {lv.u32, lv.d32, lv.res32, lv.rhs32, lv.inv_diag32};
+}
 
 // A V-cycle from a zero iterate is the same launch sequence every time (same buffers, same
 // per-level Chebyshev constants): it is captured once per (rhs, smoother, pre, post) into a CUDA
 // graph and replayed -- the coarse levels are launch-latency-bound, ~90 launches per V-cycle.
 struct VcycleGraph {
-    const double *rhs;
+    const void *rhs;
     int smoother, pre, post;
     cudaGraphExec_t exec;
     int64_t launches;
     std::vector<int> cur_after;  // each level's ping-pong parity when the V-cycle ends
     int k = 0;                   // 0: the single V-cycle; 1..SB_BLOCK_MAX: the block V-cycle on k columns
+    int bits = 64;               // 64: the FP64 V-cycle; 32: the FP32 one (k = 0)
     // exec == nullptr: a multi-rank configuration that has run eagerly once and is captured at its next use
 };
 
@@ -329,6 +355,14 @@ struct saena_b200_ctx {
     double *route_t = nullptr, *route_s = nullptr;
     int route_cap = 0;
 
+    // FP32 preconditioner (saena_b200_set_precond_precision): 64 (default) or 32.  At 32 the FP32 copies of the values
+    // in use, inv_diag32 and the levels' float work vectors exist; f32_stale: some call since their last build may
+    // have changed values, layouts, the route or the coarsest solver (set by sb_invalidate_graphs), so sb_f32_sync
+    // builds them again before the next FP32 use.  route32_*: the route's intermediates in float.
+    int precond_bits = 64;
+    bool f32_stale = false;
+    float *route32_t = nullptr, *route32_s = nullptr;
+
     // L2 flush buffer for the timing loops
     void *flush_buf = nullptr;
     size_t flush_bytes = 0;
@@ -395,10 +429,17 @@ int sb_symdiag_plan(int M, int n_offsets, const int *offsets, int64_t nnz, int64
 int sb_refresh_symdiag(saena_b200_ctx *ctx, DevOperator &op);
 // w-style application of an operator with a fused epilogue; x is the local input vector.
 int sb_apply(saena_b200_ctx *ctx, DevOperator &op, const double *x, int epi, const EpiArgs &args);
+// ---- spmv_f32.cu
+// the same on the operator's FP32 copy (precision 32: one rank, no halo, not merged, no streaming row blocks)
+int sb_apply(saena_b200_ctx *ctx, DevOperator &op, const float *x, int epi, const EpiArgs32 &args);
+// dst = (float)src / (double)src, and the FP32 copies' cast
+int sb_convert(saena_b200_ctx *ctx, size_t n, const double *src, float *dst);
+int sb_convert(saena_b200_ctx *ctx, size_t n, const float *src, double *dst);
 // ---- spmv_block.cu
 // sb_apply on k column-major vectors: x's column j at x + j * n_local_cols, the epilogue's at + j * M (inv_diag shared)
 int sb_apply_block(saena_b200_ctx *ctx, DevOperator &op, int k, const double *x, int epi, const EpiArgs &args);
-int64_t sb_operator_bytes(const DevOperator &op);
+// algorithmic bytes of one application with vb-byte values and vector elements (8: FP64, 4: FP32 preconditioner)
+int64_t sb_operator_bytes(const DevOperator &op, int vb = 8);
 
 // ---- nccl_comm.cu
 int sb_nccl_unique_id(void *out, std::string &err);
@@ -452,6 +493,10 @@ int sb_pcg_p_update(saena_b200_ctx *ctx, int n, double *p, const double *rho);
 int sb_cg_p_update(saena_b200_ctx *ctx, int n, double *p, const double *r, int num_slot, int den_slot);
 int sb_negate_copy(saena_b200_ctx *ctx, int n, const double *src, double *dst);              // dst = -src
 int sb_fill_zero(saena_b200_ctx *ctx, double *p, size_t n);
+// float forms (FP32 preconditioner)
+int sb_cheb_first_zero(saena_b200_ctx *ctx, int n, const float *rhs, const float *inv_diag, float c, float *d, float *u);
+int sb_negate_copy(saena_b200_ctx *ctx, int n, const float *src, float *dst);
+int sb_fill_zero(saena_b200_ctx *ctx, float *p, size_t n);
 int sb_scale_vector(saena_b200_ctx *ctx, int n, double *v, const double *w);                   // v *= w (scale_vector)
 int sb_coarsest_apply(saena_b200_ctx *ctx, const double *rhs, double *u);
 int sb_coarsest_cg(saena_b200_ctx *ctx, const double *rhs, double *u);  // u: initial guess in, solution out
@@ -476,13 +521,20 @@ int sb_find_eig(saena_b200_ctx *ctx, int level, int max_iter, const double *star
                 double *eig_out, int *iters_out);
 
 // ---- solve.cu
+// Each with an FP64 and an FP32 form (the FP32 preconditioner): one template, the same steps on the level's work
+// vectors of that precision (sb_level_vecs), the operators through the sb_apply of that precision.
 // level l's operator with a fused epilogue: the stored A_l, or on a route level R_{l-1} A_{l-1} P_{l-1}
 int sb_apply_level_A(saena_b200_ctx *ctx, int l, const double *x, int epi, const EpiArgs &args);
-int64_t sb_level_A_bytes(const saena_b200_ctx *ctx, int l);  // algorithmic bytes of what sb_apply_level_A streams
+int sb_apply_level_A(saena_b200_ctx *ctx, int l, const float *x, int epi, const EpiArgs32 &args);
+int64_t sb_level_A_bytes(const saena_b200_ctx *ctx, int l, int vb = 8);  // algorithmic bytes of what sb_apply_level_A streams
 int sb_smooth(saena_b200_ctx *ctx, int l, int smoother, int iters, const double *rhs, bool u_is_zero);
+int sb_smooth(saena_b200_ctx *ctx, int l, int smoother, int iters, const float *rhs, bool u_is_zero);
 int sb_vcycle(saena_b200_ctx *ctx, int l, int smoother, int pre, int post, const double *rhs, bool u_is_zero);
-// level-0 V-cycle from a zero iterate, replayed from a CUDA graph when nothing in it needs the host
+int sb_vcycle(saena_b200_ctx *ctx, int l, int smoother, int pre, int post, const float *rhs, bool u_is_zero);
+// level-0 V-cycle from a zero iterate, replayed from a CUDA graph when nothing in it needs the host (graphs keyed by
+// precision too)
 int sb_vcycle_from_zero(saena_b200_ctx *ctx, int smoother, int pre, int post, const double *rhs);
+int sb_vcycle_from_zero(saena_b200_ctx *ctx, int smoother, int pre, int post, const float *rhs);
 void sb_invalidate_graphs(saena_b200_ctx *ctx);
 // the block forms on k columns of the levels' block buffers (DevLevel::bu[bcur] is the iterate)
 int sb_apply_level_A_block(saena_b200_ctx *ctx, int l, int k, const double *x, int epi, const EpiArgs &args);
@@ -497,3 +549,10 @@ int sb_vcycle_block_from_zero(saena_b200_ctx *ctx, int k, int smoother, int pre,
 // block V-cycle); a failed allocation leaves no block buffer and the context usable for single solves
 int sb_block_reserve(saena_b200_ctx *ctx, int k);
 void sb_block_free(saena_b200_ctx *ctx);
+
+// ---- api.cu (FP32 preconditioner)
+// Before every FP32 use: when stale, checks the refusal rules again, builds every FP32 copy anew from the FP64 data
+// (values of the layout in use, inv_diag, work vectors, the route's intermediates) and drops the captured FP32 V-cycles.
+// The one place the copies are written.  On a refusal or a failed allocation the context goes back to 64.
+int sb_f32_sync(saena_b200_ctx *ctx);
+void sb_f32_free(saena_b200_ctx *ctx);

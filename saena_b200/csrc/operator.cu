@@ -72,7 +72,7 @@ static int64_t sliced_padded_est(const std::vector<int64_t> &rp) {
 }
 
 static void free_sliced(SlicedLayout &s) {
-    cudaFree(s.ptr); cudaFree(s.perm); cudaFree(s.col); cudaFree(s.val);
+    cudaFree(s.ptr); cudaFree(s.perm); cudaFree(s.col); cudaFree(s.val); cudaFree(s.val32);
     s = SlicedLayout();
 }
 
@@ -86,6 +86,7 @@ void sb_free_operator(DevOperator &op) {
     free_sliced(op.sell);
     free_sliced(op.sellp);
     cudaFree(op.sdiag_val);
+    cudaFree(op.val32); cudaFree(op.sdiag_val32);
     cudaFree(op.x_round);
     cudaFree(op.rowmid); cudaFree(op.partial);
     op = DevOperator();
@@ -1008,10 +1009,11 @@ int sb_apply(saena_b200_ctx *ctx, DevOperator &op, const double *x, int epi, con
 }
 
 // algorithmic bytes of w = Op v (SURVEY.md 8d): nnz*(8+4) + M*p (row offsets) + N*8 (x once) + M*8 (w); on the
-// symmetric diagonals each stored diagonal once (its second, lagging read is expected from L2) + x + w
-int64_t sb_operator_bytes(const DevOperator &op) {
-    if (op.mapping == SB_MAPPING_SYMDIAG) return 8 * (int64_t)op.sdiag.nd * op.M + (int64_t)op.n_local_cols * 8 + (int64_t)op.M * 8;
+// symmetric diagonals each stored diagonal once (its second, lagging read is expected from L2) + x + w.  vb = 4: the
+// FP32 copy, 4-byte values and vector elements (the column ids and row offsets stay as they are)
+int64_t sb_operator_bytes(const DevOperator &op, int vb) {
+    if (op.mapping == SB_MAPPING_SYMDIAG) return vb * (int64_t)op.sdiag.nd * op.M + (int64_t)op.n_local_cols * vb + (int64_t)op.M * vb;
     const int64_t p = op.wide_offsets ? 8 : 4;
-    return (op.nnz_local + op.nnz_remote) * 12 + (int64_t)op.M * p + (int64_t)op.n_local_cols * 8 +
-           (int64_t)op.M * 8;
+    return (op.nnz_local + op.nnz_remote) * (vb + 4) + (int64_t)op.M * p + (int64_t)op.n_local_cols * vb +
+           (int64_t)op.M * vb;
 }

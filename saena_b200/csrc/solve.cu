@@ -12,9 +12,21 @@
 // ping-pongs between two buffers because a fused sweep must read the old u of other rows.  The
 // first sweep from a zero iterate (every coarse-level entry and the preconditioner's rho = 0)
 // needs no pass over A at all.  Prolongation is fused with the correction u -= P e.
+//
+// The FP32 preconditioner (saena_b200_set_precond_precision 32) runs the same smoother and V-cycle on float vectors and
+// the operators' FP32 copies: sb_apply_level_A, sb_smooth, sb_vcycle and sb_vcycle_from_zero are templates on the value
+// type V, instantiated for double and float.  Steps that only exist in FP64 -- repartitions, scaling, the fused residual
+// + restriction -- are compiled into the double form only (sb_f32_sync refuses hierarchies that need them), and the
+// coarsest level runs its FP64 solve between two conversions.
 #include <math.h>
 
+#include <type_traits>
+
 #include "common.h"
+
+// the route's two fine-level intermediates of each precision
+static double *route_buf(saena_b200_ctx *ctx, int i, double) { return i ? ctx->route_s : ctx->route_t; }
+static float *route_buf(saena_b200_ctx *ctx, int i, float) { return i ? ctx->route32_s : ctx->route32_t; }
 
 // Level l's operator.  Pairwise aggregation halves the rows of the fine level, but the Galerkin product A_l = R A P
 // of a short-row operator has far longer rows: on the 256^3 Poisson hierarchy A_1 has 68 entries a row and five times
@@ -22,48 +34,59 @@
 // is therefore applied as three SpMVs, each operator on its own mapping, through two fine-level intermediates; R's
 // rows are level l's rows, so the epilogue (residual, smoother update) fuses into the last one unchanged.  A_{l-1} is
 // always the stored operator.
-int sb_apply_level_A(saena_b200_ctx *ctx, int l, const double *x, int epi, const EpiArgs &args) {
+template <typename V>
+static int apply_level_A(saena_b200_ctx *ctx, int l, const V *x, int epi, const EpiArgsT<V> &args) {
     DevLevel &lv = ctx->levels[l];
     if (!lv.route) return sb_apply(ctx, lv.A, x, epi, args);
     DevLevel &fl = ctx->levels[l - 1];
     if (ctx->route_cap < fl.M) SB_FAIL("apply: route level without its intermediate vectors");
-    EpiArgs e{};
-    e.out = ctx->route_t;
+    V *t = route_buf(ctx, 0, V()), *s = route_buf(ctx, 1, V());
+    EpiArgsT<V> e{};
+    e.out = t;
     SB_TRY(sb_apply(ctx, fl.P, x, EPI_PLAIN, e));
-    e.out = ctx->route_s;
-    SB_TRY(sb_apply(ctx, fl.A, ctx->route_t, EPI_PLAIN, e));
-    return sb_apply(ctx, fl.R, ctx->route_s, epi, args);
+    e.out = s;
+    SB_TRY(sb_apply(ctx, fl.A, t, EPI_PLAIN, e));
+    return sb_apply(ctx, fl.R, s, epi, args);
 }
 
-int64_t sb_level_A_bytes(const saena_b200_ctx *ctx, int l) {
+int sb_apply_level_A(saena_b200_ctx *ctx, int l, const double *x, int epi, const EpiArgs &args) {
+    return apply_level_A(ctx, l, x, epi, args);
+}
+int sb_apply_level_A(saena_b200_ctx *ctx, int l, const float *x, int epi, const EpiArgs32 &args) {
+    return apply_level_A(ctx, l, x, epi, args);
+}
+
+int64_t sb_level_A_bytes(const saena_b200_ctx *ctx, int l, int vb) {
     const DevLevel &lv = ctx->levels[l];
-    if (!lv.route) return sb_operator_bytes(lv.A);
+    if (!lv.route) return sb_operator_bytes(lv.A, vb);
     const DevLevel &fl = ctx->levels[l - 1];
-    return sb_operator_bytes(fl.P) + sb_operator_bytes(fl.A) + sb_operator_bytes(fl.R);
+    return sb_operator_bytes(fl.P, vb) + sb_operator_bytes(fl.A, vb) + sb_operator_bytes(fl.R, vb);
 }
 
-int sb_smooth(saena_b200_ctx *ctx, int l, int smoother, int iters, const double *rhs, bool u_is_zero) {
+template <typename V>
+static int smooth(saena_b200_ctx *ctx, int l, int smoother, int iters, const V *rhs, bool u_is_zero) {
     DevLevel &lv = ctx->levels[l];
     if (iters <= 0 || lv.M == 0) {
         if (iters > 0 && (!lv.A.sends.empty() || !lv.A.recvs.empty())) SB_FAIL("smooth: empty rank with a halo plan");
         return 0;
     }
-    EpiArgs e{};
+    const LevelVecs<V> v = sb_level_vecs(lv, V());
+    EpiArgsT<V> e{};
     e.rhs = rhs;
-    e.inv_diag = lv.inv_diag;
+    e.inv_diag = v.inv_diag;
     if (smoother == SAENA_B200_JACOBI) {
         // u -= (omega D^-1)(A u - rhs), omega = float(2.0/3) promoted (saena_matrix.h:182)
-        e.c1 = (double)(float)(2.0 / 3);
+        e.c1 = V((double)(float)(2.0 / 3));
         int j = 0;
         if (u_is_zero) {
             // A*0 = 0: u = 0 - (0 - rhs)*(invd*omega) = (omega*invd)*rhs, no pass over A
-            SB_TRY(sb_cheb_first_zero(ctx, lv.M, rhs, lv.inv_diag, e.c1, lv.d, lv.u[lv.cur]));
+            SB_TRY(sb_cheb_first_zero(ctx, lv.M, rhs, v.inv_diag, e.c1, v.d, v.u[lv.cur]));
             j = 1;
         }
         for (; j < iters; ++j) {
-            e.u_in = lv.u[lv.cur];
-            e.out = lv.u[lv.cur ^ 1];
-            SB_TRY(sb_apply_level_A(ctx, l, lv.u[lv.cur], EPI_JACOBI, e));
+            e.u_in = v.u[lv.cur];
+            e.out = v.u[lv.cur ^ 1];
+            SB_TRY(sb_apply_level_A(ctx, l, v.u[lv.cur], EPI_JACOBI, e));
             lv.cur ^= 1;
         }
         return 0;
@@ -78,16 +101,16 @@ int sb_smooth(saena_b200_ctx *ctx, int l, int smoother, int iters, const double 
     const double s1 = theta / delta;
     const double twos1 = 2.0 * s1;
     double rhok = 1.0 / s1;
-    e.d_in = lv.d;
-    e.d_out = lv.d;
+    e.d_in = v.d;
+    e.d_out = v.d;
     // first sweep: d = (1/theta) D^-1 (rhs - A u); u += d
     if (u_is_zero) {
-        SB_TRY(sb_cheb_first_zero(ctx, lv.M, rhs, lv.inv_diag, 1.0 / theta, lv.d, lv.u[lv.cur]));
+        SB_TRY(sb_cheb_first_zero(ctx, lv.M, rhs, v.inv_diag, V(1.0 / theta), v.d, v.u[lv.cur]));
     } else {
-        e.c1 = 1.0 / theta;
-        e.u_in = lv.u[lv.cur];
-        e.out = lv.u[lv.cur ^ 1];
-        SB_TRY(sb_apply_level_A(ctx, l, lv.u[lv.cur], EPI_CHEB_FIRST, e));
+        e.c1 = V(1.0 / theta);
+        e.u_in = v.u[lv.cur];
+        e.out = v.u[lv.cur ^ 1];
+        SB_TRY(sb_apply_level_A(ctx, l, v.u[lv.cur], EPI_CHEB_FIRST, e));
         lv.cur ^= 1;
     }
     for (int i = 1; i < iters; ++i) {
@@ -96,38 +119,61 @@ int sb_smooth(saena_b200_ctx *ctx, int l, int smoother, int iters, const double 
         const double d1 = rhokp1 * rhok;
         const double d2 = two_rhokp1 / delta;
         rhok = rhokp1;
-        e.c1 = d1;
-        e.c2 = d2;
-        e.u_in = lv.u[lv.cur];
-        e.out = lv.u[lv.cur ^ 1];
-        SB_TRY(sb_apply_level_A(ctx, l, lv.u[lv.cur], EPI_CHEB_NEXT, e));
+        e.c1 = V(d1);
+        e.c2 = V(d2);
+        e.u_in = v.u[lv.cur];
+        e.out = v.u[lv.cur ^ 1];
+        SB_TRY(sb_apply_level_A(ctx, l, v.u[lv.cur], EPI_CHEB_NEXT, e));
         lv.cur ^= 1;
     }
     return 0;
 }
 
-// V-cycle on grid l with right-hand side `rhs`; the iterate is lv.u[lv.cur] on entry and exit.
-int sb_vcycle(saena_b200_ctx *ctx, int l, int smoother, int pre, int post, const double *rhs, bool u_is_zero) {
+int sb_smooth(saena_b200_ctx *ctx, int l, int smoother, int iters, const double *rhs, bool u_is_zero) {
+    return smooth(ctx, l, smoother, iters, rhs, u_is_zero);
+}
+int sb_smooth(saena_b200_ctx *ctx, int l, int smoother, int iters, const float *rhs, bool u_is_zero) {
+    return smooth(ctx, l, smoother, iters, rhs, u_is_zero);
+}
+
+// V-cycle on grid l with right-hand side `rhs`; the iterate is lv.u[lv.cur] (FP32: lv.u32[lv.cur]) on entry and exit.
+template <typename V>
+static int vcycle(saena_b200_ctx *ctx, int l, int smoother, int pre, int post, const V *rhs, bool u_is_zero) {
+    constexpr bool F64 = std::is_same<V, double>::value;
     const int max_level = (int)ctx->levels.size() - 1;
     DevLevel &lv = ctx->levels[l];
+    const LevelVecs<V> v = sb_level_vecs(lv, V());
     // solve.cpp:991-1057 coarsest level: direct solve on the rank that owns it
     if (l == max_level) {
-        SbRange rg(ctx, "coarsest", l);
-        if (lv.M > 0 && ctx->coarsest_cg) {
-            // direct_solver == "CG" (:998-999): u is the initial guess of solve_coarsest_CG
-            if (!lv.A.sends.empty() || !lv.A.recvs.empty()) SB_FAIL("vcycle: the coarsest level must live on one rank");
-            if (u_is_zero) SB_TRY(sb_fill_zero(ctx, lv.u[lv.cur], lv.M));
-            SB_TRY(sb_coarsest_cg(ctx, rhs, lv.u[lv.cur]));
-        } else if (lv.M > 0) {
-            if (ctx->coarse_n != lv.M) SB_FAIL("vcycle: no coarsest factor was uploaded for the coarsest level");
-            SB_TRY(sb_coarsest_apply(ctx, rhs, lv.u[lv.cur]));
+        if constexpr (!F64) {
+            // FP32: the FP64 solve between two conversions (res, unused on the coarsest level, holds the FP64 rhs); CG
+            // starts from the current iterate
+            if (lv.M > 0) {
+                SB_TRY(sb_convert(ctx, lv.M, rhs, lv.res));
+                if (ctx->coarsest_cg && !u_is_zero) SB_TRY(sb_convert(ctx, lv.M, v.u[lv.cur], lv.u[lv.cur]));
+                SB_TRY(sb_vcycle(ctx, l, smoother, pre, post, (const double *)lv.res, u_is_zero));
+                SB_TRY(sb_convert(ctx, lv.M, lv.u[lv.cur], v.u[lv.cur]));
+            }
+            return 0;
+        } else {
+            SbRange rg(ctx, "coarsest", l);
+            if (lv.M > 0 && ctx->coarsest_cg) {
+                // direct_solver == "CG" (:998-999): u is the initial guess of solve_coarsest_CG
+                if (!lv.A.sends.empty() || !lv.A.recvs.empty()) SB_FAIL("vcycle: the coarsest level must live on one rank");
+                if (u_is_zero) SB_TRY(sb_fill_zero(ctx, lv.u[lv.cur], lv.M));
+                SB_TRY(sb_coarsest_cg(ctx, rhs, lv.u[lv.cur]));
+            } else if (lv.M > 0) {
+                if (ctx->coarse_n != lv.M) SB_FAIL("vcycle: no coarsest factor was uploaded for the coarsest level");
+                SB_TRY(sb_coarsest_apply(ctx, rhs, lv.u[lv.cur]));
+            }
+            return 0;
         }
-        return 0;
     }
     DevLevel &cl = ctx->levels[l + 1];
+    const LevelVecs<V> cv = sb_level_vecs(cl, V());
     // 1. pre-smooth (:1105-1107)
     if (pre) { SbRange rg(ctx, "pre-smooth", l); SB_TRY(sb_smooth(ctx, l, smoother, pre, rhs, u_is_zero)); }
-    else if (u_is_zero) SB_TRY(sb_fill_zero(ctx, lv.u[lv.cur], lv.M));
+    else if (u_is_zero) SB_TRY(sb_fill_zero(ctx, v.u[lv.cur], lv.M));
     // 2. + 3. residual res = A u - rhs (:1140) and restriction (:1175) into the coarse grid's rhs, through the old
     //    partition if they differ.  Opt-in (saena_b200_set_fused_restrict): both as ONE pass over A that scatters every
     //    fine residual through its row of P and never writes res (fused_restrict.cu; measured in
@@ -135,7 +181,7 @@ int sb_vcycle(saena_b200_ctx *ctx, int l, int smoother, int pre, int post, const
     //    atomics make the coarse vector's last bits depend on the run).  Not on a route level: the fused kernel
     //    walks the stored A.
     bool fused_rr = false;
-    if (!(pre == 0 && u_is_zero) && ctx->fused_restrict_levels > l && !lv.route) {
+    if constexpr (F64) if (!(pre == 0 && u_is_zero) && ctx->fused_restrict_levels > l && !lv.route) {
         const bool ident = lv.repart.identity();
         const int rc = sb_residual_restrict_fused(ctx, l, lv.u[lv.cur], rhs, ident ? cl.rhs : lv.xfer_old);
         if (rc < 0) SB_FAIL("vcycle: fused residual + restriction failed to launch");
@@ -145,39 +191,40 @@ int sb_vcycle(saena_b200_ctx *ctx, int l, int smoother, int pre, int post, const
     // with a zero iterate and no pre-smoothing the residual is -rhs
     if (fused_rr) {
     } else if (pre == 0 && u_is_zero) {
-        SB_TRY(sb_negate_copy(ctx, lv.M, rhs, lv.res));
+        SB_TRY(sb_negate_copy(ctx, lv.M, rhs, v.res));
     } else {
         SbRange rg(ctx, "residual", l);
-        EpiArgs e{};
+        EpiArgsT<V> e{};
         e.rhs = rhs;
-        e.out = lv.res;
-        SB_TRY(sb_apply_level_A(ctx, l, lv.u[lv.cur], EPI_RESIDUAL, e));
+        e.out = v.res;
+        SB_TRY(sb_apply_level_A(ctx, l, v.u[lv.cur], EPI_RESIDUAL, e));
     }
     if (!fused_rr) {
         SbRange rg(ctx, "Rtransfer", l);
-        EpiArgs e{};
+        EpiArgsT<V> e{};
         const bool ident = lv.repart.identity();
-        e.out = ident ? cl.rhs : lv.xfer_old;
-        SB_TRY(sb_apply(ctx, lv.R, lv.res, EPI_PLAIN, e));
-        if (!ident) SB_TRY(sb_repart(ctx, lv.repart, false, lv.xfer_old, cl.rhs, ctx->stream));  // :1201-1203
+        e.out = cv.rhs;
+        if constexpr (F64) if (!ident) e.out = lv.xfer_old;
+        SB_TRY(sb_apply(ctx, lv.R, v.res, EPI_PLAIN, e));
+        if constexpr (F64) if (!ident) SB_TRY(sb_repart(ctx, lv.repart, false, lv.xfer_old, cl.rhs, ctx->stream));  // :1201-1203
     }
     // scale the next level's rhs (:1245-1247)
-    if (ctx->scale) SB_TRY(sb_scale_vector(ctx, cl.M, cl.rhs, cl.inv_sq_diag));
+    if constexpr (F64) if (ctx->scale) SB_TRY(sb_scale_vector(ctx, cl.M, cl.rhs, cl.inv_sq_diag));
     // 4. recurse with a zero initial correction (:1249, :1256)
-    SB_TRY(sb_vcycle(ctx, l + 1, smoother, pre, post, cl.rhs, true));
+    SB_TRY(sb_vcycle(ctx, l + 1, smoother, pre, post, (const V *)cv.rhs, true));
     // scale the coarse correction (:1264-1266)
-    if (ctx->scale) SB_TRY(sb_scale_vector(ctx, cl.M, cl.u[cl.cur], cl.inv_sq_diag));
+    if constexpr (F64) if (ctx->scale) SB_TRY(sb_scale_vector(ctx, cl.M, cl.u[cl.cur], cl.inv_sq_diag));
     // 5. + 6. prolong and correct: u -= P e_c (:1301-1303, :1325, :1360-1361)
     {
         SbRange rg(ctx, "Ptransfer", l);
-        const double *ec = cl.u[cl.cur];
-        if (!lv.repart.identity()) {
+        const V *ec = cv.u[cl.cur];
+        if constexpr (F64) if (!lv.repart.identity()) {
             SB_TRY(sb_repart(ctx, lv.repart, true, ec, lv.xfer_old, ctx->stream));
             ec = lv.xfer_old;
         }
-        EpiArgs e{};
-        e.u_in = lv.u[lv.cur];
-        e.out = lv.u[lv.cur];  // row i reads and writes only u[i]: in place
+        EpiArgsT<V> e{};
+        e.u_in = v.u[lv.cur];
+        e.out = v.u[lv.cur];  // row i reads and writes only u[i]: in place
         SB_TRY(sb_apply(ctx, lv.P, ec, EPI_SUB, e));
     }
     // 7. post-smooth (:1397-1399)
@@ -185,10 +232,21 @@ int sb_vcycle(saena_b200_ctx *ctx, int l, int smoother, int pre, int post, const
     return 0;
 }
 
+int sb_vcycle(saena_b200_ctx *ctx, int l, int smoother, int pre, int post, const double *rhs, bool u_is_zero) {
+    return vcycle(ctx, l, smoother, pre, post, rhs, u_is_zero);
+}
+int sb_vcycle(saena_b200_ctx *ctx, int l, int smoother, int pre, int post, const float *rhs, bool u_is_zero) {
+    return vcycle(ctx, l, smoother, pre, post, rhs, u_is_zero);
+}
+
+// Every call that changes what a captured V-cycle would run -- values, layouts, mappings, the route, the coarsest
+// solver, Chebyshev bounds -- comes through here, so the FP32 copies are marked stale at the same points
+// (sb_f32_sync builds them again before their next use).
 void sb_invalidate_graphs(saena_b200_ctx *ctx) {
     for (VcycleGraph &g : ctx->graphs)
         if (g.exec) cudaGraphExecDestroy(g.exec);
     ctx->graphs.clear();
+    ctx->f32_stale = true;
 }
 
 // Multi-rank capture.  The halo's comm stream is forked from the compute stream by an event at
@@ -206,7 +264,9 @@ static int join_comm_stream(saena_b200_ctx *ctx) {
     return 0;
 }
 
-int sb_vcycle_from_zero(saena_b200_ctx *ctx, int smoother, int pre, int post, const double *rhs) {
+template <typename V>
+static int vcycle_from_zero(saena_b200_ctx *ctx, int smoother, int pre, int post, const V *rhs) {
+    const int bits = std::is_same<V, double>::value ? 64 : 32;
     // a zero iterate is overwritten, so every level may start in buffer 0: the launch sequence
     // (pointers included) is then identical from one V-cycle to the next
     for (DevLevel &lv : ctx->levels) lv.cur = 0;
@@ -214,7 +274,8 @@ int sb_vcycle_from_zero(saena_b200_ctx *ctx, int smoother, int pre, int post, co
     if (!capturable) return sb_vcycle(ctx, 0, smoother, pre, post, rhs, true);
     VcycleGraph *known = nullptr;
     for (VcycleGraph &g : ctx->graphs)
-        if (g.k == 0 && g.rhs == rhs && g.smoother == smoother && g.pre == pre && g.post == post) known = &g;
+        if (g.k == 0 && g.bits == bits && g.rhs == rhs && g.smoother == smoother && g.pre == pre && g.post == post)
+            known = &g;
     if (known && known->exec) {
         SB_CUDA(cudaGraphLaunch(known->exec, ctx->stream));
         ctx->launches += known->launches;
@@ -225,7 +286,7 @@ int sb_vcycle_from_zero(saena_b200_ctx *ctx, int smoother, int pre, int post, co
     if (!known && ctx->nranks > 1) {
         // several ranks: the first V-cycle of a configuration runs eagerly (NCCL opens its
         // point-to-point channels, every lazy allocation happens), the next one is captured
-        ctx->graphs.push_back(VcycleGraph{rhs, smoother, pre, post, nullptr, 0, {}});
+        ctx->graphs.push_back(VcycleGraph{rhs, smoother, pre, post, nullptr, 0, {}, 0, bits});
         return sb_vcycle(ctx, 0, smoother, pre, post, rhs, true);
     }
     // first use of this configuration (second on several ranks): capture, instantiate, launch
@@ -250,7 +311,7 @@ int sb_vcycle_from_zero(saena_b200_ctx *ctx, int smoother, int pre, int post, co
         ctx->error.clear();
         return sb_vcycle(ctx, 0, smoother, pre, post, rhs, true);
     }
-    VcycleGraph g{rhs, smoother, pre, post, nullptr, ctx->launches - before, {}};
+    VcycleGraph g{rhs, smoother, pre, post, nullptr, ctx->launches - before, {}, 0, bits};
     const cudaError_t ie = cudaGraphInstantiate(&g.exec, graph, 0);
     cudaGraphDestroy(graph);
     if (ie != cudaSuccess) {
@@ -267,6 +328,13 @@ int sb_vcycle_from_zero(saena_b200_ctx *ctx, int smoother, int pre, int post, co
     SB_CUDA(cudaGraphLaunch(g.exec, ctx->stream));
     ++ctx->graph_replays;
     return 0;
+}
+
+int sb_vcycle_from_zero(saena_b200_ctx *ctx, int smoother, int pre, int post, const double *rhs) {
+    return vcycle_from_zero(ctx, smoother, pre, post, rhs);
+}
+int sb_vcycle_from_zero(saena_b200_ctx *ctx, int smoother, int pre, int post, const float *rhs) {
+    return vcycle_from_zero(ctx, smoother, pre, post, rhs);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -31,33 +31,34 @@
 // (No caller passes u_in aliasing d_out; out may be u_in, d_out may be d_in: same element, read first either way.)
 // Row i of the operator; o: where row i's entries of the epilogue's vectors are (i, or i + j * ld in column j of a
 // block: inv_diag, one per row, is shared by the columns).
-template <int EPI, typename IdxT>
-__device__ __forceinline__ void sb_epilogue_at(int i, IdxT o, double ax, const EpiArgs &e) {
+// V: the value type (double; float in the FP32 preconditioner's instantiations, spmv_f32.cu).
+template <int EPI, typename IdxT, typename V>
+__device__ __forceinline__ void sb_epilogue_at(int i, IdxT o, V ax, const EpiArgsT<V> &e) {
     if (EPI == EPI_PLAIN) {
         e.out[o] = ax;
     } else if (EPI == EPI_RESIDUAL) {
         e.out[o] = ax - e.rhs[o];
     } else if (EPI == EPI_CHEB_FIRST) {
-        const double u = e.u_in[o];
-        const double d = e.c1 * e.inv_diag[i] * (e.rhs[o] - ax);
+        const V u = e.u_in[o];
+        const V d = e.c1 * e.inv_diag[i] * (e.rhs[o] - ax);
         e.d_out[o] = d;
         e.out[o] = u + d;
     } else if (EPI == EPI_CHEB_NEXT) {
-        const double u = e.u_in[o];
-        const double res = e.c2 * e.inv_diag[i] * (e.rhs[o] - ax);
-        const double d = (e.c1 * e.d_in[o]) + res;
+        const V u = e.u_in[o];
+        const V res = e.c2 * e.inv_diag[i] * (e.rhs[o] - ax);
+        const V d = (e.c1 * e.d_in[o]) + res;
         e.d_out[o] = d;
         e.out[o] = u + d;
     } else if (EPI == EPI_JACOBI) {
-        const double t = (ax - e.rhs[o]) * (e.inv_diag[i] * e.c1);
+        const V t = (ax - e.rhs[o]) * (e.inv_diag[i] * e.c1);
         e.out[o] = e.u_in[o] - t;
     } else if (EPI == EPI_SUB) {
         e.out[o] = e.u_in[o] - ax;
     }
 }
 
-template <int EPI>
-__device__ __forceinline__ void sb_epilogue(int i, double ax, const EpiArgs &e) {
+template <int EPI, typename V>
+__device__ __forceinline__ void sb_epilogue(int i, V ax, const EpiArgsT<V> &e) {
     sb_epilogue_at<EPI>(i, i, ax, e);
 }
 
@@ -71,6 +72,7 @@ __device__ __forceinline__ bool sb_row_skipped(const uint32_t *__restrict__ mask
 // streaming loads of the matrix arrays: read once, do not pollute L1
 __device__ __forceinline__ double sb_ld_stream(const double *p) { return __ldcs(p); }
 __device__ __forceinline__ int sb_ld_stream(const int *p) { return __ldcs(p); }
+__device__ __forceinline__ float sb_ld_stream(const float *p) { return __ldcs(p); }
 
 // Where the gathered operand comes from.  XLocal: the rank's own vector.  XGhost (merged mode of the
 // fused halo kernel, csrc/fused_halo.cu): columns >= n_local are ghost values the neighbours stored
@@ -78,10 +80,12 @@ __device__ __forceinline__ int sb_ld_stream(const int *p) { return __ldcs(p); }
 // values across rows as much as local ones (deep levels: thousands of entries per row), and no
 // line of the landing area can be stale in L1 -- L1 is invalidated at every launch and within a
 // launch nothing reads the area before the `arrived` flag has been observed.
-struct XLocal {
-    const double *x;
-    __device__ __forceinline__ double ld(int c) const { return __ldg(x + c); }
+template <typename V>
+struct XLocalT {
+    const V *x;
+    __device__ __forceinline__ V ld(int c) const { return __ldg(x + c); }
 };
+using XLocal = XLocalT<double>;
 struct XGhost {
     const double *x;
     const double *ghost;
@@ -101,10 +105,10 @@ struct XGhost {
 // ---------------------------------------------------------------------------------------------
 constexpr int VEC_UNROLL = 4;
 
-template <int LANES, int EPI, typename OffT, typename XS>
+template <int LANES, int EPI, typename OffT, typename XS, typename V>
 __device__ __forceinline__ void
 spmv_vec_body(int vb, int row_begin, int M, const OffT *__restrict__ rowptr, const int *__restrict__ col,
-              const double *__restrict__ val, const XS xs, const EpiArgs &e,
+              const V *__restrict__ val, const XS xs, const EpiArgsT<V> &e,
               const uint32_t *__restrict__ skip_mask) {
     constexpr int G = 32 / LANES;  // rows in flight per warp per step
     const int lane = threadIdx.x & 31;
@@ -118,7 +122,7 @@ spmv_vec_body(int vb, int row_begin, int M, const OffT *__restrict__ rowptr, con
         my_start = rowptr[my_row];
         my_end = rowptr[my_row + 1];
     }
-    double mine = 0.0;
+    V mine = V(0);
     const int g = lane / LANES;   // which row of the step this lane works on
     const int sub = lane % LANES;
 #pragma unroll
@@ -126,17 +130,17 @@ spmv_vec_body(int vb, int row_begin, int M, const OffT *__restrict__ rowptr, con
         const int src = t * G + g;  // lane that owns the row this group works on in step t
         const OffT start = __shfl_sync(0xffffffffu, my_start, src);
         const OffT end = __shfl_sync(0xffffffffu, my_end, src);
-        double sum = 0.0;
+        V sum = V(0);
         for (OffT k = start + sub; k < end; k += LANES * VEC_UNROLL) {
             // issue all loads of the trip before the first use: VEC_UNROLL independent chains
             int c[VEC_UNROLL];
-            double a[VEC_UNROLL];
+            V a[VEC_UNROLL];
 #pragma unroll
             for (int q = 0; q < VEC_UNROLL; ++q) {
                 const OffT kk = k + q * LANES;
                 const bool in = kk < end;
                 c[q] = in ? sb_ld_stream(col + kk) : 0;
-                a[q] = in ? sb_ld_stream(val + kk) : 0.0;
+                a[q] = in ? sb_ld_stream(val + kk) : V(0);
             }
 #pragma unroll
             for (int q = 0; q < VEC_UNROLL; ++q) sum += a[q] * xs.ld(c[q]);
@@ -144,18 +148,18 @@ spmv_vec_body(int vb, int row_begin, int M, const OffT *__restrict__ rowptr, con
 #pragma unroll
         for (int o = LANES / 2; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
         // lane j = t*G + g' wants the sum of group g' = j % G
-        const double v = __shfl_sync(0xffffffffu, sum, (lane % G) * LANES);
+        const V v = __shfl_sync(0xffffffffu, sum, (lane % G) * LANES);
         if (lane / G == t) mine = v;
     }
     if (my_row < M && !sb_row_skipped(skip_mask, my_row)) sb_epilogue<EPI>(my_row, mine, e);
 }
 
-template <int LANES, int EPI, typename OffT>
+template <int LANES, int EPI, typename OffT, typename V = double>
 __global__ void __launch_bounds__(256)
 spmv_vec_kernel(int row_begin, int M, const OffT *__restrict__ rowptr, const int *__restrict__ col,
-                const double *__restrict__ val, const double *__restrict__ x, EpiArgs e,
+                const V *__restrict__ val, const V *__restrict__ x, EpiArgsT<V> e,
                 const uint32_t *__restrict__ skip_mask) {
-    spmv_vec_body<LANES, EPI, OffT>(blockIdx.x, row_begin, M, rowptr, col, val, XLocal{x}, e, skip_mask);
+    spmv_vec_body<LANES, EPI, OffT>(blockIdx.x, row_begin, M, rowptr, col, val, XLocalT<V>{x}, e, skip_mask);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -164,28 +168,28 @@ spmv_vec_kernel(int row_begin, int M, const OffT *__restrict__ rowptr, const int
 // (256^3 Poisson: level 4 has 21 466 rows x 3025 nnz/row).  One row per warp-group keeps all SMs
 // busy where the 32-rows-per-warp mapping above would leave most of the chip idle.
 // ---------------------------------------------------------------------------------------------
-template <int TPR, int EPI, typename OffT, typename XS>
+template <int TPR, int EPI, typename OffT, typename XS, typename V>
 __device__ __forceinline__ void
 spmv_rowgroup_body(int vb, int row_begin, int M, const OffT *__restrict__ rowptr, const int *__restrict__ col,
-                   const double *__restrict__ val, const XS xs, const EpiArgs &e,
+                   const V *__restrict__ val, const XS xs, const EpiArgsT<V> &e,
                    const uint32_t *__restrict__ skip_mask) {
     constexpr int ROWS = 256 / TPR;
     constexpr int WPR = TPR / 32;  // warps per row
-    __shared__ double s_part[8];
+    __shared__ V s_part[8];
     const int g = threadIdx.x / TPR, sub = threadIdx.x % TPR;
     const int row = row_begin + vb * ROWS + g;  // rows [row_begin, M)
-    double sum = 0.0;
+    V sum = V(0);
     if (row < M) {
         const OffT start = rowptr[row], end = rowptr[row + 1];
         for (OffT k = start + sub; k < end; k += TPR * VEC_UNROLL) {
             int c[VEC_UNROLL];
-            double a[VEC_UNROLL];
+            V a[VEC_UNROLL];
 #pragma unroll
             for (int q = 0; q < VEC_UNROLL; ++q) {
                 const OffT kk = k + q * TPR;
                 const bool in = kk < end;
                 c[q] = in ? sb_ld_stream(col + kk) : 0;
-                a[q] = in ? sb_ld_stream(val + kk) : 0.0;
+                a[q] = in ? sb_ld_stream(val + kk) : V(0);
             }
 #pragma unroll
             for (int q = 0; q < VEC_UNROLL; ++q) sum += a[q] * xs.ld(c[q]);
@@ -199,7 +203,7 @@ spmv_rowgroup_body(int vb, int row_begin, int M, const OffT *__restrict__ rowptr
         if ((threadIdx.x & 31) == 0) s_part[threadIdx.x >> 5] = sum;
         __syncthreads();
         if (sub == 0 && row < M && !sb_row_skipped(skip_mask, row)) {
-            double tot = 0.0;
+            V tot = V(0);
 #pragma unroll
             for (int w = 0; w < WPR; ++w) tot += s_part[g * WPR + w];
             sb_epilogue<EPI>(row, tot, e);
@@ -207,12 +211,12 @@ spmv_rowgroup_body(int vb, int row_begin, int M, const OffT *__restrict__ rowptr
     }
 }
 
-template <int TPR, int EPI, typename OffT>
+template <int TPR, int EPI, typename OffT, typename V = double>
 __global__ void __launch_bounds__(256)
 spmv_rowgroup_kernel(int row_begin, int M, const OffT *__restrict__ rowptr, const int *__restrict__ col,
-                     const double *__restrict__ val, const double *__restrict__ x, EpiArgs e,
+                     const V *__restrict__ val, const V *__restrict__ x, EpiArgsT<V> e,
                      const uint32_t *__restrict__ skip_mask) {
-    spmv_rowgroup_body<TPR, EPI, OffT>(blockIdx.x, row_begin, M, rowptr, col, val, XLocal{x}, e, skip_mask);
+    spmv_rowgroup_body<TPR, EPI, OffT>(blockIdx.x, row_begin, M, rowptr, col, val, XLocalT<V>{x}, e, skip_mask);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -318,17 +322,17 @@ spmv_stream_kernel(int M, const OffT *__restrict__ rowptr, const int *__restrict
 // per entry (256^3 Poisson on a B200: level-0 SpMV 0.292 -> 0.259 ms, profiles/r04_sliced_depth.md).
 constexpr int SELL_UNROLL = 8;
 
-template <int DEPTH, typename XS>
-__device__ __forceinline__ double sb_sliced_row_sum(const int *cp, const double *vp, int len, const XS &xs) {
-    double sum = 0.0;
+template <int DEPTH, typename XS, typename V>
+__device__ __forceinline__ V sb_sliced_row_sum(const int *cp, const V *vp, int len, const XS &xs) {
+    V sum = V(0);
     for (int j = 0; j < len; j += DEPTH) {
         int c[DEPTH];
-        double a[DEPTH];
+        V a[DEPTH];
 #pragma unroll
         for (int q = 0; q < DEPTH; ++q) {
             const bool in = j + q < len;
             c[q] = in ? sb_ld_stream(cp + (j + q) * 32) : 0;
-            a[q] = in ? sb_ld_stream(vp + (j + q) * 32) : 0.0;
+            a[q] = in ? sb_ld_stream(vp + (j + q) * 32) : V(0);
         }
 #pragma unroll
         for (int q = 0; q < DEPTH; ++q)
@@ -338,10 +342,10 @@ __device__ __forceinline__ double sb_sliced_row_sum(const int *cp, const double 
 }
 
 // DEPTH: SELL_UNROLL, or 4 in the fused halo kernel, which runs 8 CTAs an SM (32 registers) and would spill at 8
-template <int EPI, typename XS, int DEPTH = SELL_UNROLL>
+template <int EPI, typename XS, int DEPTH = SELL_UNROLL, typename V>
 __device__ __forceinline__ void
 spmv_sell_body(int vb, int row_begin, int M, const long long *__restrict__ slice_ptr, const int *__restrict__ col,
-               const double *__restrict__ val, const XS xs, const EpiArgs &e,
+               const V *__restrict__ val, const XS xs, const EpiArgsT<V> &e,
                const uint32_t *__restrict__ skip_mask) {
     const int row = row_begin + vb * blockDim.x + threadIdx.x;  // rows [row_begin, M), row_begin % 32 == 0
     const int lane = threadIdx.x & 31;
@@ -349,16 +353,16 @@ spmv_sell_body(int vb, int row_begin, int M, const long long *__restrict__ slice
     if ((slice << 5) >= M) return;
     const long long base = slice_ptr[slice];
     const int len = (int)((slice_ptr[slice + 1] - base) >> 5);
-    const double sum = sb_sliced_row_sum<DEPTH>(col + base + lane, val + base + lane, len, xs);
+    const V sum = sb_sliced_row_sum<DEPTH>(col + base + lane, val + base + lane, len, xs);
     if (row < M && !sb_row_skipped(skip_mask, row)) sb_epilogue<EPI>(row, sum, e);
 }
 
-template <int EPI>
+template <int EPI, typename V = double>
 __global__ void __launch_bounds__(256)
 spmv_sell_kernel(int row_begin, int M, const long long *__restrict__ slice_ptr, const int *__restrict__ col,
-                 const double *__restrict__ val, const double *__restrict__ x, EpiArgs e,
+                 const V *__restrict__ val, const V *__restrict__ x, EpiArgsT<V> e,
                  const uint32_t *__restrict__ skip_mask) {
-    spmv_sell_body<EPI>(blockIdx.x, row_begin, M, slice_ptr, col, val, XLocal{x}, e, skip_mask);
+    spmv_sell_body<EPI>(blockIdx.x, row_begin, M, slice_ptr, col, val, XLocalT<V>{x}, e, skip_mask);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -368,18 +372,18 @@ spmv_sell_kernel(int row_begin, int M, const long long *__restrict__ slice_ptr, 
 // order through shared memory, so the epilogue's vector streams are as coalesced as in spmv_sell.  Each row is
 // summed by one lane in column order, exactly as in spmv_sell: same result, bit for bit.
 // ---------------------------------------------------------------------------------------------
-template <int EPI, typename XS>
+template <int EPI, typename XS, typename V>
 __device__ __forceinline__ void
 spmv_sellp_body(int vb, int M, const long long *__restrict__ slice_ptr, const int *__restrict__ perm,
-                const int *__restrict__ col, const double *__restrict__ val, const XS xs, const EpiArgs &e) {
+                const int *__restrict__ col, const V *__restrict__ val, const XS xs, const EpiArgsT<V> &e) {
     // blockDim.x == 256 == the window; the grid holds exactly ceil(M / 256) CTAs, so every slot exists
-    __shared__ double s_sum[256];
+    __shared__ V s_sum[256];
     const int slot = vb * 256 + threadIdx.x;
     const int lane = threadIdx.x & 31;
     const int slice = slot >> 5;
     const long long base = slice_ptr[slice];
     const int len = (int)((slice_ptr[slice + 1] - base) >> 5);
-    const double sum = sb_sliced_row_sum<SELL_UNROLL>(col + base + lane, val + base + lane, len, xs);
+    const V sum = sb_sliced_row_sum<SELL_UNROLL>(col + base + lane, val + base + lane, len, xs);
     // back to row order through shared memory: the window's rows are the 256 consecutive rows from vb * 256, each in
     // exactly one slot, so thread t finishes row vb * 256 + t and the epilogue's vector streams stay coalesced
     const int wbase = vb * 256;
@@ -390,11 +394,11 @@ spmv_sellp_body(int vb, int M, const long long *__restrict__ slice_ptr, const in
     if (mine < M) sb_epilogue<EPI>(mine, s_sum[threadIdx.x], e);
 }
 
-template <int EPI>
+template <int EPI, typename V = double>
 __global__ void __launch_bounds__(256)
 spmv_sellp_kernel(int M, const long long *__restrict__ slice_ptr, const int *__restrict__ perm,
-                  const int *__restrict__ col, const double *__restrict__ val, const double *__restrict__ x, EpiArgs e) {
-    spmv_sellp_body<EPI>(blockIdx.x, M, slice_ptr, perm, col, val, XLocal{x}, e);
+                  const int *__restrict__ col, const V *__restrict__ val, const V *__restrict__ x, EpiArgsT<V> e) {
+    spmv_sellp_body<EPI>(blockIdx.x, M, slice_ptr, perm, col, val, XLocalT<V>{x}, e);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -406,33 +410,33 @@ spmv_sellp_kernel(int M, const long long *__restrict__ slice_ptr, const int *__r
 // Loads: d_q[i] is the first touch of its line and stays cached in L2 (.cg) until d_q[i-k], k rows later, reads it
 // again as the last use (.cs, evict first).  ND: the kernel's bucket (4, 8, 16 diagonals), s.nd <= ND of them stored.
 // ---------------------------------------------------------------------------------------------
-template <int ND, int EPI>
+template <int ND, int EPI, typename V = double>
 __global__ void __launch_bounds__(256)
-spmv_symdiag_kernel(int M, const double *__restrict__ d, const SymDiagOffsets s, const double *__restrict__ x,
-                    EpiArgs e) {
+spmv_symdiag_kernel(int M, const V *__restrict__ d, const SymDiagOffsets s, const V *__restrict__ x,
+                    EpiArgsT<V> e) {
     const int i = blockIdx.x * 256 + threadIdx.x;
     if (i >= M) return;
     const size_t m = (size_t)M;
     // every load of the row in flight before the first use
-    double la[ND], lx[ND], ua[ND], ux[ND];
+    V la[ND], lx[ND], ua[ND], ux[ND];
     // (in the reverse of the order the terms are summed: the first multiply-add needs the last load issued, so the
     // compiler has no partial sum to start before every load is in flight)
 #pragma unroll
     for (int q = ND - 1; q >= 1; --q) {
         const bool up = q < s.nd && i < M - s.off[q];
-        ua[q] = up ? __ldcg(d + q * m + i) : 0.0;
-        ux[q] = up ? __ldg(x + (i + s.off[q])) : 0.0;
+        ua[q] = up ? __ldcg(d + q * m + i) : V(0);
+        ux[q] = up ? __ldg(x + (i + s.off[q])) : V(0);
     }
-    const double a0 = __ldcg(d + i), x0 = __ldg(x + i);
+    const V a0 = __ldcg(d + i), x0 = __ldg(x + i);
 #pragma unroll
     for (int q = 1; q < ND; ++q) {
         const bool lo = q < s.nd && i >= s.off[q];
-        la[q] = lo ? __ldcs(d + q * m + (i - s.off[q])) : 0.0;
-        lx[q] = lo ? __ldg(x + (i - s.off[q])) : 0.0;
+        la[q] = lo ? __ldcs(d + q * m + (i - s.off[q])) : V(0);
+        lx[q] = lo ? __ldg(x + (i - s.off[q])) : V(0);
     }
     // a skipped term is 0.0 * 0.0: adding +0 leaves a non-zero sum as it is, and keeps the chain free of branches
     // (with a branch per term the compiler issues the upper loads only after the lower terms are summed)
-    double sum = 0.0;
+    V sum = V(0);
 #pragma unroll
     for (int q = ND - 1; q >= 1; --q) sum += la[q] * lx[q];
     sum += a0 * x0;

@@ -150,16 +150,17 @@ ccg_update_kernel(int n, double *__restrict__ u, double *__restrict__ res, const
 }
 
 // first Chebyshev sweep from a zero iterate: A*0 = 0, so d = (1/theta) D^-1 rhs and u = d
-// (saena_matrix.cpp:1099-1109 with u == 0; bit-identical to running the SpMV on zeros)
+// (saena_matrix.cpp:1099-1109 with u == 0; bit-identical to running the SpMV on zeros); V = float: the FP32 V-cycle's
+template <typename V>
 __global__ void __launch_bounds__(256)
-cheb_first_zero_kernel(int n, long long ld, const double *__restrict__ rhs, const double *__restrict__ inv_diag,
-                       double c, double *__restrict__ d, double *__restrict__ u) {
+cheb_first_zero_kernel(int n, long long ld, const V *__restrict__ rhs, const V *__restrict__ inv_diag,
+                       V c, V *__restrict__ d, V *__restrict__ u) {
     const long long o = blockIdx.y * ld;
     rhs += o;
     d += o;
     u += o;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-        const double v = c * inv_diag[i] * rhs[i];
+        const V v = c * inv_diag[i] * rhs[i];
         d[i] = v;
         u[i] = v;
     }
@@ -172,8 +173,9 @@ scale_vector_kernel(int n, long long ld, double *__restrict__ v, const double *_
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) v[i] *= w[i];
 }
 
+template <typename V>
 __global__ void __launch_bounds__(256)
-negate_copy_kernel(int n, long long ld, const double *__restrict__ src, double *__restrict__ dst) {
+negate_copy_kernel(int n, long long ld, const V *__restrict__ src, V *__restrict__ dst) {
     src += blockIdx.y * ld;
     dst += blockIdx.y * ld;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) dst[i] = -src[i];
@@ -271,6 +273,27 @@ int sb_negate_copy(saena_b200_ctx *ctx, int n, const double *src, double *dst) {
     ++ctx->launches;
     negate_copy_kernel<<<red_blocks(ctx, n), 256, 0, ctx->stream>>>(n, 0, src, dst);
     SB_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int sb_cheb_first_zero(saena_b200_ctx *ctx, int n, const float *rhs, const float *inv_diag, float c, float *d, float *u) {
+    if (n == 0) return 0;
+    ++ctx->launches;
+    cheb_first_zero_kernel<<<red_blocks(ctx, n), 256, 0, ctx->stream>>>(n, 0, rhs, inv_diag, c, d, u);
+    SB_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int sb_negate_copy(saena_b200_ctx *ctx, int n, const float *src, float *dst) {
+    if (n == 0) return 0;
+    ++ctx->launches;
+    negate_copy_kernel<<<red_blocks(ctx, n), 256, 0, ctx->stream>>>(n, 0, src, dst);
+    SB_CUDA(cudaGetLastError());
+    return 0;
+}
+
+int sb_fill_zero(saena_b200_ctx *ctx, float *p, size_t n) {
+    if (n) SB_CUDA(cudaMemsetAsync(p, 0, n * sizeof(float), ctx->stream));
     return 0;
 }
 

@@ -127,6 +127,12 @@ def load_library(path: Optional[str] = None):
     L.saena_b200_get_level_route.argtypes = [vp, i, ctypes.POINTER(ctypes.c_float), ctypes.POINTER(ctypes.c_float)]
     L.saena_b200_operator_bytes.restype = ctypes.c_int64
     L.saena_b200_operator_bytes.argtypes = [vp, i, i]
+    L.saena_b200_set_precond_precision.argtypes = [vp, i]
+    L.saena_b200_get_precond_precision.argtypes = [vp]
+    L.saena_b200_matvec_f32.argtypes = [vp, i, i, vp, vp]
+    L.saena_b200_residual_f32.argtypes = [vp, i, vp, vp, vp]
+    L.saena_b200_smooth_f32.argtypes = [vp, i, i, i, vp, vp]
+    L.saena_b200_vcycle_f32.argtypes = [vp, i, i, i, i, vp, vp]
     _lib = L
     return L
 
@@ -143,6 +149,8 @@ EXPORTED_SYMBOLS = [
     "saena_b200_set_level_route", "saena_b200_get_level_route", "saena_b200_operator_bytes",
     "saena_b200_solve_pcg_block", "saena_b200_solve_pcg_block_dev", "saena_b200_matvec_block",
     "saena_b200_residual_block", "saena_b200_smooth_block", "saena_b200_vcycle_block",
+    "saena_b200_set_precond_precision", "saena_b200_get_precond_precision", "saena_b200_matvec_f32",
+    "saena_b200_residual_f32", "saena_b200_smooth_f32", "saena_b200_vcycle_f32",
 ]
 
 
@@ -523,6 +531,43 @@ class Context:
         u, rhs = self._block(u, n).copy(), self._block(rhs, n)
         self._ck(self._L.saena_b200_vcycle_block(self._h, level, smoother_id(smoother), int(pre), int(post),
                                                  u.shape[0], _vp(u), _vp(rhs)))
+        return u
+
+    # ---- FP32 preconditioner ----
+    def set_precond_precision(self, bits: int):
+        """64 (default) or 32: solve_pcg / solve_pcg_dev apply the preconditioner as an FP32 V-cycle (the Krylov loop
+        stays FP64).  Raises, leaving 64, where the hierarchy cannot run it (see saena_b200_set_precond_precision)."""
+        self._ck(self._L.saena_b200_set_precond_precision(self._h, int(bits)))
+
+    def get_precond_precision(self) -> int:
+        return int(self._L.saena_b200_get_precond_precision(self._h))
+
+    def matvec_f32(self, level: int, kind: int, v) -> np.ndarray:
+        """the hooks below on the FP32 path (precision 32 only): float32 arrays in and out"""
+        op = self._op(level, kind)
+        v = np.ascontiguousarray(v, np.float32)
+        assert len(v) == op.n_local_cols
+        w = np.zeros(op.M, np.float32)
+        self._ck(self._L.saena_b200_matvec_f32(self._h, level, kind, _vp(v), _vp(w)))
+        return w
+
+    def residual_f32(self, level, u, rhs) -> np.ndarray:
+        u, rhs = np.ascontiguousarray(u, np.float32), np.ascontiguousarray(rhs, np.float32)
+        res = np.zeros_like(u)
+        self._ck(self._L.saena_b200_residual_f32(self._h, level, _vp(u), _vp(rhs), _vp(res)))
+        return res
+
+    def smooth_f32(self, level, smoother, iters, u, rhs) -> np.ndarray:
+        u = np.array(u, np.float32, copy=True)
+        rhs = np.ascontiguousarray(rhs, np.float32)
+        self._ck(self._L.saena_b200_smooth_f32(self._h, level, smoother_id(smoother), int(iters), _vp(u), _vp(rhs)))
+        return u
+
+    def vcycle_f32(self, level, u, rhs, pre=3, post=3, smoother="chebyshev") -> np.ndarray:
+        u = np.array(u, np.float32, copy=True)
+        rhs = np.ascontiguousarray(rhs, np.float32)
+        self._ck(self._L.saena_b200_vcycle_f32(self._h, level, smoother_id(smoother), int(pre), int(post), _vp(u),
+                                               _vp(rhs)))
         return u
 
     # ---- hooks ----
