@@ -274,6 +274,47 @@ int saena_b200_solve_pcg_dev(saena_b200_ctx *ctx, const double *rhs_dev, double 
                              int smoother, int pre, int post, int *iters, double *hist, int hist_cap,
                              int *hist_len);
 
+/* ---- flexible GMRES: nonsymmetric operators, one rank -----------------------------------------------------------
+ * Right-preconditioned restarted flexible GMRES(restart) (Saad's FGMRES) with the AMG V-cycle as the preconditioner.
+ * For an operator that is not symmetric positive definite, where solve_pcg's CG does not apply: convection-diffusion,
+ * a Newton Jacobian with an upwinded term, a Helmholtz-type operator in general form.  The conventions of solve_pcg:
+ * zero initial guess, r = A u - rhs, the stop test ||r|| < tol * ||r0|| with r0 = -rhs, the direct solve alone on a
+ * one-level hierarchy (iters = 1, hist = {||r0||, ||r||}), and u scaled with level 0's inv_sq_diag_orig at the end on
+ * a scaled hierarchy.
+ *   Cycle.  v_0 = r / ||r||; inner iteration j: z_j = M^-1 v_j (the V-cycle from a zero iterate, FP32 while
+ *   saena_b200_set_precond_precision is 32, as for solve_pcg), w = A z_j, w orthogonalised against v_0 .. v_j by
+ *   classical Gram-Schmidt applied twice (h_{i,j} = the sum of both passes' coefficients), h_{j+1,j} = ||w||,
+ *   v_{j+1} = w / h_{j+1,j}.  Z = [z_0 ..] is kept next to V, so the preconditioner may change between applications
+ *   (the FP32 V-cycle); with the FP64 one this is plain right-preconditioned GMRES.  The small least-squares problem
+ *   is solved on the host by Givens rotations; its residual estimate |g_{j+1}| is hist's entry for the iteration.  A
+ *   cycle ends when that estimate is below tol * ||r0||, after `restart` inner iterations, at max_iter inner iterations
+ *   in all, or at a happy breakdown (h_{j+1,j} = 0 or <= 1e-300 * ||w|| before the orthogonalisation).  Then u -= Z y
+ *   (y from the rotated triangle; a zero pivot contributes nothing), the true residual is computed, and the solve
+ *   stops if it meets the test or max_iter is reached, else restarts from it.
+ *   Outputs.  iters = inner iterations run; hist[0] = ||r0||, hist[k] = the residual estimate after inner iteration k,
+ *   so hist_len = iters + 1 (a restart adds no entry).  A zero rhs returns u = 0, iters = 0, hist_len = 1,
+ *   hist[0] = 0.  A NaN stops the solve at once: a NaN ||r0|| returns u = 0, iters = 0, hist = {NaN}; a NaN estimate
+ *   is its iteration's hist entry and u keeps the iterate of the last finished cycle.
+ *   Workspace.  2 * restart + 2 vectors of level 0's length (V, Z and the preconditioner's input), allocated at the
+ *   first call with a larger restart than before and freed by finalize and destroy; growing it drops nothing else.
+ *   A failed allocation returns non-zero and leaves the context usable for every other solver.
+ *   Refused (non-zero, the hierarchy untouched): restart outside 1..64, max_iter < 1, several ranks or a detached share,
+ *   a context that is not finalized.
+ * Every reduction runs in a fixed order with partials and counters of its own: a repeated solve gives the same bits,
+ * with graphs on or off (the V-cycle is replayed from its graph; the Arnoldi step is not captured). */
+int saena_b200_solve_gmres(saena_b200_ctx *ctx, const double *rhs, double *u, int restart, int max_iter, double tol,
+                           int smoother, int pre, int post, int *iters, double *hist, int hist_cap, int *hist_len);
+/* the same with rhs / u in device memory (complete before the call) */
+int saena_b200_solve_gmres_dev(saena_b200_ctx *ctx, const double *rhs_dev, double *u_dev, int restart, int max_iter,
+                               double tol, int smoother, int pre, int post, int *iters, double *hist, int hist_cap,
+                               int *hist_len);
+/* Test hook: one orthogonalisation step of the solve's kernels on host vectors.  V: nv (0..64) vectors of n entries
+ * back to back; w (n) is replaced by w'' = w' - V h2, where w' = w - V h1.  h1[0..nv) = V^T w with h1[nv] = <w, w>;
+ * h2[0..nv) = V^T w' with h2[nv] = <w', w'>; col[0..nv) = h1 + h2, col[nv] = ||w''||, col[nv + 1] = ||w||.  Needs an
+ * initialised context only (no hierarchy). */
+int saena_b200_gmres_orthogonalize(saena_b200_ctx *ctx, int n, int nv, const double *V, double *w, double *h1,
+                                   double *h2, double *col);
+
 /* ---- per-operator hooks (saena::matrix::matvec and the parity tests) --------------------- */
 int saena_b200_matvec(saena_b200_ctx *ctx, int level, int kind, const double *v, double *w);
 int saena_b200_residual(saena_b200_ctx *ctx, int level, const double *u, const double *rhs, double *res);
@@ -345,6 +386,9 @@ int saena_b200_timer_start(saena_b200_ctx *ctx);
  * precision is 32 (saena_b200_set_precond_precision) it times the FP32 V-cycle, which is what the solve runs. */
 int saena_b200_time_vcycle(saena_b200_ctx *ctx, int level, int smoother, int pre, int post, int reps, float *ms_out);
 int saena_b200_timer_stop(saena_b200_ctx *ctx, float *ms_out);
+/* median ms of one GMRES orthogonalisation step with nv (1..64) basis vectors of level 0's length: the three CGS2
+ * passes and the normalisation, on seeded unit vectors in the solve's workspace (one rank) */
+int saena_b200_time_gmres_step(saena_b200_ctx *ctx, int nv, int reps, float *ms_out);
 /* kernels launched by this context since init (bench.py's gpu_launches) */
 int64_t saena_b200_launch_count(const saena_b200_ctx *ctx);
 /* Force one operator's SpMV row mapping (tuning / profiling / tests): 0 = heuristic from nnz/row;

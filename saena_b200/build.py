@@ -11,7 +11,7 @@ PKG = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(PKG)
 CSRC = os.path.join(PKG, "csrc")
 LIB = os.path.join(PKG, "libsaena_b200.so")
-SOURCES = ["api.cu", "operator.cu", "vector_ops.cu", "solve.cu", "nccl_comm.cu", "p2p_halo.cu", "fused_halo.cu", "fused_restrict.cu", "lanczos.cu", "spgemm.cu", "refresh.cu", "spmv_block.cu", "spmv_f32.cu"]
+SOURCES = ["api.cu", "operator.cu", "vector_ops.cu", "solve.cu", "nccl_comm.cu", "p2p_halo.cu", "fused_halo.cu", "fused_restrict.cu", "lanczos.cu", "spgemm.cu", "refresh.cu", "spmv_block.cu", "spmv_f32.cu", "krylov.cu"]
 HEADERS = ["common.h", "spmv_kernels.cuh", "halo_sync.cuh"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 

@@ -126,6 +126,7 @@ int saena_b200_destroy(saena_b200_ctx *ctx) {
     cudaFree(ctx->tune_dev);
     cudaFree(ctx->route_t); cudaFree(ctx->route_s);
     sb_block_free(ctx);
+    sb_gmres_free(ctx);
     sb_nccl_destroy(ctx);
     cudaEventDestroy(ctx->ev_packed); cudaEventDestroy(ctx->ev_halo);
     cudaEventDestroy(ctx->ev_t0); cudaEventDestroy(ctx->ev_t1);
@@ -512,6 +513,7 @@ int saena_b200_finalize(saena_b200_ctx *ctx) {
     }
     route_free(ctx);
     sb_block_free(ctx);
+    sb_gmres_free(ctx);
     sb_f32_free(ctx);
     ctx->precond_bits = 64;
     SB_TRY(sb_arena_build(ctx));  // ghost buffers of every operator, one allocation (p2p_halo.cu)
@@ -1896,3 +1898,247 @@ int sb_recheck_routes(saena_b200_ctx *ctx) {
     route_release_if_unused(ctx);
     return 0;
 }
+
+// ---------------------------------------------------------------------------------------------
+// Flexible GMRES(m) with the V-cycle as its right preconditioner (Saad's FGMRES), one rank.  The basis V, the
+// preconditioned vectors Z and the preconditioner's input t are the GMRES workspace (ctx->gm_vec); the Arnoldi
+// kernels and their reduction state are krylov.cu's.  The small least-squares problem is solved on the host with
+// Givens rotations from the Hessenberg column each step reads back.
+// ---------------------------------------------------------------------------------------------
+static long long gmres_ld(int n) { return std::max<long long>(32, ((long long)n + 31) / 32 * 32); }
+
+static void gmres_free(saena_b200_ctx *ctx) {
+    cudaFree(ctx->gm_vec);
+    ctx->gm_vec = nullptr;
+    ctx->gm_cap = 0;
+    ctx->gm_ld = 0;
+}
+
+// 2 * restart + 2 level-0 vectors, grown to the largest restart so far; a failed allocation leaves none and the
+// context usable for every other solver
+static int gmres_reserve(saena_b200_ctx *ctx, int restart) {
+    SB_TRY(sb_gmres_state(ctx));
+    const long long ld = gmres_ld(ctx->levels[0].M);
+    if (restart <= ctx->gm_cap && ld == ctx->gm_ld) return 0;
+    const int cap = std::max(restart, ld == ctx->gm_ld ? ctx->gm_cap : 0);
+    gmres_free(ctx);
+    const size_t bytes = sizeof(double) * (size_t)(2 * cap + 2) * (size_t)ld;
+    if (cudaMalloc((void **)&ctx->gm_vec, bytes) != cudaSuccess ||
+        cudaMemsetAsync(ctx->gm_vec, 0, bytes, ctx->stream) != cudaSuccess) {
+        cudaGetLastError();   // an out-of-memory status is not sticky
+        gmres_free(ctx);
+        SB_FAIL("solve_gmres: not enough device memory for " + std::to_string(2 * cap + 2) + " work vectors");
+    }
+    ctx->gm_cap = cap;
+    ctx->gm_ld = ld;
+    return 0;
+}
+
+void sb_gmres_free(saena_b200_ctx *ctx) {
+    gmres_free(ctx);
+    sb_gmres_state_free(ctx);
+}
+
+static void push_norm(double v, double *hist, int cap, int &n) {
+    if (hist && n < cap) hist[n] = v;
+    ++n;
+}
+
+// the norm of the last sb_gmres_norm2
+static int gmres_norm(saena_b200_ctx *ctx, int n, const double *w, double *out) {
+    SB_TRY(sb_gmres_norm2(ctx, n, w));
+    SB_TRY(sb_gmres_read(ctx));
+    *out = sqrt(sb_gmres_norm2_host(ctx));
+    return 0;
+}
+
+static int gmres_device(saena_b200_ctx *ctx, const double *rhs, double *u, int m, int max_iter, double tol,
+                        int smoother, int pre, int post, int *iters, double *hist, int hist_cap, int *hist_len) {
+    DevLevel &l0 = ctx->levels[0];
+    const int n = l0.M;
+    SB_TRY(gmres_reserve(ctx, m));
+    const long long ld = ctx->gm_ld;
+    double *V = ctx->gm_vec, *Z = V + (ctx->gm_cap + 1) * ld, *t = Z + ctx->gm_cap * ld;
+    int nh = 0, it = 0;
+    *iters = 0;
+    *hist_len = 0;
+    // u = 0; r0 = A u - rhs = -rhs (the library's sign convention, as pcg_device)
+    SB_TRY(sb_fill_zero(ctx, u, n));
+    SB_TRY(sb_negate_copy(ctx, n, rhs, V));
+    double beta = 0.0;
+    SB_TRY(gmres_norm(ctx, n, V, &beta));
+    push_norm(beta, hist, hist_cap, nh);
+    const double thr = tol * beta;
+    if (!(beta > 0.0)) {   // a zero right-hand side (u = 0 solves it) or a NaN: no iteration
+        *hist_len = nh;
+        return 0;
+    }
+    if (ctx->levels.size() == 1) {
+        // direct solver only (pcg_device's shortcut): u = A^-1 rhs, one iteration
+        l0.cur = 0;
+        SB_TRY(sb_vcycle(ctx, 0, smoother, pre, post, rhs, true));
+        if (n) SB_CUDA(cudaMemcpyAsync(u, l0.u[l0.cur], sizeof(double) * n, cudaMemcpyDeviceToDevice, ctx->stream));
+        EpiArgs e{};
+        e.rhs = rhs;
+        e.out = t;
+        SB_TRY(sb_apply(ctx, l0.A, u, EPI_RESIDUAL, e));
+        double rn = 0.0;
+        SB_TRY(gmres_norm(ctx, n, t, &rn));
+        push_norm(rn, hist, hist_cap, nh);
+        if (ctx->scale) SB_TRY(sb_scale_vector(ctx, n, u, l0.inv_sq_diag));
+        *iters = 1;
+        *hist_len = nh;
+        return 0;
+    }
+    // H: the (m + 1) x m Hessenberg matrix column by column, rotated in place into R; g: the rotated beta e_1
+    std::vector<double> H((size_t)(m + 1) * m, 0.0), cs(m, 1.0), sn(m, 0.0), g(m + 1, 0.0), y(m, 0.0);
+    auto h = [&](int i, int j) -> double & { return H[(size_t)j * (m + 1) + i]; };
+    SB_TRY(sb_gmres_normalize(ctx, n, V, beta, t));   // v_0 = r / beta
+    for (;;) {   // one cycle: at most m inner iterations from the current u
+        std::fill(g.begin(), g.end(), 0.0);
+        g[0] = beta;
+        int k = 0;
+        bool nan = false;
+        for (int j = 0; j < m && it < max_iter; ++j) {
+            double *z = Z + j * ld, *w = V + (j + 1) * ld;
+            { SbRange rg(ctx, "vcycle_gmres"); SB_TRY(precondition(ctx, smoother, pre, post, t)); }   // z_j = M^-1 v_j
+            if (n) SB_CUDA(cudaMemcpyAsync(z, l0.u[l0.cur], sizeof(double) * n, cudaMemcpyDeviceToDevice, ctx->stream));
+            EpiArgs e{};
+            e.out = w;
+            { SbRange rg(ctx, "L0matvec"); SB_TRY(sb_apply(ctx, l0.A, z, EPI_PLAIN, e)); }            // w = A z_j
+            { SbRange rg(ctx, "arnoldi"); SB_TRY(sb_gmres_orthogonalize(ctx, n, ld, V, j + 1, w)); }
+            SB_TRY(sb_gmres_read(ctx));
+            const double *col = sb_gmres_column_host(ctx);
+            for (int i = 0; i <= j; ++i) h(i, j) = col[i];
+            const double hn = col[j + 1], wn = col[j + 2];   // ||w|| after and before the orthogonalisation
+            ++it;
+            k = j + 1;
+            for (int i = 0; i < j; ++i) {   // the earlier rotations
+                const double a = h(i, j), b = h(i + 1, j);
+                h(i, j) = cs[i] * a + sn[i] * b;
+                h(i + 1, j) = -sn[i] * a + cs[i] * b;
+            }
+            const double a = h(j, j), r = hypot(a, hn);
+            cs[j] = r > 0.0 ? a / r : 1.0;
+            sn[j] = r > 0.0 ? hn / r : 0.0;
+            h(j, j) = r;
+            g[j + 1] = -sn[j] * g[j];
+            g[j] = cs[j] * g[j];
+            const double est = fabs(g[j + 1]);   // ||r|| of the least-squares solution so far
+            push_norm(est, hist, hist_cap, nh);
+            if (est != est) {   // a NaN stops the solve at once (u keeps the last cycle's iterate)
+                nan = true;
+                break;
+            }
+            if (!(est >= thr)) break;
+            if (!(hn > 0.0) || hn <= 1e-300 * wn) break;   // happy breakdown: A z_j lies in the span of the basis
+            if (j + 1 == m || it == max_iter) break;
+            SB_TRY(sb_gmres_normalize(ctx, n, w, hn, t));   // v_{j+1} = w / h_{j+1,j}
+        }
+        if (nan) break;
+        // y = R^-1 g[0..k) (R: the rotated upper triangle); a zero pivot (a singular step) contributes nothing
+        for (int i = k - 1; i >= 0; --i) {
+            double s = g[i];
+            for (int l = i + 1; l < k; ++l) s -= h(i, l) * y[l];
+            y[i] = h(i, i) != 0.0 ? s / h(i, i) : 0.0;
+        }
+        // r(u + Z y') = V (beta e_1 + Hbar y'): the minimiser is y' = -y, so u -= Z y
+        SB_TRY(sb_gmres_update(ctx, n, ld, Z, k, y.data(), u));
+        EpiArgs e{};
+        e.rhs = rhs;
+        e.out = V;
+        SB_TRY(sb_apply(ctx, l0.A, u, EPI_RESIDUAL, e));   // the true residual r = A u - rhs
+        double rn = 0.0;
+        SB_TRY(gmres_norm(ctx, n, V, &rn));
+        if (!(rn >= thr) || it >= max_iter) break;
+        beta = rn;   // restart from r
+        SB_TRY(sb_gmres_normalize(ctx, n, V, beta, t));
+    }
+    if (ctx->scale) SB_TRY(sb_scale_vector(ctx, n, u, l0.inv_sq_diag));
+    *iters = it;
+    *hist_len = nh;
+    return 0;
+}
+
+extern "C" {
+
+static int gmres_enter(saena_b200_ctx *ctx, int restart, int max_iter, const int *iters, const int *hist_len) {
+    if (restart < 1 || restart > SB_GMRES_MAX) SB_FAIL("solve_gmres: restart must be in 1..64");
+    if (max_iter < 1) SB_FAIL("solve_gmres: max_iter must be at least 1");
+    // the multi-dot would need an all-reduce of its j + 1 sums per pass
+    if (ctx->nranks > 1 || ctx->detached) SB_FAIL("solve_gmres: one rank only");
+    if (!iters || !hist_len) SB_FAIL("solve_gmres: null argument");
+    return 0;
+}
+
+int saena_b200_solve_gmres_dev(saena_b200_ctx *ctx, const double *rhs_dev, double *u_dev, int restart, int max_iter,
+                               double tol, int smoother, int pre, int post, int *iters, double *hist, int hist_cap,
+                               int *hist_len) {
+    SB_ENTER();
+    SB_TRY(gmres_enter(ctx, restart, max_iter, iters, hist_len));
+    if (!rhs_dev || !u_dev) SB_FAIL("solve_gmres: null argument");
+    SB_TRY(gmres_device(ctx, rhs_dev, u_dev, restart, max_iter, tol, smoother, pre, post, iters, hist, hist_cap,
+                        hist_len));
+    return sb_sync_stream(ctx, ctx->stream);
+}
+
+int saena_b200_solve_gmres(saena_b200_ctx *ctx, const double *rhs, double *u, int restart, int max_iter, double tol,
+                           int smoother, int pre, int post, int *iters, double *hist, int hist_cap, int *hist_len) {
+    SB_ENTER();
+    SB_TRY(gmres_enter(ctx, restart, max_iter, iters, hist_len));
+    if (!rhs || !u) SB_FAIL("solve_gmres: null argument");
+    const int n = ctx->levels[0].M;
+    SB_TRY(h2d(ctx, ctx->pcg_rhs, rhs, n));
+    SB_TRY(gmres_device(ctx, ctx->pcg_rhs, ctx->pcg_u, restart, max_iter, tol, smoother, pre, post, iters, hist,
+                        hist_cap, hist_len));
+    return d2h(ctx, u, ctx->pcg_u, n);
+}
+
+// Test hook: one CGS2 step of the solve's kernels on host vectors (V: nv vectors of n, back to back)
+int saena_b200_gmres_orthogonalize(saena_b200_ctx *ctx, int n, int nv, const double *V, double *w, double *h1,
+                                   double *h2, double *col) {
+    if (!ctx) return 1;
+    SB_CUDA(cudaSetDevice(ctx->device));
+    if (n < 1 || nv < 0 || nv > SB_GMRES_MAX) SB_FAIL("gmres_orthogonalize: n >= 1 and nv in 0..64");
+    if ((nv && !V) || !w || !h1 || !h2 || !col) SB_FAIL("gmres_orthogonalize: null argument");
+    SB_TRY(sb_gmres_state(ctx));
+    const long long ld = gmres_ld(n);   // the solve's stride
+    SB_TRY(stage_buf(ctx, 0, (size_t)std::max(nv, 1) * ld));
+    SB_TRY(stage_buf(ctx, 1, n));
+    if (nv)
+        SB_CUDA(cudaMemcpy2DAsync(ctx->stage[0], sizeof(double) * ld, V, sizeof(double) * n, sizeof(double) * n, nv,
+                                  cudaMemcpyHostToDevice, ctx->stream));
+    SB_TRY(h2d(ctx, ctx->stage[1], (const double *)w, n));
+    SB_TRY(sb_gmres_orthogonalize(ctx, n, ld, ctx->stage[0], nv, ctx->stage[1]));
+    SB_TRY(sb_gmres_read(ctx));
+    memcpy(h1, sb_gmres_h1_host(ctx), sizeof(double) * (nv + 1));
+    memcpy(h2, sb_gmres_h2_host(ctx), sizeof(double) * (nv + 1));
+    memcpy(col, sb_gmres_column_host(ctx), sizeof(double) * (nv + 2));
+    return d2h(ctx, w, ctx->stage[1], n);
+}
+
+// Measurement: median ms of one Arnoldi step's orthogonalisation with nv basis vectors (the three CGS2 passes and the
+// normalisation) on the solve's workspace for level 0, on unit vectors from a seeded generator
+int saena_b200_time_gmres_step(saena_b200_ctx *ctx, int nv, int reps, float *ms_out) {
+    SB_ENTER();
+    if (nv < 1 || nv > SB_GMRES_MAX) SB_FAIL("time_gmres_step: nv must be in 1..64");
+    if (ctx->nranks > 1 || ctx->detached) SB_FAIL("time_gmres_step: one rank only");
+    if (!ms_out) SB_FAIL("time_gmres_step: null argument");
+    SB_TRY(gmres_reserve(ctx, nv));
+    const int n = ctx->levels[0].M;
+    const long long ld = ctx->gm_ld;
+    double *V = ctx->gm_vec, *t = V + (2 * ctx->gm_cap + 1) * ld, *w = V + nv * ld;
+    for (int i = 0; i <= nv; ++i) {
+        double *v = V + i * ld, nrm = 0.0;
+        SB_TRY(sb_fill_random(ctx, n, 0, 0x6A55ull + i, v));
+        SB_TRY(gmres_norm(ctx, n, v, &nrm));
+        if (nrm > 0.0) SB_TRY(sb_gmres_normalize(ctx, n, v, nrm, t));
+    }
+    // w stays a unit vector orthogonal to the others up to rounding: every repetition does the same work
+    return time_median(ctx, reps < 1 ? 20 : reps, false, [&]() {
+        SB_TRY(sb_gmres_orthogonalize(ctx, n, ld, V, nv, w));
+        return sb_gmres_normalize(ctx, n, w, 1.0, t);
+    }, ms_out);
+}
+
+}  // extern "C"

@@ -383,6 +383,17 @@ struct saena_b200_ctx {
     double *blk_scal_host = nullptr;  // pinned mirror
     int *blk_active = nullptr;        // [SB_BLOCK_MAX] 1: the column still iterates (the PCG updates skip the others)
     int *blk_active_host = nullptr;   // pinned mirror
+
+    // GMRES (saena_b200_solve_gmres, sb_gmres_reserve): one allocation of 2 * gm_cap + 2 level-0 vectors at stride
+    // gm_ld -- the basis v_0 .. v_cap, the preconditioned vectors z_0 .. z_{cap-1} and the preconditioner's input t --
+    // grown to the largest restart so far; and the reduction state of the Arnoldi kernels (krylov.cu), its own
+    int gm_cap = 0;
+    long long gm_ld = 0;
+    double *gm_vec = nullptr;
+    double *gm_partials = nullptr;      // [(SB_GMRES_MAX + 2) * RED_MAX_BLOCKS]
+    unsigned int *gm_counter = nullptr;
+    double *gm_scal = nullptr;          // krylov.cu: the reductions' sums and the Hessenberg column
+    double *gm_scal_host = nullptr;     // pinned mirror
 };
 
 // scalar slots
@@ -399,6 +410,7 @@ static const int STREAM_TILE = 2048;      // nnz per row block of the streaming 
 static const int STREAM_THREADS = 256;
 static const int RED_MAX_BLOCKS = 1184;   // 148 SMs x 8
 static const int SB_BLOCK_MAX = 8;        // right-hand sides of one block solve
+static const int SB_GMRES_MAX = 64;       // largest GMRES restart length
 
 // ---------------------------------------------------------------------------------------------
 // NVTX ranges (SAENA_B200_NVTX=1): the stages the reference's PROFILE_PCG / PROFILE_VCYCLE builds time
@@ -513,6 +525,22 @@ int sb_cheb_first_zero_block(saena_b200_ctx *ctx, int n, int k, const double *rh
 int sb_negate_copy_block(saena_b200_ctx *ctx, int n, int k, const double *src, double *dst);
 int sb_scale_vector_block(saena_b200_ctx *ctx, int n, int k, double *v, const double *w);
 int sb_read_block_scalars(saena_b200_ctx *ctx);  // blk_scal -> blk_scal_host (synchronises the stream)
+
+// ---- krylov.cu (GMRES's Arnoldi process; every pass on level-0 vectors of n rows at stride ld)
+int sb_gmres_state(saena_b200_ctx *ctx);        // the reduction state, allocated once
+void sb_gmres_state_free(saena_b200_ctx *ctx);
+void sb_gmres_free(saena_b200_ctx *ctx);        // api.cu: the workspace and the reduction state
+// w = A z_j orthogonalised in place against the nv vectors V (CGS2); the Hessenberg column h_0 .. h_{nv-1}, ||w||
+// after and ||w|| before the orthogonalisation land in the device scalars (sb_gmres_read, sb_gmres_column_host)
+int sb_gmres_orthogonalize(saena_b200_ctx *ctx, int n, long long ld, const double *V, int nv, double *w);
+int sb_gmres_norm2(saena_b200_ctx *ctx, int n, const double *w);   // <w, w> (sb_gmres_norm2_host after a read)
+int sb_gmres_normalize(saena_b200_ctx *ctx, int n, double *v, double h, double *t);   // v /= h; t = v
+int sb_gmres_update(saena_b200_ctx *ctx, int n, long long ld, const double *Z, int k, const double *y, double *x);
+int sb_gmres_read(saena_b200_ctx *ctx);         // device scalars -> pinned mirror (synchronises the stream)
+double sb_gmres_norm2_host(const saena_b200_ctx *ctx);
+const double *sb_gmres_h1_host(const saena_b200_ctx *ctx);      // first pass's dots, |w|^2 after them
+const double *sb_gmres_h2_host(const saena_b200_ctx *ctx);      // second pass's dots, |w'|^2 after them
+const double *sb_gmres_column_host(const saena_b200_ctx *ctx);  // h1 + h2, ||w''||, ||w||
 
 // ---- lanczos.cu
 // out = uniform(-1, 1) from a counter-based generator on the global row index (row_offset + i)

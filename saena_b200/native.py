@@ -90,6 +90,11 @@ def load_library(path: Optional[str] = None):
     L.saena_b200_solve_vcycle.argtypes = solve_args
     L.saena_b200_solve_smoother.argtypes = solve_args
     L.saena_b200_solve_cg.argtypes = [vp, vp, vp, i, d, ip, dp, i, ip]
+    gmres_args = [vp, vp, vp, i, i, d, i, i, i, ip, dp, i, ip]
+    L.saena_b200_solve_gmres.argtypes = gmres_args
+    L.saena_b200_solve_gmres_dev.argtypes = gmres_args
+    L.saena_b200_gmres_orthogonalize.argtypes = [vp, i, i, vp, vp, dp, dp, dp]
+    L.saena_b200_time_gmres_step.argtypes = [vp, i, i, ctypes.POINTER(ctypes.c_float)]
     L.saena_b200_matvec.argtypes = [vp, i, i, vp, vp]
     L.saena_b200_residual.argtypes = [vp, i, vp, vp, vp]
     L.saena_b200_smooth.argtypes = [vp, i, i, i, vp, vp]
@@ -151,6 +156,8 @@ EXPORTED_SYMBOLS = [
     "saena_b200_residual_block", "saena_b200_smooth_block", "saena_b200_vcycle_block",
     "saena_b200_set_precond_precision", "saena_b200_get_precond_precision", "saena_b200_matvec_f32",
     "saena_b200_residual_f32", "saena_b200_smooth_f32", "saena_b200_vcycle_f32",
+    "saena_b200_solve_gmres", "saena_b200_solve_gmres_dev", "saena_b200_gmres_orthogonalize",
+    "saena_b200_time_gmres_step",
 ]
 
 
@@ -471,6 +478,40 @@ class Context:
                                              ctypes.byref(iters), _f64p(hist), len(hist), ctypes.byref(n)))
         return u, iters.value, hist[:n.value]
 
+    def _gmres(self, fn, rhs, u, restart, max_iter, tol, smoother, pre, post):
+        iters, n = ctypes.c_int(0), ctypes.c_int(0)
+        hist = np.zeros(max_iter + 2, F64)
+        self._ck(fn(self._h, _vp(rhs), _vp(u), int(restart), int(max_iter), float(tol), smoother_id(smoother), int(pre),
+                    int(post), ctypes.byref(iters), _f64p(hist), len(hist), ctypes.byref(n)))
+        return iters.value, hist[:n.value]
+
+    def solve_gmres(self, rhs, restart=30, max_iter=100, tol=1e-8, smoother="chebyshev", pre=3, post=3):
+        """saena_b200_solve_gmres: restarted flexible GMRES with the V-cycle as right preconditioner, for operators
+        that are not symmetric positive definite -> (u, inner iterations, history: ||r0|| and the residual estimate
+        after each inner iteration).  Honours set_precond_precision like solve_pcg."""
+        rhs = np.ascontiguousarray(rhs, F64)
+        u = np.zeros(self.level_rows[0], F64)
+        it, hist = self._gmres(self._L.saena_b200_solve_gmres, rhs, u, restart, max_iter, tol, smoother, pre, post)
+        return u, it, hist
+
+    def solve_gmres_dev(self, rhs_ptr: int, u_ptr: int, restart=30, max_iter=100, tol=1e-8, smoother="chebyshev",
+                        pre=3, post=3):
+        """rhs / u are raw device pointers (e.g. torch.Tensor.data_ptr()) -> (iterations, history)"""
+        return self._gmres(self._L.saena_b200_solve_gmres_dev, rhs_ptr, u_ptr, restart, max_iter, tol, smoother, pre,
+                           post)
+
+    def gmres_orthogonalize(self, V, w):
+        """test hook of the Arnoldi kernels (saena_b200_gmres_orthogonalize): V (nv, n), w (n) ->
+        (w'', h1 [nv + 1], h2 [nv + 1], col [nv + 2])"""
+        w = np.array(w, F64, copy=True)
+        n = len(w)
+        V = np.ascontiguousarray(V, F64).reshape(-1, n)
+        nv = V.shape[0]
+        h1, h2, col = np.zeros(nv + 1, F64), np.zeros(nv + 1, F64), np.zeros(nv + 2, F64)
+        self._ck(self._L.saena_b200_gmres_orthogonalize(self._h, n, nv, _vp(V) if nv else None, _vp(w), _f64p(h1),
+                                                        _f64p(h2), _f64p(col)))
+        return w, h1, h2, col
+
     # ---- block solve: k = 1..8 right-hand sides as (k, n) arrays (row j = column j of the C ABI's block) ----
     @staticmethod
     def _block(a, n: int) -> np.ndarray:
@@ -642,6 +683,12 @@ class Context:
     def time_vcycle(self, level: int, smoother="chebyshev", pre=3, post=3, reps=10) -> float:
         ms = ctypes.c_float(0)
         self._ck(self._L.saena_b200_time_vcycle(self._h, level, smoother_id(smoother), pre, post, reps, ctypes.byref(ms)))
+        return ms.value
+
+    def time_gmres_step(self, nv: int, reps: int = 20) -> float:
+        """median ms of one GMRES orthogonalisation step against nv level-0 basis vectors"""
+        ms = ctypes.c_float(0)
+        self._ck(self._L.saena_b200_time_gmres_step(self._h, int(nv), int(reps), ctypes.byref(ms)))
         return ms.value
 
     def timer_start(self):

@@ -388,6 +388,25 @@ def poisson3d_coo(n: int):
     return n ** 3, np.concatenate(rows), np.concatenate(cols), np.concatenate(vals)
 
 
+def convdiff3d_coo(n: int, wind=(1.0, 0.5, 0.25), peclet: float = 20.0):
+    """Nonsymmetric 7-point convection-diffusion operator -lap(u) + b . grad(u) on the n^3 interior nodes of the unit
+    cube, b = peclet * wind, first-order upwind differences for the convection term: diag 6/h^2 + sum|b|/h, neighbour
+    -1/h^2, and -|b_d|/h more on the upstream neighbour of each direction d, h = 1/(n+1).  An M-matrix, not
+    symmetric (the GMRES solve's test and measurement input)."""
+    h = 1.0 / (n + 1)
+    b = peclet * np.asarray(wind, np.float64)
+    idx = np.arange(n ** 3, dtype=np.int64)
+    coord = (idx % n, (idx // n) % n, idx // (n * n))
+    rows, cols, vals = [idx], [idx], [np.full(idx.shape, 6.0 / h ** 2 + np.abs(b).sum() / h)]
+    for d, stride in enumerate((1, n, n * n)):
+        for s in (-1, 1):
+            ok = coord[d] > 0 if s < 0 else coord[d] < n - 1
+            upstream = (b[d] > 0) == (s < 0)
+            v = -1.0 / h ** 2 - (abs(b[d]) / h if upstream else 0.0)
+            rows.append(idx[ok]); cols.append(idx[ok] + s * stride); vals.append(np.full(int(ok.sum()), v))
+    return n ** 3, np.concatenate(rows), np.concatenate(cols), np.concatenate(vals)
+
+
 def poisson3d_rhs(n: int) -> np.ndarray:
     """laplacian3D_set_rhs restricted to interior nodes (src/aux_functions2.cpp:629-700):
     12 pi^2 sin(2 pi x) sin(2 pi y) sin(2 pi z) at x = i/(mx-1)"""
